@@ -14,6 +14,15 @@ larger than the 126 MB L2, so no flush is needed between iterations.
   cpu_baseline the oracle's C++ restatement of the C# SIMD FIR on the host cores (bounded sample)
 
 `--impl reference` times that CPU restatement alone (the C# reference cannot run here: no .NET).
+
+`--steps` and `--warmup` set the timed and warm-up steps of the FIR sweep, the decimate-by-D leg, the chain and modulator
+legs and the host-pointer (e2e) legs.  Fixed in size: the pageable / registered variants (one timed call each), the stream
+leg (a fixed 400 blocks through each API) and the CPU baselines (a fixed sample of samples or bursts).
+
+`--dump-outputs DIR` writes, after the timed steps, what each of the four filters returned in the last timed step, so that
+two builds run with the same arguments (identical inputs) can be compared output for output: DIR/fir_taps<N>.npy holds
+float32 (I, Q) pairs at the output positions listed in DIR/sample_index.npy (float64): the first 4096 outputs (the delay
+line carried over from the step before) and a fixed random sample (seed 0) of 2^20 of the others, about 42 MB in all.
 """
 from __future__ import annotations
 
@@ -27,11 +36,13 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (no __pycache__ of its imports)
 
 TAPS = [(16, 2), (16, 4), (16, 8), (16, 16)]  # (span, sps) -> 33, 65, 129, 257 taps
 ALPHA = 0.35
 LOG2_SAMPLES = 28
 METRIC = "Msamples/s RRC FIR sweep (taps 33-257) on 2^28 cf32 samples"
+DUMP_HEAD, DUMP_SAMPLE = 4096, 1 << 20          # outputs per filter kept by --dump-outputs: 4 x ~8 MB of cf32
 
 
 def peaks():
@@ -70,6 +81,11 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        try:
+            self.proc.wait(timeout=10)       # reaped here, so no sampler outlives the benchmark
+        except subprocess.TimeoutExpired:
+            self.proc.kill()
+            self.proc.wait()
         sm, mx, reasons = [], [], set()
         for ln in self.lines:
             f = [x.strip() for x in ln.split(",")]
@@ -228,7 +244,13 @@ def main():
     ap.add_argument("--no-decimate", action="store_true")
     ap.add_argument("--no-scaling-legs", action="store_true", help="skip the 16384-channel strong / saturated chain legs")
     ap.add_argument("--channels-total", type=int, default=16384, help="BASELINE.json configs[3]: size of the fixed channel set")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's filter outputs to DIR "
+                                                            "as .npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the GPU filters' outputs; the reference arm has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -277,8 +299,16 @@ def main():
     stream = tstream.cuda_stream
     assert stream != 0
     x = torch.empty(2 * n, dtype=torch.float32, device="cuda")
-    y = torch.empty(2 * n, dtype=torch.float32, device="cuda")
+    # one output buffer per filter, so that all four outputs of the last timed step survive it (--dump-outputs)
+    ys = [torch.empty(2 * n, dtype=torch.float32, device="cuda") for _ in TAPS]
+    y = ys[-1]
     Q.fill_uniform_dev(1, rank, 0, 2 * n, x.data_ptr(), stream)
+
+    def history(nt):
+        """The delay line a streaming filter of nt taps carries into its last call over x: the tail of x, or zeros when
+        (--warmup 0 --steps 1) that call was its first."""
+        tail = x[2 * (n - (nt - 1)):]
+        return tail if args.warmup + args.steps > 1 else torch.zeros_like(tail)
     filters = []
     for span, sps in TAPS:
         t = taps_for(Q, span, sps)
@@ -293,7 +323,7 @@ def main():
         for i, (nt, f) in enumerate(filters):
             if ev is not None:
                 ev[i][0].record()
-            f.filter_dev(x.data_ptr(), y.data_ptr(), 2 * n, stream=stream)
+            f.filter_dev(x.data_ptr(), ys[i].data_ptr(), 2 * n, stream=stream)
             if ev is not None:
                 ev[i][1].record()
 
@@ -320,6 +350,18 @@ def main():
     launches = Q.launch_count()
     ms = e0.elapsed_time(e1)
     kernels = {nt: f.last_kernel() for nt, f in filters}     # what the library actually launched for each tap count
+    if args.dump_outputs and rank == 0:
+        if n <= DUMP_HEAD + DUMP_SAMPLE:
+            idx = np.arange(n)
+        else:
+            rest = np.random.default_rng(0).choice(n - DUMP_HEAD, DUMP_SAMPLE, replace=False) + DUMP_HEAD
+            idx = np.concatenate([np.arange(DUMP_HEAD), np.sort(rest)])
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "sample_index.npy"), idx.astype(np.float64))
+        idx_dev = torch.from_numpy(idx).cuda()
+        for (nt, _), yo in zip(filters, ys):
+            np.save(os.path.join(args.dump_outputs, f"fir_taps{nt}.npy"), yo.view(-1, 2).index_select(0, idx_dev).cpu().numpy())
+        del idx_dev
     # in-run parity of the timed output: y still holds what the LAST timed launch wrote (the longest filter, delay line carried
     # from the step before = the tail of x).  Two windows — the head of the stream and one across tile seams deep inside — are
     # recomputed by the CPU oracle (checker only) from the same samples; north_star's tolerance 1e-5 * max|y|.
@@ -332,7 +374,7 @@ def main():
         worst, scale = 0.0, 0.0
         for lo in (0, n // 3):
             if lo == 0:
-                seg = torch.cat([x[2 * (n - (nt_last - 1)):], x[:2 * wlen]]).cpu().numpy()
+                seg = torch.cat([history(nt_last), x[:2 * wlen]]).cpu().numpy()
             else:
                 seg = x[2 * (lo - (nt_last - 1)): 2 * (lo + wlen)].cpu().numpy()
             want = O.ComplexFIRFilter(taps_last).Filter(seg)[2 * (nt_last - 1):]
@@ -411,10 +453,10 @@ def main():
             t = taps_for(Q, span, sps)
             nt = t.size // 2
             f = Q.ComplexFIRFilter(t)
-            for _ in range(2):
+            for _ in range(args.warmup):
                 f.decimate_dev(x.data_ptr(), 2 * n, dec, y.data_ptr(), 2 * n, stream=stream)
             ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            reps = 5
+            reps = args.steps
             ev0.record()
             for _ in range(reps):
                 f.decimate_dev(x.data_ptr(), 2 * n, dec, y.data_ptr(), 2 * n, stream=stream)
@@ -430,7 +472,7 @@ def main():
                 # tail of x; n is a multiple of D, so the kept-output phase is 0) — oracle filter at full rate, every D-th kept
                 import oracle as O
                 wo = 2048
-                seg = torch.cat([x[2 * (n - (nt - 1)):], x[:2 * wo * dec]]).cpu().numpy()
+                seg = torch.cat([history(nt), x[:2 * wo * dec]]).cpu().numpy()
                 want = O.decimate(O.ComplexFIRFilter(t).Filter(seg)[2 * (nt - 1):], dec)
                 got = y[:2 * wo].cpu().numpy()
                 err = float(np.abs(got - want).max() / max(float(np.abs(want).max()), 1e-30))
@@ -455,7 +497,7 @@ def main():
         for _, f in filters:
             f.reset()
         pcie = copy_ceiling(torch, hin, hout, 1 << 30)
-        k_e2e = max(1, min(args.steps, 5))
+        k_e2e = args.steps
         for _, f in filters:                                    # one untimed full step: slot buffers, streams, first DMA
             f.Filter(hin.array, hout.array)
             f.reset()
@@ -510,14 +552,13 @@ def main():
         import bench_chain
         d = dist if world > 1 else None
         torch.cuda.synchronize()
-        del y
+        del y, ys
         torch.cuda.empty_cache()
-        k = max(1, min(args.steps, 10))
         cpu_legs = rank == 0 and world == 1 and not args.no_cpu
         # config 3 / config 4's per-GPU share: 2048 channels per GPU (weak: 16384 channels at N = 8).  At N = 1 every
         # channel is replayed through the oracle; at N > 1, 128 channels per rank.
         par = None if world == 1 else 128
-        common = dict(steps=k, warmup=3, hbm_peak=hbm_peak, comm=comm)
+        common = dict(steps=args.steps, warmup=args.warmup, hbm_peak=hbm_peak, comm=comm)
         chain = bench_chain.run_chain(Q, torch, d, world, rank, stream, use_fll=False, cpu=cpu_legs, parity_channels=par,
                                       label="weak: 2048 channels per GPU", **common)
         chain_fll = bench_chain.run_chain(Q, torch, d, world, rank, stream, use_fll=True, cpu=cpu_legs, parity_channels=par,
@@ -539,14 +580,13 @@ def main():
                     scaling_legs[key + "_saturated"] = bench_chain.run_chain(
                         Q, torch, d, world, rank, stream, use_fll=fll, channels_per_gpu=tot, parity_channels=0,
                         label=f"saturated weak: {tot} channels per GPU", **common)
-        modulator = bench_chain.run_modulator(Q, torch, d, world, rank, stream, steps=k, warmup=3, hbm_peak=hbm_peak,
-                                              parity=cpu_legs)
+        modulator = bench_chain.run_modulator(Q, torch, d, world, rank, stream, steps=args.steps, warmup=args.warmup,
+                                              hbm_peak=hbm_peak, parity=cpu_legs)
         chain_e2e = chain_fll_e2e = modulator_e2e = None
         if not args.no_e2e:
-            ks = max(1, min(args.steps, 5))
-            chain_e2e = bench_chain.run_chain_e2e(Q, torch, d, world, rank, stream, steps=ks, use_fll=False)
-            chain_fll_e2e = bench_chain.run_chain_e2e(Q, torch, d, world, rank, stream, steps=ks, use_fll=True)
-            modulator_e2e = bench_chain.run_modulator_e2e(Q, torch, d, world, rank, steps=min(ks, 3))
+            chain_e2e = bench_chain.run_chain_e2e(Q, torch, d, world, rank, stream, steps=args.steps, use_fll=False)
+            chain_fll_e2e = bench_chain.run_chain_e2e(Q, torch, d, world, rank, stream, steps=args.steps, use_fll=True)
+            modulator_e2e = bench_chain.run_modulator_e2e(Q, torch, d, world, rank, steps=args.steps)
         stream_leg = bench_chain.run_stream(Q) if (rank == 0 and world == 1 and not args.no_cpu) else None
 
     cpu = None
