@@ -178,6 +178,37 @@ QPSK_API int qpsk_costas_process_dev(qpsk_costas* c, const float* d_in, float* d
 /* GetState() :130, per channel */
 QPSK_API int qpsk_costas_get_state(qpsk_costas* c, double* theta, double* freq);
 
+/* ---- symbol-spaced blind CMA equalizer ---------------------------------------------------------------- */
+/* Not in the reference (its receive chain has no equalizer); the block a GNU Radio PSK receiver puts between clock
+ * recovery and the Costas loop, for multipath channels.  One output per input symbol, group delay D = (n_taps-1)/2.
+ * fp32, every product and sum rounded separately (no FMA).  State per channel: taps w[0..N-1] (at creation and reset
+ * w[D] = 1+0j, the others 0) and the last N-1 inputs (zero before the stream starts).  For each input x_n, with
+ * v_k = x_{n-k} (k = 0..N-1):
+ *   P_k = w_k * v_k                        re = w.re*v.re - w.im*v.im, im = w.re*v.im + w.im*v.re
+ *   s_l = +0.0f, then s_l = s_l + P_k      for k = l (mod 8), k increasing (l = 0..7, re and im separately)
+ *   y   = ((s_0 + s_1) + (s_2 + s_3)) + ((s_4 + s_5) + (s_6 + s_7))
+ *   d   = (y.re*y.re + y.im*y.im) - modulus
+ *   e   = (fminf(fmaxf(y.re*d, -1), 1), fminf(fmaxf(y.im*d, -1), 1))
+ *   g_k = e * conj(v_k)                    re = e.re*v.re + e.im*v.im, im = e.im*v.re - e.re*v.im
+ *   w_k = w_k - mu*g_k                     (re and im separately, every k, after y is formed);  output y
+ * State persists across calls: any chunking of a stream gives the same outputs bit for bit.
+ * n_taps 1..64 (else QPSK_ERR_UNSUPPORTED); mu finite and >= 0, modulus finite and > 0 (else QPSK_ERR_RANGE).  modulus
+ * 1.0 is |symbol|^2 at this modem's matched-filter output for unit channel gain.  A refused call consumes no state. */
+typedef struct qpsk_eq qpsk_eq;
+QPSK_API int qpsk_eq_create(int n_taps, float mu, float modulus, qpsk_eq** out);
+QPSK_API int qpsk_eq_create_batch(int n_taps, float mu, float modulus, int channels, qpsk_eq** out);
+QPSK_API int qpsk_eq_destroy(qpsk_eq* eq);
+QPSK_API int qpsk_eq_reset(qpsk_eq* eq);                      /* taps to the centre spike, window zeroed */
+/* host memory, iq_in / iq_out [channels][n_floats]; odd n_floats -> QPSK_ERR_ARG, out_cap_floats < n_floats -> QPSK_ERR_CAPACITY */
+QPSK_API int qpsk_eq_process(qpsk_eq* eq, const float* iq_in, float* iq_out, int64_t n_floats, int64_t out_cap_floats);
+/* device memory, strides in floats; d_n_sym[channels] valid complex symbols per channel (NULL = n_floats/2 for all) */
+QPSK_API int qpsk_eq_process_dev(qpsk_eq* eq, const float* d_in, float* d_out, int64_t n_floats, int64_t in_stride_floats,
+                                 int64_t out_stride_floats, const int* d_n_sym, void* stream);
+/* taps [channels][2*n_taps] interleaved IQ; get: cap_floats < channels*2*n_taps -> QPSK_ERR_CAPACITY; set: n_floats must be
+ * exactly channels*2*n_taps (else QPSK_ERR_ARG), every value finite (else QPSK_ERR_RANGE) */
+QPSK_API int qpsk_eq_get_taps(qpsk_eq* eq, float* taps_iq, int64_t cap_floats);
+QPSK_API int qpsk_eq_set_taps(qpsk_eq* eq, const float* taps_iq, int64_t n_floats);
+
 /* ---- a6  QPSKModulator  (MS/QPSKModulator.cs:18-168) ---------------------------------------- */
 /* tsc_bits: '0'/'1' string or NULL (null/whitespace = no TSC, :27) */
 QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha, int rrc_span,
@@ -227,6 +258,15 @@ QPSK_API int qpsk_demod_destroy(qpsk_demod* d);
  * summation order bit for bit.  QPSK_FIR_FAST accumulates with FMA (outputs within ~1e-7 relative): a decision can differ
  * only where a decision variable lies that close to zero (bench.py counts such channels on its own bursts). */
 QPSK_API int qpsk_demod_set_fir_mode(qpsk_demod* d, int mode);
+/* Opt-in CMA equalizer stage (qpsk_eq_* above) between Mueller-Muller and Costas, for multipath channels; n_taps 0 = off
+ * (the default: the chain is then exactly the reference's).  The first (n_taps-1)/2 equalizer outputs of each channel's
+ * stream are discarded once, so the k-th symbol reaching Costas is the equalized k-th Mueller-Muller symbol (bit
+ * alignment as without the stage); the last (n_taps-1)/2 symbols of a call come out at the start of the next.  May be
+ * called at any time: synchronises the handle, resets the equalizer (taps, window, discard count) and leaves every other
+ * piece of loop and framer state alone.  With the stage on, the symbol path runs as separate MM / EQ / decode kernels. */
+QPSK_API int qpsk_demod_set_equalizer(qpsk_demod* d, int n_taps, float mu, float modulus);
+/* the equalizer taps, [channels][2*n_taps]; QPSK_ERR_ARG when the stage is off */
+QPSK_API int qpsk_demod_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats);
 /* DeModulate(ReadOnlySpan<float>) :345-425 -> '0'/'1' chars (not NUL-terminated).  Batch handles:
  * iq_in [channels][n_floats], bits_out [channels][cap], n_bits[channels] (same layout rule for the
  * other host entry points below). */

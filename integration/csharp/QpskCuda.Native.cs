@@ -53,6 +53,13 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_costas_destroy(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_costas_process(IntPtr h, float* iqIn, float* iqOut, long nFloats, long outCap);
     [DllImport(Lib)] internal static extern int qpsk_costas_get_state(IntPtr h, out double theta, out double freq);
+    // symbol-spaced blind CMA equalizer              (not in the reference; spec in include/qpskcuda.h)
+    [DllImport(Lib)] internal static extern int qpsk_eq_create(int nTaps, float mu, float modulus, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_eq_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_eq_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_eq_process(IntPtr h, float* iqIn, float* iqOut, long nFloats, long outCap);
+    [DllImport(Lib)] internal static extern int qpsk_eq_get_taps(IntPtr h, float* tapsIq, long capFloats);
+    [DllImport(Lib)] internal static extern int qpsk_eq_set_taps(IntPtr h, float* tapsIq, long nFloats);
     // a6  QPSKModulator                             (MS/QPSKModulator.cs:18,54,104)
     [DllImport(Lib, CharSet = CharSet.Ansi)]
     internal static extern int qpsk_mod_create(int fs, int rs, double alpha, int span, int diff, string? tsc, out IntPtr h);
@@ -66,6 +73,8 @@ internal static unsafe partial class QpskCuda
     internal static extern int qpsk_demod_create(int fs, int rs, float alpha, int span, double symBw, double costasBw, double cfoBw,
                                                  int diff, string? tsc, int useFll, long maxFrameBytes, out IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_demod_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_demod_set_equalizer(IntPtr h, int nTaps, float mu, float modulus);
+    [DllImport(Lib)] internal static extern int qpsk_demod_equalizer_taps(IntPtr h, float* tapsIq, long capFloats);
     [DllImport(Lib)] internal static extern int qpsk_demod_bits(IntPtr h, float* iqIn, long nFloats, byte* bitsOut, long cap, out long nBits);
     [DllImport(Lib)] internal static extern int qpsk_demod_bytes(IntPtr h, float* iqIn, long nFloats, byte* start, long nStart,
                                                                  byte* end, long nEnd, byte* payloadOut, long cap, out long nBytes);

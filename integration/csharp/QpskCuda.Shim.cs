@@ -227,6 +227,59 @@ namespace QPSK.Models
         }
         public void Dispose() => _o.Dispose();
     }
+
+    // Symbol-spaced blind CMA equalizer: not a reference class (its receive chain has none); the block a GNU Radio PSK
+    // receiver puts between clock recovery and the Costas loop.  Arithmetic spec in include/qpskcuda.h.
+    public sealed unsafe class CmaEqualizer : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int NumTaps;
+        public CmaEqualizer(int nTaps, float mu, float modulus = 1.0f)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_eq_create(nTaps, mu, modulus, out IntPtr h));
+            _o = new QpskHandle(h, QpskCuda.qpsk_eq_destroy);
+            NumTaps = nTaps;
+        }
+        public int Process(ReadOnlySpan<float> iqIn, Span<float> iqOut)
+        {
+            if ((iqIn.Length & 1) != 0) throw new ArgumentException("Input must be interleaved IQ with even length.", nameof(iqIn));
+            if (iqOut.Length < iqIn.Length) throw new ArgumentException("Output span is too small.", nameof(iqOut));
+            fixed (float* i = iqIn) fixed (float* o = iqOut)
+                QpskCuda.Check(QpskCuda.qpsk_eq_process(_h, i, o, iqIn.Length, iqOut.Length), nameof(iqIn));
+            GC.KeepAlive(this);
+            return iqIn.Length >> 1;                                                 // complex symbols processed
+        }
+        public float[] Process(float[] iqIn)
+        {
+            if (iqIn == null) throw new ArgumentNullException(nameof(iqIn));
+            var y = new float[iqIn.Length];
+            Process(iqIn.AsSpan(), y.AsSpan());
+            return y;
+        }
+        public float[] Taps                                                          // interleaved IQ, 2 * NumTaps floats
+        {
+            get
+            {
+                var t = new float[2 * NumTaps];
+                fixed (float* p = t) QpskCuda.Check(QpskCuda.qpsk_eq_get_taps(_h, p, t.Length));
+                GC.KeepAlive(this);
+                return t;
+            }
+            set
+            {
+                if (value == null) throw new ArgumentNullException(nameof(value));
+                fixed (float* p = value) QpskCuda.Check(QpskCuda.qpsk_eq_set_taps(_h, p, value.Length), nameof(value));
+                GC.KeepAlive(this);
+            }
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_eq_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
 }
 
 namespace QPSK
@@ -309,6 +362,21 @@ namespace QPSK
             QpskCuda.Check(QpskCuda.qpsk_demod_create(SampleRate, SymbolRate, RrcAlpha, rrcSpan, SymbolSyncBandwith, CostasLoopBandwith,
                                                       CFOLoopBandwith, differentialEncoding ? 1 : 0, tsc, 0, 0, out IntPtr h));
             _o = new QpskHandle(h, QpskCuda.qpsk_demod_destroy);
+        }
+        // opt-in CMA equalizer between clock recovery and Costas (not in the reference; nTaps 0 = off, the default)
+        public void SetEqualizer(int nTaps, float mu, float modulus = 1.0f)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_demod_set_equalizer(_h, nTaps, mu, modulus));
+            _eqTaps = nTaps;
+            GC.KeepAlive(this);
+        }
+        int _eqTaps;
+        public float[] EqualizerTaps()
+        {
+            var t = new float[2 * _eqTaps];
+            fixed (float* p = t) QpskCuda.Check(QpskCuda.qpsk_demod_equalizer_taps(_h, p, t.Length));
+            GC.KeepAlive(this);
+            return t;
         }
         public byte[] DeModulateBytes(ReadOnlySpan<float> samplesIQ, ReadOnlySpan<byte> startMarker, ReadOnlySpan<byte> endMarker)   // :169
         {

@@ -109,6 +109,14 @@ def _signatures():
         "qpsk_costas_process": (i, [vp, vp, vp, i64, i64]),
         "qpsk_costas_process_dev": (i, [vp, vp, vp, i64, i64, i64, vp, vp]),
         "qpsk_costas_get_state": (i, [vp, f64p, f64p]),
+        "qpsk_eq_create": (i, [i, f, f, vpp]),
+        "qpsk_eq_create_batch": (i, [i, f, f, i, vpp]),
+        "qpsk_eq_destroy": (i, [vp]),
+        "qpsk_eq_reset": (i, [vp]),
+        "qpsk_eq_process": (i, [vp, vp, vp, i64, i64]),
+        "qpsk_eq_process_dev": (i, [vp, vp, vp, i64, i64, i64, vp, vp]),
+        "qpsk_eq_get_taps": (i, [vp, f32p, i64]),
+        "qpsk_eq_set_taps": (i, [vp, f32p, i64]),
         "qpsk_mod_create": (i, [i, i, d, i, i, cp, vpp]),
         "qpsk_mod_destroy": (i, [vp]),
         "qpsk_mod_taps": (i, [vp, f64p, i, i32p]),
@@ -121,6 +129,8 @@ def _signatures():
         "qpsk_demod_create_batch": (i, [i, i, f, i, d, d, d, i, cp, i, i64, i, vpp]),
         "qpsk_demod_destroy": (i, [vp]),
         "qpsk_demod_set_fir_mode": (i, [vp, i]),
+        "qpsk_demod_set_equalizer": (i, [vp, i, f, f]),
+        "qpsk_demod_equalizer_taps": (i, [vp, f32p, i64]),
         "qpsk_demod_bits": (i, [vp, vp, i64, vp, i64, vp]),
         "qpsk_demod_bits_packed": (i, [vp, vp, i64, vp, i64, vp]),
         "qpsk_demod_bytes": (i, [vp, vp, i64, vp, i64, vp, i64, vp, i64, vp]),

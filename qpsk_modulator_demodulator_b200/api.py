@@ -378,3 +378,46 @@ class CostasLoopQpsk(_Handle):
         f = np.empty(self.channels, np.float64)
         check(lib().qpsk_costas_get_state(self._h, t.ctypes.data_as(N.f64p), f.ctypes.data_as(N.f64p)))
         return (float(t[0]), float(f[0])) if self.channels == 1 else (t, f)
+
+
+# ---- symbol-spaced blind CMA equalizer (not in the reference) ---------------------------------
+class CmaEqualizer(_Handle):
+    """Symbol-spaced blind CMA equalizer on the GPU (csrc/eq.cu; arithmetic spec in include/qpskcuda.h): `n_taps` complex
+    taps (1..64) adapted by the constant-modulus rule with step `mu` towards |y|^2 = `modulus`, one output per input,
+    group delay (n_taps-1)//2 symbols.  State persists across calls."""
+    _destroy = "qpsk_eq_destroy"
+
+    def __init__(self, n_taps: int, mu: float, modulus: float = 1.0, channels: int = 1):
+        super().__init__()
+        self.n_taps, self.channels = n_taps, channels
+        check(lib().qpsk_eq_create_batch(n_taps, mu, modulus, channels, C.byref(self._h)))
+
+    def Process(self, iqIn, iqOut=None):
+        """-> the equalized symbols (interleaved IQ; [channels, n_floats] for batch handles).  With `iqOut` given the
+        outputs go there and the number of complex symbols processed is returned."""
+        x = _f32(iqIn)
+        n = x.shape[-1] if x.ndim == 2 else x.size
+        y = iqOut if iqOut is not None else np.empty(x.shape, np.float32)
+        cap = y.shape[-1] if y.ndim == 2 else y.size
+        check(lib().qpsk_eq_process(self._h, _ptr(x), _ptr(y), n, cap))
+        return (n >> 1) if iqOut is not None else y
+
+    def process_dev(self, d_in: int, d_out: int, n_floats: int, in_stride: int = 0, out_stride: int = 0, d_n_sym: int = 0,
+                    stream: int = 0):
+        check(lib().qpsk_eq_process_dev(self._h, d_in, d_out, n_floats, in_stride or n_floats, out_stride or n_floats,
+                                        d_n_sym or None, stream))
+
+    @property
+    def taps(self) -> np.ndarray:
+        """[2*n_taps] interleaved IQ ([channels, 2*n_taps] for batch handles)."""
+        out = np.empty((self.channels, 2 * self.n_taps), np.float32)
+        check(lib().qpsk_eq_get_taps(self._h, out.ctypes.data_as(N.f32p), out.size))
+        return out[0] if self.channels == 1 else out
+
+    @taps.setter
+    def taps(self, t):
+        t = _f32(t)
+        check(lib().qpsk_eq_set_taps(self._h, t.ctypes.data_as(N.f32p), t.size))
+
+    def reset(self):
+        check(lib().qpsk_eq_reset(self._h))

@@ -15,10 +15,10 @@ LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(HERE, "build")
 LIB = os.path.join(LIBDIR, "libqpskcuda.so")
 
-SOURCES = ["core.cu", "fir.cu", "util.cu", "loops.cu", "fll_duo.cu", "fll_lane.cu", "modulator.cu", "demod.cu", "chain.cu", "stream.cu", "channel.cu", "comm.cu"]
+SOURCES = ["core.cu", "fir.cu", "util.cu", "loops.cu", "eq.cu", "fll_duo.cu", "fll_lane.cu", "modulator.cu", "demod.cu", "chain.cu", "stream.cu", "channel.cu", "comm.cu"]
 
 # serial-loop kernels restate C# arithmetic in which RyuJIT never fuses a*b+c: no FMA contraction there
-PER_FILE_FLAGS = {"loops.cu": ["--fmad=false"], "fll_duo.cu": ["--fmad=false"], "fll_lane.cu": ["--fmad=false"], "demod.cu": ["--fmad=false"], "chain.cu": ["--fmad=false"], "channel.cu": ["--fmad=false"]}
+PER_FILE_FLAGS = {"loops.cu": ["--fmad=false"], "eq.cu": ["--fmad=false"], "fll_duo.cu": ["--fmad=false"], "fll_lane.cu": ["--fmad=false"], "demod.cu": ["--fmad=false"], "chain.cu": ["--fmad=false"], "channel.cu": ["--fmad=false"]}
 
 NVCC_FLAGS = [
     "-std=c++17", "-O3",

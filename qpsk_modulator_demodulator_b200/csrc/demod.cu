@@ -2,16 +2,18 @@
 // channels.  Compiled with --fmad=false (see loops.cuh).
 //
 // Chain per call (DeModulate :345-425):  [FLL (opt-in; the call at :359 is commented out upstream)] ->
-// RRC matched filter (FirEngine, fir.cu) -> Mueller-Muller (loops.cu) -> decode kernel: Costas +
-// decision + differential decode -> bits -> TSC exact-match strip (:413-422).
+// RRC matched filter (FirEngine, fir.cu) -> Mueller-Muller (loops.cu) -> [CMA equalizer (opt-in, eq.cu; not in the
+// reference)] -> decode kernel: Costas + decision + differential decode -> bits -> TSC exact-match strip (:413-422).
 // DeModulateBytes (:169-259): the bits then feed the per-channel framer kernel (8 bit-offset marker
 // hunt, MSB-first packing into a bounded ring, end-marker search).
 // All loop / framer state lives in device memory per channel and persists across calls, so arbitrary
 // chunking of a stream gives the same output as the reference object would.
 #include <stdlib.h>
 
+#include <memory>
 #include <string>
 
+#include "eq.cuh"
 #include "fir.cuh"
 #include "loops.cuh"
 
@@ -982,8 +984,12 @@ struct DemodEngine {
   FllEngine fll;
   MmEngine mm;
   CostasEngine costas;
-  DevBuf<float2> t_fll, t_rrc, t_sym;
-  DevBuf<int> d_nsym;
+  std::unique_ptr<EqEngine> eq;    // opt-in CMA stage between MM and Costas (qpsk_demod_set_equalizer); null = off
+  DevBuf<float2> t_fll, t_rrc, t_sym, t_eq;
+  DevBuf<int> d_nsym, d_neq;
+  // what front() leaves for Costas: the MM symbols, or with the equalizer on its outputs
+  float2* sym_p = nullptr;
+  int* nsym_p = nullptr;
   DevBuf<uint8_t> d_raw, d_tsc, d_bits, d_markers, d_carry, d_ring, d_pk, d_payload;
   DevBuf<long long> d_nraw, d_nbits, d_npayload;
   DevBuf<DiffState> d_diff;
@@ -1089,7 +1095,7 @@ struct DemodEngine {
   }
   long long bits_bound(int64_t L) const { return 2 * symbols_bound(L); }
 
-  // FLL? -> MF -> MM.  Symbols in t_sym [C][sym_ld], counts in d_nsym.
+  // FLL? -> MF -> MM [-> EQ].  Symbols in sym_p [C][sym_ld] (t_sym, or t_eq with the equalizer on), counts in nsym_p.
   int front(const float2* x, int64_t L, int64_t ldx, cudaStream_t s, bool run_mm = true) {
     const int64_t ld = L + (L & 1);
     QPSK_TRY(t_rrc.ensure((size_t)ld * channels));
@@ -1108,6 +1114,31 @@ struct DemodEngine {
     mf_ld = ld;
     if (!run_mm) return QPSK_OK;
     QPSK_TRY(mm.process_dev(t_rrc.p, L, ld, t_sym.p, 2 * L, sym_ld, d_nsym.p, s));   // :364-367
+    sym_p = t_sym.p;
+    nsym_p = d_nsym.p;
+    if (eq) {
+      QPSK_TRY(t_eq.ensure((size_t)sym_ld * channels));
+      QPSK_TRY(eq->process_dev(t_sym.p, t_eq.p, sym_ld, sym_ld, sym_ld, d_nsym.p, d_neq.p, true, s));
+      sym_p = t_eq.p;
+      nsym_p = d_neq.p;
+    }
+    return QPSK_OK;
+  }
+
+  // opt-in equalizer stage: n_taps 0 = off; otherwise a fresh equalizer (spike taps, zero window, discard count D)
+  int set_equalizer(int n_taps, float mu, float modulus) {
+    if (n_taps != 0) QPSK_TRY(eq_check_params(n_taps, mu, modulus));
+    QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
+    if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
+    if (n_taps == 0) {
+      eq.reset();
+      return QPSK_OK;
+    }
+    std::unique_ptr<EqEngine> e(new (std::nothrow) EqEngine());
+    if (!e) return QPSK_ERR_NOMEM;
+    QPSK_TRY(e->init(n_taps, mu, modulus, channels));
+    QPSK_TRY(d_neq.ensure((size_t)channels));
+    eq = std::move(e);
     return QPSK_OK;
   }
 
@@ -1201,7 +1232,7 @@ struct DemodEngine {
 
   // the fused MM -> Costas -> decode kernel applies when no call can run out of output room and the MM
   // queue holds at most kSsCarry samples (always true once every call has had room)
-  bool can_fuse() const { return fuse && (sps - 0.1 > 1.0) && mm.q_bound <= kSsCarry; }
+  bool can_fuse() const { return fuse && !eq && (sps - 0.1 > 1.0) && mm.q_bound <= kSsCarry; }
   // ... and it takes the matched filter in as well (MFW extra warps, see symsync_decode_kernel) when the filter runs in
   // the reference's summation order (the demodulator's default), has real taps and at most 65 of them.
   // QPSK_DEMOD_FUSE_MF=0 keeps the separate matched-filter launch (A/B runs).
@@ -1401,8 +1432,8 @@ struct DemodEngine {
       QPSK_TRY(mm.ensure_queue(8, s));
       QPSK_TRY(launch_symsync(sym_in, L, sym_in_ld, raw, ld_raw, n_raw, 0, fuse_mf, s));
     } else {
-      decode_kernel<<<(channels + 31) / 32, 32, 0, s>>>(costas.P, costas.d_state.p, d_diff.p, channels, t_sym.p, sym_ld,
-                                                        d_nsym.p, diff ? 1 : 0, raw, ld_raw, n_raw);
+      decode_kernel<<<(channels + 31) / 32, 32, 0, s>>>(costas.P, costas.d_state.p, d_diff.p, channels, sym_p, sym_ld,
+                                                        nsym_p, diff ? 1 : 0, raw, ld_raw, n_raw);
       QPSK_LAUNCH_CHECK();
     }
     if (has_tsc) {
@@ -1433,8 +1464,8 @@ struct DemodEngine {
       if (ld_out < sl) return QPSK_ERR_CAPACITY;
     }
     QPSK_TRY(front(x, L, ldx, s));
-    QPSK_TRY(costas.process_dev(t_sym.p, out, sym_ld, sym_ld, ld_out, d_nsym.p, s));   // :447-452
-    QPSK_CUDA_TRY(cudaMemcpyAsync(n_out, d_nsym.p, sizeof(int) * channels, cudaMemcpyDeviceToDevice, s));
+    QPSK_TRY(costas.process_dev(sym_p, out, sym_ld, sym_ld, ld_out, nsym_p, s));   // :447-452
+    QPSK_CUDA_TRY(cudaMemcpyAsync(n_out, nsym_p, sizeof(int) * channels, cudaMemcpyDeviceToDevice, s));
     return QPSK_OK;
   }
 
@@ -1527,6 +1558,22 @@ int qpsk_demod_set_fir_mode(qpsk_demod* d, int mode) {
   if (mode != QPSK_FIR_FAST && mode != QPSK_FIR_EXACT) return QPSK_ERR_RANGE;
   // FAST inside the modem = the tap-sequential FMA kernel: chunk-invariant bit for bit (the time-chunk pipeline relies on it)
   d->eng.mf.mode = mode == QPSK_FIR_FAST ? QPSK_FIR_FMA : mode;
+  return QPSK_OK;
+}
+int qpsk_demod_set_equalizer(qpsk_demod* d, int n_taps, float mu, float modulus) {
+  if (!d) return QPSK_ERR_NULL;
+  QPSK_TRY(ensure_device(d->eng.device));
+  return d->eng.set_equalizer(n_taps, mu, modulus);
+}
+int qpsk_demod_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats) {
+  if (!d || !taps_iq) return QPSK_ERR_NULL;
+  DemodEngine& e = d->eng;
+  if (!e.eq) return QPSK_ERR_ARG;
+  const int64_t need = (int64_t)e.channels * 2 * e.eq->P.n_taps;
+  if (cap_floats < need) return QPSK_ERR_CAPACITY;
+  QPSK_TRY(ensure_device(e.device));
+  QPSK_CUDA_TRY(cudaStreamSynchronize(e.stream));
+  QPSK_CUDA_TRY(cudaMemcpy(taps_iq, e.eq->d_taps.p, (size_t)need * 4, cudaMemcpyDeviceToHost));
   return QPSK_OK;
 }
 

@@ -169,6 +169,19 @@ class QPSKDeModulator(_Handle):
     def set_fir_mode(self, mode: int):
         check(lib().qpsk_demod_set_fir_mode(self._h, mode))
 
+    def set_equalizer(self, n_taps: int, mu: float, modulus: float = 1.0):
+        """Opt-in CMA equalizer (api.CmaEqualizer) between Mueller-Muller and Costas, for multipath channels; n_taps 0 turns
+        it off.  Resets the equalizer and leaves the other loop and framer state alone.  Its group delay is absorbed: the
+        bits keep their alignment, and the last (n_taps-1)//2 symbols of a call come out at the start of the next."""
+        check(lib().qpsk_demod_set_equalizer(self._h, n_taps, mu, modulus))
+        self._eq_taps = n_taps
+
+    def equalizer_taps(self) -> np.ndarray:
+        """[2*n_taps] interleaved IQ ([channels, 2*n_taps] for batch handles); ArgumentException when the stage is off."""
+        out = np.empty((self.channels, 2 * getattr(self, "_eq_taps", 0)), np.float32)
+        check(lib().qpsk_demod_equalizer_taps(self._h, out.ctypes.data_as(N.f32p), out.size))
+        return out[0] if self.channels == 1 else out
+
     def _in(self, SamplesIQ):
         if SamplesIQ is None:
             raise ArgumentNullException("SamplesIQ")
