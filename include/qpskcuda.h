@@ -191,14 +191,22 @@ QPSK_API int qpsk_costas_get_state(qpsk_costas* c, double* theta, double* freq);
  *   e   = (fminf(fmaxf(y.re*d, -1), 1), fminf(fmaxf(y.im*d, -1), 1))
  *   g_k = e * conj(v_k)                    re = e.re*v.re + e.im*v.im, im = e.im*v.re - e.re*v.im
  *   w_k = w_k - mu*g_k                     (re and im separately, every k, after y is formed);  output y
+ * Fractionally spaced form (qpsk_eq_create_fractional): update stride S >= 1, the samples per symbol of a T/S-spaced
+ * input.  Each channel also keeps a stream sample counter n (0 at creation and reset).  Every input sample shifts the
+ * window, forms y and outputs it as above; d, e, g and the tap update run only when n % S == 0; then n = n + 1.
+ * S = 1 is the symbol-spaced equalizer: one update per input.
  * State persists across calls: any chunking of a stream gives the same outputs bit for bit.
  * n_taps 1..64 (else QPSK_ERR_UNSUPPORTED); mu finite and >= 0, modulus finite and > 0 (else QPSK_ERR_RANGE).  modulus
  * 1.0 is |symbol|^2 at this modem's matched-filter output for unit channel gain.  A refused call consumes no state. */
 typedef struct qpsk_eq qpsk_eq;
 QPSK_API int qpsk_eq_create(int n_taps, float mu, float modulus, qpsk_eq** out);
 QPSK_API int qpsk_eq_create_batch(int n_taps, float mu, float modulus, int channels, qpsk_eq** out);
+/* T/sps-spaced (fractionally spaced) equalizer: taps update on every sps-th input sample (update stride S = sps above).
+ * One output per input sample, group delay (n_taps-1)/2 samples.  sps 1..8 (else QPSK_ERR_UNSUPPORTED); sps 1 is
+ * qpsk_eq_create_batch.  Every other qpsk_eq_* entry point works on the handle unchanged. */
+QPSK_API int qpsk_eq_create_fractional(int n_taps, float mu, float modulus, int sps, int channels, qpsk_eq** out);
 QPSK_API int qpsk_eq_destroy(qpsk_eq* eq);
-QPSK_API int qpsk_eq_reset(qpsk_eq* eq);                      /* taps to the centre spike, window zeroed */
+QPSK_API int qpsk_eq_reset(qpsk_eq* eq);                      /* taps to the centre spike, window and sample counter zeroed */
 /* host memory, iq_in / iq_out [channels][n_floats]; odd n_floats -> QPSK_ERR_ARG, out_cap_floats < n_floats -> QPSK_ERR_CAPACITY */
 QPSK_API int qpsk_eq_process(qpsk_eq* eq, const float* iq_in, float* iq_out, int64_t n_floats, int64_t out_cap_floats);
 /* device memory, strides in floats; d_n_sym[channels] valid complex symbols per channel (NULL = n_floats/2 for all) */
@@ -267,6 +275,16 @@ QPSK_API int qpsk_demod_set_fir_mode(qpsk_demod* d, int mode);
 QPSK_API int qpsk_demod_set_equalizer(qpsk_demod* d, int n_taps, float mu, float modulus);
 /* the equalizer taps, [channels][2*n_taps]; QPSK_ERR_ARG when the stage is off */
 QPSK_API int qpsk_demod_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats);
+/* Opt-in fractionally spaced CMA equalizer stage (qpsk_eq_create_fractional, S = fs/rs) between the matched filter and
+ * Mueller-Muller, so clock recovery locks on an equalized eye; n_taps 0 = off (the default).  Needs an integer rate:
+ * fs % rs == 0 and S in 2..8, else QPSK_ERR_UNSUPPORTED.  The first (n_taps-1)/2 outputs (samples) of each channel's
+ * stream are discarded once, so a centre spike with mu 0 gives the bits of the handle without the stage; the last
+ * (n_taps-1)/2 samples of a call reach Mueller-Muller in the next.  Independent of qpsk_demod_set_equalizer (both may be
+ * on: FLL? -> MF -> FSE -> MM -> EQ -> Costas).  May be called at any time: synchronises the handle, resets this stage
+ * only (taps, window, sample counter, discard count).  With the stage on, the symbol path runs as separate kernels. */
+QPSK_API int qpsk_demod_set_fractional_equalizer(qpsk_demod* d, int n_taps, float mu, float modulus);
+/* the fractional stage's taps, [channels][2*n_taps]; QPSK_ERR_ARG when the stage is off */
+QPSK_API int qpsk_demod_fractional_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats);
 /* DeModulate(ReadOnlySpan<float>) :345-425 -> '0'/'1' chars (not NUL-terminated).  Batch handles:
  * iq_in [channels][n_floats], bits_out [channels][cap], n_bits[channels] (same layout rule for the
  * other host entry points below). */

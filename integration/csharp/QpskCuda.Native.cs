@@ -55,6 +55,7 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_costas_get_state(IntPtr h, out double theta, out double freq);
     // symbol-spaced blind CMA equalizer              (not in the reference; spec in include/qpskcuda.h)
     [DllImport(Lib)] internal static extern int qpsk_eq_create(int nTaps, float mu, float modulus, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_eq_create_fractional(int nTaps, float mu, float modulus, int sps, int channels, out IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_eq_destroy(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_eq_reset(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_eq_process(IntPtr h, float* iqIn, float* iqOut, long nFloats, long outCap);
@@ -75,6 +76,8 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_demod_destroy(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_demod_set_equalizer(IntPtr h, int nTaps, float mu, float modulus);
     [DllImport(Lib)] internal static extern int qpsk_demod_equalizer_taps(IntPtr h, float* tapsIq, long capFloats);
+    [DllImport(Lib)] internal static extern int qpsk_demod_set_fractional_equalizer(IntPtr h, int nTaps, float mu, float modulus);
+    [DllImport(Lib)] internal static extern int qpsk_demod_fractional_equalizer_taps(IntPtr h, float* tapsIq, long capFloats);
     [DllImport(Lib)] internal static extern int qpsk_demod_bits(IntPtr h, float* iqIn, long nFloats, byte* bitsOut, long cap, out long nBits);
     [DllImport(Lib)] internal static extern int qpsk_demod_bytes(IntPtr h, float* iqIn, long nFloats, byte* start, long nStart,
                                                                  byte* end, long nEnd, byte* payloadOut, long cap, out long nBytes);

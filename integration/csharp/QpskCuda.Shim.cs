@@ -228,8 +228,9 @@ namespace QPSK.Models
         public void Dispose() => _o.Dispose();
     }
 
-    // Symbol-spaced blind CMA equalizer: not a reference class (its receive chain has none); the block a GNU Radio PSK
-    // receiver puts between clock recovery and the Costas loop.  Arithmetic spec in include/qpskcuda.h.
+    // Blind CMA equalizer: not a reference class (its receive chain has none); the block a GNU Radio PSK receiver puts
+    // between clock recovery and the Costas loop, or (sps 2..8) fractionally spaced ahead of it.  Arithmetic spec in
+    // include/qpskcuda.h.
     public sealed unsafe class CmaEqualizer : IDisposable
     {
         readonly QpskHandle _o;
@@ -238,6 +239,13 @@ namespace QPSK.Models
         public CmaEqualizer(int nTaps, float mu, float modulus = 1.0f)
         {
             QpskCuda.Check(QpskCuda.qpsk_eq_create(nTaps, mu, modulus, out IntPtr h));
+            _o = new QpskHandle(h, QpskCuda.qpsk_eq_destroy);
+            NumTaps = nTaps;
+        }
+        // fractionally spaced: input at sps samples per symbol, the taps update on every sps-th sample (sps 1..8)
+        public CmaEqualizer(int nTaps, float mu, float modulus, int sps)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_eq_create_fractional(nTaps, mu, modulus, sps, 1, out IntPtr h));
             _o = new QpskHandle(h, QpskCuda.qpsk_eq_destroy);
             NumTaps = nTaps;
         }
@@ -375,6 +383,22 @@ namespace QPSK
         {
             var t = new float[2 * _eqTaps];
             fixed (float* p = t) QpskCuda.Check(QpskCuda.qpsk_demod_equalizer_taps(_h, p, t.Length));
+            GC.KeepAlive(this);
+            return t;
+        }
+        // opt-in fractionally spaced CMA equalizer between the matched filter and clock recovery (not in the reference;
+        // needs SampleRate / SymbolRate an integer 2..8; nTaps 0 = off, the default)
+        public void SetFractionalEqualizer(int nTaps, float mu, float modulus = 1.0f)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_demod_set_fractional_equalizer(_h, nTaps, mu, modulus));
+            _fseTaps = nTaps;
+            GC.KeepAlive(this);
+        }
+        int _fseTaps;
+        public float[] FractionalEqualizerTaps()
+        {
+            var t = new float[2 * _fseTaps];
+            fixed (float* p = t) QpskCuda.Check(QpskCuda.qpsk_demod_fractional_equalizer_taps(_h, p, t.Length));
             GC.KeepAlive(this);
             return t;
         }

@@ -111,6 +111,7 @@ def _signatures():
         "qpsk_costas_get_state": (i, [vp, f64p, f64p]),
         "qpsk_eq_create": (i, [i, f, f, vpp]),
         "qpsk_eq_create_batch": (i, [i, f, f, i, vpp]),
+        "qpsk_eq_create_fractional": (i, [i, f, f, i, i, vpp]),
         "qpsk_eq_destroy": (i, [vp]),
         "qpsk_eq_reset": (i, [vp]),
         "qpsk_eq_process": (i, [vp, vp, vp, i64, i64]),
@@ -131,6 +132,8 @@ def _signatures():
         "qpsk_demod_set_fir_mode": (i, [vp, i]),
         "qpsk_demod_set_equalizer": (i, [vp, i, f, f]),
         "qpsk_demod_equalizer_taps": (i, [vp, f32p, i64]),
+        "qpsk_demod_set_fractional_equalizer": (i, [vp, i, f, f]),
+        "qpsk_demod_fractional_equalizer_taps": (i, [vp, f32p, i64]),
         "qpsk_demod_bits": (i, [vp, vp, i64, vp, i64, vp]),
         "qpsk_demod_bits_packed": (i, [vp, vp, i64, vp, i64, vp]),
         "qpsk_demod_bytes": (i, [vp, vp, i64, vp, i64, vp, i64, vp, i64, vp]),

@@ -380,17 +380,18 @@ class CostasLoopQpsk(_Handle):
         return (float(t[0]), float(f[0])) if self.channels == 1 else (t, f)
 
 
-# ---- symbol-spaced blind CMA equalizer (not in the reference) ---------------------------------
+# ---- blind CMA equalizer (not in the reference) ------------------------------------------------
 class CmaEqualizer(_Handle):
-    """Symbol-spaced blind CMA equalizer on the GPU (csrc/eq.cu; arithmetic spec in include/qpskcuda.h): `n_taps` complex
-    taps (1..64) adapted by the constant-modulus rule with step `mu` towards |y|^2 = `modulus`, one output per input,
-    group delay (n_taps-1)//2 symbols.  State persists across calls."""
+    """Blind CMA equalizer on the GPU (csrc/eq.cu; arithmetic spec in include/qpskcuda.h): `n_taps` complex taps (1..64)
+    adapted by the constant-modulus rule with step `mu` towards |y|^2 = `modulus`, one output per input, group delay
+    (n_taps-1)//2 inputs.  `sps` 1 (the default) is symbol-spaced; `sps` 2..8 makes it fractionally spaced on a T/sps-spaced
+    input, the taps updating on every sps-th sample of the stream.  State persists across calls."""
     _destroy = "qpsk_eq_destroy"
 
-    def __init__(self, n_taps: int, mu: float, modulus: float = 1.0, channels: int = 1):
+    def __init__(self, n_taps: int, mu: float, modulus: float = 1.0, channels: int = 1, sps: int = 1):
         super().__init__()
-        self.n_taps, self.channels = n_taps, channels
-        check(lib().qpsk_eq_create_batch(n_taps, mu, modulus, channels, C.byref(self._h)))
+        self.n_taps, self.channels, self.sps = n_taps, channels, sps
+        check(lib().qpsk_eq_create_fractional(n_taps, mu, modulus, sps, channels, C.byref(self._h)))
 
     def Process(self, iqIn, iqOut=None):
         """-> the equalized symbols (interleaved IQ; [channels, n_floats] for batch handles).  With `iqOut` given the

@@ -2,8 +2,8 @@
 // channels.  Compiled with --fmad=false (see loops.cuh).
 //
 // Chain per call (DeModulate :345-425):  [FLL (opt-in; the call at :359 is commented out upstream)] ->
-// RRC matched filter (FirEngine, fir.cu) -> Mueller-Muller (loops.cu) -> [CMA equalizer (opt-in, eq.cu; not in the
-// reference)] -> decode kernel: Costas + decision + differential decode -> bits -> TSC exact-match strip (:413-422).
+// RRC matched filter (FirEngine, fir.cu) -> [fractionally spaced CMA equalizer (opt-in, eq.cu; not in the reference)] ->
+// Mueller-Muller (loops.cu) -> [CMA equalizer (opt-in, eq.cu; not in the reference)] -> decode kernel: Costas + decision + differential decode -> bits -> TSC exact-match strip (:413-422).
 // DeModulateBytes (:169-259): the bits then feed the per-channel framer kernel (8 bit-offset marker
 // hunt, MSB-first packing into a bounded ring, end-marker search).
 // All loop / framer state lives in device memory per channel and persists across calls, so arbitrary
@@ -980,12 +980,16 @@ struct DemodEngine {
   bool diff = true, has_tsc = false, use_fll = false;
   std::string tsc;
   double sps = 0.0;
+  int int_sps = 0;             // fs / rs when rs divides fs, else 0 (the fractionally spaced stage needs an integer rate)
   FirEngine mf;
   FllEngine fll;
   MmEngine mm;
   CostasEngine costas;
   std::unique_ptr<EqEngine> eq;    // opt-in CMA stage between MM and Costas (qpsk_demod_set_equalizer); null = off
-  DevBuf<float2> t_fll, t_rrc, t_sym, t_eq;
+  // opt-in T/sps-spaced CMA stage between the matched filter and MM (qpsk_demod_set_fractional_equalizer); null = off
+  std::unique_ptr<EqEngine> fse;
+  int64_t fse_drop = 0;            // outputs the stage still discards: the same for every channel (every call feeds all L)
+  DevBuf<float2> t_fll, t_rrc, t_sym, t_eq, t_fse;
   DevBuf<int> d_nsym, d_neq;
   // what front() leaves for Costas: the MM symbols, or with the equalizer on its outputs
   float2* sym_p = nullptr;
@@ -1054,6 +1058,7 @@ struct DemodEngine {
     has_tsc = !blank_or_null(tsc_in);                          // :21
     if (has_tsc) tsc = tsc_in;
     sps = (double)fs / (double)rs;
+    int_sps = (fs % rs == 0) ? fs / rs : 0;
     if (const char* e = getenv("QPSK_DEMOD_FUSE")) fuse = (e[0] != '0');   // tuning knob: 0 = separate MM / decode kernels
     QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
     const std::vector<double> h = design_rrc((double)span, (double)alpha, fs, rs);   // :28-32
@@ -1095,7 +1100,8 @@ struct DemodEngine {
   }
   long long bits_bound(int64_t L) const { return 2 * symbols_bound(L); }
 
-  // FLL? -> MF -> MM [-> EQ].  Symbols in sym_p [C][sym_ld] (t_sym, or t_eq with the equalizer on), counts in nsym_p.
+  // FLL? -> MF [-> FSE] -> MM [-> EQ].  Symbols in sym_p [C][sym_ld] (t_sym, or t_eq with the equalizer on), counts in
+  // nsym_p.
   int front(const float2* x, int64_t L, int64_t ldx, cudaStream_t s, bool run_mm = true) {
     const int64_t ld = L + (L & 1);
     QPSK_TRY(t_rrc.ensure((size_t)ld * channels));
@@ -1113,7 +1119,18 @@ struct DemodEngine {
     QPSK_TRY(mf.filter_dev(src, t_rrc.p, L, lds, ld, s));      // :360
     mf_ld = ld;
     if (!run_mm) return QPSK_OK;
-    QPSK_TRY(mm.process_dev(t_rrc.p, L, ld, t_sym.p, 2 * L, sym_ld, d_nsym.p, s));   // :364-367
+    const float2* mm_in = t_rrc.p;
+    int64_t mm_n = L;
+    if (fse) {
+      // every channel takes L samples, so every channel discards the same dc: MM takes L - dc samples of each row
+      QPSK_TRY(t_fse.ensure((size_t)ld * channels));
+      QPSK_TRY(fse->process_dev(t_rrc.p, t_fse.p, L, ld, ld, nullptr, nullptr, true, s));
+      const int64_t dc = fse_drop < L ? fse_drop : L;
+      fse_drop -= dc;
+      mm_in = t_fse.p;
+      mm_n = L - dc;
+    }
+    QPSK_TRY(mm.process_dev(mm_in, mm_n, ld, t_sym.p, 2 * L, sym_ld, d_nsym.p, s));   // :364-367
     sym_p = t_sym.p;
     nsym_p = d_nsym.p;
     if (eq) {
@@ -1127,7 +1144,7 @@ struct DemodEngine {
 
   // opt-in equalizer stage: n_taps 0 = off; otherwise a fresh equalizer (spike taps, zero window, discard count D)
   int set_equalizer(int n_taps, float mu, float modulus) {
-    if (n_taps != 0) QPSK_TRY(eq_check_params(n_taps, mu, modulus));
+    if (n_taps != 0) QPSK_TRY(eq_check_params(n_taps, mu, modulus, 1));
     QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
     if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
     if (n_taps == 0) {
@@ -1136,9 +1153,30 @@ struct DemodEngine {
     }
     std::unique_ptr<EqEngine> e(new (std::nothrow) EqEngine());
     if (!e) return QPSK_ERR_NOMEM;
-    QPSK_TRY(e->init(n_taps, mu, modulus, channels));
+    QPSK_TRY(e->init(n_taps, mu, modulus, 1, channels));
     QPSK_TRY(d_neq.ensure((size_t)channels));
     eq = std::move(e);
+    return QPSK_OK;
+  }
+
+  // opt-in fractionally spaced stage, update stride S = fs / rs: n_taps 0 = off; otherwise a fresh equalizer (spike taps,
+  // zero window, sample counter 0, discard count D)
+  int set_fractional_equalizer(int n_taps, float mu, float modulus) {
+    if (n_taps != 0) {
+      if (int_sps < 2 || int_sps > kEqMaxSps) return QPSK_ERR_UNSUPPORTED;
+      QPSK_TRY(eq_check_params(n_taps, mu, modulus, int_sps));
+    }
+    QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
+    if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
+    if (n_taps == 0) {
+      fse.reset();
+      return QPSK_OK;
+    }
+    std::unique_ptr<EqEngine> e(new (std::nothrow) EqEngine());
+    if (!e) return QPSK_ERR_NOMEM;
+    QPSK_TRY(e->init(n_taps, mu, modulus, int_sps, channels));
+    fse = std::move(e);
+    fse_drop = (n_taps - 1) / 2;
     return QPSK_OK;
   }
 
@@ -1232,7 +1270,7 @@ struct DemodEngine {
 
   // the fused MM -> Costas -> decode kernel applies when no call can run out of output room and the MM
   // queue holds at most kSsCarry samples (always true once every call has had room)
-  bool can_fuse() const { return fuse && !eq && (sps - 0.1 > 1.0) && mm.q_bound <= kSsCarry; }
+  bool can_fuse() const { return fuse && !eq && !fse && (sps - 0.1 > 1.0) && mm.q_bound <= kSsCarry; }
   // ... and it takes the matched filter in as well (MFW extra warps, see symsync_decode_kernel) when the filter runs in
   // the reference's summation order (the demodulator's default), has real taps and at most 65 of them.
   // QPSK_DEMOD_FUSE_MF=0 keeps the separate matched-filter launch (A/B runs).
@@ -1574,6 +1612,22 @@ int qpsk_demod_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats)
   QPSK_TRY(ensure_device(e.device));
   QPSK_CUDA_TRY(cudaStreamSynchronize(e.stream));
   QPSK_CUDA_TRY(cudaMemcpy(taps_iq, e.eq->d_taps.p, (size_t)need * 4, cudaMemcpyDeviceToHost));
+  return QPSK_OK;
+}
+int qpsk_demod_set_fractional_equalizer(qpsk_demod* d, int n_taps, float mu, float modulus) {
+  if (!d) return QPSK_ERR_NULL;
+  QPSK_TRY(ensure_device(d->eng.device));
+  return d->eng.set_fractional_equalizer(n_taps, mu, modulus);
+}
+int qpsk_demod_fractional_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats) {
+  if (!d || !taps_iq) return QPSK_ERR_NULL;
+  DemodEngine& e = d->eng;
+  if (!e.fse) return QPSK_ERR_ARG;
+  const int64_t need = (int64_t)e.channels * 2 * e.fse->P.n_taps;
+  if (cap_floats < need) return QPSK_ERR_CAPACITY;
+  QPSK_TRY(ensure_device(e.device));
+  QPSK_CUDA_TRY(cudaStreamSynchronize(e.stream));
+  QPSK_CUDA_TRY(cudaMemcpy(taps_iq, e.fse->d_taps.p, (size_t)need * 4, cudaMemcpyDeviceToHost));
   return QPSK_OK;
 }
 

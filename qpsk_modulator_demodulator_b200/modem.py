@@ -182,6 +182,20 @@ class QPSKDeModulator(_Handle):
         check(lib().qpsk_demod_equalizer_taps(self._h, out.ctypes.data_as(N.f32p), out.size))
         return out[0] if self.channels == 1 else out
 
+    def set_fractional_equalizer(self, n_taps: int, mu: float, modulus: float = 1.0):
+        """Opt-in fractionally spaced CMA equalizer (api.CmaEqualizer with sps = fs/rs) between the matched filter and
+        Mueller-Muller, so clock recovery locks on an equalized eye; n_taps 0 turns it off.  Needs fs % rs == 0 and
+        fs/rs in 2..8.  Independent of set_equalizer; resets this stage only.  Its group delay of (n_taps-1)//2 samples is
+        absorbed: the last (n_taps-1)//2 samples of a call reach clock recovery in the next."""
+        check(lib().qpsk_demod_set_fractional_equalizer(self._h, n_taps, mu, modulus))
+        self._fse_taps = n_taps
+
+    def fractional_equalizer_taps(self) -> np.ndarray:
+        """[2*n_taps] interleaved IQ ([channels, 2*n_taps] for batch handles); ArgumentException when the stage is off."""
+        out = np.empty((self.channels, 2 * getattr(self, "_fse_taps", 0)), np.float32)
+        check(lib().qpsk_demod_fractional_equalizer_taps(self._h, out.ctypes.data_as(N.f32p), out.size))
+        return out[0] if self.channels == 1 else out
+
     def _in(self, SamplesIQ):
         if SamplesIQ is None:
             raise ArgumentNullException("SamplesIQ")
