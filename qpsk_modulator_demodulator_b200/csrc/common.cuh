@@ -51,7 +51,7 @@ int device_sm_count();         // of the device the calling thread has current (
 // Host side of the pageable-memory path.  cudaMemcpyAsync on memory the driver has not page-locked is a blocking, staged copy on
 // the calling thread: the H2D / kernel / D2H pipelines of the host entry points degenerate into a sequence (FIR end to end:
 // 0.85 Gsample/s against 5.6 on page-locked buffers).  Such calls go through page-locked staging slots instead, filled and
-// drained by a small pool of host threads (QPSK_HOST_COPY_THREADS, default 6) while the DMA engines work on the other slots.
+// drained by a pool of six host threads (fewer on smaller hosts) while the DMA engines work on the other slots.
 bool host_ptr_is_pageable(const void* p);            // true when the driver does not know the address as page-locked memory
 void host_parallel_copy(void* dst, const void* src, size_t bytes);   // blocking; split over the pool and the caller
 // `rows` pieces of `width` bytes, `spitch` / `dpitch` bytes apart (a time chunk of a [channels][samples] block)
@@ -361,20 +361,6 @@ __device__ __forceinline__ void sincos_rq_f64_k(double x, const SinCosK& K, doub
   const double hz = K.half * z;
   const double w = K.one - hz;
   *cr_out = w + fma(z2, Cc, (K.one - w) - hz);
-}
-// MathF.Sin/Cos model (see sincos_f32_exact) through the register-constant fast path
-__device__ __forceinline__ void sincos_f32_fast_k(float x, const SinCosK& K, float* s, float* c) {
-  double sd, cd;
-  sincos_fast_f64_k((double)x, K, &sd, &cd);
-  *s = (float)sd;
-  *c = (float)cd;
-}
-// MathF.Sin/Cos model through the fast path (|x| small: loop phases are bounded)
-__device__ __forceinline__ void sincos_f32_fast(float x, float* s, float* c) {
-  double sd, cd;
-  sincos_fast_f64((double)x, &sd, &cd);
-  *s = (float)sd;
-  *c = (float)cd;
 }
 #endif
 

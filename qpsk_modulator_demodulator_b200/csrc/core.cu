@@ -188,11 +188,6 @@ bool blank_or_null(const char* s) {
 
 // ---- host copy pool -------------------------------------------------------------------------------------------------
 bool host_ptr_is_pageable(const void* p) {
-  static const bool off = [] {
-    const char* e = getenv("QPSK_HOST_BOUNCE");          // 0: leave pageable memory to the driver's own staging (A/B runs)
-    return e && e[0] == '0';
-  }();
-  if (off) return false;
   cudaPointerAttributes at;
   if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
     cudaGetLastError();                                  // older runtimes report unknown host memory as an error
@@ -262,11 +257,9 @@ class HostCopyPool {
     cv_done_.wait(lk, [&] { return pending_ == 0; });
   }
   HostCopyPool() {
-    int n = 6;
-    if (const char* e = getenv("QPSK_HOST_COPY_THREADS")) n = atoi(e);
+    int n = 6;                                           // copy threads, the caller's included
     const int hw = (int)std::thread::hardware_concurrency();
     if (hw > 0 && n > hw) n = hw;
-    if (n < 1) n = 1;
     for (int i = 1; i < n; ++i) workers_.emplace_back([this] { run(); });
   }
   ~HostCopyPool() {

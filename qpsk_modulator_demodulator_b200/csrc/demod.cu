@@ -8,8 +8,6 @@
 // hunt, MSB-first packing into a bounded ring, end-marker search).
 // All loop / framer state lives in device memory per channel and persists across calls, so arbitrary
 // chunking of a stream gives the same output as the reference object would.
-#include <stdlib.h>
-
 #include <memory>
 #include <string>
 
@@ -93,7 +91,6 @@ constexpr int kSsCarry = 4;
 // unconditional loads at (row + kSsCarry - carried + index).  Odd pitch (float2): rows of different lanes fall in different banks.
 constexpr int kSsPitch = kSsCarry + kSsBlock + 1;
 constexpr int kSsSymCap = kSsBlock + 4;  // symbols one round can emit (advance >= 0.9 samples)
-constexpr int kSsSymPitch = kSsSymCap + 1;
 
 __device__ __forceinline__ void cp_async8(void* smem_dst, const void* gsrc) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gsrc)
@@ -287,7 +284,7 @@ __device__ __forceinline__ void mf_round(const float2* __restrict__ ring_ch, int
 // DENSE: compiled for four resident CTAs per SM (a 128-register cap: some spills in the filter warps) — the choice when
 // the batch has more 32-channel CTAs than three per SM can hold, where one wave beats two
 template <bool DIFF, int MFW, bool DENSE = false>
-__global__ void __launch_bounds__(64 + 32 * MFW, MFW == 1 ? 4 : (MFW == 2 ? (DENSE ? 4 : 3) : (MFW == 4 ? 2 : 1)))
+__global__ void __launch_bounds__(64 + 32 * MFW, MFW == 2 ? (DENSE ? 4 : 3) : (MFW == 4 ? 2 : 1))
     symsync_decode_kernel(const MmParams MP, MmState* mm_g, const float2* __restrict__ q_in, float2* __restrict__ q_out,
                           long long qcap, const CostasParams CP, CostasState* cst_g, DiffState* dst_g, int C,
                           const float2* __restrict__ x, long long L, long long ldx, uint8_t* __restrict__ bits,
@@ -1005,7 +1002,6 @@ struct DemodEngine {
   long long ring_cap = 0;
   long long sym_ld = 0;
   int64_t mf_ld = 0;
-  bool fuse = true;            // use symsync_decode_kernel when it applies
   cudaStream_t stream = nullptr;
   cudaStream_t side = nullptr;               // front-end stream of the time-chunk pipeline
   cudaStream_t copy = nullptr;               // host-source calls: the PCIe copies (and the CS16 widening) of the chunks
@@ -1059,7 +1055,6 @@ struct DemodEngine {
     if (has_tsc) tsc = tsc_in;
     sps = (double)fs / (double)rs;
     int_sps = (fs % rs == 0) ? fs / rs : 0;
-    if (const char* e = getenv("QPSK_DEMOD_FUSE")) fuse = (e[0] != '0');   // tuning knob: 0 = separate MM / decode kernels
     QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
     const std::vector<double> h = design_rrc((double)span, (double)alpha, fs, rs);   // :28-32
     const std::vector<float> iq = real_taps_as_iq(h);
@@ -1180,34 +1175,25 @@ struct DemodEngine {
     return QPSK_OK;
   }
 
-  // Time-chunk pipeline of bits_dev (FLL path): number of chunks for an L-sample call.  QPSK_DEMOD_CHUNKS overrides
-  // (1 = off).  Short calls stay on one stream: the split costs two launches and a warm-up per chunk.  The channel count
-  // does not matter: a single stream gains as much as a full batch (1.10 -> 0.84 ms for 4196 samples), because the FLL
-  // and the symbol stages are each latency-bound on their own warps.
+  // Time-chunk pipeline of bits_dev (FLL path): number of chunks for an L-sample call.  Short calls stay on one stream: the
+  // split costs two launches and a warm-up per chunk.  The channel count does not matter: a single stream gains as much as
+  // a full batch (1.10 -> 0.84 ms for 4196 samples), because the FLL and the symbol stages are each latency-bound on their
+  // own warps.
   int pipeline_chunks(int64_t L) const {
-    static const int env = [] {
-      const char* e = getenv("QPSK_DEMOD_CHUNKS");
-      return e ? atoi(e) : 0;
-    }();
     // six chunks while the FLL is latency-bound (1.22 -> 1.15 ms per step at 2048 channels: a shorter exposed tail); four once
     // it is issue-bound and every extra launch pair costs more than the tail it hides (8192 channels: 2.22 against 2.32 ms)
-    int n = env > 0 ? env : (channels <= 4096 ? 6 : 4);
-    if (n > 16) n = 16;
-    if (env <= 0 && L < 2048) n = 1;
+    int n = channels <= 4096 ? 6 : 4;
+    if (L < 2048) n = 1;
     while (n > 1 && L < (int64_t)n * 8 * kSsBlock) --n;
     return n;
   }
   // host-source calls: chunks of >= 8 MiB of samples, at most 6 — every chunk is a 2-D copy of `channels` row pieces, and short
   // pieces cost PCIe efficiency (2048 channels x 4380 samples, Gsample/s end to end at 1 / 2 / 4 / 6 / 8 / 16 chunks: cf32 4.25 /
-  // 4.91 / 5.11 / 5.13 / 5.07 / 4.96, CS16 6.03 / 7.00 / 7.47 / 7.39 / 7.17 / 6.69; tools/e2e_chunks_sweep.py)
+  // 4.91 / 5.11 / 5.13 / 5.07 / 4.96, CS16 6.03 / 7.00 / 7.47 / 7.39 / 7.17 / 6.69)
   int host_chunks(int64_t L, bool cs16) const {
-    static const int env = [] {
-      const char* e = getenv("QPSK_DEMOD_HOST_CHUNKS");
-      return e ? atoi(e) : 0;
-    }();
     const double bytes = (double)L * channels * (cs16 ? 4.0 : 8.0);
-    int n = env > 0 ? env : (int)(bytes / (8.0 * 1024 * 1024));
-    if (n > (env > 0 ? 16 : 6)) n = env > 0 ? 16 : 6;
+    int n = (int)(bytes / (8.0 * 1024 * 1024));
+    if (n > 6) n = 6;
     if (n < 1) n = 1;
     while (n > 1 && L < (int64_t)n * 8 * kSsBlock) --n;
     return n;
@@ -1270,30 +1256,19 @@ struct DemodEngine {
 
   // the fused MM -> Costas -> decode kernel applies when no call can run out of output room and the MM
   // queue holds at most kSsCarry samples (always true once every call has had room)
-  bool can_fuse() const { return fuse && !eq && !fse && (sps - 0.1 > 1.0) && mm.q_bound <= kSsCarry; }
+  bool can_fuse() const { return !eq && !fse && (sps - 0.1 > 1.0) && mm.q_bound <= kSsCarry; }
   // ... and it takes the matched filter in as well (MFW extra warps, see symsync_decode_kernel) when the filter runs in
   // the reference's summation order (the demodulator's default), has real taps and at most 65 of them.
-  // QPSK_DEMOD_FUSE_MF=0 keeps the separate matched-filter launch (A/B runs).
   bool can_fuse_mf() const {
-    static const bool env_on = [] {
-      const char* e = getenv("QPSK_DEMOD_FUSE_MF");
-      return !(e && e[0] == '0');
-    }();
     // a lone CTA gains nothing from the fusion (the separate filter launch costs ~5 us) and its rounds run ~10 % slower
     // with the filter warps on board: one radio stream (qpsk_stream_*, per-call DeModulateBytes) keeps the separate kernel
     if (channels < 32) return false;
-    return env_on && mf.mode == QPSK_FIR_EXACT && mf.real_taps && mf.n_taps <= kMfMaxTaps && mf.n_taps >= 1;
+    return mf.mode == QPSK_FIR_EXACT && mf.real_taps && mf.n_taps <= kMfMaxTaps && mf.n_taps >= 1;
   }
   // matched-filter warps per 32-channel CTA.  One round costs a Mueller-Muller warp ~340 cycles per symbol; the filter
-  // needs ~70 issue slots per tap for the round's 32 outputs.  Small batches have SMs to spare and take the latency-safe
-  // choice; from ~8192 channels on the CTAs have to share SMs, and a single filter warp keeps four CTAs resident per SM
-  // (QPSK_DEMOD_MF_WARPS overrides).
+  // needs ~70 issue slots per tap for the round's 32 outputs.  Two filter warps while the estimate below fits in 60 % of a
+  // round, else four.
   int mf_warps() const {
-    static const int env = [] {
-      const char* e = getenv("QPSK_DEMOD_MF_WARPS");
-      return e ? atoi(e) : 0;
-    }();
-    if (env == 1 || env == 2 || env == 4) return env;
     const double round_cycles = 340.0 * (double)kSsBlock / sps;
     const double mf_slots = 110.0 * mf.n_taps;       // issue slots for the 32 outputs of one round (~3.4 per tap and output)
     return (mf_slots <= 0.6 * round_cycles) ? 2 : 4;
@@ -1325,26 +1300,12 @@ struct DemodEngine {
       ma.hist_in = mf.hist[mf.cur].p; ma.hist_out = mf.hist[mf.cur ^ 1].p; ma.HL = mf.HL;
       const size_t smem = symq_bytes + (size_t)32 * (ring_n + 1) * sizeof(float2);
       const int w = mf_warps();
-      const void* kp = nullptr;
-      const bool dense = w == 2 && grid > 3 * device_sm_count();
-      if (w == 1) kp = diff ? (const void*)symsync_decode_kernel<true, 1> : (const void*)symsync_decode_kernel<false, 1>;
-      else if (w == 2 && dense) kp = diff ? (const void*)symsync_decode_kernel<true, 2, true> : (const void*)symsync_decode_kernel<false, 2, true>;
-      else if (w == 2) kp = diff ? (const void*)symsync_decode_kernel<true, 2> : (const void*)symsync_decode_kernel<false, 2>;
-      else kp = diff ? (const void*)symsync_decode_kernel<true, 4> : (const void*)symsync_decode_kernel<false, 4>;
-      QPSK_TRY(allow_max_dynamic_smem(kp));
-      if (w == 1) {
-        if (diff) symsync_decode_kernel<true, 1><<<grid, 96, smem, s>>>(QPSK_SS_ARGS);
-        else symsync_decode_kernel<false, 1><<<grid, 96, smem, s>>>(QPSK_SS_ARGS);
-      } else if (w == 2 && dense) {
-        if (diff) symsync_decode_kernel<true, 2, true><<<grid, 128, smem, s>>>(QPSK_SS_ARGS);
-        else symsync_decode_kernel<false, 2, true><<<grid, 128, smem, s>>>(QPSK_SS_ARGS);
-      } else if (w == 2) {
-        if (diff) symsync_decode_kernel<true, 2><<<grid, 128, smem, s>>>(QPSK_SS_ARGS);
-        else symsync_decode_kernel<false, 2><<<grid, 128, smem, s>>>(QPSK_SS_ARGS);
-      } else {
-        if (diff) symsync_decode_kernel<true, 4><<<grid, 192, smem, s>>>(QPSK_SS_ARGS);
-        else symsync_decode_kernel<false, 4><<<grid, 192, smem, s>>>(QPSK_SS_ARGS);
-      }
+      decltype(&symsync_decode_kernel<false, 4>) kern;
+      if (w == 4) kern = diff ? symsync_decode_kernel<true, 4> : symsync_decode_kernel<false, 4>;
+      else if (grid > 3 * device_sm_count()) kern = diff ? symsync_decode_kernel<true, 2, true> : symsync_decode_kernel<false, 2, true>;
+      else kern = diff ? symsync_decode_kernel<true, 2> : symsync_decode_kernel<false, 2>;
+      QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
+      kern<<<grid, 64 + 32 * w, smem, s>>>(QPSK_SS_ARGS);
       mf.cur ^= 1;                                   // the kernel left the advanced delay line in the other buffer
     }
 #undef QPSK_SS_ARGS

@@ -23,8 +23,6 @@
 // pointers, and tap counts beyond the parameter-space table.
 #include "fir.cuh"
 
-#include <stdlib.h>
-
 namespace qpsk {
 
 // ---------------------------------------------------------------------------------------------
@@ -185,7 +183,7 @@ struct TileWalk {
 // and TMA-stores its own 32*R outputs, so warps drift apart and their prologues/epilogues overlap the
 // other warps' FFMA2 streams.
 template <int R, int NT, bool CPLX>
-__global__ void __launch_bounds__(NT + 32, R <= 6 ? 3 : 2)
+__global__ void __launch_bounds__(NT + 32, 2)
     fir_tma_kernel(const __grid_constant__ FirArgs a, const __grid_constant__ typename TapsOf<CPLX>::type taps) {
   static_assert(R % 2 == 0, "R must be even (LDS.128 moves two samples)");
   constexpr int T = R * NT;
@@ -1518,34 +1516,19 @@ namespace {
 
 constexpr int kR = 10;
 constexpr int kNT = 256;
-constexpr int kT = kR * kNT;
+constexpr int kNTWide = 320;
 constexpr int kSmemBudget = 112 * 1024;  // per CTA, two CTAs per SM
 
-// tile geometry of the TMA kernel: R outputs per thread, NT compute threads, CTAs per SM.  The production choice is
-// (10, 256, 2); QPSK_FIR_CFG=<index> selects another entry for tuning runs.  Measured on a B200, 2^28 samples, ms for
-// 33 / 65 / 129 / 257 taps:  (10,256,2) 0.79 1.32 2.37 4.46 | (10,320,2) 0.79 1.29 2.43 4.72 | (14,224,2) 0.83 1.40
-// 2.56 4.97 | (6,256,3) 0.92 1.52 2.73 5.15 | (10,192,3) 0.88 1.52 2.78 5.35 | (14,192,2) 0.96 1.64 3.01 5.80 |
-// (10,288,2) 0.91 1.59 3.01 5.85: eight consumer warps per CTA (four per scheduler with two CTAs) beat both fewer,
-// fatter threads and warp counts that do not divide over the four schedulers.
-struct FirCfg {
-  int R, NT, per_sm;
-};
-constexpr FirCfg kFirCfgs[] = {{10, 256, 2}, {10, 320, 2}, {14, 224, 2}, {6, 256, 3}};
-// QPSK_FIR_CFG=<index> forces one entry; otherwise the tap count picks: ten consumer warps (10, 320, 2) are ahead for
-// real-tap filters of ~48-96 taps (65 taps: 1.29 against 1.32 ms in the table above), eight everywhere else.
-inline int fir_cfg_index(int G = 0, bool cplx = false) {
-  static const int forced = [] {
-    const char* e = getenv("QPSK_FIR_CFG");
-    if (!e) return -1;
-    const int i = atoi(e);
-    return (i >= 0 && i < (int)(sizeof(kFirCfgs) / sizeof(kFirCfgs[0]))) ? i : 0;
-  }();
-  if (forced >= 0) return forced;
-  return (!cplx && G >= 48 && G <= 96) ? 1 : 0;
-}
+// tile geometry of the TMA kernel: R outputs per thread, NT compute threads, two CTAs per SM.  Measured on a B200, 2^28
+// samples, ms for 33 / 65 / 129 / 257 taps (R, NT, CTAs per SM):  (10,256,2) 0.79 1.32 2.37 4.46 | (10,320,2) 0.79 1.29
+// 2.43 4.72 | (14,224,2) 0.83 1.40 2.56 4.97 | (6,256,3) 0.92 1.52 2.73 5.15 | (10,192,3) 0.88 1.52 2.78 5.35 |
+// (14,192,2) 0.96 1.64 3.01 5.80 | (10,288,2) 0.91 1.59 3.01 5.85: eight consumer warps per CTA (four per scheduler with
+// two CTAs) beat both fewer, fatter threads and warp counts that do not divide over the four schedulers.  Ten consumer
+// warps (kNTWide) are ahead for real-tap filters of ~48-96 taps (65 taps: 1.29 against 1.32 ms), eight everywhere else.
+inline bool fir_wide(int G, bool cplx) { return !cplx && G >= 48 && G <= 96; }
 
 template <int R, int NT, bool CPLX>
-int launch_tma_cfg(const FirArgs& a, const typename TapsOf<CPLX>::type& taps, size_t smem, int grid, cudaStream_t s) {
+int launch_tma(const FirArgs& a, const typename TapsOf<CPLX>::type& taps, size_t smem, int grid, cudaStream_t s) {
   auto kern = fir_tma_kernel<R, NT, CPLX>;
   QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
   kern<<<grid, NT + 32, smem, s>>>(a, taps);
@@ -1553,38 +1536,19 @@ int launch_tma_cfg(const FirArgs& a, const typename TapsOf<CPLX>::type& taps, si
   return QPSK_OK;
 }
 inline const char* tma_kernel_name(bool cplx, int G) {
-  static const char* const real_names[] = {"fir_tma_kernel<R=10,NT=256,real taps>", "fir_tma_kernel<R=10,NT=320,real taps>",
-                                           "fir_tma_kernel<R=14,NT=224,real taps>", "fir_tma_kernel<R=6,NT=256,real taps>"};
-  static const char* const cplx_names[] = {"fir_tma_kernel<R=10,NT=256,complex taps>", "fir_tma_kernel<R=10,NT=320,complex taps>",
-                                           "fir_tma_kernel<R=14,NT=224,complex taps>", "fir_tma_kernel<R=6,NT=256,complex taps>"};
-  return (cplx ? cplx_names : real_names)[fir_cfg_index(G, cplx)];
-}
-template <bool CPLX>
-int launch_tma(const FirArgs& a, const typename TapsOf<CPLX>::type& taps, size_t smem, int grid, cudaStream_t s) {
-  switch (fir_cfg_index(a.G, CPLX)) {
-    case 1: return launch_tma_cfg<10, 320, CPLX>(a, taps, smem, grid, s);
-    case 2: return launch_tma_cfg<14, 224, CPLX>(a, taps, smem, grid, s);
-    case 3: return launch_tma_cfg<6, 256, CPLX>(a, taps, smem, grid, s);
-    default: return launch_tma_cfg<kR, kNT, CPLX>(a, taps, smem, grid, s);
-  }
+  if (cplx) return "fir_tma_kernel<R=10,NT=256,complex taps>";
+  return fir_wide(G, false) ? "fir_tma_kernel<R=10,NT=320,real taps>" : "fir_tma_kernel<R=10,NT=256,real taps>";
 }
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-// fir_split2_kernel geometry and the tap count from which QPSK_FIR_FAST uses it for real taps (QPSK_FIR_SPLIT2_MIN=<G>
-// overrides, 0 = never)
+// fir_split2_kernel geometry and the tap count from which QPSK_FIR_FAST uses it for real taps
 // Measured on a B200, 2^28 samples, ms for 33 / 65 / 129 / 257 taps: FMA kernel 0.797 1.296 2.367 4.456 | split (10, 256)
 // 0.825 1.187 2.020 3.656 | split (10, 320), two ring stages only: - 1.301 2.243 4.199.  Ahead from ~48 taps on, where the
 // FMA pipe rather than HBM sets the time.
 constexpr int kS2R = 10, kS2NT = 256;
 constexpr int kS2MinForced = 14;        // QPSK_FIR_SPLIT: at least one full block of seven sub-taps
-inline int fir_split2_min_g() {
-  static const int v = [] {
-    const char* e = getenv("QPSK_FIR_SPLIT2_MIN");
-    return e && *e ? atoi(e) : 48;
-  }();
-  return v;
-}
+constexpr int kS2MinFast = 48;
 inline bool fir_mode_is_fast(int mode) { return mode != QPSK_FIR_EXACT; }
 // a: stream, delay-line and tap geometry filled in; tile geometry and the launch happen here
 template <int R2, int NT2>
@@ -1626,9 +1590,8 @@ int FirEngine::run(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t l
   const int hl = stateless ? (N - 1) : HL;
   const int G = (hl + 1 + 1) & ~1;
 
-  const FirCfg cfg = kFirCfgs[fir_cfg_index(G, !real_taps)];
-  const int T = cfg.R * cfg.NT;
-  const int smem_budget = (cfg.per_sm == 2) ? kSmemBudget : (224 * 1024 / cfg.per_sm);
+  const bool wide = fir_wide(G, !real_taps);
+  const int T = kR * (wide ? kNTWide : kNT);
   bool use_tma = (fir_mode_is_fast(mode) || stateless) && G <= kMaxG && hl <= T;
   if (use_tma) {
     if (!aligned16(x) || !aligned16(y)) use_tma = false;
@@ -1641,7 +1604,7 @@ int FirEngine::run(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t l
   float2* hout = stateless ? nullptr : hist[cur ^ 1].p;
 
   const bool want_split = (mode == QPSK_FIR_SPLIT && G >= kS2MinForced) ||
-                          (mode == QPSK_FIR_FAST && fir_split2_min_g() > 0 && G >= fir_split2_min_g());
+                          (mode == QPSK_FIR_FAST && G >= kS2MinFast);
   if (use_tma && real_taps && want_split) {
     FirArgs a;
     a.x = x; a.y = y; a.ldx = ldx; a.ldy = ldy; a.L = L;
@@ -1676,12 +1639,12 @@ int FirEngine::run(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t l
     a.stage_elems = a.E_load + 2;
     const size_t stage_bytes = (size_t)a.stage_elems * 8;
     const size_t out_bytes = (size_t)2 * T * 8;
-    int stages = (int)((smem_budget - out_bytes - 128) / stage_bytes);
+    int stages = (int)((kSmemBudget - out_bytes - 128) / stage_bytes);
     if (stages > 4) stages = 4;
     if (stages >= 2) {
       a.stages = stages;
       const size_t smem = (size_t)stages * stage_bytes + out_bytes + (size_t)stages * 16;
-      long long grid = (long long)cfg.per_sm * device_sm_count();
+      long long grid = 2LL * device_sm_count();
       if (grid > a.total_tiles) grid = a.total_tiles;
       if (real_taps) {
         TapsReal t;
@@ -1690,7 +1653,8 @@ int FirEngine::run(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t l
           const int j = hl - i;
           t.g[i] = (j < N) ? taps_iq[2 * j] : 0.0f;
         }
-        QPSK_TRY(launch_tma<false>(a, t, smem, (int)grid, s));
+        if (wide) QPSK_TRY((launch_tma<kR, kNTWide, false>(a, t, smem, (int)grid, s)));
+        else QPSK_TRY((launch_tma<kR, kNT, false>(a, t, smem, (int)grid, s)));
       } else {
         TapsCplx t;
         memset(&t, 0, sizeof t);
@@ -1699,7 +1663,7 @@ int FirEngine::run(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t l
           t.gi[i] = (j < N) ? taps_iq[2 * j] : 0.0f;
           t.gq[i] = (j < N) ? taps_iq[2 * j + 1] : 0.0f;
         }
-        QPSK_TRY(launch_tma<true>(a, t, smem, (int)grid, s));
+        QPSK_TRY((launch_tma<kR, kNT, true>(a, t, smem, (int)grid, s)));
       }
       last_kernel = tma_kernel_name(!real_taps, G);
       if (!stateless) cur ^= 1;
@@ -1820,13 +1784,8 @@ int FirEngine::decimate_dev(const float2* x, int64_t L, int64_t ldx, int dec, fl
       return QPSK_OK;
     };
     int st = QPSK_ERR_UNSUPPORTED;
-    // D = 2 on the TMA pipeline (fir_dec2_kernel) when the pointers allow bulk copies; QPSK_FIR_DEC2_TMA=0 keeps the
-    // register-staged kernel (A/B runs)
-    static const bool dec2_tma = [] {
-      const char* e = getenv("QPSK_FIR_DEC2_TMA");
-      return !(e && e[0] == '0');
-    }();
-    if (dec == 2 && dec2_tma && aligned16(x) && aligned16(y) && !(channels > 1 && ((ldx & 1) || (ldy & 1)))) {
+    // D = 2 on the TMA pipeline (fir_dec2_kernel) when the pointers allow bulk copies
+    if (dec == 2 && aligned16(x) && aligned16(y) && !(channels > 1 && ((ldx & 1) || (ldy & 1)))) {
       constexpr int R2 = 14, NT2 = 256, T2 = R2 * NT2, TO2 = T2 / 2;
       const int Gs = (HL + 1 + (int)skip + 1) & ~1;
       if (Gs <= kMaxG && HL <= T2) {
@@ -1861,7 +1820,7 @@ int FirEngine::decimate_dev(const float2* x, int64_t L, int64_t ldx, int dec, fl
       }
     }
     // D = 4, 8, 16 on the same pipeline (fir_decim_tma_kernel, dense tiles)
-    if (dec > 2 && dec2_tma && aligned16(x) && !(channels > 1 && (ldx & 1))) {
+    if (dec > 2 && aligned16(x) && !(channels > 1 && (ldx & 1))) {
       const int sk = (int)(skip & 1);
       const int Ks = (HL + 1 + sk + dec - 1) / dec;
       auto go_tma = [&](auto kern, int NTO, int NG, bool repack, const char* name) -> int {

@@ -26,8 +26,6 @@
 // from lane 7's prefix of the previous step; the last stage closes window n.
 #include "loops.cuh"
 
-#include <stdlib.h>
-
 #include <type_traits>
 
 namespace qpsk {
@@ -485,15 +483,10 @@ bool fll_duo_supported(int n_taps) { return n_taps >= 8 && n_taps <= 55; }
 
 int fll_duo_launch(const FllParams& P, const float* taps, float2* ring, int* head, float2* pf, int C, const float2* x,
                    float2* y, long long L, long long ldx, long long ldy, cudaStream_t s) {
-  static const int pairs_env = [] {
-    const char* e = getenv("QPSK_FLL_PAIRS");                // 1 or 4 warp pairs per CTA (timing experiments)
-    return e ? atoi(e) : 0;
-  }();
   // measured on a B200 (tools/fll_only.py, 40 taps): up to ~1300 streams one pair per CTA spreads the chain warps
   // over all SMs (356 cycles per sample at 1024 streams against 421); beyond that four pairs per CTA, one chain and
   // one side warp per scheduler, keep two chain warps off the same scheduler (4096 streams: 580 against 724)
-  const int pairs = pairs_env ? pairs_env : (C <= 1280 ? 1 : 4);
-  if (pairs == 1) return launch_duo<1>(P.n_taps, P, taps, ring, head, pf, C, x, y, L, ldx, ldy, s);
+  if (C <= 1280) return launch_duo<1>(P.n_taps, P, taps, ring, head, pf, C, x, y, L, ldx, ldy, s);
   return launch_duo<4>(P.n_taps, P, taps, ring, head, pf, C, x, y, L, ldx, ldy, s);
 }
 

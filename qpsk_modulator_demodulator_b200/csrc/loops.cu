@@ -1,9 +1,7 @@
-// loops.cu — K4/K5 building blocks: standalone FLL, Mueller-Muller and Costas kernels (one thread
-// per independent stream) and the qpsk_fll_* / qpsk_mm_* / qpsk_costas_* entry points.
+// loops.cu — K4/K5 building blocks: the generic FLL kernel, the Mueller-Muller and Costas kernels (one
+// thread per independent stream) and the qpsk_fll_* / qpsk_mm_* / qpsk_costas_* entry points.
 // Compiled with --fmad=false (see loops.cuh).
 #include "loops.cuh"
-
-#include <stdlib.h>
 
 namespace qpsk {
 
@@ -12,42 +10,6 @@ constexpr int kLoopThreads = 32;  // one warp per CTA: spreads few streams over 
 // ---------------------------------------------------------------------------------------------
 // FLL kernels
 // ---------------------------------------------------------------------------------------------
-// fll_kernel: one thread per stream (reference implementation of the recurrence on the GPU; used for
-// very long band-edge filters).
-__global__ void __launch_bounds__(kLoopThreads)
-    fll_kernel(const FllParams P, const float* __restrict__ taps, float2* ring_g, int* head_g, float2* pf_g, int C,
-               const float2* __restrict__ x, float2* __restrict__ y, long long L, long long ldx, long long ldy) {
-  extern __shared__ float sm[];
-  const int N = P.n_taps;
-  float* tapI = sm;
-  float* tapQ = sm + N;
-  float2* ring = reinterpret_cast<float2*>(sm + 2 * N + ((2 * N) & 1));  // 8-byte aligned
-  for (int i = threadIdx.x; i < 2 * N; i += blockDim.x) sm[i] = taps[i];
-  const int c = blockIdx.x * blockDim.x + threadIdx.x;
-  const bool live = c < C;
-  // per-thread ring in shared memory, element i at ring[i*blockDim.x + tid]: conflict-free
-  float2* myring = ring + threadIdx.x;
-  const int rs = blockDim.x;
-  if (live)
-    for (int i = 0; i < N; ++i) myring[i * rs] = ring_g[(long long)i * C + c];
-  __syncthreads();
-  if (!live) return;
-  int head = head_g[c];
-  float2 pf = pf_g[c];
-  float phase = pf.x, freq = pf.y;
-  const float2* xc = x + (long long)c * ldx;
-  float2* yc = y + (long long)c * ldy;
-  for (long long n = 0; n < L; ++n) {
-    const float2 in = xc[n];
-    float oI, oQ;
-    fll_step(P, tapI, tapQ, myring, rs, head, phase, freq, in.x, in.y, oI, oQ);
-    yc[n] = make_float2(oI, oQ);
-  }
-  for (int i = 0; i < N; ++i) ring_g[(long long)i * C + c] = myring[i * rs];
-  head_g[c] = head;
-  pf_g[c] = make_float2(phase, freq);
-}
-
 // fll_group_kernel: 8 lanes per stream — GPU lane g of a group IS lane g of the reference's
 // Vector<float> dot product (FIRFilter.cs:165-180): it accumulates window elements i = g, g+8, ... of all
 // four sums (lower I/Q, upper I/Q) in the reference's order, the eight partials are then added lane 0..7
@@ -161,178 +123,6 @@ __global__ void __launch_bounds__(kFllCtaThreads)
   }
 }
 
-// fll_group_kernel_t<K, TAIL>: the same mapping, specialised at compile time for N = 8*K + TAIL taps so
-// that one sample step is straight-line code the scheduler can interleave:
-//   * the partial sums over the N-1 OLD outputs do not depend on this sample's phase, so they (and the
-//     exchange of the eight lane partials through shared memory) run alongside the fp64 sincos chain;
-//   * only  acc = prefix + (partial + term(out[n]))  [+ nothing else] follows the rotation — in exactly the
-//     reference's order of additions: the newest window element is the LAST term of lane 7 (TAIL == 0,
-//     FIRFilter.cs:165-180) or the last scalar-tail term (TAIL > 0, :183-192);
-//   * taps live in registers, the ring is doubled (2N, like the reference's delay line :50-51) so no
-//     index wraps, sin/cos come from the branch-free sincos_fast_f64 (the loop phase is bounded by
-//     2*pi + max|freq|).
-template <int K, int TAIL>
-__global__ void __launch_bounds__(kFllCtaThreads)
-    fll_group_kernel_t(const FllParams P, const float* __restrict__ taps, float2* ring_g, int* head_g, float2* pf_g, int C,
-                       const float2* __restrict__ x, float2* __restrict__ y, long long L, long long ldx, long long ldy) {
-  constexpr int N = 8 * K + TAIL;
-  constexpr int NV = 8 * K;
-  constexpr int TOLD = TAIL > 0 ? TAIL - 1 : 0;            // old samples in the scalar tail
-  __shared__ __align__(16) float4 part[kFllCtaStreams * kFllGroup];
-  __shared__ float2 xin[kFllCtaStreams * kFllBlock];
-  __shared__ float2 yout[kFllCtaStreams * kFllBlock];
-  __shared__ float2 ring[kFllCtaStreams * 2 * N];
-  const int sl = threadIdx.x / kFllGroup;
-  const int g = threadIdx.x % kFllGroup;
-  const int c_raw = blockIdx.x * kFllCtaStreams + sl;
-  const bool live = c_raw < C;
-  const int c = live ? c_raw : C - 1;
-  float4* mypart = part + sl * kFllGroup;
-  float2* myx = xin + sl * kFllBlock;
-  float2* myy = yout + sl * kFllBlock;
-  float2* myring = ring + (size_t)sl * 2 * N;
-  // reversed lower taps: taps[i] = tapI_rev[i], taps[N+i] = tapQ_rev[i]
-  float ta[K], tb[K];
-#pragma unroll
-  for (int k = 0; k < K; ++k) {
-    ta[k] = taps[g + 8 * k];
-    tb[k] = taps[N + g + 8 * k];
-  }
-  float tla[TAIL > 0 ? TAIL : 1], tlb[TAIL > 0 ? TAIL : 1];
-#pragma unroll
-  for (int t = 0; t < TAIL; ++t) {
-    tla[t] = taps[NV + t];
-    tlb[t] = taps[N + NV + t];
-  }
-  const float newA = taps[N - 1], newB = taps[2 * N - 1];   // tap of the newest window element
-  const SinCosK SK = sincos_load_consts();
-  for (int i = g; i < N; i += kFllGroup) {
-    const float2 v = ring_g[(long long)i * C + c];
-    myring[i] = v;
-    myring[i + N] = v;
-  }
-  int pos = head_g[c];                                      // slot the next output goes to (= oldest)
-  const float2 pf = pf_g[c];
-  float phase = pf.x, freq = pf.y;
-  const float2* xc = x + (long long)c * ldx;
-  float2* yc = y + (long long)c * ldy;
-  __syncwarp();
-  for (long long n0 = 0; n0 < L; n0 += kFllBlock) {
-    const int nb = (int)((L - n0) < kFllBlock ? (L - n0) : kFllBlock);
-    for (int i = g; i < nb; i += kFllGroup) myx[i] = xc[n0 + i];
-    __syncwarp();
-    for (int n = 0; n < nb; ++n) {
-      // -- critical chain: phase -> sin/cos -> rotated sample
-      float s, co;
-      sincos_f32_fast_k(phase, SK, &s, &co);                // MathF.Cos/Sin(phase) :108-109
-      const float2 in = myx[n];
-      const float oI = in.x * co - in.y * s;                // :111
-      const float oQ = in.x * s + in.y * co;                // :112
-      // -- independent of the above: lane partials over the old outputs (window element i at ring[pos+1+i])
-      const float2* wp = myring + pos + 1 + g;
-      float loI = 0.f, loQ = 0.f, upI = 0.f, upQ = 0.f;
-#pragma unroll
-      for (int k = 0; k < K; ++k) {
-        const float2 v = wp[8 * k];
-        const float p1 = ta[k] * v.x, p2 = tb[k] * v.y, p3 = ta[k] * v.y, p4 = tb[k] * v.x;
-        if (TAIL == 0 && k == K - 1) {
-          // lane 7's last element is out[n] itself: its term is added after the rotation (below)
-          const bool skip = g == kFllGroup - 1;
-          loI = skip ? loI : loI + (p1 - p2);
-          loQ = skip ? loQ : loQ + (p3 + p4);
-          upI = skip ? upI : upI + (p1 + p2);
-          upQ = skip ? upQ : upQ + (p3 - p4);
-        } else {
-          loI = loI + (p1 - p2);
-          loQ = loQ + (p3 + p4);
-          upI = upI + (p1 + p2);
-          upQ = upQ + (p3 - p4);
-        }
-      }
-      // exchange the eight lane partials; every lane adds them in lane order 0..7 (:176-180), redundantly, so
-      // nothing but register arithmetic follows the rotation (cross-lane traffic stays off the critical path)
-      mypart[g] = make_float4(loI, loQ, upI, upQ);
-      __syncwarp();
-      float aLoI = 0.f, aLoQ = 0.f, aUpI = 0.f, aUpQ = 0.f;
-#pragma unroll
-      for (int l = 0; l < kFllGroup - 1; ++l) {
-        const float4 q = mypart[l];
-        aLoI += q.x; aLoQ += q.y; aUpI += q.z; aUpQ += q.w;
-      }
-      float4 q7 = mypart[kFllGroup - 1];
-      const float n1 = newA * oI, n2 = newB * oQ, n3 = newA * oQ, n4 = newB * oI;   // term of out[n]
-      if (TAIL == 0) {                                       // last term of lane 7, then lane 7 joins the sum
-        q7.x = q7.x + (n1 - n2); q7.y = q7.y + (n3 + n4); q7.z = q7.z + (n1 + n2); q7.w = q7.w + (n3 - n4);
-        aLoI += q7.x; aLoQ += q7.y; aUpI += q7.z; aUpQ += q7.w;
-      } else {
-        aLoI += q7.x; aLoQ += q7.y; aUpI += q7.z; aUpQ += q7.w;
-        const float2* tp = myring + pos + 1 + NV;
-#pragma unroll
-        for (int t = 0; t < TOLD; ++t) {                    // old scalar-tail terms (:183-192)
-          const float2 v = tp[t];
-          const float p1 = tla[t] * v.x, p2 = tlb[t] * v.y, p3 = tla[t] * v.y, p4 = tlb[t] * v.x;
-          aLoI += (p1 - p2); aLoQ += (p3 + p4); aUpI += (p1 + p2); aUpQ += (p3 - p4);
-        }
-        aLoI += (n1 - n2); aLoQ += (n3 + n4); aUpI += (n1 + n2); aUpQ += (n3 - n4);
-      }
-      const float powUpper = aUpI * aUpI + aUpQ * aUpQ;     // :118
-      const float powLower = aLoI * aLoI + aLoQ * aLoQ;     // :119
-      const float error = powLower - powUpper;              // :121
-      freq += P.beta * error;                               // :124
-      phase += freq + P.alpha * error;                      // :125
-      if (g == 0) {
-        const float2 o = make_float2(oI, oQ);
-        myring[pos] = o;
-        myring[pos + N] = o;
-        myy[n] = o;
-      }
-      pos = (pos + 1 == N) ? 0 : pos + 1;
-      if (phase > kTwoPiF || phase < -kTwoPiF) phase = remainderf(phase, kTwoPiF);   // :185-189
-      if (freq > P.max_freq) freq = P.max_freq;             // :191-195
-      else if (freq < P.min_freq) freq = P.min_freq;
-      __syncwarp();
-    }
-    if (live)
-      for (int i = g; i < nb; i += kFllGroup) yc[n0 + i] = myy[i];
-    __syncwarp();
-  }
-  if (live) {
-    for (int i = g; i < N; i += kFllGroup) ring_g[(long long)i * C + c] = myring[i];
-    if (g == 0) {
-      head_g[c] = pos;
-      pf_g[c] = make_float2(phase, freq);
-    }
-  }
-}
-
-typedef void (*FllGroupFn)(const FllParams, const float*, float2*, int*, float2*, int, const float2*, float2*, long long,
-                           long long, long long);
-template <int K>
-static FllGroupFn fll_group_pick_tail(int tail) {
-  switch (tail) {
-    case 0: return fll_group_kernel_t<K, 0>;
-    case 1: return fll_group_kernel_t<K, 1>;
-    case 2: return fll_group_kernel_t<K, 2>;
-    case 3: return fll_group_kernel_t<K, 3>;
-    case 4: return fll_group_kernel_t<K, 4>;
-    case 5: return fll_group_kernel_t<K, 5>;
-    case 6: return fll_group_kernel_t<K, 6>;
-    default: return fll_group_kernel_t<K, 7>;
-  }
-}
-static FllGroupFn fll_group_pick(int n_taps) {
-  const int k = n_taps / 8, tail = n_taps % 8;
-  switch (k) {
-    case 1: return fll_group_pick_tail<1>(tail);
-    case 2: return fll_group_pick_tail<2>(tail);
-    case 3: return fll_group_pick_tail<3>(tail);
-    case 4: return fll_group_pick_tail<4>(tail);
-    case 5: return fll_group_pick_tail<5>(tail);
-    case 6: return fll_group_pick_tail<6>(tail);
-    default: return nullptr;                                // N < 8 or N >= 56: generic kernel
-  }
-}
-
 FllEngine::~FllEngine() {
   if (stream) cudaStreamDestroy(stream);
 }
@@ -343,7 +133,7 @@ int FllEngine::init(float sps, float rolloff, int size, float bw, int channels_i
   if (size <= 0) return QPSK_ERR_RANGE;                      // :44
   if (!(bw > 0.0f)) return QPSK_ERR_RANGE;                   // :45
   if (channels_in <= 0) return QPSK_ERR_RANGE;
-  if (size > 2048) return QPSK_ERR_UNSUPPORTED;              // per-thread ring lives in shared memory
+  if (size > 2048) return QPSK_ERR_UNSUPPORTED;              // the ring lives in shared memory
   QPSK_TRY(ensure_device());
   device = current_device();
   channels = channels_in;
@@ -376,74 +166,33 @@ int FllEngine::process_dev(const float2* x, float2* y, int64_t L, int64_t ldx, i
   if (L == 0) return QPSK_OK;
   if (!x || !y) return QPSK_ERR_NULL;
   if (!s) s = stream;
-  static const int force_impl = [] {
-    const char* e = getenv("QPSK_FLL_IMPL");                 // "group": the single-warp kernels, "thread": one thread per
-    if (e && strcmp(e, "group") == 0) return 1;              // stream (A/B timing, tests)
-    if (e && strcmp(e, "thread") == 0) return 2;
-    if (e && strcmp(e, "lane") == 0) return 3;               // "lane": one lane per stream at any stream count
-    if (e && strcmp(e, "duo") == 0) return 4;                // "duo": never the lane kernel
-    if (e && strcmp(e, "pair") == 0) return 5;               // "pair": two lanes per stream at any stream count
-    return 0;
-  }();
   // Kernel choice by stream count (40 taps, 4196 samples, ms; tools/fll_only.py):
   //   streams   1024   2048   4096   8192   16384
   //   duo       0.76   0.90   1.25   2.46   4.49    two warps per four streams: shortest recurrence (356 cycles / sample),
   //                                                   44 warp instructions per stream and sample -> issue-bound from ~4096
   //   pair      1.45   1.45   1.45   1.47   2.35    two lanes per stream, software-pipelined (680 cycles / sample, ~21 issue
   //                                                   slots per stream and sample)
-  //   lane      2.28   2.40   2.50   2.50   2.52    one lane per stream (the general sin/cos: any |phase| < 1e5)
-  // QPSK_FLL_PAIR_MIN overrides the crossover.
-  static const int pair_min = [] {
-    const char* e = getenv("QPSK_FLL_PAIR_MIN");
-    return e ? atoi(e) : 5120;
-  }();
-  static const int lane_min = [] {
-    const char* e = getenv("QPSK_FLL_LANE_MIN");
-    return e ? atoi(e) : (1 << 30);
-  }();
-  const bool force_group = force_impl == 1 || force_impl == 2;   // (3 = lane, 4 = duo, 5 = pair)
+  constexpr int kPairMinStreams = 5120;
   // The two-warp kernel evaluates sin/cos and the phase wrap with short-range formulas (|phase| < 1e5): the loop
   // keeps |phase| <= 2*pi + max|freq|, so only a caller-set state or an absurd frequency limit (sps < 1e-3) can
-  // leave that range — those calls take the generic kernels, which use the library routines.
+  // leave that range — those calls take the generic kernel, which uses the library routines.
   const bool wild = state_wild || !(P.max_freq < 1e4f);
   state_wild = false;                                          // any kernel leaves the state wrapped and clamped
-  // the pair kernel's sin/cos is the |phase| < 64 form: a caller-set phase beyond that goes through the lane kernel once
+  // the pair kernel's sin/cos is the |phase| < 64 form: a caller-set phase beyond that goes through the two-warp kernel once
   const bool far = state_far;
   state_far = false;
-  if (!force_group && !wild && !far && fll_lane_supported(n_taps) && force_impl != 3 && force_impl != 4 &&
-      (force_impl == 5 || channels >= pair_min))
+  if (!wild && !far && fll_pair_supported(n_taps) && channels >= kPairMinStreams)
     return fll_pair_launch(P, lower, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy, s);
-  if (!force_group && !wild && fll_lane_supported(n_taps) && force_impl != 4 &&
-      (force_impl == 3 || channels >= lane_min || (far && channels >= pair_min)))
-    return fll_lane_launch(P, lower, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy, s);
-  if (!force_group && !wild && fll_duo_supported(n_taps))
+  if (!wild && fll_duo_supported(n_taps))
     return fll_duo_launch(P, d_taps.p, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy, s);
-  if (FllGroupFn fn = (wild || force_impl == 2) ? nullptr : fll_group_pick(n_taps)) {
-    // 8 lanes per stream, specialised on the tap count (the default 40-tap and the 10..55-tap filters)
-    const int blocks = (channels + kFllCtaStreams - 1) / kFllCtaStreams;
-    fn<<<blocks, kFllCtaThreads, 0, s>>>(P, d_taps.p, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy);
-    QPSK_LAUNCH_CHECK();
-    return QPSK_OK;
-  }
-  {
-    // 8 lanes per stream; ring, staging and partial sums in shared memory
-    const int Np = n_taps + (n_taps & 1);
-    const size_t smem = (size_t)(2 * Np + 4) * sizeof(float) + (size_t)kFllCtaStreams * kFllGroup * sizeof(float4) +
-                        (size_t)2 * kFllCtaStreams * kFllBlock * sizeof(float2) + (size_t)kFllCtaStreams * n_taps * sizeof(float2);
-    if (smem <= 200 * 1024 && force_impl != 2) {
-      const int blocks = (channels + kFllCtaStreams - 1) / kFllCtaStreams;
-      QPSK_TRY(allow_max_dynamic_smem((const void*)fll_group_kernel));
-      fll_group_kernel<<<blocks, kFllCtaThreads, smem, s>>>(P, d_taps.p, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy);
-      QPSK_LAUNCH_CHECK();
-      return QPSK_OK;
-    }
-  }
-  const int threads = kLoopThreads;
-  const int blocks = (channels + threads - 1) / threads;
-  const size_t smem = (size_t)(2 * n_taps + 2) * sizeof(float) + (size_t)n_taps * threads * sizeof(float2);
+  // 8 lanes per stream; ring, staging and partial sums in shared memory
+  const int Np = n_taps + (n_taps & 1);
+  const size_t smem = (size_t)(2 * Np + 4) * sizeof(float) + (size_t)kFllCtaStreams * kFllGroup * sizeof(float4) +
+                      (size_t)2 * kFllCtaStreams * kFllBlock * sizeof(float2) + (size_t)kFllCtaStreams * n_taps * sizeof(float2);
   if (smem > 200 * 1024) return QPSK_ERR_UNSUPPORTED;
-  QPSK_TRY(allow_max_dynamic_smem((const void*)fll_kernel));
-  fll_kernel<<<blocks, threads, smem, s>>>(P, d_taps.p, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy);
+  const int blocks = (channels + kFllCtaStreams - 1) / kFllCtaStreams;
+  QPSK_TRY(allow_max_dynamic_smem((const void*)fll_group_kernel));
+  fll_group_kernel<<<blocks, kFllCtaThreads, smem, s>>>(P, d_taps.p, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy);
   QPSK_LAUNCH_CHECK();
   return QPSK_OK;
 }

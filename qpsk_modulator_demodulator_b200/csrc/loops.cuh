@@ -2,7 +2,7 @@
 // sequential and in the reference's precisions.  This translation unit family is compiled with
 // --fmad=false: RyuJIT never fuses a*b+c, so every product and sum below rounds separately.
 //
-//   FllState/fll_step      FLLBandEdgeFilter.Process   MS/Models/Band-Edge Filter.cs:102-129,185-195
+//   FllParams/FllEngine    FLLBandEdgeFilter.Process   MS/Models/Band-Edge Filter.cs:102-129,185-195
 //   MmState/mm_*           MuellerMuller.Process       MS/Models/MuellerMuller.cs:52-136,160-198
 //   CostasState/costas_step CostasLoopQpsk.Process     MS/Models/CostasLoopQpsk.cs:63-92
 #pragma once
@@ -23,59 +23,7 @@ struct FllParams {
 // so one ring of past outputs and the four products a*xI, b*xQ, a*xQ, b*xI serve both; sums keep
 // ComplexDotWindow's order (8 lane partials over the chronological window, lanes 0..7, scalar
 // tail: FIRFilter.cs:165-192).  (-b)*x == -(b*x) and p - (-q) == p + q exactly, so sharing the
-// products is bit-neutral.
-//   ring:  float2 ring[n_taps] of this stream, element i at ring[i*ring_stride]
-//   tapI/tapQ: lower-filter taps reversed (rev[i] = lower[N-1-i]), shared memory
-__device__ __forceinline__ void fll_step(const FllParams& P, const float* __restrict__ tapI,
-                                         const float* __restrict__ tapQ, float2* ring, int ring_stride, int& head,
-                                         float& phase, float& freq, float inI, float inQ, float& outI, float& outQ) {
-  float s, c;
-  sincos_f32_exact(phase, &s, &c);                 // MathF.Cos/Sin(phase) :108-109
-  outI = inI * c - inQ * s;                        // :111
-  outQ = inI * s + inQ * c;                        // :112
-  const int N = P.n_taps;
-  // write the newest sample over the oldest, then the window starts at the next slot
-  ring[head * ring_stride] = make_float2(outI, outQ);
-  head = (head + 1 == N) ? 0 : head + 1;           // head = oldest element = window start
-  float loI[8], loQ[8], upI[8], upQ[8];
-#pragma unroll
-  for (int l = 0; l < 8; ++l) loI[l] = loQ[l] = upI[l] = upQ[l] = 0.f;
-  const int nVec = N - (N & 7);
-  int idx = head;
-  for (int i = 0; i < nVec; i += 8) {
-#pragma unroll
-    for (int l = 0; l < 8; ++l) {
-      const float2 x = ring[idx * ring_stride];
-      idx = (idx + 1 == N) ? 0 : idx + 1;
-      const float a = tapI[i + l], b = tapQ[i + l];
-      const float p1 = a * x.x, p2 = b * x.y, p3 = a * x.y, p4 = b * x.x;
-      loI[l] = loI[l] + (p1 - p2);
-      loQ[l] = loQ[l] + (p3 + p4);
-      upI[l] = upI[l] + (p1 + p2);
-      upQ[l] = upQ[l] + (p3 - p4);
-    }
-  }
-  float aLoI = 0.f, aLoQ = 0.f, aUpI = 0.f, aUpQ = 0.f;
-#pragma unroll
-  for (int l = 0; l < 8; ++l) {
-    aLoI += loI[l]; aLoQ += loQ[l]; aUpI += upI[l]; aUpQ += upQ[l];
-  }
-  for (int i = nVec; i < N; ++i) {
-    const float2 x = ring[idx * ring_stride];
-    idx = (idx + 1 == N) ? 0 : idx + 1;
-    const float a = tapI[i], b = tapQ[i];
-    const float p1 = a * x.x, p2 = b * x.y, p3 = a * x.y, p4 = b * x.x;
-    aLoI += (p1 - p2); aLoQ += (p3 + p4); aUpI += (p1 + p2); aUpQ += (p3 - p4);
-  }
-  const float powUpper = aUpI * aUpI + aUpQ * aUpQ;  // :118
-  const float powLower = aLoI * aLoI + aLoQ * aLoQ;  // :119
-  const float error = powLower - powUpper;           // :121
-  freq += P.beta * error;                            // :124
-  phase += freq + P.alpha * error;                   // :125
-  if (phase > kTwoPiF || phase < -kTwoPiF) phase = remainderf(phase, kTwoPiF);  // :185-189
-  if (freq > P.max_freq) freq = P.max_freq;          // :191-195
-  else if (freq < P.min_freq) freq = P.min_freq;
-}
+// products is bit-neutral.  Every FLL kernel takes the lower-filter taps reversed (rev[i] = lower[N-1-i]).
 
 // ---------------------------------------------------------------------------------------------
 // Mueller-Muller
@@ -307,16 +255,13 @@ struct FllEngine {
   int process_dev(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t ldy, cudaStream_t s);
 };
 
-// fll_duo.cu: two-warp (chain + side) FLL kernel for N = 8..48 taps, N % 8 == 0
+// fll_duo.cu: two-warp (chain + side) FLL kernel for N = 8..55 taps
 bool fll_duo_supported(int n_taps);
 int fll_duo_launch(const FllParams& P, const float* taps, float2* ring, int* head, float2* pf, int C, const float2* x,
                    float2* y, long long L, long long ldx, long long ldy, cudaStream_t s);
 
-// fll_lane.cu: one lane per stream, for large batches (40 and 10 taps)
-bool fll_lane_supported(int n_taps);
-int fll_lane_launch(const FllParams& P, const std::vector<float>& lower, float2* ring, int* head, float2* pf, int C,
-                    const float2* x, float2* y, long long L, long long ldx, long long ldy, cudaStream_t s);
-// ... and two lanes per stream (16 streams per warp): twice the warps, half the taps per lane
+// fll_pair.cu: two lanes per stream (16 streams per warp), for large batches (40 and 10 taps)
+bool fll_pair_supported(int n_taps);
 int fll_pair_launch(const FllParams& P, const std::vector<float>& lower, float2* ring, int* head, float2* pf, int C,
                     const float2* x, float2* y, long long L, long long ldx, long long ldy, cudaStream_t s);
 

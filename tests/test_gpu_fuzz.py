@@ -11,10 +11,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.mark.parametrize("tool,args,env", [("fuzz_path.py", ["16", "5"], {}), ("fuzz_fll.py", ["30", "5"], {}),
-                                           # the lane-per-stream FLL kernel (csrc/fll_lane.cu) forced at every stream count
-                                           ("fuzz_fll.py", ["40", "6"], {"QPSK_FLL_IMPL": "lane", "FUZZ_SIZES": "10,40"}),
-                                           # two lanes per stream (fll_pair_kernel), forced likewise
-                                           ("fuzz_fll.py", ["40", "7"], {"QPSK_FLL_IMPL": "pair", "FUZZ_SIZES": "10,40"})])
+                                           # two lanes per stream (csrc/fll_pair.cu): 10 or 40 taps from 5120 streams
+                                           ("fuzz_fll.py", ["40", "7"], {"FUZZ_SIZES": "10,40", "FUZZ_CHANNELS": "5120,5137"})])
 def test_fuzz_slice(gpu, tool, args, env):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "tools", tool)] + args, capture_output=True, text=True, timeout=600,
                        env=dict(os.environ, **env))

@@ -241,8 +241,8 @@ def test_costas_matches_oracle(gpu, orc, fs, bw):
 
 def test_fll_large_batch_kernel_choice_and_far_phase(gpu, orc):
     """From 5120 streams the two-lanes-per-stream kernel (fll_pair_kernel) serves the FLL.  Its sin/cos is the |phase| < 64
-    form, so a caller-set phase beyond 32 goes through the lane-per-stream kernel for one call (which leaves the phase
-    wrapped); both calls, and the loop state after them, must be the oracle's bit for bit."""
+    form, so a caller-set phase beyond 32 goes through the two-warp kernel (fll_duo_kernel) for one call (which leaves the
+    phase wrapped); both calls, and the loop state after them, must be the oracle's bit for bit."""
     C, L = 5200, 300
     rng = np.random.default_rng(21)
     x = (0.4 * rng.standard_normal((C, 2 * L))).astype(np.float32)
@@ -253,7 +253,7 @@ def test_fll_large_batch_kernel_choice_and_far_phase(gpu, orc):
     ph[probe] = np.array([50.0, -37.5, 0.3, 6.5, 1000.25, -63.0], np.float32)
     fr[probe] = np.array([0.1, -0.2, 0.0, 0.5, 0.01, -0.4], np.float32)
     g.state = (ph, fr)
-    outs = [g.Process(x), g.Process(x[:, ::-1].copy())]        # first call: lane kernel (far phase); second: pair kernel
+    outs = [g.Process(x), g.Process(x[:, ::-1].copy())]        # first call: duo kernel (far phase); second: pair kernel
     gp, gf = g.state
     for c in probe + [7, 4000]:
         o = orc.FLLBandEdgeFilter(2.0, 0.4, 40, 0.02)

@@ -23,4 +23,4 @@ for _ in range(reps):
 e1.record(ts); torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / reps
 print(json.dumps({"channels": C, "samples": L, "taps": N, "ms": ms, "cycles_per_sample_at_1965MHz": ms * 1e-3 * 1.965e9 / L,
-                  "msamples_s": C * L / ms / 1e3, "impl": os.environ.get("QPSK_FLL_IMPL", "duo")}))
+                  "msamples_s": C * L / ms / 1e3}))

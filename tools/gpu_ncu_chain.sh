@@ -6,6 +6,6 @@ WHICH=${2:-chain}
 OUT=gpurun_out
 mkdir -p $OUT
 python tools/chain_only.py $WHICH 2 > $OUT/${TAG}_plain_${WHICH}.log 2>&1 || { echo "plain run failed"; tail -5 $OUT/${TAG}_plain_${WHICH}.log; exit 1; }
-timeout 900 ncu --set full --clock-control none --import-source on -k regex:"symsync|fll_duo|fll_lane" -c 3 -f -o $OUT/${TAG}_prof_${WHICH} \
+timeout 900 ncu --set full --clock-control none --import-source on -k regex:"symsync|fll_duo|fll_pair" -c 3 -f -o $OUT/${TAG}_prof_${WHICH} \
   python tools/chain_only.py $WHICH 2 > $OUT/${TAG}_ncu_${WHICH}.log 2>&1
 echo "ncu rc=$?"; tail -3 $OUT/${TAG}_ncu_${WHICH}.log

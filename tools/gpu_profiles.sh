@@ -17,14 +17,14 @@ echo "fir rc=$?"
 python tools/decim_probe.py > $OUT/${TAG}_plain_decim.log 2>&1
 timeout 900 ncu --set full --clock-control none -k regex:fir_dec -c 6 -f -o $OUT/${TAG}_prof_decim python tools/decim_probe.py > $OUT/${TAG}_ncu_decim.log 2>&1
 echo "decim rc=$?"
-# 4. chain at 2048 channels, every stage one launch (no time-chunk pipeline): FLL (duo), fused MF + symbol stage, TSC strip, BER
-QPSK_DEMOD_CHUNKS=1 python tools/chain_only.py fll 2 > $OUT/${TAG}_plain_chain_fll.log 2>&1
-QPSK_DEMOD_CHUNKS=1 timeout 900 ncu --set full --clock-control none --import-source on -k regex:"fll_duo|symsync|tsc_strip|ber_kernel" -s 12 -c 4 -f \
+# 4. chain at 2048 channels: FLL (duo), fused MF + symbol stage, TSC strip, BER
+python tools/chain_only.py fll 2 > $OUT/${TAG}_plain_chain_fll.log 2>&1
+timeout 900 ncu --set full --clock-control none --import-source on -k regex:"fll_duo|symsync|tsc_strip|ber_kernel" -s 12 -c 4 -f \
   -o $OUT/${TAG}_prof_chain python tools/chain_only.py fll 2 > $OUT/${TAG}_ncu_chain.log 2>&1
 echo "chain rc=$?"
-# 5. the 16384-channel set on one GPU: fll_pair_kernel + the dense symbol-stage kernel
-QPSK_DEMOD_CHUNKS=1 SWEEP=16384 timeout 900 ncu --set full --clock-control none --import-source on -k regex:"fll_pair|symsync" -s 4 -c 2 -f \
-  -o $OUT/${TAG}_prof_chain16k python tools/fll_impl_sweep.py > $OUT/${TAG}_ncu_chain16k.log 2>&1
+# 5. the 16384-channel FLL on one GPU: fll_pair_kernel
+timeout 900 ncu --set full --clock-control none --import-source on -k regex:"fll_pair" -s 3 -c 1 -f \
+  -o $OUT/${TAG}_prof_chain16k python tools/fll_only.py 16384 > $OUT/${TAG}_ncu_chain16k.log 2>&1
 echo "chain16k rc=$?"
 # 6. modulator leg: mod_shape_kernel, one launch of 512 frames
 timeout 600 ncu --set full --clock-control none --import-source on -k regex:mod_shape -s 3 -c 1 -f -o $OUT/${TAG}_prof_mod python tools/mod_probe.py 512 2 > $OUT/${TAG}_ncu_mod.log 2>&1

@@ -4,8 +4,7 @@
   FIR      fir_tma_kernel (mbarrier ring, TMA bulk loads / per-warp bulk stores) over several tile seams, streaming in
            two chunks (delay-line ping-pong), real and complex taps, stateless alignment; fir_exact_real_kernel;
            fir_split2_kernel; fir_dec2_kernel / fir_decim_tma_kernel (D = 2, 4, 8, 16)
-  FLL      fll_duo_kernel (chain warp / side warp hand-off through shared memory + mbarriers), 40 and 10 taps,
-           fll_lane_kernel forced, generic group kernel (13 taps)
+  FLL      fll_duo_kernel (chain warp / side warp hand-off through shared memory + mbarriers), 40, 10 and 13 taps
   symsync  symsync_decode_kernel (cp.async double buffer, two-warp symbol queue), with TSC strip and framer
   chain    the time-chunk pipeline (two streams, events) with the FLL on
   mod      mod_tile_rot / mod_shape kernels; channel simulator; BER counters; pack / unpack; CS16
