@@ -217,6 +217,49 @@ QPSK_API int qpsk_eq_process_dev(qpsk_eq* eq, const float* d_in, float* d_out, i
 QPSK_API int qpsk_eq_get_taps(qpsk_eq* eq, float* taps_iq, int64_t cap_floats);
 QPSK_API int qpsk_eq_set_taps(qpsk_eq* eq, const float* taps_iq, int64_t n_floats);
 
+/* ---- polyphase analysis channelizer ------------------------------------------------------------------------ */
+/* Not in the reference (it receives one carrier per stream); the block that splits ONE wideband capture holding M carriers
+ * on a frequency grid into the [channels][samples] batch the demodulator takes: a critically sampled polyphase filter-bank
+ * (PFB) analysis channelizer, GNU Radio's pfb_channelizer_ccf without oversampling.
+ * Parameters: real prototype taps h[0..n_taps-1]; M channels, a power of two 2..1024; the taps are zero-padded at the end
+ * to L = P*M with P = ceil(n_taps/M) taps per branch, 1 <= P <= 32 (outside these limits: QPSK_ERR_UNSUPPORTED; n_taps <= 0:
+ * QPSK_ERR_ARG; a non-finite tap: QPSK_ERR_RANGE).
+ * Blocks: x[n] counts samples since creation or the last reset, x[n] = 0 for n < 0.  Output m exists once block m, samples
+ * mM .. mM+M-1, is complete.  With N = mM + M - 1:
+ *   y_k[m] = sum_{i=0}^{L-1} h[i] * e^{+j 2 pi k i / M} * x[N - i],   k = 0..M-1.
+ * Channel k is the band centred at +k/M cycles per input sample, rows in natural order (no fftshift: k >= M/2 are the
+ * negative frequencies k - M).  No 1/M factor: a prototype with sum h = 1 passes a carrier centred on channel k with unit
+ * gain, so the CMA `modulus 1.0` convention holds after the channelizer.  Against "mix down by k/M, filter with h, keep
+ * every M-th sample (n = N)", channel k carries the constant phase e^{-j 2 pi k / M}.
+ * Computation (the equivalent polyphase form): v_r[m] = sum_{q=0}^{P-1} h[qM + r] * x[(m - q)M + M - 1 - r], accumulated
+ * in increasing q, then y_k[m] = sum_r v_r[m] * w^{kr}, w = e^{j 2 pi / M}, by an in-place radix-2/radix-2^2 FFT.  fp32 with
+ * FMA; twiddles from an fp64 table rounded to fp32.  Against an fp64 evaluation of the definition max|err| <= 1e-5 max|y|.
+ * State: the last (P-1) complete blocks and the pending = (samples so far) mod M samples of the open block.  Any chunking of
+ * a stream (chunks shorter than M, empty calls, any pointer alignment that results) gives the same outputs bit for bit.
+ * A call of n samples gives floor((pending + n) / M) outputs per channel, known to the host without reading the device. */
+typedef struct qpsk_pfb qpsk_pfb;
+/* Kaiser-windowed sinc prototype, host fp64, unit DC gain; L = taps_per_branch*channels taps, cutoff in cycles per input
+ * sample (0 < cutoff < 0.5, else QPSK_ERR_RANGE), beta from atten_db (finite, >= 0) by Kaiser's formula.  Same as
+ * scipy.signal.firwin(L, 2*cutoff, window=("kaiser", kaiser_beta(atten_db)), scale=True).  channels / taps_per_branch
+ * outside the limits above: QPSK_ERR_UNSUPPORTED.  out==NULL or cap too small: *n still set (like qpsk_rrc_taps). */
+QPSK_API int qpsk_pfb_taps(int channels, int taps_per_branch, double cutoff, double atten_db, double* out, int cap, int* n);
+QPSK_API int qpsk_pfb_create(const float* taps, int n_taps, int channels, qpsk_pfb** out);
+QPSK_API int qpsk_pfb_destroy(qpsk_pfb* p);
+/* back to the state at creation: no history, no pending samples.  Waits for the handle's own stream only: qpsk_pfb_process_dev
+ * calls enqueued on another stream must have completed before the reset (synchronise that stream first). */
+QPSK_API int qpsk_pfb_reset(qpsk_pfb* p);
+/* host memory: iq_in n_floats (even, else QPSK_ERR_ARG) of ONE wideband stream -> iq_out [channels][out_stride_floats];
+ * *n_out_floats = floats written per channel (set on QPSK_ERR_CAPACITY too); out_stride_floats < *n_out_floats ->
+ * QPSK_ERR_CAPACITY, nothing consumed.  Floats of a row past *n_out_floats are not written. */
+QPSK_API int qpsk_pfb_process(qpsk_pfb* p, const float* iq_in, int64_t n_floats, float* iq_out,
+                              int64_t out_stride_floats, int64_t* n_out_floats);
+/* device memory (8-byte aligned), out_stride_floats even: the [channels][out_stride] rows qpsk_demod_bits_dev /
+ * qpsk_demod_bytes_dev read with in_stride = out_stride; pass both calls the same stream (NULL means each handle's own
+ * stream, and nothing then orders the demodulator's reads after these writes).  Enqueued on `stream`; the handle's state
+ * advances at enqueue, so calls on one handle must run in issue order. */
+QPSK_API int qpsk_pfb_process_dev(qpsk_pfb* p, const float* d_in, int64_t n_floats, float* d_out,
+                                  int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
+
 /* ---- a6  QPSKModulator  (MS/QPSKModulator.cs:18-168) ---------------------------------------- */
 /* tsc_bits: '0'/'1' string or NULL (null/whitespace = no TSC, :27) */
 QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha, int rrc_span,

@@ -61,6 +61,12 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_eq_process(IntPtr h, float* iqIn, float* iqOut, long nFloats, long outCap);
     [DllImport(Lib)] internal static extern int qpsk_eq_get_taps(IntPtr h, float* tapsIq, long capFloats);
     [DllImport(Lib)] internal static extern int qpsk_eq_set_taps(IntPtr h, float* tapsIq, long nFloats);
+    [DllImport(Lib)] internal static extern int qpsk_pfb_taps(int channels, int tapsPerBranch, double cutoff, double attenDb, double* taps, int cap, out int n);
+    [DllImport(Lib)] internal static extern int qpsk_pfb_create(float* taps, int nTaps, int channels, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_pfb_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_pfb_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_pfb_process(IntPtr h, float* iqIn, long nFloats, float* iqOut, long outStrideFloats, out long nOutFloats);
+    [DllImport(Lib)] internal static extern int qpsk_pfb_process_dev(IntPtr h, float* dIn, long nFloats, float* dOut, long outStrideFloats, out long nOutFloats, IntPtr stream);
     // a6  QPSKModulator                             (MS/QPSKModulator.cs:18,54,104)
     [DllImport(Lib, CharSet = CharSet.Ansi)]
     internal static extern int qpsk_mod_create(int fs, int rs, double alpha, int span, int diff, string? tsc, out IntPtr h);

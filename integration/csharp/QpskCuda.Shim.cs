@@ -288,6 +288,53 @@ namespace QPSK.Models
         }
         public void Dispose() => _o.Dispose();
     }
+
+    // Polyphase analysis channelizer (not in the reference): one wideband stream -> Channels streams at 1/Channels of the
+    // rate, channel k centred at +k/Channels cycles per input sample; rows [Channels][outStride] are what the batch
+    // QPSKDeModulator reads.  State persists across calls.
+    public sealed unsafe class PfbChannelizer : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Channels;
+        public PfbChannelizer(float[] taps, int channels)
+        {
+            if (taps == null) throw new ArgumentNullException(nameof(taps));
+            if (taps.Length == 0) throw new ArgumentException("Prototype taps must not be empty.", nameof(taps));
+            if (channels < 2 || channels > 1024 || (channels & (channels - 1)) != 0)
+                throw new ArgumentOutOfRangeException(nameof(channels), "channels must be a power of two from 2 to 1024.");
+            IntPtr h;
+            fixed (float* t = taps) QpskCuda.Check(QpskCuda.qpsk_pfb_create(t, taps.Length, channels, out h), nameof(taps));
+            _o = new QpskHandle(h, QpskCuda.qpsk_pfb_destroy);
+            Channels = channels;
+        }
+        // Kaiser-windowed sinc prototype, unit DC gain, channels * tapsPerBranch taps; cutoff in cycles per input sample
+        public static double[] DesignTaps(int channels, int tapsPerBranch, double cutoff, double attenDb = 60.0)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_pfb_taps(channels, tapsPerBranch, cutoff, attenDb, null, 0, out int n));
+            var t = new double[n];
+            fixed (double* p = t) QpskCuda.Check(QpskCuda.qpsk_pfb_taps(channels, tapsPerBranch, cutoff, attenDb, p, n, out n));
+            return t;
+        }
+        // iqIn: interleaved IQ of the wideband stream; iqOut: [Channels][outStrideFloats].  Returns floats written per channel.
+        public long Process(ReadOnlySpan<float> iqIn, Span<float> iqOut, long outStrideFloats)
+        {
+            if ((iqIn.Length & 1) != 0) throw new ArgumentException("Input must be interleaved IQ with even length.", nameof(iqIn));
+            if (outStrideFloats < 0 || iqOut.Length < Channels * outStrideFloats)
+                throw new ArgumentException("Output span is too small for Channels rows of outStrideFloats.", nameof(iqOut));
+            long n;
+            fixed (float* i = iqIn) fixed (float* o = iqOut)
+                QpskCuda.Check(QpskCuda.qpsk_pfb_process(_h, i, iqIn.Length, o, outStrideFloats, out n), nameof(iqOut));
+            GC.KeepAlive(this);
+            return n;
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_pfb_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
 }
 
 namespace QPSK

@@ -118,6 +118,12 @@ def _signatures():
         "qpsk_eq_process_dev": (i, [vp, vp, vp, i64, i64, i64, vp, vp]),
         "qpsk_eq_get_taps": (i, [vp, f32p, i64]),
         "qpsk_eq_set_taps": (i, [vp, f32p, i64]),
+        "qpsk_pfb_taps": (i, [i, i, d, d, f64p, i, i32p]),
+        "qpsk_pfb_create": (i, [f32p, i, i, vpp]),
+        "qpsk_pfb_destroy": (i, [vp]),
+        "qpsk_pfb_reset": (i, [vp]),
+        "qpsk_pfb_process": (i, [vp, vp, i64, vp, i64, i64p]),
+        "qpsk_pfb_process_dev": (i, [vp, vp, i64, vp, i64, i64p, vp]),
         "qpsk_mod_create": (i, [i, i, d, i, i, cp, vpp]),
         "qpsk_mod_destroy": (i, [vp]),
         "qpsk_mod_taps": (i, [vp, f64p, i, i32p]),

@@ -422,3 +422,55 @@ class CmaEqualizer(_Handle):
 
     def reset(self):
         check(lib().qpsk_eq_reset(self._h))
+
+
+# ---- polyphase analysis channelizer (not in the reference) -------------------------------------
+def pfb_taps(channels: int, taps_per_branch: int, cutoff: float, atten_db: float = 60.0) -> np.ndarray:
+    """Kaiser-windowed sinc prototype for PfbChannelizer (fp64, unit DC gain, channels*taps_per_branch taps); cutoff in
+    cycles per input sample, e.g. 0.5/channels for adjacent channels meeting at their -6 dB points."""
+    n = C.c_int(0)
+    check(lib().qpsk_pfb_taps(channels, taps_per_branch, cutoff, atten_db, None, 0, C.byref(n)))
+    out = np.empty(n.value, np.float64)
+    check(lib().qpsk_pfb_taps(channels, taps_per_branch, cutoff, atten_db, out.ctypes.data_as(N.f64p), n.value, C.byref(n)))
+    return out
+
+
+class PfbChannelizer(_Handle):
+    """Critically sampled polyphase analysis channelizer on the GPU (csrc/pfb.cu; definition in include/qpskcuda.h): one
+    wideband stream in, `channels` (a power of two, 2..1024) channel streams out at 1/channels of the rate, channel k
+    centred at +k/channels cycles per input sample.  `taps`: the real prototype (e.g. pfb_taps(...)), at most
+    32*channels taps.  State persists across calls: any chunking of the stream gives the same outputs."""
+    _destroy = "qpsk_pfb_destroy"
+
+    def __init__(self, taps, channels: int):
+        super().__init__()
+        if taps is None:
+            raise ArgumentNullException("taps")
+        t = _f32(taps)
+        self.channels = channels
+        check(lib().qpsk_pfb_create(t.ctypes.data_as(N.f32p), t.size, channels, C.byref(self._h)))
+
+    def process(self, x, out_stride: int = 0) -> np.ndarray:
+        """x: complex64 samples (or interleaved float32 IQ) of the wideband stream -> complex64 [channels, n_out], the
+        outputs this call completes.  `out_stride` (floats) sizes the output rows like the C call; 0 = just enough."""
+        a = np.asarray(x)
+        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        n = C.c_int64(0)
+        if not out_stride:
+            st = lib().qpsk_pfb_process(self._h, None, a.size, None, -1, C.byref(n))
+            if st != N.ERR_CAPACITY:
+                check(st)
+            out_stride = n.value
+        y = np.zeros((self.channels, max(out_stride, 0)), np.float32)
+        check(lib().qpsk_pfb_process(self._h, _ptr(a), a.size, _ptr(y), out_stride, C.byref(n)))
+        return np.ascontiguousarray(y[:, : n.value]).view(np.complex64)
+
+    def process_dev(self, d_in: int, n_floats: int, d_out: int, out_stride: int, stream: int = 0) -> int:
+        """Device pointers: n_floats of the wideband stream -> d_out [channels][out_stride] floats.  Returns the floats
+        written per channel (the n_floats to pass to QPSKDeModulator.demod_bytes_dev with in_stride = out_stride)."""
+        n = C.c_int64(0)
+        check(lib().qpsk_pfb_process_dev(self._h, d_in, n_floats, d_out, out_stride, C.byref(n), stream))
+        return n.value
+
+    def reset(self):
+        check(lib().qpsk_pfb_reset(self._h))
