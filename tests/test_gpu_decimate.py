@@ -163,3 +163,38 @@ def test_decimate_by_2_kernels_agree_across_an_odd_cut(gpu, orc, aligned):
     got = np.concatenate([dy.cpu().numpy()[:n1], dz.cpu().numpy()[:n2]])          # the counts are in floats
     assert n1 + n2 == want.size
     assert _close(got, want)
+
+
+@pytest.mark.parametrize("layout", ["offset_pointer", "odd_stride_batch"])
+@pytest.mark.parametrize("span,sps,dec", [(16, 4, 4), (16, 4, 8), (16, 4, 16), (16, 8, 4), (16, 8, 8), (16, 8, 16)])
+def test_register_staged_decimators_match_the_subsampled_oracle(gpu, orc, span, sps, dec, layout):
+    """D = 4, 8, 16 leave the bulk-copy pipeline for the register-staged fir_decim_kernel when the rows rule out bulk
+    copies: an input pointer one sample into the buffer, or a 3-channel batch whose rows are an odd number of samples
+    apart.  65 and 129 taps, over more than two tiles of every D with a ragged end."""
+    import torch
+    taps = _taps(gpu, span, sps)
+    L = 40010                                                   # 11+ tiles at every D; L + 3 is odd
+    C = 1 if layout == "offset_pointer" else 3
+    x = orc.fill_uniform(11 + dec, sps, 0, 2 * L * C).reshape(C, 2 * L)
+    if layout == "offset_pointer":
+        ld = 2 * L
+        buf = torch.zeros(2 + ld + 2, dtype=torch.float32, device="cuda")
+        buf[2:2 + ld] = torch.from_numpy(x[0]).cuda()
+        p = buf.data_ptr() + 8
+    else:
+        ld = 2 * (L + 3)                                        # floats: an odd number of samples per row
+        buf = torch.zeros(C * ld, dtype=torch.float32, device="cuda")
+        buf.view(C, ld)[:, : 2 * L] = torch.from_numpy(x).cuda()
+        p = buf.data_ptr()
+    n_out = (L + dec - 1) // dec
+    ldo = 2 * n_out + 6
+    y = torch.zeros(C * ldo, dtype=torch.float32, device="cuda")
+    f = gpu.ComplexFIRFilter(taps, channels=C)
+    torch.cuda.synchronize()
+    n = f.decimate_dev(p, 2 * L, dec, y.data_ptr(), 2 * n_out, in_stride=ld, out_stride=ldo)
+    torch.cuda.synchronize()
+    assert f.last_kernel().startswith("fir_decim_kernel<"), f.last_kernel()
+    assert n == 2 * n_out
+    yh = y.view(C, ldo).cpu().numpy()
+    for c in range(C):
+        assert _close(yh[c, :n], _sub(orc.ComplexFIRFilter(taps).Filter(x[c]), dec)), c

@@ -774,6 +774,65 @@ def test_demod_tsc_strip_lengths(gpu, orc, tlen):
         assert gpu.QPSKDeModulator(fs, rs, **kw2).DeModulate(x) == orc.QPSKDeModulator(fs, rs, **kw2).DeModulate(x)
 
 
+def _tsc_smem_bytes(L, T, sps):
+    """Shared memory DemodEngine::bits_dev asks for tsc_strip_smem_kernel on an L-sample call (rows of 2 x the symbol
+    bound, padded to 16 bytes); above 160 KB the call takes tsc_strip_kernel."""
+    sl = L if sps - 0.1 <= 1.0 else min(int((L + 4) / (sps - 0.1)) + 2, L)
+    ld_raw = (2 * max(sl, 1) + 15) & ~15
+    row_bytes = (ld_raw + 15) & ~15
+    words = (row_bytes + 31) // 32 + 4
+    return 4 * (row_bytes + ((T + 15) & ~15)) + 16 * words
+
+
+@pytest.mark.parametrize("C", [1, 33])
+@pytest.mark.parametrize("tlen", [64, 100])
+def test_demod_tsc_strip_long_calls(gpu, orc, tlen, C):
+    """Calls too long for tsc_strip_smem_kernel's shared memory take tsc_strip_kernel: three calls per channel, the first
+    with the TSC in its middle, the second without it and ending half-way through the next TSC, which the third call
+    starts in.  Bits must equal the oracle's on every call."""
+    import re
+    import symsync_dispatch as sd
+    fs, rs, span = 2000, 1000, 10
+    sps = fs / rs
+    tsc = "".join(np.random.default_rng(200 + tlen).choice(["0", "1"], tlen))
+    Lmin = next(L for L in range(20000, 60000, 16) if _tsc_smem_bytes(L, tlen, sps) > 160 * 1024)
+    n_bits = 2 * ((Lmin + 1200) // 2)                            # ~ one sample per bit at sps 2
+    # the TSC goes inside a frame's bit string: at the start of a frame the differential reference of the modulator
+    # restarts while the demodulator's carries on, and the first dibit would not decode as sent
+    mod = orc.QPSKModulator(fs, rs, 0.35, span, True, None)
+    lead = 1000                                                  # bits of t before its TSC
+    rows, cuts = [], None
+    for c in range(C):
+        a = mod.Modulate(_bits(n_bits // 2, 3 * c) + tsc + _bits(n_bits // 2, 3 * c + 1))
+        b = mod.Modulate(_bits(n_bits, 3 * c + 2))
+        t = mod.Modulate(_bits(lead, 3 * c + 3) + tsc + _bits(n_bits, 3 * c + 4))
+        rng = np.random.default_rng(c)
+        z = np.concatenate([a, b, t])
+        rows.append((z + 0.01 * rng.standard_normal(z.size)).astype(np.float32))
+        mid = lead + span * int(sps) // 2 + tlen // 2            # about the middle of t's TSC, in samples
+        cuts = [0, a.size // 2, a.size // 2 + b.size // 2 + mid, z.size // 2]
+    x = np.stack(rows)
+    assert min(q - p for p, q in zip(cuts[:-1], cuts[1:])) >= Lmin
+    kw = dict(RrcAlpha=0.35, rrcSpan=span, SymbolSyncBandwith=0.002, tsc=tsc)
+    gd = gpu.QPSKDeModulator(fs, rs, channels=C, **kw)
+    ods = [orc.QPSKDeModulator(fs, rs, **kw) for _ in range(C)]
+    for k, (p, q) in enumerate(zip(cuts[:-1], cuts[1:])):
+        xs = np.ascontiguousarray(x[:, 2 * p:2 * q])
+        arg = xs if C > 1 else xs[0]
+        if k == 0:
+            got, names = sd.launched_kernels(lambda: gd.DeModulate(arg))
+            print(f"[kernel] tsc long call T={tlen} C={C}: {sorted(set(n.split('(')[0] for n in names if 'tsc_strip' in n))}")
+            assert any(re.search(r"\btsc_strip_kernel\b", n) for n in names), names
+            assert not any("tsc_strip_smem_kernel" in n for n in names), names
+        else:
+            got = gd.DeModulate(arg)
+        got = got if C > 1 else [got]
+        for c in range(C):
+            want = ods[c].DeModulate(xs[c])
+            assert got[c] == want, (k, c)
+            assert (want != "") == (k == 0), (k, c, len(want))    # found in the first call only: absent, then cut in two
+
+
 @pytest.mark.parametrize("diff,tsc,nbits", [(True, TSC, 600), (False, None, 4096), (True, None, 13), (True, TSC, 0), (False, TSC, 7)])
 def test_modulate_packed_equals_bit_string(gpu, orc, diff, tsc, nbits):
     rng = np.random.default_rng(nbits + 1)
