@@ -260,6 +260,48 @@ QPSK_API int qpsk_pfb_process(qpsk_pfb* p, const float* iq_in, int64_t n_floats,
 QPSK_API int qpsk_pfb_process_dev(qpsk_pfb* p, const float* d_in, int64_t n_floats, float* d_out,
                                   int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
 
+/* ---- digital down-converter bank ---------------------------------------------------------------------------- */
+/* Not in the reference; the front end for carriers at arbitrary frequencies in ONE wideband capture: K digital
+ * down-converters (mix by -f_k, lowpass with a shared real prototype, keep every D-th sample) sharing one pass over the
+ * input, GNU Radio's freq_xlating_fir_filter_ccf once per carrier.  Unlike the PFB channelizer the carriers need no grid,
+ * any subset of frequencies is computed, and the output rate is 1/D whatever K is.
+ * Parameters: real taps h[0..n_taps-1], 1 <= n_taps <= 4096; K channels, 1 <= K <= 2048; decimation D, 1 <= D <= 1024;
+ * frequencies f_k in cycles per input sample, each finite and in [-0.5, 0.5) (outside the limits on K, D and n_taps:
+ * QPSK_ERR_UNSUPPORTED; n_taps <= 0: QPSK_ERR_ARG; a non-finite tap or a bad frequency: QPSK_ERR_RANGE).
+ * Phase words: inc_k = nearbyint(ldexp(f_k, 64)) mod 2^64 (uint64); the phase of stream sample n is phi_k(n) = inc_k * n
+ * mod 2^64, exact unsigned 64-bit arithmetic, n counting samples since creation or the last reset.  No phase is
+ * accumulated in floating point, so it is chunk-invariant and identical on the host, the device and in a reference.
+ * Output: x[n] = 0 for n < 0.  Output m exists once samples up to n_m = mD + D - 1 have arrived; with N = n_taps
+ *   y_k[m] = sum_{i=0}^{N-1} h[i] * x[n_m - i] * e^{-j 2 pi phi_k(n_m - i) / 2^64}
+ * ("mix down by f_k, filter with h, keep every D-th sample").  No 1/D factor: a prototype with sum h = 1 passes a tuned
+ * carrier with unit gain and no rotation, so the CMA `modulus 1.0` convention holds after the bank.
+ * Computation (exact in the phase words, phi(n - i) = phi(n) - phi(i) mod 2^64): u_k[m] = sum_i g_k[i] x[n_m - i] with
+ * rotated taps g_k[i] = h[i] e^{+j 2 pi phi_k(i) / 2^64} formed on the host in fp64 and rounded to fp32, then
+ * y_k[m] = u_k[m] e^{-j 2 pi phi_k(n_m) / 2^64}.  fp32 with FMA; against an fp64 evaluation of the definition
+ * max|err| <= 1e-5 max|y| over a call's output.
+ * Relation to the PFB channelizer: with D = M and f_k = k/M (k >= M/2 taken as k - M), row k of the bank equals row k of
+ * qpsk_pfb with the same prototype times e^{+j 2 pi k / M}.  For a full grid the PFB is the cheaper block.
+ * State: the last N-1 input samples, the pending = (samples so far) mod D samples of the open block and the 64-bit sample
+ * counter.  Any chunking of a stream (chunks shorter than D, empty calls, any pointer alignment that results) gives the
+ * same outputs bit for bit.  A call of n samples gives floor((pending + n) / D) outputs per channel, known to the host. */
+typedef struct qpsk_ddc qpsk_ddc;
+QPSK_API int qpsk_ddc_create(const float* taps, int n_taps, const double* freqs, int channels, int decim, qpsk_ddc** out);
+QPSK_API int qpsk_ddc_destroy(qpsk_ddc* p);
+/* back to the state at creation: no history, no pending samples, counter 0.  Waits for the handle's own stream only:
+ * qpsk_ddc_process_dev calls enqueued on another stream must have completed before the reset. */
+QPSK_API int qpsk_ddc_reset(qpsk_ddc* p);
+/* host memory: iq_in n_floats (even, else QPSK_ERR_ARG) of ONE wideband stream -> iq_out [channels][out_stride_floats];
+ * *n_out_floats = floats written per channel (set on QPSK_ERR_CAPACITY too); out_stride_floats < *n_out_floats ->
+ * QPSK_ERR_CAPACITY, nothing consumed.  Floats of a row past *n_out_floats are not written. */
+QPSK_API int qpsk_ddc_process(qpsk_ddc* p, const float* iq_in, int64_t n_floats, float* iq_out,
+                              int64_t out_stride_floats, int64_t* n_out_floats);
+/* device memory (8-byte aligned), out_stride_floats even: the [channels][out_stride] rows qpsk_demod_bits_dev /
+ * qpsk_demod_bytes_dev read with in_stride = out_stride; pass both calls the same stream (NULL means each handle's own
+ * stream, and nothing then orders the demodulator's reads after these writes).  Enqueued on `stream`; the handle's state
+ * advances at enqueue, so calls on one handle must run in issue order. */
+QPSK_API int qpsk_ddc_process_dev(qpsk_ddc* p, const float* d_in, int64_t n_floats, float* d_out,
+                                  int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
+
 /* ---- a6  QPSKModulator  (MS/QPSKModulator.cs:18-168) ---------------------------------------- */
 /* tsc_bits: '0'/'1' string or NULL (null/whitespace = no TSC, :27) */
 QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha, int rrc_span,

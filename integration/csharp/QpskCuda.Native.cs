@@ -67,6 +67,11 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_pfb_reset(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_pfb_process(IntPtr h, float* iqIn, long nFloats, float* iqOut, long outStrideFloats, out long nOutFloats);
     [DllImport(Lib)] internal static extern int qpsk_pfb_process_dev(IntPtr h, float* dIn, long nFloats, float* dOut, long outStrideFloats, out long nOutFloats, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_ddc_create(float* taps, int nTaps, double* freqs, int channels, int decim, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_ddc_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_ddc_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_ddc_process(IntPtr h, float* iqIn, long nFloats, float* iqOut, long outStrideFloats, out long nOutFloats);
+    [DllImport(Lib)] internal static extern int qpsk_ddc_process_dev(IntPtr h, float* dIn, long nFloats, float* dOut, long outStrideFloats, out long nOutFloats, IntPtr stream);
     // a6  QPSKModulator                             (MS/QPSKModulator.cs:18,54,104)
     [DllImport(Lib, CharSet = CharSet.Ansi)]
     internal static extern int qpsk_mod_create(int fs, int rs, double alpha, int span, int diff, string? tsc, out IntPtr h);

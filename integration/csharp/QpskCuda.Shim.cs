@@ -335,6 +335,54 @@ namespace QPSK.Models
         }
         public void Dispose() => _o.Dispose();
     }
+
+    // Digital down-converter bank (not in the reference): one wideband stream -> one channel per frequency (cycles per
+    // input sample, in [-0.5, 0.5)), each mixed down, lowpass-filtered with the shared real prototype and decimated by
+    // Decim; rows [Channels][outStride] are what the batch QPSKDeModulator reads.  State persists across calls.
+    public sealed unsafe class DdcBank : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Channels;
+        public readonly int Decim;
+        public DdcBank(float[] taps, double[] freqs, int decim)
+        {
+            if (taps == null) throw new ArgumentNullException(nameof(taps));
+            if (freqs == null) throw new ArgumentNullException(nameof(freqs));
+            if (taps.Length == 0) throw new ArgumentException("Prototype taps must not be empty.", nameof(taps));
+            if (taps.Length > 4096) throw new ArgumentOutOfRangeException(nameof(taps), "At most 4096 prototype taps.");
+            if (freqs.Length < 1 || freqs.Length > 2048)
+                throw new ArgumentOutOfRangeException(nameof(freqs), "From 1 to 2048 channel frequencies.");
+            if (decim < 1 || decim > 1024) throw new ArgumentOutOfRangeException(nameof(decim), "decim must be from 1 to 1024.");
+            foreach (var f in freqs)
+                if (!(f >= -0.5 && f < 0.5))
+                    throw new ArgumentOutOfRangeException(nameof(freqs), "Frequencies are cycles per input sample in [-0.5, 0.5).");
+            IntPtr h;
+            fixed (float* t = taps) fixed (double* f = freqs)
+                QpskCuda.Check(QpskCuda.qpsk_ddc_create(t, taps.Length, f, freqs.Length, decim, out h), nameof(taps));
+            _o = new QpskHandle(h, QpskCuda.qpsk_ddc_destroy);
+            Channels = freqs.Length;
+            Decim = decim;
+        }
+        // iqIn: interleaved IQ of the wideband stream; iqOut: [Channels][outStrideFloats].  Returns floats written per channel.
+        public long Process(ReadOnlySpan<float> iqIn, Span<float> iqOut, long outStrideFloats)
+        {
+            if ((iqIn.Length & 1) != 0) throw new ArgumentException("Input must be interleaved IQ with even length.", nameof(iqIn));
+            if (outStrideFloats < 0 || iqOut.Length < Channels * outStrideFloats)
+                throw new ArgumentException("Output span is too small for Channels rows of outStrideFloats.", nameof(iqOut));
+            long n;
+            fixed (float* i = iqIn) fixed (float* o = iqOut)
+                QpskCuda.Check(QpskCuda.qpsk_ddc_process(_h, i, iqIn.Length, o, outStrideFloats, out n), nameof(iqOut));
+            GC.KeepAlive(this);
+            return n;
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_ddc_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
 }
 
 namespace QPSK

@@ -124,6 +124,11 @@ def _signatures():
         "qpsk_pfb_reset": (i, [vp]),
         "qpsk_pfb_process": (i, [vp, vp, i64, vp, i64, i64p]),
         "qpsk_pfb_process_dev": (i, [vp, vp, i64, vp, i64, i64p, vp]),
+        "qpsk_ddc_create": (i, [f32p, i, f64p, i, i, vpp]),
+        "qpsk_ddc_destroy": (i, [vp]),
+        "qpsk_ddc_reset": (i, [vp]),
+        "qpsk_ddc_process": (i, [vp, vp, i64, vp, i64, i64p]),
+        "qpsk_ddc_process_dev": (i, [vp, vp, i64, vp, i64, i64p, vp]),
         "qpsk_mod_create": (i, [i, i, d, i, i, cp, vpp]),
         "qpsk_mod_destroy": (i, [vp]),
         "qpsk_mod_taps": (i, [vp, f64p, i, i32p]),

@@ -474,3 +474,51 @@ class PfbChannelizer(_Handle):
 
     def reset(self):
         check(lib().qpsk_pfb_reset(self._h))
+
+
+# ---- digital down-converter bank (not in the reference) ----------------------------------------
+class DdcBank(_Handle):
+    """Frequency-translating decimating filter bank on the GPU (csrc/ddc.cu; definition in include/qpskcuda.h): one
+    wideband stream in, one channel per entry of `freqs` (cycles per input sample, each in [-0.5, 0.5), 1..2048 of them)
+    out at 1/`decim` of the rate, channel k mixed down by freqs[k], filtered with the real prototype `taps` (1..4096 taps,
+    e.g. scipy.signal.firwin) and decimated.  State persists across calls: any chunking of the stream gives the same
+    outputs."""
+    _destroy = "qpsk_ddc_destroy"
+
+    def __init__(self, taps, freqs, decim: int):
+        super().__init__()
+        if taps is None:
+            raise ArgumentNullException("taps")
+        if freqs is None:
+            raise ArgumentNullException("freqs")
+        t = _f32(taps)
+        f = np.ascontiguousarray(freqs, dtype=np.float64).ravel()
+        self.channels = f.size
+        self.decim = decim
+        check(lib().qpsk_ddc_create(t.ctypes.data_as(N.f32p), t.size, f.ctypes.data_as(N.f64p), f.size, decim,
+                                    C.byref(self._h)))
+
+    def process(self, x, out_stride: int = 0) -> np.ndarray:
+        """x: complex64 samples (or interleaved float32 IQ) of the wideband stream -> complex64 [channels, n_out], the
+        outputs this call completes.  `out_stride` (floats) sizes the output rows like the C call; 0 = just enough."""
+        a = np.asarray(x)
+        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        n = C.c_int64(0)
+        if not out_stride:
+            st = lib().qpsk_ddc_process(self._h, None, a.size, None, -1, C.byref(n))
+            if st != N.ERR_CAPACITY:
+                check(st)
+            out_stride = n.value
+        y = np.zeros((self.channels, max(out_stride, 0)), np.float32)
+        check(lib().qpsk_ddc_process(self._h, _ptr(a), a.size, _ptr(y), out_stride, C.byref(n)))
+        return np.ascontiguousarray(y[:, : n.value]).view(np.complex64)
+
+    def process_dev(self, d_in: int, n_floats: int, d_out: int, out_stride: int, stream: int = 0) -> int:
+        """Device pointers: n_floats of the wideband stream -> d_out [channels][out_stride] floats.  Returns the floats
+        written per channel (the n_floats to pass to QPSKDeModulator.demod_bytes_dev with in_stride = out_stride)."""
+        n = C.c_int64(0)
+        check(lib().qpsk_ddc_process_dev(self._h, d_in, n_floats, d_out, out_stride, C.byref(n), stream))
+        return n.value
+
+    def reset(self):
+        check(lib().qpsk_ddc_reset(self._h))
