@@ -302,6 +302,42 @@ QPSK_API int qpsk_ddc_process(qpsk_ddc* p, const float* iq_in, int64_t n_floats,
 QPSK_API int qpsk_ddc_process_dev(qpsk_ddc* p, const float* d_in, int64_t n_floats, float* d_out,
                                   int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
 
+/* ---- feed-forward AGC ----------------------------------------------------------------------------------------- */
+/* Not in the reference (its chain assumes unit amplitude); the level normaliser for a batch of channels that arrive at
+ * different levels, e.g. the carriers of one capture after qpsk_pfb / qpsk_ddc.  GNU Radio's feedforward_agc_cc made
+ * causal: one gain per sample from the peak envelope of a W-sample window that looks ahead of the sample it scales.
+ * Parameters: window W, 1..4096 (else QPSK_ERR_UNSUPPORTED); ref and max_gain finite and > 0 (else QPSK_ERR_RANGE);
+ * channels >= 1 (else QPSK_ERR_RANGE).
+ * Definition, per channel, x[n] counting samples since creation or the last reset, x[n] = 0 for n < 0:
+ *   env(v) = fmaxf(fabsf(v.re), fabsf(v.im))                                  (exact)
+ *   m[n]   = fmaxf over {0, env(x[n - i]) : i = 0..W-1}                         (exact; a NaN envelope is ignored)
+ *   g[n]   = fminf(ref / m[n], max_gain)                                       (one rounding; m = 0 gives max_gain)
+ *   y[n]   = (x[n-W+1].re * g[n], x[n-W+1].im * g[n])                          (one rounding each)
+ * so the window of output n runs from the sample it scales, x[n-W+1], W-1 samples ahead to x[n]: the output stream is the
+ * input delayed by W-1 samples (its first W-1 outputs scale the zero history).  fp32, no FMA anywhere, so the GPU equals
+ * any CPU restatement bit for bit (a NaN output is NaN; its sign and payload are not specified).  Scaling the input by 2^k changes no output bit unless max_gain binds or a value
+ * leaves the normal range.  State: the last W-1 samples and the last gain of each channel.  Any chunking of a stream
+ * (empty calls, chunks shorter than W) gives the same outputs bit for bit.  One output per input sample. */
+typedef struct qpsk_agc qpsk_agc;
+QPSK_API int qpsk_agc_create_batch(int window, float ref, float max_gain, int channels, qpsk_agc** out);
+QPSK_API int qpsk_agc_destroy(qpsk_agc* p);
+/* back to the state at creation: zero history, every last gain max_gain.  Waits for the handle's own stream only:
+ * qpsk_agc_process_dev calls enqueued on another stream must have completed before the reset. */
+QPSK_API int qpsk_agc_reset(qpsk_agc* p);
+/* host memory, iq_in / iq_out [channels][n_floats]; odd n_floats -> QPSK_ERR_ARG, out_cap_floats < n_floats ->
+ * QPSK_ERR_CAPACITY.  A refused call consumes nothing. */
+QPSK_API int qpsk_agc_process(qpsk_agc* p, const float* iq_in, float* iq_out, int64_t n_floats, int64_t out_cap_floats);
+/* device memory (8-byte aligned, else QPSK_ERR_ARG), strides in floats (even; in_stride_floats >= n_floats, else
+ * QPSK_ERR_ARG; out_stride_floats < n_floats -> QPSK_ERR_CAPACITY); d_out must not overlap d_in.  Enqueued on `stream`
+ * (NULL = the handle's own); the state advances at enqueue, so calls on one handle must run in issue order.  Floats of a
+ * row past n_floats are not written. */
+QPSK_API int qpsk_agc_process_dev(qpsk_agc* p, const float* d_in, float* d_out, int64_t n_floats, int64_t in_stride_floats,
+                                  int64_t out_stride_floats, void* stream);
+/* gain of each channel's last output, gain[channels] (cap < channels -> QPSK_ERR_CAPACITY); synchronises the handle's own
+ * stream.  The _dev form copies them to d_gain[channels] on `stream` (NULL = the handle's own) in stream order. */
+QPSK_API int qpsk_agc_gain(qpsk_agc* p, float* gain, int64_t cap);
+QPSK_API int qpsk_agc_gain_dev(qpsk_agc* p, float* d_gain, void* stream);
+
 /* ---- a6  QPSKModulator  (MS/QPSKModulator.cs:18-168) ---------------------------------------- */
 /* tsc_bits: '0'/'1' string or NULL (null/whitespace = no TSC, :27) */
 QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha, int rrc_span,
@@ -370,6 +406,14 @@ QPSK_API int qpsk_demod_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t ca
 QPSK_API int qpsk_demod_set_fractional_equalizer(qpsk_demod* d, int n_taps, float mu, float modulus);
 /* the fractional stage's taps, [channels][2*n_taps]; QPSK_ERR_ARG when the stage is off */
 QPSK_API int qpsk_demod_fractional_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats);
+/* Opt-in feed-forward AGC stage (qpsk_agc_* above) ahead of everything else: AGC -> FLL? -> MF -> ..., so carriers at any
+ * level reach the loops at the level `ref` sets; window 0 = off (the default: the chain is then exactly the reference's).
+ * The first W-1 AGC outputs of each channel's stream are discarded once, so the k-th sample reaching the FLL / matched
+ * filter is the k-th input sample, scaled (bit alignment as without the stage); the last W-1 samples of a call come out
+ * at the start of the next.  The fused symbol-stage kernel and the time-chunk pipeline stay in use with the stage on.
+ * May be called at any time: synchronises the handle, resets this stage only (history, discard count).  Limits and
+ * argument codes as qpsk_agc_create_batch. */
+QPSK_API int qpsk_demod_set_agc(qpsk_demod* d, int window, float ref, float max_gain);
 /* DeModulate(ReadOnlySpan<float>) :345-425 -> '0'/'1' chars (not NUL-terminated).  Batch handles:
  * iq_in [channels][n_floats], bits_out [channels][cap], n_bits[channels] (same layout rule for the
  * other host entry points below). */

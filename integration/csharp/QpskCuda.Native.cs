@@ -72,6 +72,13 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_ddc_reset(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_ddc_process(IntPtr h, float* iqIn, long nFloats, float* iqOut, long outStrideFloats, out long nOutFloats);
     [DllImport(Lib)] internal static extern int qpsk_ddc_process_dev(IntPtr h, float* dIn, long nFloats, float* dOut, long outStrideFloats, out long nOutFloats, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_agc_create_batch(int window, float refLevel, float maxGain, int channels, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_agc_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_agc_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_agc_process(IntPtr h, float* iqIn, float* iqOut, long nFloats, long outCapFloats);
+    [DllImport(Lib)] internal static extern int qpsk_agc_process_dev(IntPtr h, float* dIn, float* dOut, long nFloats, long inStrideFloats, long outStrideFloats, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_agc_gain(IntPtr h, float* gain, long cap);
+    [DllImport(Lib)] internal static extern int qpsk_agc_gain_dev(IntPtr h, float* dGain, IntPtr stream);
     // a6  QPSKModulator                             (MS/QPSKModulator.cs:18,54,104)
     [DllImport(Lib, CharSet = CharSet.Ansi)]
     internal static extern int qpsk_mod_create(int fs, int rs, double alpha, int span, int diff, string? tsc, out IntPtr h);
@@ -88,6 +95,7 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_demod_set_equalizer(IntPtr h, int nTaps, float mu, float modulus);
     [DllImport(Lib)] internal static extern int qpsk_demod_equalizer_taps(IntPtr h, float* tapsIq, long capFloats);
     [DllImport(Lib)] internal static extern int qpsk_demod_set_fractional_equalizer(IntPtr h, int nTaps, float mu, float modulus);
+    [DllImport(Lib)] internal static extern int qpsk_demod_set_agc(IntPtr h, int window, float refLevel, float maxGain);
     [DllImport(Lib)] internal static extern int qpsk_demod_fractional_equalizer_taps(IntPtr h, float* tapsIq, long capFloats);
     [DllImport(Lib)] internal static extern int qpsk_demod_bits(IntPtr h, float* iqIn, long nFloats, byte* bitsOut, long cap, out long nBits);
     [DllImport(Lib)] internal static extern int qpsk_demod_bytes(IntPtr h, float* iqIn, long nFloats, byte* start, long nStart,

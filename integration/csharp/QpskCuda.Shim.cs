@@ -383,6 +383,54 @@ namespace QPSK.Models
         }
         public void Dispose() => _o.Dispose();
     }
+
+    // Feed-forward AGC (not in the reference; definition in qpskcuda.h): per channel every sample is scaled by
+    // min(refLevel / m, maxGain), m the peak of max(|I|, |Q|) over a Window-sample window looking Window-1 samples ahead, so
+    // the output is the input delayed by Window-1 samples, at level refLevel.  State persists across calls.
+    public sealed unsafe class Agc : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Window;
+        public readonly int Channels;
+        public Agc(int window, float refLevel = 1.0f, float maxGain = 65536.0f, int channels = 1)
+        {
+            if (window < 1 || window > 4096) throw new ArgumentOutOfRangeException(nameof(window), "window must be from 1 to 4096.");
+            if (!(refLevel > 0) || float.IsInfinity(refLevel)) throw new ArgumentOutOfRangeException(nameof(refLevel), "refLevel must be finite and > 0.");
+            if (!(maxGain > 0) || float.IsInfinity(maxGain)) throw new ArgumentOutOfRangeException(nameof(maxGain), "maxGain must be finite and > 0.");
+            if (channels < 1) throw new ArgumentOutOfRangeException(nameof(channels), "At least one channel.");
+            IntPtr h;
+            QpskCuda.Check(QpskCuda.qpsk_agc_create_batch(window, refLevel, maxGain, channels, out h), nameof(window));
+            _o = new QpskHandle(h, QpskCuda.qpsk_agc_destroy);
+            Window = window;
+            Channels = channels;
+        }
+        // iqIn / iqOut: [Channels][nFloats] interleaved IQ, nFloats = iqIn.Length / Channels.
+        public void Process(ReadOnlySpan<float> iqIn, Span<float> iqOut)
+        {
+            if (iqIn.Length % (2 * Channels) != 0)
+                throw new ArgumentException("Input must be Channels rows of interleaved IQ with even length.", nameof(iqIn));
+            if (iqOut.Length < iqIn.Length) throw new ArgumentException("Output span is shorter than the input.", nameof(iqOut));
+            long n = iqIn.Length / Channels;
+            fixed (float* i = iqIn) fixed (float* o = iqOut)
+                QpskCuda.Check(QpskCuda.qpsk_agc_process(_h, i, o, n, n), nameof(iqOut));
+            GC.KeepAlive(this);
+        }
+        // the gain of each channel's last output
+        public float[] Gain()
+        {
+            var g = new float[Channels];
+            fixed (float* p = g) QpskCuda.Check(QpskCuda.qpsk_agc_gain(_h, p, g.Length));
+            GC.KeepAlive(this);
+            return g;
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_agc_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
 }
 
 namespace QPSK
@@ -480,6 +528,12 @@ namespace QPSK
             fixed (float* p = t) QpskCuda.Check(QpskCuda.qpsk_demod_equalizer_taps(_h, p, t.Length));
             GC.KeepAlive(this);
             return t;
+        }
+        // opt-in feed-forward AGC ahead of the FLL and the matched filter (not in the reference; window 0 = off, the default)
+        public void SetAgc(int window, float refLevel = 1.0f, float maxGain = 65536.0f)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_demod_set_agc(_h, window, refLevel, maxGain));
+            GC.KeepAlive(this);
         }
         // opt-in fractionally spaced CMA equalizer between the matched filter and clock recovery (not in the reference;
         // needs SampleRate / SymbolRate an integer 2..8; nTaps 0 = off, the default)

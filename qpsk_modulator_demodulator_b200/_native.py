@@ -129,6 +129,13 @@ def _signatures():
         "qpsk_ddc_reset": (i, [vp]),
         "qpsk_ddc_process": (i, [vp, vp, i64, vp, i64, i64p]),
         "qpsk_ddc_process_dev": (i, [vp, vp, i64, vp, i64, i64p, vp]),
+        "qpsk_agc_create_batch": (i, [i, f, f, i, vpp]),
+        "qpsk_agc_destroy": (i, [vp]),
+        "qpsk_agc_reset": (i, [vp]),
+        "qpsk_agc_process": (i, [vp, vp, vp, i64, i64]),
+        "qpsk_agc_process_dev": (i, [vp, vp, vp, i64, i64, i64, vp]),
+        "qpsk_agc_gain": (i, [vp, f32p, i64]),
+        "qpsk_agc_gain_dev": (i, [vp, vp, vp]),
         "qpsk_mod_create": (i, [i, i, d, i, i, cp, vpp]),
         "qpsk_mod_destroy": (i, [vp]),
         "qpsk_mod_taps": (i, [vp, f64p, i, i32p]),
@@ -145,6 +152,7 @@ def _signatures():
         "qpsk_demod_equalizer_taps": (i, [vp, f32p, i64]),
         "qpsk_demod_set_fractional_equalizer": (i, [vp, i, f, f]),
         "qpsk_demod_fractional_equalizer_taps": (i, [vp, f32p, i64]),
+        "qpsk_demod_set_agc": (i, [vp, i, f, f]),
         "qpsk_demod_bits": (i, [vp, vp, i64, vp, i64, vp]),
         "qpsk_demod_bits_packed": (i, [vp, vp, i64, vp, i64, vp]),
         "qpsk_demod_bytes": (i, [vp, vp, i64, vp, i64, vp, i64, vp, i64, vp]),

@@ -424,6 +424,51 @@ class CmaEqualizer(_Handle):
         check(lib().qpsk_eq_reset(self._h))
 
 
+# ---- feed-forward AGC (not in the reference) -----------------------------------------------------
+class Agc(_Handle):
+    """Feed-forward AGC on the GPU (csrc/agc.cu; definition in include/qpskcuda.h): per channel, each sample is scaled by
+    fminf(ref / m, max_gain), m the peak of max(|re|, |im|) over a `window`-sample window (1..4096) that looks window-1
+    samples ahead of it, so the output is the input delayed by window-1 samples, at level `ref`.  State persists across
+    calls: any chunking of the stream gives the same outputs bit for bit."""
+    _destroy = "qpsk_agc_destroy"
+
+    def __init__(self, window: int, ref: float = 1.0, max_gain: float = 65536.0, channels: int = 1):
+        super().__init__()
+        self.window, self.channels = window, channels
+        check(lib().qpsk_agc_create_batch(window, ref, max_gain, channels, C.byref(self._h)))
+
+    def process(self, x) -> np.ndarray:
+        """x: complex64 [channels, n] (or [n] for one channel; interleaved float32 IQ also taken) -> complex64 outputs of
+        the same shape, one per input sample."""
+        a = np.asarray(x)
+        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        rows = a.reshape(self.channels, -1)
+        y = np.empty(rows.shape, np.float32)
+        check(lib().qpsk_agc_process(self._h, _ptr(rows), _ptr(y), rows.shape[1], rows.shape[1]))
+        out = y.view(np.complex64)
+        return out[0] if (self.channels == 1 and a.ndim == 1) else out
+
+    def process_dev(self, d_in: int, d_out: int, n_floats: int, in_stride: int = 0, out_stride: int = 0, stream: int = 0):
+        """Device pointers: [channels][in_stride] floats -> [channels][out_stride], n_floats per channel (strides in
+        floats, 0 = n_floats).  d_out must not overlap d_in."""
+        check(lib().qpsk_agc_process_dev(self._h, d_in, d_out, n_floats, in_stride or n_floats, out_stride or n_floats,
+                                         stream))
+
+    @property
+    def gain(self) -> np.ndarray:
+        """float32 [channels]: the gain of each channel's last output (max_gain before any sample)."""
+        out = np.empty(self.channels, np.float32)
+        check(lib().qpsk_agc_gain(self._h, out.ctypes.data_as(N.f32p), out.size))
+        return out
+
+    def gain_dev(self, d_gain: int, stream: int = 0):
+        """Copy the last gains to d_gain[channels] (float32, device) in stream order."""
+        check(lib().qpsk_agc_gain_dev(self._h, d_gain, stream))
+
+    def reset(self):
+        check(lib().qpsk_agc_reset(self._h))
+
+
 # ---- polyphase analysis channelizer (not in the reference) -------------------------------------
 def pfb_taps(channels: int, taps_per_branch: int, cutoff: float, atten_db: float = 60.0) -> np.ndarray:
     """Kaiser-windowed sinc prototype for PfbChannelizer (fp64, unit DC gain, channels*taps_per_branch taps); cutoff in

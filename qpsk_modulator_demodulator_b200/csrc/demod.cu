@@ -1,7 +1,8 @@
 // demod.cu — K5: QPSKDeModulator on the GPU (MS/QPSKDeModulator.cs:11-456), batched over independent
 // channels.  Compiled with --fmad=false (see loops.cuh).
 //
-// Chain per call (DeModulate :345-425):  [FLL (opt-in; the call at :359 is commented out upstream)] ->
+// Chain per call (DeModulate :345-425):  [feed-forward AGC (opt-in, agc.cu; not in the reference)] ->
+// [FLL (opt-in; the call at :359 is commented out upstream)] ->
 // RRC matched filter (FirEngine, fir.cu) -> [fractionally spaced CMA equalizer (opt-in, eq.cu; not in the reference)] ->
 // Mueller-Muller (loops.cu) -> [CMA equalizer (opt-in, eq.cu; not in the reference)] -> decode kernel: Costas + decision + differential decode -> bits -> TSC exact-match strip (:413-422).
 // DeModulateBytes (:169-259): the bits then feed the per-channel framer kernel (8 bit-offset marker
@@ -11,6 +12,7 @@
 #include <memory>
 #include <string>
 
+#include "agc.cuh"
 #include "eq.cuh"
 #include "fir.cuh"
 #include "loops.cuh"
@@ -986,7 +988,11 @@ struct DemodEngine {
   // opt-in T/sps-spaced CMA stage between the matched filter and MM (qpsk_demod_set_fractional_equalizer); null = off
   std::unique_ptr<EqEngine> fse;
   int64_t fse_drop = 0;            // outputs the stage still discards: the same for every channel (every call feeds all L)
-  DevBuf<float2> t_fll, t_rrc, t_sym, t_eq, t_fse;
+  // opt-in feed-forward AGC ahead of everything else (qpsk_demod_set_agc); null = off.  It writes t_agc, which the
+  // unchanged path then reads in place of the input.
+  std::unique_ptr<AgcEngine> agc;
+  int64_t agc_drop = 0;            // AGC outputs still to discard (W-1 once per stream), the same for every channel
+  DevBuf<float2> t_fll, t_rrc, t_sym, t_eq, t_fse, t_agc;
   DevBuf<int> d_nsym, d_neq;
   // what front() leaves for Costas: the MM symbols, or with the equalizer on its outputs
   float2* sym_p = nullptr;
@@ -1175,6 +1181,35 @@ struct DemodEngine {
     return QPSK_OK;
   }
 
+  // opt-in AGC stage: window 0 = off; otherwise a fresh AGC (zero history, discard count W-1)
+  int set_agc(int window, float ref, float max_gain) {
+    if (window != 0) QPSK_TRY(agc_check_params(window, ref, max_gain));
+    QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
+    if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
+    if (window == 0) {
+      agc.reset();
+      return QPSK_OK;
+    }
+    std::unique_ptr<AgcEngine> a(new (std::nothrow) AgcEngine());
+    if (!a) return QPSK_ERR_NOMEM;
+    QPSK_TRY(a->init(window, ref, max_gain, channels));
+    agc = std::move(a);
+    agc_drop = window - 1;
+    return QPSK_OK;
+  }
+  // the AGC over a whole call on `s`: x / ldx then point at its outputs past this call's discard, L counts them
+  int agc_front(const float2*& x, int64_t& L, int64_t& ldx, cudaStream_t s) {
+    const int64_t ld = L + (L & 1);
+    QPSK_TRY(t_agc.ensure((size_t)ld * channels));
+    QPSK_TRY(agc->process_dev(x, L, ldx, t_agc.p, ld, s));
+    const int64_t dc = agc_drop < L ? agc_drop : L;
+    agc_drop -= dc;
+    x = t_agc.p + dc;
+    ldx = ld;
+    L -= dc;
+    return QPSK_OK;
+  }
+
   // Time-chunk pipeline of bits_dev (FLL path): number of chunks for an L-sample call.  Short calls stay on one stream: the
   // split costs two launches and a warm-up per chunk.  The channel count does not matter: a single stream gains as much as
   // a full batch (1.10 -> 0.84 ms for 4196 samples), because the FLL and the symbol stages are each latency-bound on their
@@ -1349,6 +1384,18 @@ struct DemodEngine {
       if (hsrc.pageable) QPSK_TRY(ensure_bounce((size_t)channels * (size_t)hs->ld * (hs->cs16 ? 4 : 8)));
       if (chunks == 1) QPSK_TRY(stage_host_chunk(hsrc, 0, L, ld, s));
     }
+    int64_t agc_dc = 0;                              // time-chunk pipeline: samples of this call the AGC discards
+    if (agc && chunks == 1) {
+      QPSK_TRY(agc_front(x, L, ldx, s));
+      if (L == 0) {
+        QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(long long) * channels, s));
+        return QPSK_OK;
+      }
+    } else if (agc) {
+      QPSK_TRY(t_agc.ensure((size_t)(L + (L & 1)) * channels));
+      agc_dc = agc_drop < L ? agc_drop : L;
+      agc_drop -= agc_dc;
+    }
     const float2* sym_in = nullptr;                  // what the symbol-stage kernel reads in the single-launch case
     int64_t sym_in_ld = 0;
     if (chunks > 1) {
@@ -1404,8 +1451,9 @@ struct DemodEngine {
       // copy and FLL would take turns (3.3 ms per step where 1.3 + tail is possible).
       if (from_host) QPSK_CUDA_TRY(cudaStreamWaitEvent(copy, ev_in, 0));
       int t = 0;
+      bool launched = false;
       for (int64_t n0 = 0; n0 < L; n0 += step, ++t) {
-        const int64_t len = (L - n0 < step) ? (L - n0) : step;
+        int64_t len = (L - n0 < step) ? (L - n0) : step;
         if (from_host) {
           QPSK_TRY(stage_host_chunk(hsrc, n0, len, mf_ld, copy));      // pageable source: the host gathers the chunk first
           QPSK_CUDA_TRY(cudaEventRecord(ev_copy[(size_t)t], copy));
@@ -1413,20 +1461,33 @@ struct DemodEngine {
         }
         const float2* src = x + n0;
         int64_t lds = ldx;
-        if (use_fll) {
-          QPSK_TRY(fll.process_dev(src, t_fll.p + n0, len, lds, mf_ld, side));           // the call at :359
-          src = t_fll.p + n0;
+        int64_t o = n0;                              // where this chunk's samples sit in the scratch rows
+        if (agc) {
+          QPSK_TRY(agc->process_dev(src, len, lds, t_agc.p + n0, mf_ld, side));
+          const int64_t skip = agc_dc > n0 ? std::min<int64_t>(agc_dc - n0, len) : 0;
+          o = n0 + skip;
+          len -= skip;
+          src = t_agc.p + o;
           lds = mf_ld;
         }
-        if (!fuse_mf) {
-          QPSK_TRY(mf.filter_dev(src, t_rrc.p + n0, len, lds, mf_ld, side));             // :360
-          src = t_rrc.p + n0;
+        if (len > 0 && use_fll) {
+          QPSK_TRY(fll.process_dev(src, t_fll.p + o, len, lds, mf_ld, side));            // the call at :359
+          src = t_fll.p + o;
+          lds = mf_ld;
+        }
+        if (len > 0 && !fuse_mf) {
+          QPSK_TRY(mf.filter_dev(src, t_rrc.p + o, len, lds, mf_ld, side));              // :360
+          src = t_rrc.p + o;
           lds = mf_ld;
         }
         QPSK_CUDA_TRY(cudaEventRecord(ev_chunk[(size_t)t], side));
         QPSK_CUDA_TRY(cudaStreamWaitEvent(s, ev_chunk[(size_t)t], 0));
-        QPSK_TRY(launch_symsync(src, len, lds, raw, ld_raw, n_raw, t > 0 ? 1 : 0, fuse_mf, s));
+        if (len > 0) {
+          QPSK_TRY(launch_symsync(src, len, lds, raw, ld_raw, n_raw, launched ? 1 : 0, fuse_mf, s));
+          launched = true;
+        }
       }
+      if (!launched) QPSK_CUDA_TRY(cudaMemsetAsync(n_raw, 0, sizeof(long long) * channels, s));
     } else if (fused) {
       QPSK_TRY(mm.ensure_queue(8, s));
       QPSK_TRY(launch_symsync(sym_in, L, sym_in_ld, raw, ld_raw, n_raw, 0, fuse_mf, s));
@@ -1461,6 +1522,13 @@ struct DemodEngine {
       long long sl = symbols_bound(L);                         // refuse before any stage consumes the samples
       if (sl < 1) sl = 1;
       if (ld_out < sl) return QPSK_ERR_CAPACITY;
+    }
+    if (agc) {
+      QPSK_TRY(agc_front(x, L, ldx, s));
+      if (L == 0) {
+        QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(int) * channels, s));
+        return QPSK_OK;
+      }
     }
     QPSK_TRY(front(x, L, ldx, s));
     QPSK_TRY(costas.process_dev(sym_p, out, sym_ld, sym_ld, ld_out, nsym_p, s));   // :447-452
@@ -1563,6 +1631,11 @@ int qpsk_demod_set_equalizer(qpsk_demod* d, int n_taps, float mu, float modulus)
   if (!d) return QPSK_ERR_NULL;
   QPSK_TRY(ensure_device(d->eng.device));
   return d->eng.set_equalizer(n_taps, mu, modulus);
+}
+int qpsk_demod_set_agc(qpsk_demod* d, int window, float ref, float max_gain) {
+  if (!d) return QPSK_ERR_NULL;
+  QPSK_TRY(ensure_device(d->eng.device));
+  return d->eng.set_agc(window, ref, max_gain);
 }
 int qpsk_demod_equalizer_taps(qpsk_demod* d, float* taps_iq, int64_t cap_floats) {
   if (!d || !taps_iq) return QPSK_ERR_NULL;

@@ -196,6 +196,12 @@ class QPSKDeModulator(_Handle):
         check(lib().qpsk_demod_fractional_equalizer_taps(self._h, out.ctypes.data_as(N.f32p), out.size))
         return out[0] if self.channels == 1 else out
 
+    def set_agc(self, window: int, ref: float = 1.0, max_gain: float = 65536.0):
+        """Opt-in feed-forward AGC (api.Agc) ahead of the FLL and the matched filter, so carriers at any level reach the
+        loops at the level `ref` sets; window 0 turns it off.  Resets this stage only.  Its delay of window-1 samples is
+        absorbed: the bits keep their alignment, and the last window-1 samples of a call reach the chain in the next."""
+        check(lib().qpsk_demod_set_agc(self._h, window, ref, max_gain))
+
     def _in(self, SamplesIQ):
         if SamplesIQ is None:
             raise ArgumentNullException("SamplesIQ")
