@@ -134,6 +134,9 @@ QPSK_API int qpsk_fir_set_state(qpsk_fir* f, const float* hist_iq, int64_t n_flo
 /* ---- a7-a8  FLLBandEdgeFilter  (MS/Models/Band-Edge Filter.cs:14-203) ---------------------- */
 /* DesignFilter :132-183, host-side fp32.  lower/upper: 2*filter_size floats each. */
 QPSK_API int qpsk_fll_design(float sps, float rolloff, int filter_size, float* lower_iq, float* upper_iq);
+/* filter_size 1..1430: every size must run in the generic kernel, whose ring of filter_size past outputs per stream lives
+   in shared memory (16 streams per CTA, within 200 KiB).  Larger sizes return QPSK_ERR_UNSUPPORTED, here, in
+   qpsk_fll_create_batch and in qpsk_chain_create (fll_size). */
 QPSK_API int qpsk_fll_create(float sps, float rolloff, int filter_size, float bandwidth, qpsk_fll** out);
 QPSK_API int qpsk_fll_create_batch(float sps, float rolloff, int filter_size, float bandwidth,
                                    int channels, qpsk_fll** out);
@@ -344,7 +347,9 @@ QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha,
                              int differential, const char* tsc_bits, qpsk_mod** out);
 QPSK_API int qpsk_mod_destroy(qpsk_mod* m);
 QPSK_API int qpsk_mod_taps(const qpsk_mod* m, double* out, int cap, int* n);       /* getCoeef() :32 */
-/* Modulate(string,bool) :104-167.  out==NULL: size query (*n_floats set). */
+/* Modulate(string,bool) :104-167.  out==NULL: size query (*n_floats set).  The modulate calls return
+   QPSK_ERR_UNSUPPORTED for sample_rate / symbol_rate > 256 and for more than 96 filter taps per phase
+   (ceil(taps / (sample_rate / symbol_rate))); the output is not written then. */
 QPSK_API int qpsk_mod_modulate_bits(qpsk_mod* m, const char* bits, int64_t n_bits, int pulse_shaping,
                                     float* iq_out, int64_t cap_floats, int64_t* n_floats);
 /* ModulateBytes :54-72 (ModulateTextUtf8 :74-89 = this over UTF-8 bytes) */

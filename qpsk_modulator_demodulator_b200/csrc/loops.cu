@@ -19,6 +19,16 @@ constexpr int kFllGroup = 8;
 constexpr int kFllCtaThreads = 128;                       // 16 streams per CTA
 constexpr int kFllCtaStreams = kFllCtaThreads / kFllGroup;
 constexpr int kFllBlock = 32;                             // samples staged per round and stream
+constexpr size_t kFllGroupMaxSmem = 200 * 1024;           // dynamic shared memory the generic kernel may ask for
+
+// Dynamic shared memory of fll_group_kernel for an N-tap filter: taps (padded to even, + alignment), lane partials, input
+// and output staging, and the ring of N past outputs per stream.  Every filter size must fit it: a caller-set phase sends
+// any size to this kernel.
+static size_t fll_group_smem(int n_taps) {
+  const size_t n = (size_t)n_taps, np = n + (n & 1);
+  return (2 * np + 4) * sizeof(float) + (size_t)kFllCtaStreams * kFllGroup * sizeof(float4) +
+         (size_t)2 * kFllCtaStreams * kFllBlock * sizeof(float2) + (size_t)kFllCtaStreams * n * sizeof(float2);
+}
 
 __global__ void __launch_bounds__(kFllCtaThreads)
     fll_group_kernel(const FllParams P, const float* __restrict__ taps, float2* ring_g, int* head_g, float2* pf_g, int C,
@@ -133,7 +143,7 @@ int FllEngine::init(float sps, float rolloff, int size, float bw, int channels_i
   if (size <= 0) return QPSK_ERR_RANGE;                      // :44
   if (!(bw > 0.0f)) return QPSK_ERR_RANGE;                   // :45
   if (channels_in <= 0) return QPSK_ERR_RANGE;
-  if (size > 2048) return QPSK_ERR_UNSUPPORTED;              // the ring lives in shared memory
+  if (fll_group_smem(size) > kFllGroupMaxSmem) return QPSK_ERR_UNSUPPORTED;   // the ring lives in shared memory: N <= 1430
   QPSK_TRY(ensure_device());
   device = current_device();
   channels = channels_in;
@@ -186,10 +196,8 @@ int FllEngine::process_dev(const float2* x, float2* y, int64_t L, int64_t ldx, i
   if (!wild && fll_duo_supported(n_taps))
     return fll_duo_launch(P, d_taps.p, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy, s);
   // 8 lanes per stream; ring, staging and partial sums in shared memory
-  const int Np = n_taps + (n_taps & 1);
-  const size_t smem = (size_t)(2 * Np + 4) * sizeof(float) + (size_t)kFllCtaStreams * kFllGroup * sizeof(float4) +
-                      (size_t)2 * kFllCtaStreams * kFllBlock * sizeof(float2) + (size_t)kFllCtaStreams * n_taps * sizeof(float2);
-  if (smem > 200 * 1024) return QPSK_ERR_UNSUPPORTED;
+  const size_t smem = fll_group_smem(n_taps);
+  if (smem > kFllGroupMaxSmem) return QPSK_ERR_UNSUPPORTED;
   const int blocks = (channels + kFllCtaStreams - 1) / kFllCtaStreams;
   QPSK_TRY(allow_max_dynamic_smem((const void*)fll_group_kernel));
   fll_group_kernel<<<blocks, kFllCtaThreads, smem, s>>>(P, d_taps.p, d_ring.p, d_head.p, d_pf.p, channels, x, y, L, ldx, ldy);

@@ -6,6 +6,7 @@ import ctypes as C_
 import numpy as np
 import pytest
 
+import kernel_variants as kv
 from fse_oracle import FseBatch, FseDemod
 from test_gpu_equalizer import BENCH_CHANNEL, _bursts
 from test_gpu_guards import Guarded
@@ -22,9 +23,13 @@ def _rows(orc, C, L, seed):
 
 
 # ---- the block ---------------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("sps", [2, 4, 3, 8])
-@pytest.mark.parametrize("n_taps", [1, 7, 21, 64])
-@pytest.mark.parametrize("channels", [1, 5, 64, 2048])
+# The grid of channel counts, tap counts and rates, plus every cma_eq_kernel<J, S> instantiation at 37 channels (8 per CTA:
+# the last CTA is partial), S = 0 through sps 3 and 7 (tests/kernel_variants.py: EQ_ROWS).
+_BLOCK_CASES = ([(c, n, s) for c in (1, 5, 64, 2048) for n in (1, 7, 21, 64) for s in (2, 4, 3, 8)] +
+                [(kv.EQ_ROWS_C, n, s) for n, s in kv.EQ_ROWS])
+
+
+@pytest.mark.parametrize("channels,n_taps,sps", _BLOCK_CASES, ids=[f"{c}-{n}-{s}" for c, n, s in _BLOCK_CASES])
 def test_block_matches_oracle(gpu, orc, sps, n_taps, channels):
     L = 151 if channels == 2048 else 701                 # odd: the call ends in the middle of a symbol
     x = _rows(orc, channels, L, n_taps)
@@ -110,6 +115,11 @@ def test_block_reset_and_arguments(gpu, orc):
     h = C_.c_void_p()
     assert gpu._native.lib().qpsk_eq_create_fractional(5, 0.1, 1.0, 2, 0, C_.byref(h)) == gpu._native.ERR_RANGE
     assert gpu._native.lib().qpsk_eq_create_fractional(5, 0.1, 1.0, 2, 1, None) == gpu._native.ERR_NULL
+
+
+def test_block_launches_the_predicted_kernels(gpu):
+    import os
+    assert kv.launched_in_child("eq", int(os.environ.get("LOCAL_RANK", "0"))) == kv.predicted_launches("eq")
 
 
 # ---- the demodulator stage ---------------------------------------------------------------------------------------------

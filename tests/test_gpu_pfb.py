@@ -6,6 +6,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
+import kernel_variants as kv
 from pfb_oracle import SCENE_FS, SCENE_RS, TSC, PfbPoly, qpsk_fdm_scene, scene_channels
 
 pytestmark = pytest.mark.gpu
@@ -25,17 +26,22 @@ def _check(got, want):
     assert np.abs(got.astype(np.complex128) - want).max() <= 1e-5 * np.abs(want).max()
 
 
-@pytest.mark.parametrize("M", [2, 4, 8, 16, 32, 64, 128, 256, 512, 1024])
-@pytest.mark.parametrize("P", [1, 2, 8, 16, 32])
+# the M x P grid, plus every pfb_kernel<P> at M = 4 and at M = 1024, whose tiles differ in shape (tests/kernel_variants.py)
+@pytest.mark.parametrize("P,M", kv.PFB_ROWS, ids=[f"{P}-{M}" for P, M in kv.PFB_ROWS])
 def test_matches_polyphase_oracle(gpu, M, P):
     rng = np.random.default_rng(M * 100 + P)
-    n_taps = P * M - (M // 3 if P > 1 else 0)                   # not a multiple of M (pads to P taps per branch)
+    n_taps = kv.pfb_taps(P, M)                                  # not a multiple of M (pads to P taps per branch)
     h = rng.standard_normal(n_taps) / np.sqrt(n_taps)
     n = max(40, 2 * _tile_blocks(M) + 3) * M + M // 2 + 1       # more than two tiles for every M, ragged end
     x = _cx64(rng, n)
     got = gpu.PfbChannelizer(h, M).process(x)
     want = PfbPoly(h.astype(np.float32), M).process(x)
     _check(got, want)
+
+
+def test_launches_the_predicted_kernels(gpu):
+    import os
+    assert kv.launched_in_child("pfb", int(os.environ.get("LOCAL_RANK", "0"))) == kv.predicted_launches("pfb")
 
 
 @pytest.mark.parametrize("M,P", [(4, 3), (16, 8), (64, 5), (1024, 2)])
