@@ -341,6 +341,47 @@ QPSK_API int qpsk_agc_process_dev(qpsk_agc* p, const float* d_in, float* d_out, 
 QPSK_API int qpsk_agc_gain(qpsk_agc* p, float* gain, int64_t cap);
 QPSK_API int qpsk_agc_gain_dev(qpsk_agc* p, float* d_gain, void* stream);
 
+/* ---- rational resampler ------------------------------------------------------------------------------------- */
+/* Not in the reference; moves a batch of channel streams between sample rates that are not integer multiples of each
+ * other (a fixed ADC / DAC rate against the symbol rate), GNU Radio's rational_resampler_ccf once per channel: interpolate
+ * by L, filter with a real prototype, decimate by M.
+ * Parameters: real taps h[0..N-1], 1 <= N <= 16384; interpolation L and decimation M, each 1..1024 (not necessarily
+ * coprime); P = ceil(N / L) taps per branch, P <= 64; channels 1..16384 (outside these limits: QPSK_ERR_UNSUPPORTED;
+ * N <= 0: QPSK_ERR_ARG; a non-finite tap: QPSK_ERR_RANGE).
+ * Definition, per channel, x[n] counting input samples since creation or the last reset, x[n] = 0 for n < 0, x_up = x
+ * zero-stuffed by L (x_up[nL] = x[n], zero elsewhere):
+ *   y[m] = sum_{i=0}^{N-1} h[i] * x_up[mM - i]                       (scipy.signal.upfirdn(h, x, L, M) taken literally)
+ * Computation (the polyphase form): n_m = floor(mM / L), phi_m = mM mod L, exact integer arithmetic on 64-bit counters (no
+ * position is accumulated in floating point), and y[m] = sum_{q=0}^{P-1} h[phi_m + qL] * x[n_m - q] with h zero past N,
+ * accumulated in increasing q with fp32 FMA, re and im separately.  Against an fp64 evaluation of the definition
+ * max|err| <= 1e-5 max|y| over a call's output.
+ * No L factor: a prototype with sum h = L (e.g. L * firwin(..., scale=True)) passes a carrier with unit gain, so the CMA
+ * `modulus 1.0` convention holds after the resampler.
+ * Output m exists once x[n_m] has arrived: after n_in inputs there are n_in == 0 ? 0 : floor((n_in L - 1) / M) + 1
+ * outputs, and a call's count is that difference, known to the host without reading the device.
+ * State: the last P-1 input samples of each channel and the input and output counters.  Any chunking of a stream (empty
+ * calls, chunks shorter than M / L, any sample offset) gives the same outputs bit for bit, and row c of a batch equals a
+ * one-channel handle fed that row, bit for bit. */
+typedef struct qpsk_resamp qpsk_resamp;
+QPSK_API int qpsk_resamp_create(const float* taps, int n_taps, int interp, int decim, int channels, qpsk_resamp** out);
+QPSK_API int qpsk_resamp_destroy(qpsk_resamp* p);
+/* back to the state at creation: zero history, counters 0.  Waits for the handle's own stream only:
+ * qpsk_resamp_process_dev calls enqueued on another stream must have completed before the reset. */
+QPSK_API int qpsk_resamp_reset(qpsk_resamp* p);
+/* host memory: iq_in [channels][n_floats] (n_floats even, else QPSK_ERR_ARG) -> iq_out [channels][out_stride_floats];
+ * *n_out_floats = floats written per channel (set on QPSK_ERR_CAPACITY too); out_stride_floats < *n_out_floats ->
+ * QPSK_ERR_CAPACITY, nothing consumed.  Floats of a row past *n_out_floats are not written. */
+QPSK_API int qpsk_resamp_process(qpsk_resamp* p, const float* iq_in, int64_t n_floats, float* iq_out,
+                                 int64_t out_stride_floats, int64_t* n_out_floats);
+/* device memory (8-byte aligned, else QPSK_ERR_ARG), strides in floats (even; in_stride_floats >= n_floats, else
+ * QPSK_ERR_ARG; out_stride_floats < *n_out_floats -> QPSK_ERR_CAPACITY with *n_out_floats set and nothing consumed); the
+ * rows written must not overlap the rows read (QPSK_ERR_ARG).  d_out's rows are the [channels][out_stride] rows
+ * qpsk_demod_bytes_dev reads with in_stride = out_stride, and d_in's can be the rows qpsk_ddc_process_dev writes.
+ * Enqueued on `stream` (NULL = the handle's own); the state advances at enqueue, so calls on one handle must run in issue
+ * order.  Floats of a row past *n_out_floats are not written. */
+QPSK_API int qpsk_resamp_process_dev(qpsk_resamp* p, const float* d_in, int64_t n_floats, int64_t in_stride_floats,
+                                     float* d_out, int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
+
 /* ---- a6  QPSKModulator  (MS/QPSKModulator.cs:18-168) ---------------------------------------- */
 /* tsc_bits: '0'/'1' string or NULL (null/whitespace = no TSC, :27) */
 QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha, int rrc_span,

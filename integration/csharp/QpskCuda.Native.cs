@@ -79,6 +79,11 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_agc_process_dev(IntPtr h, float* dIn, float* dOut, long nFloats, long inStrideFloats, long outStrideFloats, IntPtr stream);
     [DllImport(Lib)] internal static extern int qpsk_agc_gain(IntPtr h, float* gain, long cap);
     [DllImport(Lib)] internal static extern int qpsk_agc_gain_dev(IntPtr h, float* dGain, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_resamp_create(float* taps, int nTaps, int interp, int decim, int channels, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_resamp_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_resamp_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_resamp_process(IntPtr h, float* iqIn, long nFloats, float* iqOut, long outStrideFloats, out long nOutFloats);
+    [DllImport(Lib)] internal static extern int qpsk_resamp_process_dev(IntPtr h, float* dIn, long nFloats, long inStrideFloats, float* dOut, long outStrideFloats, out long nOutFloats, IntPtr stream);
     // a6  QPSKModulator                             (MS/QPSKModulator.cs:18,54,104)
     [DllImport(Lib, CharSet = CharSet.Ansi)]
     internal static extern int qpsk_mod_create(int fs, int rs, double alpha, int span, int diff, string? tsc, out IntPtr h);

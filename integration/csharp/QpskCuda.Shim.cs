@@ -431,6 +431,58 @@ namespace QPSK.Models
         }
         public void Dispose() => _o.Dispose();
     }
+
+    // Rational resampler (not in the reference; definition in qpskcuda.h): Channels streams, each interpolated by Interp,
+    // filtered with a real prototype and decimated by Decim (scipy.signal.upfirdn per channel, streamed).  No Interp factor:
+    // taps summing to Interp pass a carrier with unit gain.  State persists across calls: any chunking gives the same outputs.
+    public sealed unsafe class Resampler : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Interp;
+        public readonly int Decim;
+        public readonly int Channels;
+        public Resampler(float[] taps, int interp, int decim, int channels = 1)
+        {
+            if (taps == null) throw new ArgumentNullException(nameof(taps));
+            if (taps.Length == 0) throw new ArgumentException("Prototype taps must not be empty.", nameof(taps));
+            if (taps.Length > 16384) throw new ArgumentOutOfRangeException(nameof(taps), "At most 16384 prototype taps.");
+            if (interp < 1 || interp > 1024) throw new ArgumentOutOfRangeException(nameof(interp), "interp must be from 1 to 1024.");
+            if (decim < 1 || decim > 1024) throw new ArgumentOutOfRangeException(nameof(decim), "decim must be from 1 to 1024.");
+            if ((taps.Length + interp - 1) / interp > 64)
+                throw new ArgumentOutOfRangeException(nameof(taps), "At most 64 taps per branch (taps.Length <= 64 * interp).");
+            if (channels < 1 || channels > 16384) throw new ArgumentOutOfRangeException(nameof(channels), "From 1 to 16384 channels.");
+            foreach (var t in taps)
+                if (!float.IsFinite(t)) throw new ArgumentOutOfRangeException(nameof(taps), "Taps must be finite.");
+            IntPtr h;
+            fixed (float* t = taps)
+                QpskCuda.Check(QpskCuda.qpsk_resamp_create(t, taps.Length, interp, decim, channels, out h), nameof(taps));
+            _o = new QpskHandle(h, QpskCuda.qpsk_resamp_destroy);
+            Interp = interp;
+            Decim = decim;
+            Channels = channels;
+        }
+        // iqIn: [Channels][nFloats] interleaved IQ, nFloats = iqIn.Length / Channels; iqOut: [Channels][outStrideFloats].
+        // Returns floats written per channel.
+        public long Process(ReadOnlySpan<float> iqIn, Span<float> iqOut, long outStrideFloats)
+        {
+            if (iqIn.Length % (2 * Channels) != 0)
+                throw new ArgumentException("Input must be Channels rows of interleaved IQ with even length.", nameof(iqIn));
+            if (outStrideFloats < 0 || iqOut.Length < Channels * outStrideFloats)
+                throw new ArgumentException("Output span is too small for Channels rows of outStrideFloats.", nameof(iqOut));
+            long n;
+            fixed (float* i = iqIn) fixed (float* o = iqOut)
+                QpskCuda.Check(QpskCuda.qpsk_resamp_process(_h, i, iqIn.Length / Channels, o, outStrideFloats, out n), nameof(iqOut));
+            GC.KeepAlive(this);
+            return n;
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_resamp_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
 }
 
 namespace QPSK

@@ -136,6 +136,11 @@ def _signatures():
         "qpsk_agc_process_dev": (i, [vp, vp, vp, i64, i64, i64, vp]),
         "qpsk_agc_gain": (i, [vp, f32p, i64]),
         "qpsk_agc_gain_dev": (i, [vp, vp, vp]),
+        "qpsk_resamp_create": (i, [f32p, i, i, i, i, vpp]),
+        "qpsk_resamp_destroy": (i, [vp]),
+        "qpsk_resamp_reset": (i, [vp]),
+        "qpsk_resamp_process": (i, [vp, vp, i64, vp, i64, i64p]),
+        "qpsk_resamp_process_dev": (i, [vp, vp, i64, i64, vp, i64, i64p, vp]),
         "qpsk_mod_create": (i, [i, i, d, i, i, cp, vpp]),
         "qpsk_mod_destroy": (i, [vp]),
         "qpsk_mod_taps": (i, [vp, f64p, i, i32p]),

@@ -567,3 +567,52 @@ class DdcBank(_Handle):
 
     def reset(self):
         check(lib().qpsk_ddc_reset(self._h))
+
+
+# ---- rational resampler (not in the reference) --------------------------------------------------
+class Resampler(_Handle):
+    """Batched rational resampler on the GPU (csrc/resamp.cu; definition in include/qpskcuda.h): `channels` streams, each
+    interpolated by `interp` (L), filtered with the real prototype `taps` and decimated by `decim` (M), i.e.
+    scipy.signal.upfirdn(taps, x, L, M) per channel, streamed.  No L factor: taps summing to L (e.g.
+    L * scipy.signal.firwin(..., scale=True)) pass a carrier with unit gain.  L, M in 1..1024, 1..16384 taps with
+    ceil(len(taps) / L) <= 64.  State persists across calls: any chunking of the stream gives the same outputs."""
+    _destroy = "qpsk_resamp_destroy"
+
+    def __init__(self, taps, interp: int, decim: int, channels: int = 1):
+        super().__init__()
+        if taps is None:
+            raise ArgumentNullException("taps")
+        t = _f32(taps).ravel()
+        self.interp, self.decim, self.channels = interp, decim, channels
+        check(lib().qpsk_resamp_create(t.ctypes.data_as(N.f32p), t.size, interp, decim, channels, C.byref(self._h)))
+
+    def process(self, x, out_stride: int = 0) -> np.ndarray:
+        """x: complex64 [channels, n] (or [n] for one channel; interleaved float32 IQ also taken) -> complex64
+        [channels, n_out] (or [n_out]), the outputs this call completes.  `out_stride` (floats) sizes the output rows like
+        the C call; 0 = just enough."""
+        a = np.asarray(x)
+        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        rows = a.reshape(self.channels, -1)
+        n = C.c_int64(0)
+        if not out_stride:
+            st = lib().qpsk_resamp_process(self._h, None, rows.shape[1], None, -1, C.byref(n))
+            if st != N.ERR_CAPACITY:
+                check(st)
+            out_stride = n.value
+        y = np.zeros((self.channels, max(out_stride, 0)), np.float32)
+        check(lib().qpsk_resamp_process(self._h, _ptr(rows), rows.shape[1], _ptr(y), out_stride, C.byref(n)))
+        out = np.ascontiguousarray(y[:, : n.value]).view(np.complex64)
+        return out[0] if (self.channels == 1 and a.ndim == 1) else out
+
+    def process_dev(self, d_in: int, n_floats: int, d_out: int, out_stride: int, in_stride: int = 0,
+                    stream: int = 0) -> int:
+        """Device pointers: [channels][in_stride] floats (0 = n_floats), n_floats per channel -> d_out
+        [channels][out_stride].  Returns the floats written per channel (the n_floats to pass to
+        QPSKDeModulator.demod_bytes_dev with in_stride = out_stride)."""
+        n = C.c_int64(0)
+        check(lib().qpsk_resamp_process_dev(self._h, d_in, n_floats, in_stride or n_floats, d_out, out_stride,
+                                            C.byref(n), stream))
+        return n.value
+
+    def reset(self):
+        check(lib().qpsk_resamp_reset(self._h))
