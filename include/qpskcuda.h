@@ -236,7 +236,10 @@ QPSK_API int qpsk_eq_set_taps(qpsk_eq* eq, const float* taps_iq, int64_t n_float
  * every M-th sample (n = N)", channel k carries the constant phase e^{-j 2 pi k / M}.
  * Computation (the equivalent polyphase form): v_r[m] = sum_{q=0}^{P-1} h[qM + r] * x[(m - q)M + M - 1 - r], accumulated
  * in increasing q, then y_k[m] = sum_r v_r[m] * w^{kr}, w = e^{j 2 pi / M}, by an in-place radix-2/radix-2^2 FFT.  fp32 with
- * FMA; twiddles from an fp64 table rounded to fp32.  Against an fp64 evaluation of the definition max|err| <= 1e-5 max|y|.
+ * FMA; twiddles from an fp64 table rounded to fp32.  Against an fp64 evaluation of the definition max|err| <= 1e-5 max|y|,
+ * and per output (re and im, every channel k of block m), with u = 2^-24, gamma_n = nu / (1 - nu), S = log2 M and
+ * eta = 4u + O(u^2): |err| <= (1+eta)^S sum_r gamma_P |(sum_q |h||x.re|, sum_q |h||x.im|)| + ((1+eta)^S - 1) sum_r |v_r[m]|
+ * (derivation: tests/bank_bounds.py).
  * State: the last (P-1) complete blocks and the pending = (samples so far) mod M samples of the open block.  Any chunking of
  * a stream (chunks shorter than M, empty calls, any pointer alignment that results) gives the same outputs bit for bit.
  * A call of n samples gives floor((pending + n) / M) outputs per channel, known to the host without reading the device. */
@@ -281,7 +284,9 @@ QPSK_API int qpsk_pfb_process_dev(qpsk_pfb* p, const float* d_in, int64_t n_floa
  * Computation (exact in the phase words, phi(n - i) = phi(n) - phi(i) mod 2^64): u_k[m] = sum_i g_k[i] x[n_m - i] with
  * rotated taps g_k[i] = h[i] e^{+j 2 pi phi_k(i) / 2^64} formed on the host in fp64 and rounded to fp32, then
  * y_k[m] = u_k[m] e^{-j 2 pi phi_k(n_m) / 2^64}.  fp32 with FMA; against an fp64 evaluation of the definition
- * max|err| <= 1e-5 max|y| over a call's output.
+ * max|err| <= 1e-5 max|y| over a call's output, and per output (re and im), with u = 2^-24 and A = sum_i |h[i]|
+ * (|x[n_m - i].re| + |x[n_m - i].im|): |err| <= about sqrt2 (N + 1) u A + (5u + pi (2^-31 + 2^-25)) |u_k[m]| (the exact
+ * constants and their derivation: tests/bank_bounds.py).
  * Relation to the PFB channelizer: with D = M and f_k = k/M (k >= M/2 taken as k - M), row k of the bank equals row k of
  * qpsk_pfb with the same prototype times e^{+j 2 pi k / M}.  For a full grid the PFB is the cheaper block.
  * State: the last N-1 input samples, the pending = (samples so far) mod D samples of the open block and the 64-bit sample
@@ -354,7 +359,8 @@ QPSK_API int qpsk_agc_gain_dev(qpsk_agc* p, float* d_gain, void* stream);
  * Computation (the polyphase form): n_m = floor(mM / L), phi_m = mM mod L, exact integer arithmetic on 64-bit counters (no
  * position is accumulated in floating point), and y[m] = sum_{q=0}^{P-1} h[phi_m + qL] * x[n_m - q] with h zero past N,
  * accumulated in increasing q with fp32 FMA, re and im separately.  Against an fp64 evaluation of the definition
- * max|err| <= 1e-5 max|y| over a call's output.
+ * max|err| <= 1e-5 max|y| over a call's output, and per output |err.re| <= gamma_P sum_q |h[phi_m + qL]| |x[n_m - q].re|
+ * (the same for im), gamma_P = Pu / (1 - Pu), u = 2^-24.
  * No L factor: a prototype with sum h = L (e.g. L * firwin(..., scale=True)) passes a carrier with unit gain, so the CMA
  * `modulus 1.0` convention holds after the resampler.
  * Output m exists once x[n_m] has arrived: after n_in inputs there are n_in == 0 ? 0 : floor((n_in L - 1) / M) + 1

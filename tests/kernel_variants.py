@@ -1,11 +1,12 @@
-"""Which instantiation of the FLL, modulator, equalizer, channelizer and FIR kernels a call runs, predicted from its public
-inputs, listed from the built library, and read back from the profiler.
+"""Which instantiation of the FLL, modulator, equalizer, channelizer, DDC bank, resampler and FIR kernels a call runs,
+predicted from its public inputs, listed from the built library, and read back from the profiler.
 
 Every launcher picks a template instantiation from the shape of its input, and each instantiation is separately compiled
 code (its own unrolling, tail stages and register window), so each is tested on its own.  Per family:
   * `*_predict` restates the launcher's dispatch in plain Python and returns the instantiation's name, or UNSUPPORTED
     (`fir_predict`: the list of kernels the call launches, in order);
-  * `*_ROWS` is the table of public inputs the GPU parity tests run, at least one row per instantiation;
+  * `*_ROWS` is the table of public inputs the GPU parity tests run, at least one row per instantiation (the DDC,
+    resampler and channelizer rows are the ones tests/bank_bounds.py checks against per-output error bounds);
   * `*_launch_rows` runs those rows once each, in order, so that the profiler can list what ran.
 `compiled()` lists the instantiations in the built library (cuobjdump -sass | cu++filt).  tests/test_kernel_variants.py
 checks on the CPU that the dispatch reaches exactly the compiled set and that the tables cover it; the GPU tests check the
@@ -29,6 +30,9 @@ FAMILIES = {
     "mod": ("mod_shape_kernel",),
     "eq": ("cma_eq_kernel",),
     "pfb": ("pfb_kernel",),
+    # the history copies next to the DDC and resampler kernels (ddc_history_kernel, resamp_history_kernel) are left out
+    "ddc": ("ddc_kernel",),
+    "resamp": ("resamp_kernel",),
     # fir_hist_update_kernel (the delay-line copy next to the generic and decimating kernels) is left out
     "fir": ("fir_tma_kernel", "fir_split2_kernel", "fir_exact_real_kernel", "fir_generic_kernel", "fir_dec2_kernel",
             "fir_decim_tma_kernel", "fir_decim_kernel", "fir_subsample_kernel"),
@@ -178,6 +182,63 @@ def pfb_taps(P, M):
 
 PFB_GRID = [(P, M) for P in (1, 2, 8, 16, 32) for M in (2, 4, 8, 16, 32, 64, 128, 256, 512, 1024)]
 PFB_ROWS = PFB_GRID + [(P, M) for M in (4, 1024) for P in range(1, PFB_MAX_P + 1) if (P, M) not in PFB_GRID]
+
+
+# ---- DDC bank: qpsk_ddc_create, DdcEngine::process_dev (csrc/ddc.cu) ------------------------------------------------------
+DDC_MAX_TAPS, DDC_MAX_CHANNELS, DDC_MAX_DECIM = 4096, 2048, 1024
+DDC_SMALL_K = 8                         # kDdcSmallK: K <= 8 runs the 4-channel x 1024-output shape
+DDC_TILE = {True: 1024, False: 128}     # outputs per CTA, K <= 8 / K > 8
+
+
+def ddc_predict(n_taps, channels, decim):
+    """The kernel a call that completes at least one output runs (the history copy is left out)."""
+    if (not 1 <= n_taps <= DDC_MAX_TAPS or not 1 <= channels <= DDC_MAX_CHANNELS or
+            not 1 <= decim <= DDC_MAX_DECIM):
+        return UNSUPPORTED
+    return "ddc_kernel<1, 1, 8>" if channels <= DDC_SMALL_K else "ddc_kernel<4, 2, 32>"
+
+
+# (K, D, N, taps): both shapes (K = 8 | 9) at D = 1, odd D, D = 16 and 64; taps "rand" (fir_row_taps' recipe) or "kaiser"
+# (ddc_oracle.scene_taps, the prototype of the library's scenes)
+DDC_ROWS = [(K, D, N, kind) for D, N, kind in ((1, 17, "rand"), (5, 33, "rand"), (16, 100, "rand"), (64, 300, "rand"),
+                                               (16, 128, "kaiser")) for K in (8, 9)]
+
+
+def ddc_row_calls(row):
+    """Input samples of a row's two calls: three tiles of outputs and a ragged end each; the first leaves D//2 + 1 samples
+    of an open block pending (D > 2), so the second call's first output reads history and pending samples."""
+    K, D = row[:2]
+    n_out = 3 * DDC_TILE[K <= DDC_SMALL_K] + 37
+    return [n_out * D + (D // 2 + 1) % D, n_out * D + 3]
+
+
+# ---- rational resampler: qpsk_resamp_create, ResampEngine::process_dev (csrc/resamp.cu) ------------------------------------
+RESAMP_MAX_TAPS, RESAMP_MAX_FACTOR, RESAMP_MAX_BRANCH, RESAMP_MAX_CHANNELS = 16384, 1024, 64, 16384
+RESAMP_SMALL_K = 8                      # kResampSmallK: K <= 8 runs the one-channel x 256-output shape
+RESAMP_TILE = {True: 256, False: 32}    # outputs per CTA, K <= 8 / K > 8
+
+
+def resamp_predict(n_taps, L, M, channels):
+    """The kernel a call that completes at least one output runs (the history copy is left out)."""
+    if (not 1 <= n_taps <= RESAMP_MAX_TAPS or not 1 <= L <= RESAMP_MAX_FACTOR or not 1 <= M <= RESAMP_MAX_FACTOR or
+            not 1 <= channels <= RESAMP_MAX_CHANNELS or -(-n_taps // L) > RESAMP_MAX_BRANCH):
+        return UNSUPPORTED
+    return "resamp_kernel<1, 1, 1, 2048>" if channels <= RESAMP_SMALL_K else "resamp_kernel<32, 2, 4, 64>"
+
+
+# (K, L, M, N, taps): both shapes (K = 8 | 9); L < M, L > M, L = 1; P = 1, 24, 64; every ratio coprime, so that every
+# branch is used; taps "rand" or "kaiser" (resamp_oracle.resamp_taps)
+RESAMP_ROWS = [(K, L, M, N, kind) for L, M, N, kind in ((5, 8, 120, "rand"), (8, 5, 507, "rand"), (1, 3, 1, "rand"),
+                                                        (1, 1, 64, "rand"), (3, 1, 190, "rand"), (125, 128, 3000, "kaiser"))
+               for K in (8, 9)]
+RESAMP_CALL_OUT = 3 * 256 + 37          # outputs per call: >= 3 tiles of either shape, ragged in both
+
+
+def resamp_row_calls(row):
+    """Input samples per channel of a row's two calls, each completing about RESAMP_CALL_OUT outputs."""
+    L, M = row[1:3]
+    n = RESAMP_CALL_OUT * M // L
+    return [n + 3, n + 11]
 
 
 # ---- FIR: FirEngine::run / decimate_dev, launch_split2 (csrc/fir.cu) ----------------------------------------------------
@@ -599,6 +660,10 @@ def predicted_launches(family):
         return [eq_predict(n, sps) for n, sps in EQ_ROWS]
     if family == "pfb":
         return [pfb_predict(pfb_taps(P, M), M) for P, M in PFB_ROWS]
+    if family == "ddc":
+        return [ddc_predict(N, K, D) for K, D, N, _ in DDC_ROWS for _ in ddc_row_calls((K, D))]
+    if family == "resamp":
+        return [resamp_predict(N, L, M, K) for K, L, M, N, _ in RESAMP_ROWS for _ in resamp_row_calls((K, L, M))]
     if family == "fir":
         return [k for r in FIR_ROWS for call in fir_row_dispatch(r) for k, _ in call]
     raise ValueError(family)
@@ -693,7 +758,24 @@ def _fir_launch_rows(Q):
         fir_run_row(Q, r, fir_row_inputs(r))
 
 
-LAUNCH_ROWS = {"fir": _fir_launch_rows, "fll": _fll_launch_rows, "mod": _mod_launch_rows, "eq": _eq_launch_rows, "pfb": _pfb_launch_rows}
+def _ddc_launch_rows(Q):
+    for K, D, N, _ in DDC_ROWS:
+        bank = Q.DdcBank(np.ones(N, np.float32) / N, [0.1] * K, D)
+        for n in ddc_row_calls((K, D)):
+            bank.process(np.ones(n, np.complex64))
+        bank.close()
+
+
+def _resamp_launch_rows(Q):
+    for K, L, M, N, _ in RESAMP_ROWS:
+        r = Q.Resampler(np.ones(N, np.float32), L, M, K)
+        for n in resamp_row_calls((K, L, M)):
+            r.process(np.ones((K, n), np.complex64))
+        r.close()
+
+
+LAUNCH_ROWS = {"fir": _fir_launch_rows, "fll": _fll_launch_rows, "mod": _mod_launch_rows, "eq": _eq_launch_rows,
+               "pfb": _pfb_launch_rows, "ddc": _ddc_launch_rows, "resamp": _resamp_launch_rows}
 
 
 def launched_in_child(family, device=0, timeout=900):

@@ -6,13 +6,11 @@ the full batch; untouched guard bands; argument checks; 64-bit counters and outp
 5/8 and 8/5; and a receive chain DdcBank -> Resampler -> QPSKDeModulator on one stream at 4.096 samples per symbol."""
 import ctypes as C
 import os
-import re
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
+import kernel_variants as kv
 from ddc_oracle import TSC, scene_taps
 from resamp_oracle import (SCENE_D, SCENE_FREQS, SCENE_FS, SCENE_L, SCENE_M, SCENE_RS, ResampPoly, resamp_count,
                            resamp_scene, resamp_taps)
@@ -61,48 +59,14 @@ def test_matches_polyphase_oracle(gpu, K, L, M, N):
     _check(got, want)
 
 
-def _compiled_instantiations(lib_path):
-    from kernel_variants import _tool
-    sass = subprocess.check_output([_tool("cuobjdump"), "-sass", lib_path], text=True)
-    mangled = sorted(set(re.findall(r"Function : (\S+)", sass)))
-    demangled = subprocess.run([_tool("cu++filt")], input="\n".join(mangled) + "\n", capture_output=True, text=True,
-                               check=True).stdout.splitlines()
-    out = set()
-    for d in demangled:
-        m = re.search(r"\bresamp_kernel<([^<>]*)>", d)
-        if m:
-            out.add("resamp_kernel<" + ", ".join(re.sub(r"\(int\)", "", a).strip() for a in m.group(1).split(",")) + ">")
-    return out
-
-
-_PROFILE_CHILD = """
-import sys
-sys.path[:0] = {paths!r}
-import numpy as np
-import qpsk_modulator_demodulator_b200 as Q
-from symsync_dispatch import launched_kernels
-Q.set_device({device})
-rs = [Q.Resampler(np.ones(40, np.float32), 5, 8, K) for K in (1, 9)]
-xs = [np.ones((K, 2000), np.complex64) for K in (1, 9)]
-_, names = launched_kernels(lambda: [r.process(x) for r, x in zip(rs, xs)])
-print("KERNELS", repr(sorted(set(names))))
-"""
-
-
 def test_every_instantiation_is_compiled_tested_and_runs(gpu):
-    """The instantiations in the library are exactly the two shapes the parity cases reach, and both run (profiler, in a
-    child process: a profiler session in the pytest process leaves later profiled tests recording nothing)."""
-    import ast
-    got = _compiled_instantiations(gpu._native.LIB_PATH)
+    """The instantiations in the library are exactly the two shapes the parity cases reach, and the profiler (in a child
+    process) sees the predicted one run for every call of the resampler rows in tests/kernel_variants.py."""
+    got = kv.compiled(gpu._native.LIB_PATH)["resamp"]
     assert got == set(SHAPES.values()), got
     assert {SHAPES[K <= SMALL_K] for K, _, _, _ in CASES} == got
-    here = os.path.dirname(os.path.abspath(__file__))
-    code = _PROFILE_CHILD.format(paths=[os.path.dirname(here), here], device=int(os.environ.get("LOCAL_RANK", "0")))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-4000:]
-    names = ast.literal_eval([ln for ln in r.stdout.splitlines() if ln.startswith("KERNELS ")][-1][len("KERNELS "):])
-    ran = {"resamp_kernel<" + m.group(1) + ">" for n in names for m in [re.search(r"resamp_kernel<([^<>]*)>", n)] if m}
-    assert ran == got, names
+    ran = kv.launched_in_child("resamp", int(os.environ.get("LOCAL_RANK", "0")))
+    assert ran == kv.predicted_launches("resamp") and set(ran) == got, ran
 
 
 @pytest.mark.parametrize("K,L,M,N", [(3, 5, 8, 100), (40, 8, 5, 300), (5, 1, 1024, 64), (70, 125, 128, 1000),

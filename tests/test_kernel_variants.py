@@ -36,6 +36,13 @@ def _reachable(family):
             out.add(kv.pfb_predict(n, M))
         for n in range(1, 34 * 1024, 97):
             out.add(kv.pfb_predict(n, 1024))
+    elif family == "ddc":
+        for n, c, d in itertools.product((0, 1, 100, 4096, 4097), list(range(0, 40)) + [2047, 2048, 2049], (0, 1, 1024, 1025)):
+            out.add(kv.ddc_predict(n, c, d))
+    elif family == "resamp":
+        for n, L, M, c in itertools.product((0, 1, 64, 65, 16384, 16385), (0, 1, 256, 1024, 1025), (0, 1, 1024, 1025),
+                                            list(range(0, 40)) + [16383, 16384, 16385]):
+            out.add(kv.resamp_predict(n, L, M, c))
     elif family == "fir":
         sizes = sorted(set(range(1, 140)) | set(range(140, 1100, 13)) |
                        {n + d for n in (256, 512, 536, 560, 600, 889, 1039) for d in (-1, 0, 1, 2)})
@@ -74,6 +81,8 @@ def test_instantiation_counts():
     assert len(_reachable("mod")) == 52
     assert len(_reachable("eq")) == 40
     assert len(_reachable("pfb")) == 32
+    assert len(_reachable("ddc")) == 2                    # ddc_kernel<1, 1, 8> for K <= 8, <4, 2, 32> above
+    assert len(_reachable("resamp")) == 2                 # resamp_kernel<1, 1, 1, 2048> for K <= 8, <32, 2, 4, 64> above
     assert len(_reachable("fir")) == 3 + 1 + 1 + 2 + 1 + 3 + 4 + 1    # ... + fir_decim_kernel<D = 2..16>, fir_subsample_kernel
 
 
@@ -146,6 +155,17 @@ def test_channelizer_spot_values():
     assert p(4, 4) == "pfb_kernel<1>" and p(5, 4) == "pfb_kernel<2>" and p(32 * 1024, 1024) == "pfb_kernel<32>"
     assert p(32 * 1024 + 1, 1024) == kv.UNSUPPORTED and p(16, 6) == kv.UNSUPPORTED
     assert all(p(kv.pfb_taps(P, M), M) == f"pfb_kernel<{P}>" for P in range(1, 33) for M in (4, 1024))
+
+
+def test_ddc_and_resampler_spot_values():
+    d, r = kv.ddc_predict, kv.resamp_predict
+    assert d(128, 8, 16) == "ddc_kernel<1, 1, 8>" and d(128, 9, 16) == "ddc_kernel<4, 2, 32>"
+    assert d(4096, 2048, 1024) == "ddc_kernel<4, 2, 32>" and d(1, 1, 1) == "ddc_kernel<1, 1, 8>"
+    assert d(4097, 8, 16) == d(128, 2049, 16) == d(128, 8, 1025) == d(0, 8, 16) == kv.UNSUPPORTED
+    assert r(3000, 125, 128, 8) == "resamp_kernel<1, 1, 1, 2048>" and r(3000, 125, 128, 9) == "resamp_kernel<32, 2, 4, 64>"
+    assert r(64, 1, 1, 16384) == "resamp_kernel<32, 2, 4, 64>" and r(65, 1, 1, 1) == kv.UNSUPPORTED    # P = 65
+    assert r(16384, 256, 1, 1) == "resamp_kernel<1, 1, 1, 2048>" and r(16385, 1024, 1, 1) == kv.UNSUPPORTED
+    assert r(8, 1025, 1, 1) == r(8, 1, 1025, 1) == r(8, 1, 1, 16385) == r(0, 1, 1, 1) == kv.UNSUPPORTED
 
 
 def test_fir_spot_values():
