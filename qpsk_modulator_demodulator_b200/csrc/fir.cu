@@ -5,22 +5,29 @@
 // y[i] = conv(x,h)[i+N-1].  Both are the same correlation  y[n0+q] = sum_i g[i] * xs[q+i]  over a
 // shared-memory tile xs (tile + halo), with g[i] = h[HL-i]; only the tile origin differs.
 //
-// fir_tma_kernel (the hot kernel)
-//   * persistent CTAs (2 per SM), each walking tiles  blockIdx.x + k*gridDim.x  of T = NT*R samples;
-//   * input tile + halo staged by TMA bulk copies (cp.async.bulk -> SASS UBLKCP) into a 2-4 deep
-//     mbarrier ring, so loads for the next tiles are in flight while the current one is computed;
+// The tile ring (TileRing, ring_produce): five kernels — fir_tma_kernel, fir_split2_kernel, fir_dec2_kernel,
+// fir_exact_real_kernel, fir_decim_tma_kernel — share one pipeline and differ only in their consumer arithmetic:
+//   * persistent CTAs, each walking tiles  blockIdx.x + k*gridDim.x  of a channel-major tile grid;
+//   * one producer warp stages input tile + halo by TMA bulk copies (cp.async.bulk -> SASS UBLKCP) into a 2-4 deep
+//     full/empty mbarrier ring, so loads for the next tiles are in flight while the current one is computed;
+//   * the four that store per warp stage each consumer warp's outputs in shared memory and write them back with one
+//     bulk store per warp and tile (warp_store).
+// On the host, plan_ring sizes the ring from a shared-memory budget and launch_ring starts the persistent grid.
+//
+// fir_tma_kernel (the hot kernel): tiles of T = NT*R samples, 2 CTAs per SM;
 //   * each thread owns R consecutive outputs and slides a register window over the tile: one
 //     LDS.128 (two new samples) feeds 2*R packed FFMA2 (fma.rn.f32x2: I and Q of one sample in one
 //     issue slot, the real tap broadcast from a uniform register);
 //   * R = 10 -> thread stride 80 B = 5 x 16 B chunks, odd, so the LDS.128/STS.128 of a quarter-warp
-//     hit 8 distinct 16-byte bank groups: conflict-free on a dense (TMA-compatible) layout;
-//   * results staged in shared memory and written back with one TMA bulk store per tile.
+//     hit 8 distinct 16-byte bank groups: conflict-free on a dense (TMA-compatible) layout.
 //   Algorithmic traffic: 8 B read + 8 B written per complex sample; 4*N flop (real taps) or
 //   8*N flop (complex taps) per sample.
 //
 // fir_generic_kernel: one thread per output straight from global memory.  Serves QPSK_FIR_EXACT
 // (the reference's 8-lane summation order, no FMA: FIRFilter.cs:165-192), unaligned device
 // pointers, and tap counts beyond the parameter-space table.
+#include <algorithm>
+
 #include "fir.cuh"
 
 namespace qpsk {
@@ -95,7 +102,7 @@ struct FirArgs {
   int E_load;       // samples staged per tile (even)
   int stage_elems;  // float2 slots per stage (even)
   int stages;
-  long long n_out;  // fir_dec2_kernel: decimated outputs per channel
+  long long n_out;  // outputs per channel (L for the full-rate kernels), counted in tiles by launch_ring
 };
 struct TapsReal {
   float g[kMaxG];
@@ -178,10 +185,148 @@ struct TileWalk {
   }
 };
 
-// NT compute threads (NT/32 consumer warps) + one producer warp.  No CTA-wide barrier in the steady
-// state: the input ring is handed over with full/empty mbarriers, and every consumer warp stages
-// and TMA-stores its own 32*R outputs, so warps drift apart and their prologues/epilogues overlap the
-// other warps' FFMA2 streams.
+// ---------------------------------------------------------------------------------------------
+// The tile ring shared by the five TMA-pipelined kernels
+// ---------------------------------------------------------------------------------------------
+// A CTA is NW consumer warps and one producer warp.  The producer stages each tile's input (tile + halo) into the next of
+// `stages` shared-memory slots by bulk copies and signals the slot's `full` mbarrier; each consumer warp waits on it, reads
+// the slot and arrives on its `empty` mbarrier, which the producer waits on before it refills the slot.  No CTA-wide
+// barrier in the steady state, so warps drift apart and one warp's prologue / epilogue overlaps the others' arithmetic.
+// Dynamic shared memory: the slots, then the kernel's own region (output staging, ...), then 2 * stages mbarriers.
+
+// A position in the ring: the slot and the phase parity its mbarriers are at
+struct RingCursor {
+  int stage = 0;
+  uint32_t parity = 0;
+  __device__ __forceinline__ void next(int stages) {
+    if (++stage == stages) {
+      stage = 0;
+      parity ^= 1u;
+    }
+  }
+};
+
+struct TileRing {
+  // stages and stage_elems are read from the kernel parameters where they are used: copies held in registers across the
+  // consumer loop cost up to six registers in fir_tma_kernel
+  const FirArgs* a;
+  float2* slots;     // a->stages x a->stage_elems samples
+  uint64_t* full;    // [stages] the slot's copies have landed (one producer arrival + the bytes)
+  uint64_t* empty;   // [stages] every consumer warp is done with the slot
+
+  __device__ __forceinline__ float2* slot(int stage) const { return slots + (size_t)stage * a->stage_elems; }
+  // the kernel's own region, right after the slots
+  __device__ __forceinline__ float2* region() const { return slot(a->stages); }
+
+  // consumer warp: the samples of the cursor's slot, once they have landed
+  __device__ __forceinline__ const float2* acquire(const RingCursor& c) const {
+    mbar_wait(&full[c.stage], c.parity);
+    return slot(c.stage);
+  }
+  // consumer warp: done reading the slot — hand it back to the producer, move the cursor on
+  __device__ __forceinline__ void release(RingCursor& c, int lane) const {
+    __syncwarp();
+    if (lane == 0) mbar_arrive(&empty[c.stage]);
+    c.next(a->stages);
+  }
+};
+
+// Every thread of the CTA calls this: the ring over `smem` with a kernel region of `region_elems` float2, its mbarriers
+// initialised (`empty` counts one arrival per consumer warp) and visible to the whole CTA.
+__device__ __forceinline__ TileRing ring_init(unsigned char* smem, const FirArgs& a, int region_elems, int consumer_warps) {
+  TileRing r;
+  r.a = &a;
+  r.slots = reinterpret_cast<float2*>(smem);
+  r.full = reinterpret_cast<uint64_t*>(r.region() + region_elems);   // float2 granules: 8-byte aligned as mbarriers need
+  r.empty = r.full + a.stages;
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < a.stages; ++s) {
+      mbar_init(&r.full[s], 1);
+      mbar_init(&r.empty[s], consumer_warps);
+    }
+    fence_mbar_init();
+  }
+  __syncthreads();
+  return r;
+}
+
+// The producer warp's loop.  Tile k of a channel covers stream indices s0 .. s0 + E_load, s0 = advance + k*T_IN - HL
+// (even): T_IN input samples per tile, HL delay-line samples in front of the first.  The part before the stream start
+// comes from hist_in by a bulk copy (zeros when hist_in is null: a stateless call), the in-range part by a bulk copy of an
+// even count plus one plain load for an odd one, and plain zero stores fill what lies past the stream end.
+template <int T_IN>
+__device__ __forceinline__ void ring_produce(const FirArgs& a, const TileRing& ring) {
+  const int lane = threadIdx.x & 31;
+  RingCursor c;
+  TileWalk w(a.tiles_per_ch);
+  for (int it = 0; w.tile < a.total_tiles; ++it, w.next()) {
+    if (it >= a.stages) mbar_wait(&ring.empty[c.stage], c.parity ^ 1u);   // consumers released this slot
+    const int ch = w.ch;
+    const long long s0 = (long long)a.advance + (long long)w.k * T_IN - a.HL;
+    float2* dst = ring.slot(c.stage);
+    const float2* xch = a.x + (long long)ch * a.ldx;
+    uint64_t* bar = &ring.full[c.stage];
+    const int E = a.E_load;
+    uint32_t tx = 0;
+    int nA = 0;
+    if (s0 < 0) {
+      nA = (int)((-s0) < (long long)E ? (-s0) : (long long)E);
+      if (a.hist_in) {
+        if (lane == 0) bulk_g2s(dst, a.hist_in + (long long)ch * a.HL + (a.HL + s0), (uint32_t)nA * 8u, bar);
+        tx += (uint32_t)nA * 8u;
+      } else {
+        for (int i = lane; i < nA; i += 32) dst[i] = make_float2(0.f, 0.f);
+      }
+    }
+    const long long m0 = s0 + nA;
+    long long avail = a.L - m0;
+    if (avail < 0) avail = 0;
+    const int nB = (int)(avail < (long long)(E - nA) ? avail : (long long)(E - nA));
+    const int nB2 = nB & ~1;
+    if (nB2 > 0) {
+      if (lane == 0) bulk_g2s(dst + nA, xch + m0, (uint32_t)nB2 * 8u, bar);
+      tx += (uint32_t)nB2 * 8u;
+    }
+    if ((nB & 1) && lane == 0) dst[nA + nB2] = xch[m0 + nB2];
+    for (int i = nA + nB + lane; i < E; i += 32) dst[i] = make_float2(0.f, 0.f);
+    __syncwarp();
+    if (lane == 0) mbar_arrive_expect_tx(bar, tx);
+    c.next(a.stages);
+  }
+}
+
+// Delay-line carry of a kernel that filters at the full rate: the last tile of a channel (first output n0) holds the
+// stream's final HL samples, which the next call reads as hist_in.
+template <int NT>
+__device__ __forceinline__ void carry_history(const FirArgs& a, const float2* xs, int ch, int k, long long n0) {
+  if (a.hist_out && k == a.tiles_per_ch - 1) {
+    const int off = (int)(a.L - n0);
+    float2* ho = a.hist_out + (long long)ch * a.HL;
+    for (int i = threadIdx.x; i < a.HL; i += NT) ho[i] = xs[off + i];
+  }
+}
+
+// A consumer warp's store of the WS outputs it staged at ys: the first `left` (clamped to 0..WS) go to yg by one bulk
+// store, or by lane-strided stores when their count is odd (a bulk copy moves a multiple of 16 bytes).  Either way the
+// warp commits one bulk group per tile, which the caller's bulk_wait_read<> before it next writes ys counts.
+template <int WS>
+__device__ __forceinline__ void warp_store(float2* yg, const float2* ys, int left, int lane) {
+  fence_proxy_async_smem();
+  __syncwarp();
+  const int n = left < 0 ? 0 : (left > WS ? WS : left);
+  if ((n & 1) == 0) {
+    if (lane == 0) {
+      if (n > 0) bulk_s2g(yg, ys, (uint32_t)n * 8u);
+      bulk_commit();
+    }
+  } else {
+    for (int i = lane; i < n; i += 32) yg[i] = ys[i];
+    if (lane == 0) bulk_commit();
+  }
+}
+
+// fir_tma_kernel: NT compute threads on the tile ring, R consecutive outputs each; every consumer warp stages its 32*R
+// outputs in one of two shared-memory buffers and bulk-stores them.
 template <int R, int NT, bool CPLX>
 __global__ void __launch_bounds__(NT + 32, 2)
     fir_tma_kernel(const __grid_constant__ FirArgs a, const __grid_constant__ typename TapsOf<CPLX>::type taps) {
@@ -191,95 +336,26 @@ __global__ void __launch_bounds__(NT + 32, 2)
   constexpr int WS = 32 * R; // outputs per consumer warp and tile
   constexpr int NW = NT / 32;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  float2* xs_base = reinterpret_cast<float2*>(smem_raw);
-  float2* ys_base = xs_base + (size_t)a.stages * a.stage_elems;
-  uint64_t* full = reinterpret_cast<uint64_t*>(ys_base + 2 * T);
-  uint64_t* empty = full + a.stages;
+  const TileRing ring = ring_init(smem_raw, a, 2 * T, NW);
 
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int warp = tid >> 5;
-
-  if (tid == 0) {
-    for (int s = 0; s < a.stages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], NW);
-    }
-    fence_mbar_init();
-  }
-  __syncthreads();
-
   if (warp == NW) {
-    // ---------------- producer warp: stages tile + halo into the ring ----------------
-    // TMA bulk copies for the in-range part, plain zero stores for what lies before the stream start
-    // (stateless) or past its end.
-    int stage = 0;
-    uint32_t parity = 0;
-    TileWalk w(a.tiles_per_ch);
-    for (int it = 0; w.tile < a.total_tiles; ++it, w.next()) {
-      if (it >= a.stages) mbar_wait(&empty[stage], parity ^ 1u);   // consumers released this slot
-      const int ch = w.ch;
-      const int k = w.k;
-      const long long n0 = (long long)k * T;
-      const long long s0 = n0 + a.advance - a.HL;  // stream index of xs[0] (even)
-      float2* dst = xs_base + (size_t)stage * a.stage_elems;
-      const float2* xch = a.x + (long long)ch * a.ldx;
-      uint64_t* bar = &full[stage];
-      const int E = a.E_load;
-      uint32_t tx = 0;
-      int nA = 0;
-      if (s0 < 0) {
-        nA = (int)((-s0) < (long long)E ? (-s0) : (long long)E);
-        if (a.hist_in) {
-          if (lane == 0) bulk_g2s(dst, a.hist_in + (long long)ch * a.HL + (a.HL + s0), (uint32_t)nA * 8u, bar);
-          tx += (uint32_t)nA * 8u;
-        } else {
-          for (int i = lane; i < nA; i += 32) dst[i] = make_float2(0.f, 0.f);
-        }
-      }
-      const long long m0 = s0 + nA;
-      long long avail = a.L - m0;
-      if (avail < 0) avail = 0;
-      const int nB = (int)(avail < (long long)(E - nA) ? avail : (long long)(E - nA));
-      const int nB2 = nB & ~1;
-      if (nB2 > 0) {
-        if (lane == 0) bulk_g2s(dst + nA, xch + m0, (uint32_t)nB2 * 8u, bar);
-        tx += (uint32_t)nB2 * 8u;
-      }
-      if ((nB & 1) && lane == 0) dst[nA + nB2] = xch[m0 + nB2];
-      for (int i = nA + nB + lane; i < E; i += 32) dst[i] = make_float2(0.f, 0.f);
-      __syncwarp();
-      if (lane == 0) mbar_arrive_expect_tx(bar, tx);
-      if (++stage == a.stages) {
-        stage = 0;
-        parity ^= 1u;
-      }
-    }
+    ring_produce<T>(a, ring);
     return;
   }
 
   // ---------------- consumer warps ----------------
   const int base = tid * R;
-  float2* ys_warp = ys_base + (size_t)warp * (2 * WS);   // two buffers of WS outputs
-  int stage = 0;
-  uint32_t parity = 0;
+  float2* ys_warp = ring.region() + (size_t)warp * (2 * WS);   // two buffers of WS outputs
+  RingCursor cur;
   TileWalk tw(a.tiles_per_ch);
   for (int it = 0; tw.tile < a.total_tiles; ++it, tw.next()) {
-    mbar_wait(&full[stage], parity);
-    const float2* xs = xs_base + (size_t)stage * a.stage_elems;
-
+    const float2* xs = ring.acquire(cur);
     const int ch = tw.ch;
-    const int k = tw.k;
-    const long long n0 = (long long)k * T;
-    const long long left = a.L - n0;
-    const int valid = (int)(left < (long long)T ? left : (long long)T);
-
-    // delay-line carry: the last tile of a channel holds the stream's final HL samples
-    if (a.hist_out && k == a.tiles_per_ch - 1) {
-      const int off = (int)(a.L - n0);
-      float2* ho = a.hist_out + (long long)ch * a.HL;
-      for (int i = tid; i < a.HL; i += NT) ho[i] = xs[off + i];
-    }
+    const long long n0 = (long long)tw.k * T;
+    carry_history<NT>(a, xs, ch, tw.k, n0);
 
     // ---- register-tiled correlation ----
     float2 w[W];
@@ -309,9 +385,7 @@ __global__ void __launch_bounds__(NT + 32, 2)
         default: break;
       }
     }
-    // this warp is done reading the input slot
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&empty[stage]);
+    ring.release(cur, lane);
 
     // ---- epilogue: registers -> this warp's smem slice -> TMA bulk store ----
     float2* ys = ys_warp + (size_t)(it & 1) * WS;
@@ -331,24 +405,9 @@ __global__ void __launch_bounds__(NT + 32, 2)
       }
       yv[r >> 1] = make_float4(o0.x, o0.y, o1.x, o1.y);
     }
-    fence_proxy_async_smem();
-    __syncwarp();
-    int wvalid = valid - warp * WS;
-    wvalid = wvalid < 0 ? 0 : (wvalid > WS ? WS : wvalid);
-    float2* yg = a.y + (long long)ch * a.ldy + n0 + (long long)warp * WS;
-    if ((wvalid & 1) == 0) {
-      if (lane == 0) {
-        if (wvalid > 0) bulk_s2g(yg, ys, (uint32_t)wvalid * 8u);
-        bulk_commit();
-      }
-    } else {
-      for (int i = lane; i < wvalid; i += 32) yg[i] = ys[i];
-      if (lane == 0) bulk_commit();
-    }
-    if (++stage == a.stages) {
-      stage = 0;
-      parity ^= 1u;
-    }
+    const long long left = a.L - n0;
+    const int valid = (int)(left < (long long)T ? left : (long long)T);
+    warp_store<WS>(a.y + (long long)ch * a.ldy + n0 + (long long)warp * WS, ys, valid - warp * WS, lane);
   }
   if (lane == 0) bulk_wait<0>();
 }
@@ -425,97 +484,31 @@ __global__ void __launch_bounds__(NT + 32, 2)
   constexpr int W = P + 2;
   constexpr int WS = 32 * R;   // outputs per consumer warp and tile
   constexpr int NW = NT / 32;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  float2* xs_base = reinterpret_cast<float2*>(smem_raw);
-  float2* ys_base = xs_base + (size_t)a.stages * a.stage_elems;     // one buffer of WS outputs per warp
   const int spw = (WS + a.G) / 2 + 1;                                 // S values per warp (odd or even: 8-byte accesses only)
-  float2* sp_base = ys_base + T;
-  uint64_t* full = reinterpret_cast<uint64_t*>(sp_base + (size_t)NW * spw);   // float2 slots: 8-byte aligned as mbarriers need
-  uint64_t* empty = full + a.stages;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  const TileRing ring = ring_init(smem_raw, a, T + NW * spw, NW);    // region: one buffer of WS outputs per warp, S planes
 
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int warp = tid >> 5;
-
-  if (tid == 0) {
-    for (int s = 0; s < a.stages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], NW);
-    }
-    fence_mbar_init();
-  }
-  __syncthreads();
-
   if (warp == NW) {
-    // ---------------- producer warp: the FMA kernel's staging ----------------
-    int stage = 0;
-    uint32_t parity = 0;
-    TileWalk w(a.tiles_per_ch);
-    for (int it = 0; w.tile < a.total_tiles; ++it, w.next()) {
-      if (it >= a.stages) mbar_wait(&empty[stage], parity ^ 1u);
-      const int ch = w.ch;
-      const long long n0 = (long long)w.k * T;
-      const long long s0 = n0 + a.advance - a.HL;
-      float2* dst = xs_base + (size_t)stage * a.stage_elems;
-      const float2* xch = a.x + (long long)ch * a.ldx;
-      uint64_t* bar = &full[stage];
-      const int E = a.E_load;
-      uint32_t tx = 0;
-      int nA = 0;
-      if (s0 < 0) {
-        nA = (int)((-s0) < (long long)E ? (-s0) : (long long)E);
-        if (a.hist_in) {
-          if (lane == 0) bulk_g2s(dst, a.hist_in + (long long)ch * a.HL + (a.HL + s0), (uint32_t)nA * 8u, bar);
-          tx += (uint32_t)nA * 8u;
-        } else {
-          for (int i = lane; i < nA; i += 32) dst[i] = make_float2(0.f, 0.f);
-        }
-      }
-      const long long m0 = s0 + nA;
-      long long avail = a.L - m0;
-      if (avail < 0) avail = 0;
-      const int nB = (int)(avail < (long long)(E - nA) ? avail : (long long)(E - nA));
-      const int nB2 = nB & ~1;
-      if (nB2 > 0) {
-        if (lane == 0) bulk_g2s(dst + nA, xch + m0, (uint32_t)nB2 * 8u, bar);
-        tx += (uint32_t)nB2 * 8u;
-      }
-      if ((nB & 1) && lane == 0) dst[nA + nB2] = xch[m0 + nB2];
-      for (int i = nA + nB + lane; i < E; i += 32) dst[i] = make_float2(0.f, 0.f);
-      __syncwarp();
-      if (lane == 0) mbar_arrive_expect_tx(bar, tx);
-      if (++stage == a.stages) {
-        stage = 0;
-        parity ^= 1u;
-      }
-    }
+    ring_produce<T>(a, ring);
     return;
   }
 
   // ---------------- consumer warps ----------------
   const int base = tid * R;
   const int wbase = warp * WS;
-  float2* ys = ys_base + (size_t)warp * WS;
-  float2* sp = sp_base + (size_t)warp * spw;
+  float2* ys = ring.region() + (size_t)warp * WS;
+  float2* sp = ring.region() + T + (size_t)warp * spw;
   const int Gh = a.G >> 1;
-  int stage = 0;
-  uint32_t parity = 0;
+  RingCursor cur;
   TileWalk tw(a.tiles_per_ch);
-  for (int it = 0; tw.tile < a.total_tiles; ++it, tw.next()) {
-    mbar_wait(&full[stage], parity);
-    const float2* xs = xs_base + (size_t)stage * a.stage_elems;
-
+  for (; tw.tile < a.total_tiles; tw.next()) {
+    const float2* xs = ring.acquire(cur);
     const int ch = tw.ch;
-    const int k = tw.k;
-    const long long n0 = (long long)k * T;
-    const long long left = a.L - n0;
-    const int valid = (int)(left < (long long)T ? left : (long long)T);
-
-    if (a.hist_out && k == a.tiles_per_ch - 1) {
-      const int off = (int)(a.L - n0);
-      float2* ho = a.hist_out + (long long)ch * a.HL;
-      for (int i = tid; i < a.HL; i += NT) ho[i] = xs[off + i];
-    }
+    const long long n0 = (long long)tw.k * T;
+    carry_history<NT>(a, xs, ch, tw.k, n0);
 
     // ---- this warp's S plane: S[q] = xs[wbase + 2q + 1] + xs[wbase + 2q + 2] ----
     {
@@ -569,8 +562,7 @@ __global__ void __launch_bounds__(NT + 32, 2)
       default: break;
     }
     // this warp is done reading the input slot and its S plane
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&empty[stage]);
+    ring.release(cur, lane);
 
     // ---- epilogue: recombine, registers -> this warp's smem slice -> TMA bulk store ----
     if (lane == 0) bulk_wait_read<0>();   // the previous tile's store has drained the slice
@@ -582,24 +574,9 @@ __global__ void __launch_bounds__(NT + 32, 2)
       const float2 yo = fir_sub2(fir_sub2(C[m], A[m + 1]), B[m]);
       yv[m] = make_float4(ye.x, ye.y, yo.x, yo.y);
     }
-    fence_proxy_async_smem();
-    __syncwarp();
-    int wvalid = valid - wbase;
-    wvalid = wvalid < 0 ? 0 : (wvalid > WS ? WS : wvalid);
-    float2* yg = a.y + (long long)ch * a.ldy + n0 + (long long)wbase;
-    if ((wvalid & 1) == 0) {
-      if (lane == 0) {
-        if (wvalid > 0) bulk_s2g(yg, ys, (uint32_t)wvalid * 8u);
-        bulk_commit();
-      }
-    } else {
-      for (int i = lane; i < wvalid; i += 32) yg[i] = ys[i];
-      if (lane == 0) bulk_commit();
-    }
-    if (++stage == a.stages) {
-      stage = 0;
-      parity ^= 1u;
-    }
+    const long long left = a.L - n0;
+    const int valid = (int)(left < (long long)T ? left : (long long)T);
+    warp_store<WS>(a.y + (long long)ch * a.ldy + n0 + (long long)wbase, ys, valid - wbase, lane);
   }
   if (lane == 0) bulk_wait<0>();
 }
@@ -610,8 +587,7 @@ __global__ void __launch_bounds__(NT + 32, 2)
 // The even outputs of the split above need neither C nor S: y[b+2m] = (H0*X0)[m] + (H1*X1)[m] is the polyphase decimator
 // itself, G/2 multiply-adds per input sample = the algorithmic count.  With D = 2 the thread stride on a DENSE tile is
 // 8R bytes, an odd multiple of 16 for R = 10 / 14 — so, unlike D >= 4 (fir_decim_kernel's padded layout, filled through
-// registers), the tile can arrive by TMA: producer warp, full/empty mbarrier ring and per-warp bulk store exactly as in
-// fir_tma_kernel.  A kept-output phase of 1 (dec_skip) is a leading zero tap (host side), so the tile grid stays on even
+// registers), the tile can arrive on the tile ring read in place, with the per-warp bulk store.  A kept-output phase of 1 (dec_skip) is a leading zero tap (host side), so the tile grid stays on even
 // sample indices.  Windows: two circular windows of P + 1 slots (P = R/2 outputs per thread), P + 1 sub-taps per unrolled
 // block; one LDS.128 (X0 and X1 of one position) per sub-tap feeds 2P FFMA2.  Measured, 2^28 samples, ms at 33 / 65 / 129 taps:
 // (R, NT) = (14, 256) with two output buffers per warp (two ring stages) 0.492 0.773 1.368 | one output buffer (three stages)
@@ -645,80 +621,26 @@ __global__ void __launch_bounds__(NT + 32, 2)
   constexpr int WSO = 32 * P;     // outputs per consumer warp and tile
   constexpr int NW = NT / 32;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  float2* xs_base = reinterpret_cast<float2*>(smem_raw);
-  float2* ys_base = xs_base + (size_t)a.stages * a.stage_elems;     // two buffers of WSO outputs per warp
-  uint64_t* full = reinterpret_cast<uint64_t*>(ys_base + 2 * TO);
-  uint64_t* empty = full + a.stages;
+  const TileRing ring = ring_init(smem_raw, a, 2 * TO, NW);        // region: two buffers of WSO outputs per warp
 
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int warp = tid >> 5;
-
-  if (tid == 0) {
-    for (int s = 0; s < a.stages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], NW);
-    }
-    fence_mbar_init();
-  }
-  __syncthreads();
-
   if (warp == NW) {
-    // ---------------- producer warp: the FMA kernel's staging ----------------
-    int stage = 0;
-    uint32_t parity = 0;
-    TileWalk w(a.tiles_per_ch);
-    for (int it = 0; w.tile < a.total_tiles; ++it, w.next()) {
-      if (it >= a.stages) mbar_wait(&empty[stage], parity ^ 1u);
-      const int ch = w.ch;
-      const long long n0 = (long long)w.k * T;
-      const long long s0 = n0 - a.HL;
-      float2* dst = xs_base + (size_t)stage * a.stage_elems;
-      const float2* xch = a.x + (long long)ch * a.ldx;
-      uint64_t* bar = &full[stage];
-      const int E = a.E_load;
-      uint32_t tx = 0;
-      int nA = 0;
-      if (s0 < 0) {
-        nA = (int)((-s0) < (long long)E ? (-s0) : (long long)E);
-        if (lane == 0) bulk_g2s(dst, a.hist_in + (long long)ch * a.HL + (a.HL + s0), (uint32_t)nA * 8u, bar);
-        tx += (uint32_t)nA * 8u;
-      }
-      const long long m0 = s0 + nA;
-      long long avail = a.L - m0;
-      if (avail < 0) avail = 0;
-      const int nB = (int)(avail < (long long)(E - nA) ? avail : (long long)(E - nA));
-      const int nB2 = nB & ~1;
-      if (nB2 > 0) {
-        if (lane == 0) bulk_g2s(dst + nA, xch + m0, (uint32_t)nB2 * 8u, bar);
-        tx += (uint32_t)nB2 * 8u;
-      }
-      if ((nB & 1) && lane == 0) dst[nA + nB2] = xch[m0 + nB2];
-      for (int i = nA + nB + lane; i < E; i += 32) dst[i] = make_float2(0.f, 0.f);
-      __syncwarp();
-      if (lane == 0) mbar_arrive_expect_tx(bar, tx);
-      if (++stage == a.stages) {
-        stage = 0;
-        parity ^= 1u;
-      }
-    }
+    ring_produce<T>(a, ring);
     return;
   }
 
   // ---------------- consumer warps ----------------
   const int base = tid * R;
-  float2* ys_warp = ys_base + (size_t)warp * (2 * WSO);
+  float2* ys_warp = ring.region() + (size_t)warp * (2 * WSO);
   const int Gh = a.G >> 1;
-  int stage = 0;
-  uint32_t parity = 0;
+  RingCursor cur;
   TileWalk tw(a.tiles_per_ch);
   for (int it = 0; tw.tile < a.total_tiles; ++it, tw.next()) {
-    mbar_wait(&full[stage], parity);
-    const float2* xs = xs_base + (size_t)stage * a.stage_elems;
+    const float2* xs = ring.acquire(cur);
     const int ch = tw.ch;
     const long long o0 = (long long)tw.k * TO;               // first output of the tile
-    const long long left = a.n_out - o0;
-    const int valid = (int)(left < (long long)TO ? left : (long long)TO);
 
     float2 wa[W], wb[W], A[P], B[P];
 #pragma unroll
@@ -741,8 +663,7 @@ __global__ void __launch_bounds__(NT + 32, 2)
 #undef QPSK_TAILD
       default: break;
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&empty[stage]);
+    ring.release(cur, lane);
 
     // ---- epilogue: y = A + B -> this warp's smem slice -> TMA bulk store ----
     float2* ys = ys_warp + (size_t)(it & 1) * WSO;
@@ -750,24 +671,9 @@ __global__ void __launch_bounds__(NT + 32, 2)
     __syncwarp();
 #pragma unroll
     for (int m = 0; m < P; ++m) ys[lane * P + m] = fir_add2(A[m], B[m]);
-    fence_proxy_async_smem();
-    __syncwarp();
-    int wvalid = valid - warp * WSO;
-    wvalid = wvalid < 0 ? 0 : (wvalid > WSO ? WSO : wvalid);
-    float2* yg = a.y + (long long)ch * a.ldy + o0 + (long long)warp * WSO;
-    if ((wvalid & 1) == 0) {
-      if (lane == 0) {
-        if (wvalid > 0) bulk_s2g(yg, ys, (uint32_t)wvalid * 8u);
-        bulk_commit();
-      }
-    } else {
-      for (int i = lane; i < wvalid; i += 32) yg[i] = ys[i];
-      if (lane == 0) bulk_commit();
-    }
-    if (++stage == a.stages) {
-      stage = 0;
-      parity ^= 1u;
-    }
+    const long long left = a.n_out - o0;
+    const int valid = (int)(left < (long long)TO ? left : (long long)TO);
+    warp_store<WSO>(a.y + (long long)ch * a.ldy + o0 + (long long)warp * WSO, ys, valid - warp * WSO, lane);
   }
   if (lane == 0) bulk_wait<0>();
 }
@@ -784,8 +690,7 @@ __global__ void __launch_bounds__(NT + 32, 2)
 // output (one mul.rn.f32x2 and two add.rn.f32) instead of eight scalar ones — about half the speed of the FMA kernel, against a
 // fourteenth for the one-thread-per-output kernel below.
 // Thread = 2 consecutive outputs (16-byte stride: conflict-free LDS/STS), 8 lane partials each, 8 taps per block with
-// a 9-sample register window; the tile pipeline (producer warp, full/empty mbarriers, per-warp TMA store) is the FMA
-// kernel's.
+// a 9-sample register window, on the tile ring with the per-warp bulk store.
 __device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
   float2 d;
   asm("mul.rn.f32x2 %0, %1, %2;"
@@ -822,65 +727,12 @@ __global__ void __launch_bounds__(NT + 32, 3)
   constexpr int WS = 32 * R;   // outputs per consumer warp and tile
   constexpr int NW = NT / 32;
   extern __shared__ __align__(128) unsigned char smem_raw[];
-  float2* xs_base = reinterpret_cast<float2*>(smem_raw);
-  float2* ys_base = xs_base + (size_t)a.stages * a.stage_elems;
-  uint64_t* full = reinterpret_cast<uint64_t*>(ys_base + 2 * T);
-  uint64_t* empty = full + a.stages;
+  const TileRing ring = ring_init(smem_raw, a, 2 * T, NW);         // region: two buffers of WS outputs per warp
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int warp = tid >> 5;
-  if (tid == 0) {
-    for (int s = 0; s < a.stages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], NW);
-    }
-    fence_mbar_init();
-  }
-  __syncthreads();
-
   if (warp == NW) {
-    // producer warp: the FMA kernel's staging (tile + halo by TMA bulk copies, zeros outside the stream)
-    int stage = 0;
-    uint32_t parity = 0;
-    TileWalk w(a.tiles_per_ch);
-    for (int it = 0; w.tile < a.total_tiles; ++it, w.next()) {
-      if (it >= a.stages) mbar_wait(&empty[stage], parity ^ 1u);
-      const int ch = w.ch;
-      const long long n0 = (long long)w.k * T;
-      const long long s0 = n0 + a.advance - a.HL;
-      float2* dst = xs_base + (size_t)stage * a.stage_elems;
-      const float2* xch = a.x + (long long)ch * a.ldx;
-      uint64_t* bar = &full[stage];
-      const int E = a.E_load;
-      uint32_t tx = 0;
-      int nA = 0;
-      if (s0 < 0) {
-        nA = (int)((-s0) < (long long)E ? (-s0) : (long long)E);
-        if (a.hist_in) {
-          if (lane == 0) bulk_g2s(dst, a.hist_in + (long long)ch * a.HL + (a.HL + s0), (uint32_t)nA * 8u, bar);
-          tx += (uint32_t)nA * 8u;
-        } else {
-          for (int i = lane; i < nA; i += 32) dst[i] = make_float2(0.f, 0.f);
-        }
-      }
-      const long long m0 = s0 + nA;
-      long long avail = a.L - m0;
-      if (avail < 0) avail = 0;
-      const int nB = (int)(avail < (long long)(E - nA) ? avail : (long long)(E - nA));
-      const int nB2 = nB & ~1;
-      if (nB2 > 0) {
-        if (lane == 0) bulk_g2s(dst + nA, xch + m0, (uint32_t)nB2 * 8u, bar);
-        tx += (uint32_t)nB2 * 8u;
-      }
-      if ((nB & 1) && lane == 0) dst[nA + nB2] = xch[m0 + nB2];
-      for (int i = nA + nB + lane; i < E; i += 32) dst[i] = make_float2(0.f, 0.f);
-      __syncwarp();
-      if (lane == 0) mbar_arrive_expect_tx(bar, tx);
-      if (++stage == a.stages) {
-        stage = 0;
-        parity ^= 1u;
-      }
-    }
+    ring_produce<T>(a, ring);
     return;
   }
 
@@ -890,22 +742,14 @@ __global__ void __launch_bounds__(NT + 32, 3)
   const int lead = a.HL - (n_taps - 1);      // 0 or 1: xs index of window element 0 relative to the output index
   const int n_vec = n_taps & ~7;
   const int base = tid * R;
-  float2* ys_warp = ys_base + (size_t)warp * (2 * WS);
-  int stage = 0;
-  uint32_t parity = 0;
+  float2* ys_warp = ring.region() + (size_t)warp * (2 * WS);
+  RingCursor cur;
   TileWalk tw(a.tiles_per_ch);
   for (int it = 0; tw.tile < a.total_tiles; ++it, tw.next()) {
-    mbar_wait(&full[stage], parity);
-    const float2* xs = xs_base + (size_t)stage * a.stage_elems;
+    const float2* xs = ring.acquire(cur);
     const int ch = tw.ch;
     const long long n0 = (long long)tw.k * T;
-    const long long left = a.L - n0;
-    const int valid = (int)(left < (long long)T ? left : (long long)T);
-    if (a.hist_out && tw.k == a.tiles_per_ch - 1) {
-      const int off = (int)(a.L - n0);
-      float2* ho = a.hist_out + (long long)ch * a.HL;
-      for (int i = tid; i < a.HL; i += NT) ho[i] = xs[off + i];
-    }
+    carry_history<NT>(a, xs, ch, tw.k, n0);
     float2 lp[R][8];
 #pragma unroll
     for (int r = 0; r < R; ++r)
@@ -968,31 +812,15 @@ __global__ void __launch_bounds__(NT + 32, 3)
         acc[r] = make_float2(aI, aQ);
       }
     }
-    __syncwarp();
-    if (lane == 0) mbar_arrive(&empty[stage]);
+    ring.release(cur, lane);
 
     float2* ys = ys_warp + (size_t)(it & 1) * WS;
     if (lane == 0) bulk_wait_read<1>();
     __syncwarp();
     *reinterpret_cast<float4*>(ys + lane * R) = make_float4(acc[0].x, acc[0].y, acc[1].x, acc[1].y);
-    fence_proxy_async_smem();
-    __syncwarp();
-    int wvalid = valid - warp * WS;
-    wvalid = wvalid < 0 ? 0 : (wvalid > WS ? WS : wvalid);
-    float2* yg = a.y + (long long)ch * a.ldy + n0 + (long long)warp * WS;
-    if ((wvalid & 1) == 0) {
-      if (lane == 0) {
-        if (wvalid > 0) bulk_s2g(yg, ys, (uint32_t)wvalid * 8u);
-        bulk_commit();
-      }
-    } else {
-      for (int i = lane; i < wvalid; i += 32) yg[i] = ys[i];
-      if (lane == 0) bulk_commit();
-    }
-    if (++stage == a.stages) {
-      stage = 0;
-      parity ^= 1u;
-    }
+    const long long left = a.L - n0;
+    const int valid = (int)(left < (long long)T ? left : (long long)T);
+    warp_store<WS>(a.y + (long long)ch * a.ldy + n0 + (long long)warp * WS, ys, valid - warp * WS, lane);
   }
   if (lane == 0) bulk_wait<0>();
 }
@@ -1263,9 +1091,9 @@ __global__ void __launch_bounds__(NTO * NG, 4)
   }
 }
 
-// fir_decim_kernel's arithmetic on the TMA pipeline, D = 4, 8, 16: one producer warp stages the DENSE tile (+ halo) by bulk
-// copies into a full/empty mbarrier ring, so the loads of tile t+1 are in flight under the arithmetic of tile t (the
-// register-staged kernel alternates the two inside a CTA and leans on four resident CTAs).  Read in place, a dense tile costs
+// fir_decim_kernel's arithmetic on the tile ring, D = 4, 8, 16: the DENSE tile (+ halo) arrives by bulk copies, so the
+// loads of tile t+1 are in flight under the arithmetic of tile t (the register-staged kernel alternates the two inside a
+// CTA and leans on four resident CTAs).  The groups' partial sums leave through its own epilogue, not warp_store.  Read in place, a dense tile costs
 // 2- / 4- / 8-way bank conflicts on every LDS.128 for D = 4 / 8 / 16 (thread span 56*D bytes = 14 / 28 / 56 sixteen-byte chunks;
 // measured: 0.56 / 0.87 / 1.64 ms against 0.68 / 0.65 / 0.62 for the padded register-staged kernel) — so the compute threads
 // first move the tile into the PADDED layout of fir_decim_kernel (one LDS.128 + STS.128 per sample pair, both conflict-free),
@@ -1288,73 +1116,25 @@ __global__ void __launch_bounds__(NTO * NG + 32, 2)
   constexpr int PP = DEC / 2 / NG;
   constexpr int PADS = 2;
   constexpr int PITCH = SPAN + PADS;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  float2* xs_base = reinterpret_cast<float2*>(smem_raw);
-  float2* ys = xs_base + (size_t)a.stages * a.stage_elems;            // [NG][T_OUT] partial sums
-  float2* xpad = ys + NG * T_OUT;                                     // REPACK: the tile in the padded layout
   const int pad_elems = REPACK ? ((a.E_load + PADS * (a.E_load / SPAN + 1) + 1) & ~1) : 0;
-  uint64_t* full = reinterpret_cast<uint64_t*>(xpad + pad_elems);
-  uint64_t* empty = full + a.stages;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  const TileRing ring = ring_init(smem_raw, a, NG * T_OUT + pad_elems, NW);
+  float2* ys = ring.region();                                         // [NG][T_OUT] partial sums
+  float2* xpad = ys + NG * T_OUT;                                     // REPACK: the tile in the padded layout
   const int tid = threadIdx.x;
   const int lane = tid & 31;
   const int warp = tid >> 5;
   const int K = a.G;                                                  // polyphase taps per phase
-  if (tid == 0) {
-    for (int s = 0; s < a.stages; ++s) {
-      mbar_init(&full[s], 1);
-      mbar_init(&empty[s], NW);
-    }
-    fence_mbar_init();
-  }
-  __syncthreads();
-
   if (warp == NW) {
-    int stage = 0;
-    uint32_t parity = 0;
-    TileWalk w(a.tiles_per_ch);
-    for (int it = 0; w.tile < a.total_tiles; ++it, w.next()) {
-      if (it >= a.stages) mbar_wait(&empty[stage], parity ^ 1u);
-      const int ch = w.ch;
-      const long long s0 = (long long)a.advance + (long long)w.k * T_IN - a.HL;   // advance = the even part of the kept-output phase
-      float2* dst = xs_base + (size_t)stage * a.stage_elems;
-      const float2* xch = a.x + (long long)ch * a.ldx;
-      uint64_t* bar = &full[stage];
-      const int E = a.E_load;
-      uint32_t tx = 0;
-      int nA = 0;
-      if (s0 < 0) {
-        nA = (int)((-s0) < (long long)E ? (-s0) : (long long)E);
-        if (lane == 0) bulk_g2s(dst, a.hist_in + (long long)ch * a.HL + (a.HL + s0), (uint32_t)nA * 8u, bar);
-        tx += (uint32_t)nA * 8u;
-      }
-      const long long m0 = s0 + nA;
-      long long avail = a.L - m0;
-      if (avail < 0) avail = 0;
-      const int nB = (int)(avail < (long long)(E - nA) ? avail : (long long)(E - nA));
-      const int nB2 = nB & ~1;
-      if (nB2 > 0) {
-        if (lane == 0) bulk_g2s(dst + nA, xch + m0, (uint32_t)nB2 * 8u, bar);
-        tx += (uint32_t)nB2 * 8u;
-      }
-      if ((nB & 1) && lane == 0) dst[nA + nB2] = xch[m0 + nB2];
-      for (int i = nA + nB + lane; i < E; i += 32) dst[i] = make_float2(0.f, 0.f);
-      __syncwarp();
-      if (lane == 0) mbar_arrive_expect_tx(bar, tx);
-      if (++stage == a.stages) {
-        stage = 0;
-        parity ^= 1u;
-      }
-    }
+    ring_produce<T_IN>(a, ring);                                      // advance = the even part of the kept-output phase
     return;
   }
 
   const int to = tid % NTO, grp = tid / NTO;
-  int stage = 0;
-  uint32_t parity = 0;
+  RingCursor cur;
   TileWalk tw(a.tiles_per_ch);
-  for (int it = 0; tw.tile < a.total_tiles; ++it, tw.next()) {
-    mbar_wait(&full[stage], parity);
-    const float2* xs = xs_base + (size_t)stage * a.stage_elems;
+  for (; tw.tile < a.total_tiles; tw.next()) {
+    const float2* xs = ring.acquire(cur);
     const int ch = tw.ch;
     const long long m0 = (long long)tw.k * T_OUT;
     // dense ring slot -> padded layout (a pair never straddles a pad: spans are an even number of samples)
@@ -1374,8 +1154,7 @@ __global__ void __launch_bounds__(NTO * NG + 32, 2)
           if (p < np) *reinterpret_cast<float4*>(xpad + 2 * p + PADS * ((2 * p) / SPAN)) = v4[u];
         }
       }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&empty[stage]);                      // the ring slot goes back before the arithmetic starts
+      ring.release(cur, lane);                                        // the ring slot goes back before the arithmetic starts
       named_bar_sync(1, NT);
     }
     constexpr int PD = REPACK ? PADS : 0;                             // pad slots per span in the layout the loops read
@@ -1406,10 +1185,7 @@ __global__ void __launch_bounds__(NTO * NG + 32, 2)
         default: break;
       }
     }
-    if constexpr (!REPACK) {
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&empty[stage]);                      // this warp is done with the ring slot
-    }
+    if constexpr (!REPACK) ring.release(cur, lane);                   // this warp is done with the ring slot
     float2* yp = ys + grp * T_OUT + to * RO;
 #pragma unroll
     for (int r = 0; r < RO; ++r) yp[r] = acc[r];
@@ -1427,10 +1203,6 @@ __global__ void __launch_bounds__(NTO * NG + 32, 2)
       yc[o] = sum;
     }
     named_bar_sync(1, NT);                                            // the partial sums and the padded tile are dead
-    if (++stage == a.stages) {
-      stage = 0;
-      parity ^= 1u;
-    }
   }
 }
 
@@ -1527,19 +1299,6 @@ constexpr int kSmemBudget = 112 * 1024;  // per CTA, two CTAs per SM
 // warps (kNTWide) are ahead for real-tap filters of ~48-96 taps (65 taps: 1.29 against 1.32 ms), eight everywhere else.
 inline bool fir_wide(int G, bool cplx) { return !cplx && G >= 48 && G <= 96; }
 
-template <int R, int NT, bool CPLX>
-int launch_tma(const FirArgs& a, const typename TapsOf<CPLX>::type& taps, size_t smem, int grid, cudaStream_t s) {
-  auto kern = fir_tma_kernel<R, NT, CPLX>;
-  QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
-  kern<<<grid, NT + 32, smem, s>>>(a, taps);
-  QPSK_LAUNCH_CHECK();
-  return QPSK_OK;
-}
-inline const char* tma_kernel_name(bool cplx, int G) {
-  if (cplx) return "fir_tma_kernel<R=10,NT=256,complex taps>";
-  return fir_wide(G, false) ? "fir_tma_kernel<R=10,NT=320,real taps>" : "fir_tma_kernel<R=10,NT=256,real taps>";
-}
-
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 // fir_split2_kernel geometry and the tap count from which QPSK_FIR_FAST uses it for real taps
@@ -1550,30 +1309,47 @@ constexpr int kS2R = 10, kS2NT = 256;
 constexpr int kS2MinForced = 14;        // QPSK_FIR_SPLIT: at least one full block of seven sub-taps
 constexpr int kS2MinFast = 48;
 inline bool fir_mode_is_fast(int mode) { return mode != QPSK_FIR_EXACT; }
-// a: stream, delay-line and tap geometry filled in; tile geometry and the launch happen here
-template <int R2, int NT2>
-int launch_split2(FirArgs a, const TapsSplit& t, int channels, cudaStream_t s, const char** name) {
-  constexpr int T2 = R2 * NT2, NW2 = NT2 / 32, WS2 = 32 * R2;
-  if (a.HL > T2) return QPSK_ERR_UNSUPPORTED;
-  a.tiles_per_ch = (int)((a.L + T2 - 1) / T2);
-  a.total_tiles = (long long)a.tiles_per_ch * channels;
-  a.E_load = T2 + a.G;
+
+// fir_exact_real_kernel geometry: two outputs per thread, three CTAs per SM in 72 KiB each
+constexpr int kENT = 256, kET = 2 * kENT;
+constexpr int kExactSmemBudget = 72 * 1024;
+
+// The correlation taps of a delay line of hl samples: g[i + shift] = h[hl - i] for 0 <= i <= hl (zero where hl - i >= N),
+// zero elsewhere; im = 0 / 1 takes the real / imaginary parts of h.  shift = 1 is one leading zero tap: a decimator's odd
+// kept-output phase, so that its tiles stay on even sample indices.
+void corr_taps(float (&g)[kMaxG], const std::vector<float>& taps_iq, int hl, int shift = 0, int im = 0) {
+  std::fill(g, g + kMaxG, 0.0f);
+  const int N = (int)(taps_iq.size() / 2);
+  for (int i = 0; i <= hl; ++i)
+    if (hl - i < N) g[i + shift] = taps_iq[2 * (hl - i) + im];
+}
+
+// The ring of a kernel whose tiles stage `span` input samples plus a `halo`, next to the kernel's own `fixed` bytes of
+// shared memory (ring_init's region): as many stages as `budget` holds, at most four.  Fewer than two (no tile's loads
+// in flight under another's arithmetic) does not fit.  Fills a's ring fields; returns the dynamic shared-memory size, or 0
+// when the ring does not fit.
+size_t plan_ring(FirArgs& a, int span, int halo, size_t fixed, size_t budget) {
+  a.E_load = span + halo;
   a.stage_elems = a.E_load + 2;
   const size_t stage_bytes = (size_t)a.stage_elems * 8;
-  const int spw = (WS2 + a.G) / 2 + 1;
-  const size_t fixed = (size_t)T2 * 8 + (size_t)NW2 * spw * 8;
-  if (fixed + 128 + 2 * stage_bytes > (size_t)kSmemBudget) return QPSK_ERR_UNSUPPORTED;
-  int stages = (int)(((size_t)kSmemBudget - fixed - 128) / stage_bytes);
-  if (stages > 4) stages = 4;
-  a.stages = stages;
-  const size_t smem = (size_t)stages * stage_bytes + fixed + (size_t)stages * 16;
-  long long grid = 2LL * device_sm_count();
+  if (fixed + 128 + 2 * stage_bytes > budget) return 0;
+  a.stages = (int)std::min<size_t>(4, (budget - fixed - 128) / stage_bytes);
+  return (size_t)a.stages * stage_bytes + fixed + (size_t)a.stages * 16;
+}
+
+// Launches a ring kernel over tiles of `tile_out` of the a.n_out outputs per channel: a persistent grid of `per_sm` CTAs
+// per SM, never more CTAs than tiles.  On success `last_kernel` names it.
+template <typename Kern, typename... Taps>
+int launch_ring(Kern kern, const char* name, int threads, int per_sm, int tile_out, size_t smem, FirArgs a, int channels,
+                cudaStream_t s, const char*& last_kernel, const Taps&... taps) {
+  a.tiles_per_ch = (int)((a.n_out + tile_out - 1) / tile_out);
+  a.total_tiles = (long long)a.tiles_per_ch * channels;
+  long long grid = (long long)per_sm * device_sm_count();
   if (grid > a.total_tiles) grid = a.total_tiles;
-  auto kern = fir_split2_kernel<R2, NT2>;
   QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
-  kern<<<(int)grid, NT2 + 32, smem, s>>>(a, t);
+  kern<<<(int)grid, threads, smem, s>>>(a, taps...);
   QPSK_LAUNCH_CHECK();
-  *name = "fir_split2_kernel<R=10,NT=256,real taps>";
+  last_kernel = name;
   return QPSK_OK;
 }
 
@@ -1589,148 +1365,90 @@ int FirEngine::run(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t l
   const int advance = stateless ? (N - 1) : 0;
   const int hl = stateless ? (N - 1) : HL;
   const int G = (hl + 1 + 1) & ~1;
+  // the kernels read hist[cur] and leave the updated delay line in hist[cur^1]
+  const float2* hin = stateless ? nullptr : hist[cur].p;
+  float2* hout = stateless ? nullptr : hist[cur ^ 1].p;
+  // bulk copies need 16-byte aligned rows
+  const bool rows_ok = aligned16(x) && aligned16(y) && !(channels > 1 && ((ldx & 1) || (ldy & 1)));
+  FirArgs a = {};
+  a.x = x; a.y = y; a.ldx = ldx; a.ldy = ldy; a.L = L; a.n_out = L;
+  a.hist_in = hin; a.hist_out = hout;
+  a.HL = hl; a.G = G; a.advance = advance;
 
   const bool wide = fir_wide(G, !real_taps);
   const int T = kR * (wide ? kNTWide : kNT);
-  bool use_tma = (fir_mode_is_fast(mode) || stateless) && G <= kMaxG && hl <= T;
-  if (use_tma) {
-    if (!aligned16(x) || !aligned16(y)) use_tma = false;
-    if (channels > 1 && ((ldx & 1) || (ldy & 1))) use_tma = false;
-  }
-  if (!stateless) {
-    // the kernels read hist[cur] and leave the updated delay line in hist[cur^1]
-  }
-  const float2* hin = stateless ? nullptr : hist[cur].p;
-  float2* hout = stateless ? nullptr : hist[cur ^ 1].p;
-
+  const bool use_tma = (fir_mode_is_fast(mode) || stateless) && G <= kMaxG && hl <= T && rows_ok;
   const bool want_split = (mode == QPSK_FIR_SPLIT && G >= kS2MinForced) ||
                           (mode == QPSK_FIR_FAST && G >= kS2MinFast);
-  if (use_tma && real_taps && want_split) {
-    FirArgs a;
-    a.x = x; a.y = y; a.ldx = ldx; a.ldy = ldy; a.L = L;
-    a.hist_in = hin; a.hist_out = hout;
-    a.HL = hl; a.G = G; a.advance = advance;
-    TapsSplit t;
-    memset(&t, 0, sizeof t);
-    for (int i = 0; i <= hl; ++i) {
-      const int j = hl - i;
-      const float g = (j < N) ? taps_iq[2 * j] : 0.0f;
-      ((i & 1) ? t.h1 : t.h0)[i >> 1] = g;
-    }
-    for (int j = 0; j < G / 2; ++j) t.h2[j] = t.h0[j] + t.h1[j];
-    const char* name = nullptr;
-    const int st = launch_split2<kS2R, kS2NT>(a, t, channels, s, &name);
-    if (st != QPSK_ERR_UNSUPPORTED) {              // UNSUPPORTED: the ring does not fit, the FMA kernel takes the call
-      QPSK_TRY(st);
-      last_kernel = name;
-      if (!stateless) cur ^= 1;
-      return QPSK_OK;
+  int st = QPSK_ERR_UNSUPPORTED;   // UNSUPPORTED: no kernel launched yet, the next one in line takes the call
+  constexpr int T2 = kS2R * kS2NT;
+  if (use_tma && real_taps && want_split && hl <= T2) {
+    const size_t fixed = (size_t)T2 * 8 + (size_t)(kS2NT / 32) * ((32 * kS2R + G) / 2 + 1) * 8;   // outputs, S planes
+    if (const size_t smem = plan_ring(a, T2, G, fixed, kSmemBudget)) {
+      TapsReal g;
+      corr_taps(g.g, taps_iq, hl);
+      TapsSplit t;
+      for (int j = 0; j < kMaxGh; ++j) {
+        t.h0[j] = g.g[2 * j];
+        t.h1[j] = g.g[2 * j + 1];
+        t.h2[j] = t.h0[j] + t.h1[j];
+      }
+      st = launch_ring(fir_split2_kernel<kS2R, kS2NT>, "fir_split2_kernel<R=10,NT=256,real taps>", kS2NT + 32, 2, T2, smem,
+                       a, channels, s, last_kernel, t);
     }
   }
-
-  if (use_tma) {
-    FirArgs a;
-    a.x = x; a.y = y; a.ldx = ldx; a.ldy = ldy; a.L = L;
-    a.hist_in = hin; a.hist_out = hout;
-    a.tiles_per_ch = (int)((L + T - 1) / T);
-    a.total_tiles = (long long)a.tiles_per_ch * channels;
-    a.HL = hl; a.G = G; a.advance = advance;
-    a.E_load = T + G;
-    a.stage_elems = a.E_load + 2;
-    const size_t stage_bytes = (size_t)a.stage_elems * 8;
-    const size_t out_bytes = (size_t)2 * T * 8;
-    int stages = (int)((kSmemBudget - out_bytes - 128) / stage_bytes);
-    if (stages > 4) stages = 4;
-    if (stages >= 2) {
-      a.stages = stages;
-      const size_t smem = (size_t)stages * stage_bytes + out_bytes + (size_t)stages * 16;
-      long long grid = 2LL * device_sm_count();
-      if (grid > a.total_tiles) grid = a.total_tiles;
-      if (real_taps) {
-        TapsReal t;
-        memset(&t, 0, sizeof t);
-        for (int i = 0; i <= hl; ++i) {
-          const int j = hl - i;
-          t.g[i] = (j < N) ? taps_iq[2 * j] : 0.0f;
-        }
-        if (wide) QPSK_TRY((launch_tma<kR, kNTWide, false>(a, t, smem, (int)grid, s)));
-        else QPSK_TRY((launch_tma<kR, kNT, false>(a, t, smem, (int)grid, s)));
-      } else {
+  if (st == QPSK_ERR_UNSUPPORTED && use_tma) {
+    if (const size_t smem = plan_ring(a, T, G, (size_t)2 * T * 8, kSmemBudget)) {
+      if (!real_taps) {
         TapsCplx t;
-        memset(&t, 0, sizeof t);
-        for (int i = 0; i <= hl; ++i) {
-          const int j = hl - i;
-          t.gi[i] = (j < N) ? taps_iq[2 * j] : 0.0f;
-          t.gq[i] = (j < N) ? taps_iq[2 * j + 1] : 0.0f;
-        }
-        QPSK_TRY((launch_tma<kR, kNT, true>(a, t, smem, (int)grid, s)));
-      }
-      last_kernel = tma_kernel_name(!real_taps, G);
-      if (!stateless) cur ^= 1;
-      return QPSK_OK;
-    }
-  }
-
-  // QPSK_FIR_EXACT with real taps: the reference's summation order on the TMA pipeline (fir_exact_real_kernel)
-  if (mode == QPSK_FIR_EXACT && !stateless && real_taps && N >= 8 && aligned16(x) && aligned16(y) &&
-      !(channels > 1 && ((ldx & 1) || (ldy & 1)))) {
-    constexpr int kENT = 256, kET = 2 * kENT;
-    const int GE = (HL + 1 + 1) & ~1;
-    if (GE <= kMaxG && HL <= kET) {
-      FirArgs a;
-      a.x = x; a.y = y; a.ldx = ldx; a.ldy = ldy; a.L = L;
-      a.hist_in = hin; a.hist_out = hout;
-      a.tiles_per_ch = (int)((L + kET - 1) / kET);
-      a.total_tiles = (long long)a.tiles_per_ch * channels;
-      a.HL = HL; a.G = GE; a.advance = 0;
-      a.E_load = kET + GE;
-      a.stage_elems = a.E_load + 2;
-      const size_t stage_bytes = (size_t)a.stage_elems * 8;
-      const size_t out_bytes = (size_t)2 * kET * 8;
-      int stages = (int)((72 * 1024 - out_bytes - 128) / stage_bytes);
-      if (stages > 4) stages = 4;
-      if (stages >= 2) {
-        a.stages = stages;
-        const size_t smem = (size_t)stages * stage_bytes + out_bytes + (size_t)stages * 16;
-        long long grid = 3LL * device_sm_count();
-        if (grid > a.total_tiles) grid = a.total_tiles;
+        corr_taps(t.gi, taps_iq, hl, 0, 0);
+        corr_taps(t.gq, taps_iq, hl, 0, 1);
+        st = launch_ring(fir_tma_kernel<kR, kNT, true>, "fir_tma_kernel<R=10,NT=256,complex taps>", kNT + 32, 2, T, smem, a,
+                         channels, s, last_kernel, t);
+      } else {
         TapsReal t;
-        memset(&t, 0, sizeof t);
-        for (int i = 0; i <= HL; ++i) {
-          const int j = HL - i;
-          t.g[i] = (j < N) ? taps_iq[2 * j] : 0.0f;
-        }
-        auto kern = fir_exact_real_kernel<kENT>;
-        QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
-        kern<<<(int)grid, kENT + 32, smem, s>>>(a, t, N);
-        QPSK_LAUNCH_CHECK();
-        last_kernel = "fir_exact_real_kernel<NT=256>";
-        cur ^= 1;
-        return QPSK_OK;
+        corr_taps(t.g, taps_iq, hl);
+        st = wide ? launch_ring(fir_tma_kernel<kR, kNTWide, false>, "fir_tma_kernel<R=10,NT=320,real taps>", kNTWide + 32, 2,
+                                T, smem, a, channels, s, last_kernel, t)
+                  : launch_ring(fir_tma_kernel<kR, kNT, false>, "fir_tma_kernel<R=10,NT=256,real taps>", kNT + 32, 2, T, smem,
+                                a, channels, s, last_kernel, t);
       }
     }
   }
-
-  GenArgs g;
-  g.x = x; g.y = y; g.ldx = ldx; g.ldy = ldy; g.L = L;
-  g.hist_in = hin; g.hI = d_taps.p; g.hQ = d_taps.p + N;
-  g.C = channels; g.N = N; g.HL = HL; g.advance = advance;
-  const long long total = (long long)channels * L;
-  long long blocks = (total + 255) / 256;
-  const long long cap = 32LL * device_sm_count();
-  if (blocks > cap) blocks = cap;
-  if (mode == QPSK_FIR_EXACT && !stateless)
-    fir_generic_kernel<true><<<(int)blocks, 256, 0, s>>>(g);
-  else
-    fir_generic_kernel<false><<<(int)blocks, 256, 0, s>>>(g);
-  QPSK_LAUNCH_CHECK();
-  last_kernel = (mode == QPSK_FIR_EXACT && !stateless) ? "fir_generic_kernel<EXACT>" : "fir_generic_kernel";
-  if (!stateless) {
-    const int tot = channels * HL;
-    fir_hist_update_kernel<<<(tot + 255) / 256, 256, 0, s>>>(x, ldx, L, hin, hout, channels, HL);
-    QPSK_LAUNCH_CHECK();
-    cur ^= 1;
+  // QPSK_FIR_EXACT with real taps: the reference's summation order on the tile ring (streaming: hl = HL, advance = 0)
+  if (st == QPSK_ERR_UNSUPPORTED && mode == QPSK_FIR_EXACT && !stateless && real_taps && N >= 8 && rows_ok && G <= kMaxG &&
+      HL <= kET) {
+    if (const size_t smem = plan_ring(a, kET, G, (size_t)2 * kET * 8, kExactSmemBudget)) {
+      TapsReal t;
+      corr_taps(t.g, taps_iq, HL);
+      st = launch_ring(fir_exact_real_kernel<kENT>, "fir_exact_real_kernel<NT=256>", kENT + 32, 3, kET, smem, a, channels, s,
+                       last_kernel, t, N);
+    }
   }
+  if (st == QPSK_ERR_UNSUPPORTED) {
+    GenArgs g;
+    g.x = x; g.y = y; g.ldx = ldx; g.ldy = ldy; g.L = L;
+    g.hist_in = hin; g.hI = d_taps.p; g.hQ = d_taps.p + N;
+    g.C = channels; g.N = N; g.HL = HL; g.advance = advance;
+    const long long total = (long long)channels * L;
+    long long blocks = (total + 255) / 256;
+    const long long cap = 32LL * device_sm_count();
+    if (blocks > cap) blocks = cap;
+    if (mode == QPSK_FIR_EXACT && !stateless)
+      fir_generic_kernel<true><<<(int)blocks, 256, 0, s>>>(g);
+    else
+      fir_generic_kernel<false><<<(int)blocks, 256, 0, s>>>(g);
+    QPSK_LAUNCH_CHECK();
+    last_kernel = (mode == QPSK_FIR_EXACT && !stateless) ? "fir_generic_kernel<EXACT>" : "fir_generic_kernel";
+    if (!stateless) {
+      const int tot = channels * HL;
+      fir_hist_update_kernel<<<(tot + 255) / 256, 256, 0, s>>>(x, ldx, L, hin, hout, channels, HL);
+      QPSK_LAUNCH_CHECK();
+    }
+  } else {
+    QPSK_TRY(st);
+  }
+  if (!stateless) cur ^= 1;
   return QPSK_OK;
 }
 
@@ -1751,109 +1469,45 @@ int FirEngine::decimate_dev(const float2* x, int64_t L, int64_t ldx, int dec, fl
   QPSK_TRY(ensure_device(device));
   if (!s) s = stream;
   const int64_t skip = dec_skip;
-  const int N = n_taps;
   int K = (HL + 1 + dec - 1) / dec;
   const bool fast = fir_mode_is_fast(mode) && real_taps && (dec == 2 || dec == 4 || dec == 8 || dec == 16) &&
                     (long long)K * dec <= kMaxG && nout > 0;
-  bool launched = false;
+  int st = QPSK_ERR_UNSUPPORTED;   // UNSUPPORTED: no kernel launched yet, the next one in line takes the call
   if (fast) {
-    DecArgs a;
-    a.x = x; a.y = y; a.ldx = ldx; a.ldy = ldy; a.L = L;
-    a.hist_in = hist[cur].p; a.n_out = nout; a.HL = HL; a.skip = (int)skip; a.K = K; a.tiles_per_ch = 0; a.total_tiles = 0;
-    TapsReal t;
-    memset(&t, 0, sizeof t);
-    for (int i = 0; i <= HL; ++i) {
-      const int j = HL - i;
-      t.g[i] = (j < N) ? taps_iq[2 * j] : 0.0f;
-    }
-    auto go = [&](auto kern, int NTO, int NG, int PADS) -> int {
-      const int T_OUT = 7 * NTO, SPAN = 7 * dec;
-      a.tiles_per_ch = (int)((nout + T_OUT - 1) / T_OUT);
-      a.total_tiles = (long long)a.tiles_per_ch * channels;
-      const int E = (T_OUT + K) * dec;
-      const size_t smem = (size_t)(NG * T_OUT + E + PADS * (E / SPAN + 1)) * sizeof(float2);
-      if (smem > 200 * 1024) return QPSK_ERR_UNSUPPORTED;
-      QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
-      long long per_sm = (long long)(224 * 1024) / (long long)(smem + 1024);
-      if (per_sm > 4) per_sm = 4;
-      if (per_sm < 1) per_sm = 1;
-      long long grid = per_sm * device_sm_count();
-      if (grid > a.total_tiles) grid = a.total_tiles;
-      kern<<<(int)grid, NTO * NG, smem, s>>>(a, t);
-      QPSK_LAUNCH_CHECK();
-      return QPSK_OK;
-    };
-    int st = QPSK_ERR_UNSUPPORTED;
-    // D = 2 on the TMA pipeline (fir_dec2_kernel) when the pointers allow bulk copies
-    if (dec == 2 && aligned16(x) && aligned16(y) && !(channels > 1 && ((ldx & 1) || (ldy & 1)))) {
+    const bool x_ok = aligned16(x) && !(channels > 1 && (ldx & 1));
+    const bool y_ok = aligned16(y) && !(channels > 1 && (ldy & 1));
+    // the ring kernels: an odd kept-output phase is a leading zero tap (sk), the even part of it the ring's advance, so
+    // that the tiles stay on even sample indices
+    const int sk = (int)(skip & 1);
+    FirArgs fa = {};
+    fa.x = x; fa.y = y; fa.ldx = ldx; fa.ldy = ldy; fa.L = L; fa.n_out = nout;
+    fa.hist_in = hist[cur].p; fa.hist_out = nullptr;
+    fa.HL = HL; fa.advance = (int)(skip & ~1LL);
+    if (dec == 2 && x_ok && y_ok) {
+      // D = 2: fir_dec2_kernel
       constexpr int R2 = 14, NT2 = 256, T2 = R2 * NT2, TO2 = T2 / 2;
-      const int Gs = (HL + 1 + (int)skip + 1) & ~1;
-      if (Gs <= kMaxG && HL <= T2) {
-        FirArgs fa;
-        fa.x = x; fa.y = y; fa.ldx = ldx; fa.ldy = ldy; fa.L = L;
-        fa.hist_in = hist[cur].p; fa.hist_out = nullptr;
-        fa.n_out = nout;
-        fa.tiles_per_ch = (int)((nout + TO2 - 1) / TO2);
-        fa.total_tiles = (long long)fa.tiles_per_ch * channels;
-        fa.HL = HL; fa.G = Gs; fa.advance = 0;
-        fa.E_load = T2 + Gs;
-        fa.stage_elems = fa.E_load + 2;
-        const size_t stage_bytes = (size_t)fa.stage_elems * 8;
-        const size_t out_bytes = (size_t)2 * TO2 * 8;
-        int stages = (int)((kSmemBudget - out_bytes - 128) / stage_bytes);
-        if (stages > 4) stages = 4;
-        if (stages >= 2) {
-          fa.stages = stages;
-          const size_t smem = (size_t)stages * stage_bytes + out_bytes + (size_t)stages * 16;
-          TapsReal ts;                                        // a kept-output phase of 1 = one leading zero tap
-          memset(&ts, 0, sizeof ts);
-          for (int i = 0; i <= HL; ++i) ts.g[i + (int)skip] = t.g[i];
-          long long grid = 2LL * device_sm_count();
-          if (grid > fa.total_tiles) grid = fa.total_tiles;
-          auto kern = fir_dec2_kernel<R2, NT2>;
-          QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
-          kern<<<(int)grid, NT2 + 32, smem, s>>>(fa, ts);
-          QPSK_LAUNCH_CHECK();
-          last_kernel = "fir_dec2_kernel<R=14,NT=256,D=2>";
-          st = QPSK_OK;
+      fa.G = (HL + 1 + sk + 1) & ~1;
+      if (fa.G <= kMaxG && HL <= T2) {
+        if (const size_t smem = plan_ring(fa, T2, fa.G, (size_t)2 * TO2 * 8, kSmemBudget)) {
+          TapsReal t;
+          corr_taps(t.g, taps_iq, HL, sk);
+          st = launch_ring(fir_dec2_kernel<R2, NT2>, "fir_dec2_kernel<R=14,NT=256,D=2>", NT2 + 32, 2, TO2, smem, fa, channels,
+                           s, last_kernel, t);
         }
       }
-    }
-    // D = 4, 8, 16 on the same pipeline (fir_decim_tma_kernel, dense tiles)
-    if (dec > 2 && aligned16(x) && !(channels > 1 && (ldx & 1))) {
-      const int sk = (int)(skip & 1);
-      const int Ks = (HL + 1 + sk + dec - 1) / dec;
+    } else if (dec > 2 && x_ok) {
+      // D = 4, 8, 16: fir_decim_tma_kernel on dense tiles
+      fa.G = (HL + 1 + sk + dec - 1) / dec;          // polyphase taps per phase
       auto go_tma = [&](auto kern, int NTO, int NG, bool repack, const char* name) -> int {
-        const int T_OUT = 7 * NTO;
-        if ((long long)Ks * dec > kMaxG) return QPSK_ERR_UNSUPPORTED;
-        FirArgs fa;
-        fa.x = x; fa.y = y; fa.ldx = ldx; fa.ldy = ldy; fa.L = L;
-        fa.hist_in = hist[cur].p; fa.hist_out = nullptr;
-        fa.n_out = nout;
-        fa.tiles_per_ch = (int)((nout + T_OUT - 1) / T_OUT);
-        fa.total_tiles = (long long)fa.tiles_per_ch * channels;
-        fa.HL = HL; fa.G = Ks; fa.advance = (int)(skip & ~1LL);
-        fa.E_load = (T_OUT + Ks) * dec;
-        fa.stage_elems = fa.E_load + 2;
-        const size_t stage_bytes = (size_t)fa.stage_elems * 8;
-        const int span = 7 * dec;
-        const size_t pad_elems = repack ? (size_t)((fa.E_load + 2 * (fa.E_load / span + 1) + 1) & ~1) : 0;
-        const size_t fixed = (size_t)NG * T_OUT * 8 + pad_elems * 8;
-        if (fixed + 128 + 2 * stage_bytes > (size_t)kSmemBudget) return QPSK_ERR_UNSUPPORTED;
-        int stages = (int)(((size_t)kSmemBudget - fixed - 128) / stage_bytes);
-        if (stages > 4) stages = 4;
-        fa.stages = stages;
-        const size_t smem = (size_t)stages * stage_bytes + fixed + (size_t)stages * 16;
-        TapsReal ts;
-        memset(&ts, 0, sizeof ts);
-        for (int i = 0; i <= HL; ++i) ts.g[i + sk] = t.g[i];
-        long long grid = 2LL * device_sm_count();
-        if (grid > fa.total_tiles) grid = fa.total_tiles;
-        QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
-        kern<<<(int)grid, NTO * NG + 32, smem, s>>>(fa, ts);
-        QPSK_LAUNCH_CHECK();
-        last_kernel = name;
-        return QPSK_OK;
+        const int T_OUT = 7 * NTO, T_IN = T_OUT * dec, halo = fa.G * dec;
+        if (halo > kMaxG) return QPSK_ERR_UNSUPPORTED;
+        const int E = T_IN + halo;
+        const size_t pad_elems = repack ? (size_t)((E + 2 * (E / (7 * dec) + 1) + 1) & ~1) : 0;
+        const size_t smem = plan_ring(fa, T_IN, halo, (size_t)NG * T_OUT * 8 + pad_elems * 8, kSmemBudget);
+        if (!smem) return QPSK_ERR_UNSUPPORTED;
+        TapsReal t;
+        corr_taps(t.g, taps_iq, HL, sk);
+        return launch_ring(kern, name, NTO * NG + 32, 2, T_OUT, smem, fa, channels, s, last_kernel, t);
       };
       switch (dec) {
         // D = 4 reads the dense tile in place (2-way conflicts cost less than the repack and its barrier: 0.558 against
@@ -1862,18 +1516,42 @@ int FirEngine::decimate_dev(const float2* x, int64_t L, int64_t ldx, int dec, fl
         case 8: st = go_tma(fir_decim_tma_kernel<7, 64, 4, 8, true>, 64, 4, true, "fir_decim_tma_kernel<RO=7,NTO=64,NG=4,D=8,repack>"); break;
         case 16: st = go_tma(fir_decim_tma_kernel<7, 32, 8, 16, true>, 32, 8, true, "fir_decim_tma_kernel<RO=7,NTO=32,NG=8,D=16,repack>"); break;
       }
-      if (st != QPSK_OK && st != QPSK_ERR_UNSUPPORTED) return st;
     }
-    if (st != QPSK_OK) switch (dec) {
-      case 2: st = go(fir_decim_kernel<7, 256, 1, 2>, 256, 1, 0); last_kernel = "fir_decim_kernel<RO=7,NTO=256,NG=1,D=2>"; break;
-      case 4: st = go(fir_decim_kernel<7, 128, 2, 4>, 128, 2, 2); last_kernel = "fir_decim_kernel<RO=7,NTO=128,NG=2,D=4>"; break;
-      case 8: st = go(fir_decim_kernel<7, 64, 4, 8>, 64, 4, 2); last_kernel = "fir_decim_kernel<RO=7,NTO=64,NG=4,D=8>"; break;
-      case 16: st = go(fir_decim_kernel<7, 32, 8, 16>, 32, 8, 2); last_kernel = "fir_decim_kernel<RO=7,NTO=32,NG=8,D=16>"; break;
+    if (st == QPSK_ERR_UNSUPPORTED) {
+      // the register-staged kernel (fir_decim_kernel): any alignment
+      DecArgs a;
+      a.x = x; a.y = y; a.ldx = ldx; a.ldy = ldy; a.L = L;
+      a.hist_in = hist[cur].p; a.n_out = nout; a.HL = HL; a.skip = (int)skip; a.K = K; a.tiles_per_ch = 0; a.total_tiles = 0;
+      TapsReal t;
+      corr_taps(t.g, taps_iq, HL);
+      auto go = [&](auto kern, int NTO, int NG, int PADS, const char* name) -> int {
+        const int T_OUT = 7 * NTO, SPAN = 7 * dec;
+        a.tiles_per_ch = (int)((nout + T_OUT - 1) / T_OUT);
+        a.total_tiles = (long long)a.tiles_per_ch * channels;
+        const int E = (T_OUT + K) * dec;
+        const size_t smem = (size_t)(NG * T_OUT + E + PADS * (E / SPAN + 1)) * sizeof(float2);
+        if (smem > 200 * 1024) return QPSK_ERR_UNSUPPORTED;
+        QPSK_TRY(allow_max_dynamic_smem((const void*)kern));
+        long long per_sm = (long long)(224 * 1024) / (long long)(smem + 1024);
+        if (per_sm > 4) per_sm = 4;
+        if (per_sm < 1) per_sm = 1;
+        long long grid = per_sm * device_sm_count();
+        if (grid > a.total_tiles) grid = a.total_tiles;
+        kern<<<(int)grid, NTO * NG, smem, s>>>(a, t);
+        QPSK_LAUNCH_CHECK();
+        last_kernel = name;
+        return QPSK_OK;
+      };
+      switch (dec) {
+        case 2: st = go(fir_decim_kernel<7, 256, 1, 2>, 256, 1, 0, "fir_decim_kernel<RO=7,NTO=256,NG=1,D=2>"); break;
+        case 4: st = go(fir_decim_kernel<7, 128, 2, 4>, 128, 2, 2, "fir_decim_kernel<RO=7,NTO=128,NG=2,D=4>"); break;
+        case 8: st = go(fir_decim_kernel<7, 64, 4, 8>, 64, 4, 2, "fir_decim_kernel<RO=7,NTO=64,NG=4,D=8>"); break;
+        case 16: st = go(fir_decim_kernel<7, 32, 8, 16>, 32, 8, 2, "fir_decim_kernel<RO=7,NTO=32,NG=8,D=16>"); break;
+      }
     }
-    if (st == QPSK_OK) launched = true;
-    else if (st != QPSK_ERR_UNSUPPORTED) return st;
+    if (st != QPSK_OK && st != QPSK_ERR_UNSUPPORTED) return st;
   }
-  if (launched) {
+  if (st == QPSK_OK) {
     // the delay line advances exactly as Filter() would advance it
     const int tot = channels * HL;
     fir_hist_update_kernel<<<(tot + 255) / 256, 256, 0, s>>>(x, ldx, L, hist[cur].p, hist[cur ^ 1].p, channels, HL);
