@@ -9,6 +9,10 @@
 // hunt, MSB-first packing into a bounded ring, end-marker search).
 // All loop / framer state lives in device memory per channel and persists across calls, so arbitrary
 // chunking of a stream gives the same output as the reference object would.
+// Every call runs one loop over time chunks (DemodEngine::bits_dev): the front end of a chunk (front_chunk: host copy ->
+// AGC -> FLL -> matched filter), then its symbol stage.  Long fused calls pipeline the chunks over a side stream; a single
+// launch is the one-chunk case of the same loop, on the caller's stream.
+#include <functional>
 #include <memory>
 #include <string>
 
@@ -993,10 +997,7 @@ struct DemodEngine {
   std::unique_ptr<AgcEngine> agc;
   int64_t agc_drop = 0;            // AGC outputs still to discard (W-1 once per stream), the same for every channel
   DevBuf<float2> t_fll, t_rrc, t_sym, t_eq, t_fse, t_agc;
-  DevBuf<int> d_nsym, d_neq;
-  // what front() leaves for Costas: the MM symbols, or with the equalizer on its outputs
-  float2* sym_p = nullptr;
-  int* nsym_p = nullptr;
+  DevBuf<int> d_nsym, d_neq, d_ncon;   // d_ncon: symbol counts of qpsk_demod_constellation
   DevBuf<uint8_t> d_raw, d_tsc, d_bits, d_markers, d_carry, d_ring, d_pk, d_payload;
   DevBuf<long long> d_nraw, d_nbits, d_npayload;
   DevBuf<DiffState> d_diff;
@@ -1006,8 +1007,6 @@ struct DemodEngine {
   std::vector<uint8_t> markers_host;
   std::vector<long long> last_np;   // payload lengths of the last host framer call (qpsk_demod_last_payload)
   long long ring_cap = 0;
-  long long sym_ld = 0;
-  int64_t mf_ld = 0;
   cudaStream_t stream = nullptr;
   cudaStream_t side = nullptr;               // front-end stream of the time-chunk pipeline
   cudaStream_t copy = nullptr;               // host-source calls: the PCIe copies (and the CS16 widening) of the chunks
@@ -1027,14 +1026,34 @@ struct DemodEngine {
     h_land_bytes = bytes;
     return QPSK_OK;
   }
-  // rows of `width` bytes, `ld_dev` apart on the device, to rows `ld_host` apart in caller memory; synchronises `s`
-  int fetch_rows(void* host, size_t ld_host, const void* dev, size_t ld_dev, size_t width, cudaStream_t s) {
-    if (width == 0) return QPSK_OK;
+  // The result tail of the host entry points: the per-channel counts d_n[C] to n[C], then the rows `ld_dev` bytes apart on
+  // the device to rows `cap` bytes apart in caller memory, in one copy as wide as the widest row that fits (a row's bytes
+  // past its own count are unspecified, like the rest of the caller's buffer).  A row is `bits` bits per count; one
+  // longer than `cap` bytes is not copied and makes the call QPSK_ERR_CAPACITY, its count still reported.  `prep` runs on
+  // `s` first, when there is a row to copy.  Synchronises `s`.
+  template <typename Count>
+  int fetch_results(const Count* d_n, int64_t* n, int bits, void* out, int64_t cap, const void* dev, size_t ld_dev,
+                    cudaStream_t s, const std::function<int()>& prep = nullptr) {
+    std::vector<Count> h((size_t)channels);
+    QPSK_CUDA_TRY(cudaMemcpyAsync(h.data(), d_n, sizeof(Count) * channels, cudaMemcpyDeviceToHost, s));
+    QPSK_CUDA_TRY(cudaStreamSynchronize(s));
+    int st = QPSK_OK;
+    long long widest = 0;
+    for (int c = 0; c < channels; ++c) {
+      n[c] = h[(size_t)c];
+      const long long bytes = ((long long)h[(size_t)c] * bits + 7) / 8;
+      if (bytes > cap) st = QPSK_ERR_CAPACITY;
+      else if (bytes > widest) widest = bytes;
+    }
+    if (widest == 0) return st;
+    if (!out) return QPSK_ERR_NULL;
+    if (prep) QPSK_TRY(prep());
+    const size_t width = (size_t)widest;
     QPSK_TRY(landing(width * (size_t)channels));
     QPSK_CUDA_TRY(cudaMemcpy2DAsync(h_land, width, dev, ld_dev, width, (size_t)channels, cudaMemcpyDeviceToHost, s));
     QPSK_CUDA_TRY(cudaStreamSynchronize(s));
-    for (int c = 0; c < channels; ++c) memcpy((uint8_t*)host + (size_t)c * ld_host, h_land + (size_t)c * width, width);
-    return QPSK_OK;
+    for (int c = 0; c < channels; ++c) memcpy((uint8_t*)out + (size_t)c * (size_t)cap, h_land + (size_t)c * width, width);
+    return st;
   }
 
   ~DemodEngine() {
@@ -1101,65 +1120,29 @@ struct DemodEngine {
   }
   long long bits_bound(int64_t L) const { return 2 * symbols_bound(L); }
 
-  // FLL? -> MF [-> FSE] -> MM [-> EQ].  Symbols in sym_p [C][sym_ld] (t_sym, or t_eq with the equalizer on), counts in
-  // nsym_p.
-  int front(const float2* x, int64_t L, int64_t ldx, cudaStream_t s, bool run_mm = true) {
-    const int64_t ld = L + (L & 1);
-    QPSK_TRY(t_rrc.ensure((size_t)ld * channels));
-    sym_ld = symbols_bound(L);
-    if (sym_ld < 1) sym_ld = 1;
-    QPSK_TRY(t_sym.ensure((size_t)sym_ld * channels));
-    const float2* src = x;
-    int64_t lds = ldx;
-    if (use_fll) {
-      QPSK_TRY(t_fll.ensure((size_t)ld * channels));
-      QPSK_TRY(fll.process_dev(x, t_fll.p, L, ldx, ld, s));    // the call at :359
-      src = t_fll.p;
-      lds = ld;
+  // switches an opt-in stage once both streams are idle: off (`on` false), or a fresh one set up by init(stage)
+  template <typename E, typename Init>
+  int replace_stage(std::unique_ptr<E>& stage, bool on, Init init) {
+    QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
+    if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
+    if (!on) {
+      stage.reset();
+      return QPSK_OK;
     }
-    QPSK_TRY(mf.filter_dev(src, t_rrc.p, L, lds, ld, s));      // :360
-    mf_ld = ld;
-    if (!run_mm) return QPSK_OK;
-    const float2* mm_in = t_rrc.p;
-    int64_t mm_n = L;
-    if (fse) {
-      // every channel takes L samples, so every channel discards the same dc: MM takes L - dc samples of each row
-      QPSK_TRY(t_fse.ensure((size_t)ld * channels));
-      QPSK_TRY(fse->process_dev(t_rrc.p, t_fse.p, L, ld, ld, nullptr, nullptr, true, s));
-      const int64_t dc = fse_drop < L ? fse_drop : L;
-      fse_drop -= dc;
-      mm_in = t_fse.p;
-      mm_n = L - dc;
-    }
-    QPSK_TRY(mm.process_dev(mm_in, mm_n, ld, t_sym.p, 2 * L, sym_ld, d_nsym.p, s));   // :364-367
-    sym_p = t_sym.p;
-    nsym_p = d_nsym.p;
-    if (eq) {
-      QPSK_TRY(t_eq.ensure((size_t)sym_ld * channels));
-      QPSK_TRY(eq->process_dev(t_sym.p, t_eq.p, sym_ld, sym_ld, sym_ld, d_nsym.p, d_neq.p, true, s));
-      sym_p = t_eq.p;
-      nsym_p = d_neq.p;
-    }
+    std::unique_ptr<E> e(new (std::nothrow) E());
+    if (!e) return QPSK_ERR_NOMEM;
+    QPSK_TRY(init(*e));
+    stage = std::move(e);
     return QPSK_OK;
   }
-
   // opt-in equalizer stage: n_taps 0 = off; otherwise a fresh equalizer (spike taps, zero window, discard count D)
   int set_equalizer(int n_taps, float mu, float modulus) {
     if (n_taps != 0) QPSK_TRY(eq_check_params(n_taps, mu, modulus, 1));
-    QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
-    if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
-    if (n_taps == 0) {
-      eq.reset();
-      return QPSK_OK;
-    }
-    std::unique_ptr<EqEngine> e(new (std::nothrow) EqEngine());
-    if (!e) return QPSK_ERR_NOMEM;
-    QPSK_TRY(e->init(n_taps, mu, modulus, 1, channels));
-    QPSK_TRY(d_neq.ensure((size_t)channels));
-    eq = std::move(e);
-    return QPSK_OK;
+    return replace_stage(eq, n_taps != 0, [&](EqEngine& e) {
+      QPSK_TRY(e.init(n_taps, mu, modulus, 1, channels));
+      return d_neq.ensure((size_t)channels);
+    });
   }
-
   // opt-in fractionally spaced stage, update stride S = fs / rs: n_taps 0 = off; otherwise a fresh equalizer (spike taps,
   // zero window, sample counter 0, discard count D)
   int set_fractional_equalizer(int n_taps, float mu, float modulus) {
@@ -1167,47 +1150,20 @@ struct DemodEngine {
       if (int_sps < 2 || int_sps > kEqMaxSps) return QPSK_ERR_UNSUPPORTED;
       QPSK_TRY(eq_check_params(n_taps, mu, modulus, int_sps));
     }
-    QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
-    if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
-    if (n_taps == 0) {
-      fse.reset();
+    return replace_stage(fse, n_taps != 0, [&](EqEngine& e) {
+      QPSK_TRY(e.init(n_taps, mu, modulus, int_sps, channels));
+      fse_drop = (n_taps - 1) / 2;
       return QPSK_OK;
-    }
-    std::unique_ptr<EqEngine> e(new (std::nothrow) EqEngine());
-    if (!e) return QPSK_ERR_NOMEM;
-    QPSK_TRY(e->init(n_taps, mu, modulus, int_sps, channels));
-    fse = std::move(e);
-    fse_drop = (n_taps - 1) / 2;
-    return QPSK_OK;
+    });
   }
-
   // opt-in AGC stage: window 0 = off; otherwise a fresh AGC (zero history, discard count W-1)
   int set_agc(int window, float ref, float max_gain) {
     if (window != 0) QPSK_TRY(agc_check_params(window, ref, max_gain));
-    QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
-    if (side) QPSK_CUDA_TRY(cudaStreamSynchronize(side));
-    if (window == 0) {
-      agc.reset();
+    return replace_stage(agc, window != 0, [&](AgcEngine& a) {
+      QPSK_TRY(a.init(window, ref, max_gain, channels));
+      agc_drop = window - 1;
       return QPSK_OK;
-    }
-    std::unique_ptr<AgcEngine> a(new (std::nothrow) AgcEngine());
-    if (!a) return QPSK_ERR_NOMEM;
-    QPSK_TRY(a->init(window, ref, max_gain, channels));
-    agc = std::move(a);
-    agc_drop = window - 1;
-    return QPSK_OK;
-  }
-  // the AGC over a whole call on `s`: x / ldx then point at its outputs past this call's discard, L counts them
-  int agc_front(const float2*& x, int64_t& L, int64_t& ldx, cudaStream_t s) {
-    const int64_t ld = L + (L & 1);
-    QPSK_TRY(t_agc.ensure((size_t)ld * channels));
-    QPSK_TRY(agc->process_dev(x, L, ldx, t_agc.p, ld, s));
-    const int64_t dc = agc_drop < L ? agc_drop : L;
-    agc_drop -= dc;
-    x = t_agc.p + dc;
-    ldx = ld;
-    L -= dc;
-    return QPSK_OK;
+    });
   }
 
   // Time-chunk pipeline of bits_dev (FLL path): number of chunks for an L-sample call.  Short calls stay on one stream: the
@@ -1350,6 +1306,118 @@ struct DemodEngine {
     return QPSK_OK;
   }
 
+  // What one call runs and the sizes it works in, fixed before its first launch.  Every route runs the same loop over
+  // `chunks` time chunks (front_chunk, then the symbol stage of the chunk); a single launch is the one-chunk case.
+  struct CallPlan {
+    bool fused = false;          // the symbol stage is symsync_decode_kernel (else FSE -> MM -> EQ -> decode_kernel)
+    bool fuse_mf = false;        // ... with the matched filter inside it
+    bool from_host = false;      // samples staged from `hs` into h_in chunk by chunk
+    int chunks = 1;
+    HostSrc hs;
+    int64_t ld = 0;              // pitch of every scratch row of the call
+    int64_t agc_dc = 0;          // leading samples of the call the AGC discards
+    long long sym_ld = 1;        // symbol rows
+  };
+  // refuses nothing: the callers check their arguments first, and the plan only sizes scratch and picks the route
+  int plan(CallPlan& p, int64_t L, const HostSrc* hs, bool fused) {
+    p.fused = fused;
+    p.fuse_mf = fused && can_fuse_mf();
+    p.from_host = hs != nullptr && hs->p != nullptr;
+    p.chunks = (fused && use_fll) ? pipeline_chunks(L) : 1;
+    if (fused && p.from_host) p.chunks = std::max(p.chunks, host_chunks(L, hs->cs16));
+    p.ld = L + (L & 1);
+    p.agc_dc = agc ? std::min(agc_drop, L) : 0;
+    // a single launch sizes the symbol rows from the samples it keeps: Mueller-Muller's room rule reads that size (and
+    // with it how many symbols a call leaves queued for the next one)
+    p.sym_ld = std::max(1LL, symbols_bound(p.chunks > 1 ? L : L - p.agc_dc));
+    const size_t rows = (size_t)p.ld * channels;
+    if (p.from_host) {
+      p.hs = *hs;
+      p.hs.pageable = host_ptr_is_pageable(hs->p);
+      QPSK_TRY(h_in.ensure(rows));
+      if (hs->cs16) QPSK_TRY(h_cs16.ensure(2 * rows));
+      if (p.hs.pageable) QPSK_TRY(ensure_bounce((size_t)channels * (size_t)hs->ld * (hs->cs16 ? 4 : 8)));
+    }
+    if (agc) QPSK_TRY(t_agc.ensure(rows));
+    if (use_fll) QPSK_TRY(t_fll.ensure(rows));
+    if (!p.fuse_mf) QPSK_TRY(t_rrc.ensure(rows));
+    if (!fused) {
+      QPSK_TRY(t_sym.ensure((size_t)p.sym_ld * channels));
+      if (fse) QPSK_TRY(t_fse.ensure(rows));
+      if (eq) QPSK_TRY(t_eq.ensure((size_t)p.sym_ld * channels));
+    }
+    if (p.chunks > 1) QPSK_TRY(ensure_pipeline(p.chunks, p.from_host));
+    return QPSK_OK;
+  }
+
+  // The front end of time chunk t, samples [n0, n0 + len) of the call: staged from the host (from_host) -> AGC -> its
+  // discard -> FLL -> matched filter (unless the symbol stage runs it).  The AGC writes the chunk's outputs from column n0
+  // of t_agc, so the kept ones sit at n0 + skip; the FLL and the filter write theirs from column n0.  x / ldx (the call's
+  // device source) come back pointing at what the symbol stage reads, len as the number of samples kept.  In the
+  // pipeline it runs on the side stream and the host copies on the copy stream, and the caller's stream waits for it.
+  int front_chunk(const CallPlan& p, int t, int64_t n0, int64_t& len, const float2*& x, int64_t& ldx, cudaStream_t s) {
+    const bool pipe = p.chunks > 1;
+    cudaStream_t fs = pipe ? side : s;
+    if (p.from_host) {
+      QPSK_TRY(stage_host_chunk(p.hs, n0, len, p.ld, pipe ? copy : s));   // pageable source: the host gathers the chunk first
+      if (pipe) {
+        QPSK_CUDA_TRY(cudaEventRecord(ev_copy[(size_t)t], copy));
+        QPSK_CUDA_TRY(cudaStreamWaitEvent(side, ev_copy[(size_t)t], 0));
+      }
+      x = h_in.p;
+      ldx = p.ld;
+    }
+    x += n0;
+    if (agc) {
+      QPSK_TRY(agc->process_dev(x, len, ldx, t_agc.p + n0, p.ld, fs));
+      const int64_t skip = p.agc_dc > n0 ? std::min(p.agc_dc - n0, len) : 0;
+      agc_drop -= skip;
+      len -= skip;
+      x = t_agc.p + n0 + skip;
+      ldx = p.ld;
+    }
+    if (len > 0 && use_fll) {
+      QPSK_TRY(fll.process_dev(x, t_fll.p + n0, len, ldx, p.ld, fs));   // the call at :359
+      x = t_fll.p + n0;
+      ldx = p.ld;
+    }
+    if (len > 0 && !p.fuse_mf) {
+      QPSK_TRY(mf.filter_dev(x, t_rrc.p + n0, len, ldx, p.ld, fs));     // :360
+      x = t_rrc.p + n0;
+      ldx = p.ld;
+    }
+    if (pipe) {
+      QPSK_CUDA_TRY(cudaEventRecord(ev_chunk[(size_t)t], side));
+      QPSK_CUDA_TRY(cudaStreamWaitEvent(s, ev_chunk[(size_t)t], 0));
+    }
+    return QPSK_OK;
+  }
+
+  // [FSE ->] MM [-> EQ] over the matched-filter output of an unfused call (one chunk, len samples at x / ldx): the
+  // symbols Costas reads, sym [C][sym_ld], and their counts
+  int symbols(const CallPlan& p, const float2* x, int64_t len, int64_t ldx, const float2*& sym, const int*& nsym,
+              cudaStream_t s) {
+    int64_t mm_n = len;
+    if (fse) {
+      // every channel takes len samples, so every channel discards the same dc: MM takes len - dc samples of each row
+      QPSK_TRY(fse->process_dev(x, t_fse.p, len, ldx, p.ld, nullptr, nullptr, true, s));
+      const int64_t dc = std::min(fse_drop, len);
+      fse_drop -= dc;
+      x = t_fse.p;
+      ldx = p.ld;
+      mm_n = len - dc;
+    }
+    QPSK_TRY(mm.process_dev(x, mm_n, ldx, t_sym.p, 2 * len, p.sym_ld, d_nsym.p, s));   // :364-367
+    sym = t_sym.p;
+    nsym = d_nsym.p;
+    if (eq) {
+      QPSK_TRY(eq->process_dev(t_sym.p, t_eq.p, p.sym_ld, p.sym_ld, p.sym_ld, d_nsym.p, d_neq.p, true, s));
+      sym = t_eq.p;
+      nsym = d_neq.p;
+    }
+    return QPSK_OK;
+  }
+
   // DeModulate: bits (bytes 0/1) to out [C][ld_out], counts to n_out[C]
   // hs != nullptr: the samples are in host memory (x / ldx ignored): staged into h_in chunk by chunk
   int bits_dev(const float2* x, int64_t L, int64_t ldx, uint8_t* out, int64_t ld_out, long long* n_out, cudaStream_t s,
@@ -1358,143 +1426,63 @@ struct DemodEngine {
       QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(long long) * channels, s));   // :350-351
       return QPSK_OK;
     }
-    // every capacity / alignment check comes BEFORE the first stage that advances state (matched-filter delay line, loop
-    // state, MM queue): a refused call must leave the stream where it was
-    {
-      long long sl = symbols_bound(L);
-      if (sl < 1) sl = 1;
-      if (ld_out < 2 * sl) return QPSK_ERR_CAPACITY;
-      if (!has_tsc && ((reinterpret_cast<uintptr_t>(out) & 1) || (ld_out & 1))) return QPSK_ERR_ARG;   // uchar2 stores
-    }
-    const bool fused = can_fuse();
-    const bool fuse_mf = fused && can_fuse_mf();
-    const bool from_host = hs != nullptr && hs->p != nullptr;
-    int chunks = (fused && use_fll) ? pipeline_chunks(L) : 1;
-    HostSrc hsrc;
-    if (from_host) {
-      const int64_t ld = L + (L & 1);
-      QPSK_TRY(h_in.ensure((size_t)ld * channels));
-      if (hs->cs16) QPSK_TRY(h_cs16.ensure((size_t)2 * ld * channels));
-      x = h_in.p;
-      ldx = ld;
-      const int hc = fused ? host_chunks(L, hs->cs16) : 1;
-      if (hc > chunks) chunks = hc;
-      hsrc = *hs;
-      hsrc.pageable = host_ptr_is_pageable(hs->p);
-      if (hsrc.pageable) QPSK_TRY(ensure_bounce((size_t)channels * (size_t)hs->ld * (hs->cs16 ? 4 : 8)));
-      if (chunks == 1) QPSK_TRY(stage_host_chunk(hsrc, 0, L, ld, s));
-    }
-    int64_t agc_dc = 0;                              // time-chunk pipeline: samples of this call the AGC discards
-    if (agc && chunks == 1) {
-      QPSK_TRY(agc_front(x, L, ldx, s));
-      if (L == 0) {
-        QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(long long) * channels, s));
-        return QPSK_OK;
-      }
-    } else if (agc) {
-      QPSK_TRY(t_agc.ensure((size_t)(L + (L & 1)) * channels));
-      agc_dc = agc_drop < L ? agc_drop : L;
-      agc_drop -= agc_dc;
-    }
-    const float2* sym_in = nullptr;                  // what the symbol-stage kernel reads in the single-launch case
-    int64_t sym_in_ld = 0;
-    if (chunks > 1) {
-      // sizes only; the front end runs chunk by chunk below
-      const int64_t ld = L + (L & 1);
-      if (!fuse_mf) QPSK_TRY(t_rrc.ensure((size_t)ld * channels));
-      if (use_fll) QPSK_TRY(t_fll.ensure((size_t)ld * channels));
-      sym_ld = symbols_bound(L);
-      if (sym_ld < 1) sym_ld = 1;
-      mf_ld = ld;
-    } else if (fuse_mf) {
-      // FLL (when on) in front; the matched filter runs inside the symbol-stage kernel
-      const int64_t ld = L + (L & 1);
-      sym_ld = symbols_bound(L);
-      if (sym_ld < 1) sym_ld = 1;
-      sym_in = x;
-      sym_in_ld = ldx;
-      if (use_fll) {
-        QPSK_TRY(t_fll.ensure((size_t)ld * channels));
-        QPSK_TRY(fll.process_dev(x, t_fll.p, L, ldx, ld, s));   // the call at :359
-        sym_in = t_fll.p;
-        sym_in_ld = ld;
-      }
-    } else {
-      QPSK_TRY(front(x, L, ldx, s, !fused));
-      sym_in = t_rrc.p;
-      sym_in_ld = mf_ld;
-    }
-    const long long need = 2 * sym_ld;
-    if (ld_out < need) return QPSK_ERR_CAPACITY;
+    // every check comes BEFORE the first stage that advances state (AGC history, FLL ring, matched-filter delay line, MM
+    // queue, loop state): a refused call must leave the stream where it was
+    if (ld_out < 2 * std::max(1LL, symbols_bound(L))) return QPSK_ERR_CAPACITY;
+    // uchar2 stores; with a TSC the symbol stage writes the engine's own 16-byte rows
+    if (!has_tsc && ((reinterpret_cast<uintptr_t>(out) & 1) || (ld_out & 1))) return QPSK_ERR_ARG;
+    CallPlan p;
+    QPSK_TRY(plan(p, L, hs, can_fuse()));
     uint8_t* raw = out;
     long long ld_raw = ld_out;
     long long* n_raw = n_out;
     if (has_tsc) {
-      const long long ldr = (need + 15) & ~15LL;
-      QPSK_TRY(d_raw.ensure((size_t)ldr * channels));
-      raw = d_raw.p; ld_raw = ldr; n_raw = d_nraw.p;
+      ld_raw = (2 * p.sym_ld + 15) & ~15LL;
+      QPSK_TRY(d_raw.ensure((size_t)ld_raw * channels));
+      raw = d_raw.p;
+      n_raw = d_nraw.p;
     }
-    if ((reinterpret_cast<uintptr_t>(raw) & 1) || (ld_raw & 1)) return QPSK_ERR_ARG;   // uchar2 stores
-    if (fused && chunks > 1) {
-      // FLL -> MF of time chunk t+1 on the side stream while MM -> Costas -> decode of chunk t runs on the caller's:
-      // every stage carries its state from chunk to chunk exactly (FLL ring/phase, MF delay line, MM queue, Costas,
-      // differential reference), so the split changes nothing but the schedule.
-      QPSK_TRY(mm.ensure_queue(8, s));
-      QPSK_TRY(ensure_pipeline(chunks, from_host));
-      // equal chunks except a half-size last one: the FLL on the side stream is the critical resource throughout, so
-      // what is left exposed at the end is the last chunk's MM -> Costas -> decode
-      const int64_t step = ((2 * L + 2 * chunks - 2) / (2 * chunks - 1) + kSsBlock - 1) / kSsBlock * kSsBlock;
+    if (p.chunks > 1) {
+      // the time-chunk pipeline: the front end of chunk t+1 on the side stream while the symbol stage of chunk t runs on
+      // the caller's.  Every stage carries its state from chunk to chunk exactly (AGC history, FLL ring/phase, MF delay
+      // line, MM queue, Costas, differential reference), so the split changes nothing but the schedule.
       QPSK_CUDA_TRY(cudaEventRecord(ev_in, s));
       QPSK_CUDA_TRY(cudaStreamWaitEvent(side, ev_in, 0));     // inputs (and the previous call) are complete
       // the PCIe copies run on a stream of their own: chunk t+1 crosses the bus while the FLL (side stream) works on chunk t
       // and the symbol stage (caller's stream) on chunk t-1.  On the side stream they would queue behind the FLL launches:
       // copy and FLL would take turns (3.3 ms per step where 1.3 + tail is possible).
-      if (from_host) QPSK_CUDA_TRY(cudaStreamWaitEvent(copy, ev_in, 0));
-      int t = 0;
-      bool launched = false;
-      for (int64_t n0 = 0; n0 < L; n0 += step, ++t) {
-        int64_t len = (L - n0 < step) ? (L - n0) : step;
-        if (from_host) {
-          QPSK_TRY(stage_host_chunk(hsrc, n0, len, mf_ld, copy));      // pageable source: the host gathers the chunk first
-          QPSK_CUDA_TRY(cudaEventRecord(ev_copy[(size_t)t], copy));
-          QPSK_CUDA_TRY(cudaStreamWaitEvent(side, ev_copy[(size_t)t], 0));
-        }
-        const float2* src = x + n0;
-        int64_t lds = ldx;
-        int64_t o = n0;                              // where this chunk's samples sit in the scratch rows
-        if (agc) {
-          QPSK_TRY(agc->process_dev(src, len, lds, t_agc.p + n0, mf_ld, side));
-          const int64_t skip = agc_dc > n0 ? std::min<int64_t>(agc_dc - n0, len) : 0;
-          o = n0 + skip;
-          len -= skip;
-          src = t_agc.p + o;
-          lds = mf_ld;
-        }
-        if (len > 0 && use_fll) {
-          QPSK_TRY(fll.process_dev(src, t_fll.p + o, len, lds, mf_ld, side));            // the call at :359
-          src = t_fll.p + o;
-          lds = mf_ld;
-        }
-        if (len > 0 && !fuse_mf) {
-          QPSK_TRY(mf.filter_dev(src, t_rrc.p + o, len, lds, mf_ld, side));              // :360
-          src = t_rrc.p + o;
-          lds = mf_ld;
-        }
-        QPSK_CUDA_TRY(cudaEventRecord(ev_chunk[(size_t)t], side));
-        QPSK_CUDA_TRY(cudaStreamWaitEvent(s, ev_chunk[(size_t)t], 0));
-        if (len > 0) {
-          QPSK_TRY(launch_symsync(src, len, lds, raw, ld_raw, n_raw, launched ? 1 : 0, fuse_mf, s));
-          launched = true;
-        }
+      if (p.from_host) QPSK_CUDA_TRY(cudaStreamWaitEvent(copy, ev_in, 0));
+    }
+    // equal chunks except a half-size last one: the FLL on the side stream is the critical resource throughout, so what is
+    // left exposed at the end is the last chunk's symbol stage.  One chunk: the whole call.
+    const int chunks = p.chunks;
+    const int64_t step = ((2 * L + 2 * chunks - 2) / (2 * chunks - 1) + kSsBlock - 1) / kSsBlock * kSsBlock;
+    bool launched = false;
+    int t = 0;
+    for (int64_t n0 = 0; n0 < L; n0 += step, ++t) {
+      int64_t len = std::min(step, L - n0);
+      const float2* y = x;
+      int64_t ldy = ldx;
+      QPSK_TRY(front_chunk(p, t, n0, len, y, ldy, s));
+      if (len == 0) continue;
+      if (p.fused) {
+        QPSK_TRY(launch_symsync(y, len, ldy, raw, ld_raw, n_raw, launched ? 1 : 0, p.fuse_mf, s));
+      } else {
+        const float2* sym;
+        const int* nsym;
+        QPSK_TRY(symbols(p, y, len, ldy, sym, nsym, s));
+        decode_kernel<<<(channels + 31) / 32, 32, 0, s>>>(costas.P, costas.d_state.p, d_diff.p, channels, sym, p.sym_ld, nsym,
+                                                          diff ? 1 : 0, raw, ld_raw, n_raw);
+        QPSK_LAUNCH_CHECK();
       }
-      if (!launched) QPSK_CUDA_TRY(cudaMemsetAsync(n_raw, 0, sizeof(long long) * channels, s));
-    } else if (fused) {
-      QPSK_TRY(mm.ensure_queue(8, s));
-      QPSK_TRY(launch_symsync(sym_in, L, sym_in_ld, raw, ld_raw, n_raw, 0, fuse_mf, s));
-    } else {
-      decode_kernel<<<(channels + 31) / 32, 32, 0, s>>>(costas.P, costas.d_state.p, d_diff.p, channels, sym_p, sym_ld,
-                                                        nsym_p, diff ? 1 : 0, raw, ld_raw, n_raw);
-      QPSK_LAUNCH_CHECK();
+      launched = true;
+    }
+    if (!launched) {                                 // the AGC discarded every sample of the call
+      if (chunks == 1) {
+        QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(long long) * channels, s));
+        return QPSK_OK;
+      }
+      QPSK_CUDA_TRY(cudaMemsetAsync(n_raw, 0, sizeof(long long) * channels, s));
     }
     if (has_tsc) {
       const int T = (int)tsc.size();
@@ -1513,26 +1501,27 @@ struct DemodEngine {
     return QPSK_OK;
   }
 
-  int constellation_dev(const float2* x, int64_t L, int64_t ldx, float2* out, int64_t ld_out, int* n_out, cudaStream_t s) {
+  // symbols after Costas (:447-452) to out [C][ld_out], counts to n_out[C]; hs as for bits_dev
+  int constellation_dev(const float2* x, int64_t L, int64_t ldx, float2* out, int64_t ld_out, int* n_out, cudaStream_t s,
+                        const HostSrc* hs = nullptr) {
     if (L == 0) {
       QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(int) * channels, s));
       return QPSK_OK;
     }
-    {
-      long long sl = symbols_bound(L);                         // refuse before any stage consumes the samples
-      if (sl < 1) sl = 1;
-      if (ld_out < sl) return QPSK_ERR_CAPACITY;
+    if (ld_out < std::max(1LL, symbols_bound(L))) return QPSK_ERR_CAPACITY;   // refuse before any stage consumes the samples
+    CallPlan p;
+    QPSK_TRY(plan(p, L, hs, false));
+    int64_t len = L;
+    QPSK_TRY(front_chunk(p, 0, 0, len, x, ldx, s));
+    if (len == 0) {                                  // the AGC discarded every sample of the call
+      QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(int) * channels, s));
+      return QPSK_OK;
     }
-    if (agc) {
-      QPSK_TRY(agc_front(x, L, ldx, s));
-      if (L == 0) {
-        QPSK_CUDA_TRY(cudaMemsetAsync(n_out, 0, sizeof(int) * channels, s));
-        return QPSK_OK;
-      }
-    }
-    QPSK_TRY(front(x, L, ldx, s));
-    QPSK_TRY(costas.process_dev(sym_p, out, sym_ld, sym_ld, ld_out, nsym_p, s));   // :447-452
-    QPSK_CUDA_TRY(cudaMemcpyAsync(n_out, nsym_p, sizeof(int) * channels, cudaMemcpyDeviceToDevice, s));
+    const float2* sym;
+    const int* nsym;
+    QPSK_TRY(symbols(p, x, len, ldx, sym, nsym, s));
+    QPSK_TRY(costas.process_dev(sym, out, p.sym_ld, p.sym_ld, ld_out, nsym, s));   // :447-452
+    QPSK_CUDA_TRY(cudaMemcpyAsync(n_out, nsym, sizeof(int) * channels, cudaMemcpyDeviceToDevice, s));
     return QPSK_OK;
   }
 
@@ -1673,16 +1662,6 @@ static int demod_check_in(qpsk_demod* d, const void* in, int64_t n_floats) {
   return QPSK_OK;
 }
 
-// host staging: [C][n_floats] -> device
-static int demod_stage_in(DemodEngine& e, const float* iq_in, int64_t L, cudaStream_t s) {
-  const int64_t ld = L + (L & 1);
-  QPSK_TRY(e.h_in.ensure((size_t)(ld > 0 ? ld : 2) * e.channels));
-  if (L > 0)
-    QPSK_CUDA_TRY(cudaMemcpy2DAsync(e.h_in.p, (size_t)ld * 8, iq_in, (size_t)L * 8, (size_t)L * 8, (size_t)e.channels,
-                                    cudaMemcpyHostToDevice, s));
-  return QPSK_OK;
-}
-
 int qpsk_demod_bits(qpsk_demod* d, const float* iq_in, int64_t n_floats, char* bits_out, int64_t cap, int64_t* n_bits) {
   QPSK_TRY(demod_check_in(d, iq_in, n_floats));
   if (!n_bits) return QPSK_ERR_NULL;
@@ -1697,29 +1676,16 @@ int qpsk_demod_bits(qpsk_demod* d, const float* iq_in, int64_t n_floats, char* b
   HostSrc hs;
   hs.p = iq_in; hs.ld = L; hs.cs16 = false;
   QPSK_TRY(e.bits_dev(nullptr, L, 0, e.d_bits.p, ldb, e.d_nbits.p, s, &hs));
-  std::vector<long long> nb((size_t)e.channels);
-  QPSK_CUDA_TRY(cudaMemcpyAsync(nb.data(), e.d_nbits.p, sizeof(long long) * e.channels, cudaMemcpyDeviceToHost, s));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(s));
-  int st = QPSK_OK;
-  long long widest = 0;
-  for (int c = 0; c < e.channels; ++c) {
-    n_bits[c] = nb[(size_t)c];
-    if (nb[(size_t)c] > cap) st = QPSK_ERR_CAPACITY;
-    else if (nb[(size_t)c] > widest) widest = nb[(size_t)c];
-  }
-  if (widest > 0) {
-    if (!bits_out) return QPSK_ERR_NULL;
-    // bytes 0/1 -> '0'/'1' on the device, then ONE 2-D copy as wide as the longest string of the call (a channel's
-    // characters past its own n_bits are unspecified, like the rest of the caller's buffer)
+  // bytes 0/1 -> '0'/'1' on the device before the rows come back
+  return e.fetch_results(e.d_nbits.p, n_bits, 8, bits_out, cap, e.d_bits.p, (size_t)ldb, s, [&] {
     const long long tot = ldb * e.channels;
     long long blocks = (tot + 255) / 256;
     const long long capb = 32LL * device_sm_count();
     if (blocks > capb) blocks = capb;
     bits_to_chars_kernel<<<(int)blocks, 256, 0, s>>>(e.d_bits.p, reinterpret_cast<char*>(e.d_bits.p), tot);
     QPSK_LAUNCH_CHECK();
-    QPSK_TRY(e.fetch_rows(bits_out, (size_t)cap, e.d_bits.p, (size_t)ldb, (size_t)widest, s));
-  }
-  return st;
+    return QPSK_OK;
+  });
 }
 
 int qpsk_demod_bits_packed(qpsk_demod* d, const float* iq_in, int64_t n_floats, uint8_t* packed_out, int64_t cap_bytes,
@@ -1732,30 +1698,16 @@ int qpsk_demod_bits_packed(qpsk_demod* d, const float* iq_in, int64_t n_floats, 
   if (n_floats == 0) return QPSK_OK;                         // :350-351
   QPSK_TRY(ensure_device(d->eng.device));
   cudaStream_t s = e.stream;
-  const int64_t L = n_floats >> 1, ld = L + (L & 1);
-  QPSK_TRY(demod_stage_in(e, iq_in, L, s));
+  const int64_t L = n_floats >> 1;
   const long long ldb = (e.bits_bound(L) + 2 + 7) & ~7LL;    // 8-byte aligned rows for the pack kernel's wide loads
   QPSK_TRY(e.d_bits.ensure((size_t)ldb * e.channels));
-  QPSK_TRY(e.bits_dev(e.h_in.p, L, ld, e.d_bits.p, ldb, e.d_nbits.p, s));
+  HostSrc hs;
+  hs.p = iq_in; hs.ld = L; hs.cs16 = false;
+  QPSK_TRY(e.bits_dev(nullptr, L, 0, e.d_bits.p, ldb, e.d_nbits.p, s, &hs));
   const long long ldp = ldb / 8;
   QPSK_TRY(e.d_pk.ensure((size_t)ldp * e.channels));
   QPSK_TRY(qpsk_pack_bits_dev(e.d_bits.p, ldb, (const int64_t*)e.d_nbits.p, ldb, e.channels, e.d_pk.p, ldp, s));
-  std::vector<long long> nb((size_t)e.channels);
-  QPSK_CUDA_TRY(cudaMemcpyAsync(nb.data(), e.d_nbits.p, sizeof(long long) * e.channels, cudaMemcpyDeviceToHost, s));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(s));
-  int st = QPSK_OK;
-  long long widest = 0;
-  for (int c = 0; c < e.channels; ++c) {
-    n_bits[c] = nb[(size_t)c];
-    const long long bytes = (nb[(size_t)c] + 7) / 8;
-    if (bytes > cap_bytes) st = QPSK_ERR_CAPACITY;
-    else if (bytes > widest) widest = bytes;
-  }
-  if (widest > 0) {
-    if (!packed_out) return QPSK_ERR_NULL;
-    QPSK_TRY(e.fetch_rows(packed_out, (size_t)cap_bytes, e.d_pk.p, (size_t)ldp, (size_t)widest, s));
-  }
-  return st;
+  return e.fetch_results(e.d_nbits.p, n_bits, 1, packed_out, cap_bytes, e.d_pk.p, (size_t)ldp, s);
 }
 
 // host samples -> payload bytes: the chain runs as a pipeline over time chunks (HostSrc), the payloads come back in one
@@ -1768,21 +1720,9 @@ static int demod_bytes_host(qpsk_demod* d, const HostSrc& hs, int64_t L, const u
   const int64_t pcap = cap > 0 ? (cap < e.ring_cap ? cap : e.ring_cap) : 1;
   QPSK_TRY(e.d_payload.ensure((size_t)pcap * e.channels));
   QPSK_TRY(e.bytes_dev(nullptr, L, 0, start_marker, n_start, end_marker, n_end, e.d_payload.p, pcap, e.d_npayload.p, s, &hs));
-  std::vector<long long>& np = e.last_np;
-  np.assign((size_t)e.channels, 0);
-  QPSK_CUDA_TRY(cudaMemcpyAsync(np.data(), e.d_npayload.p, sizeof(long long) * e.channels, cudaMemcpyDeviceToHost, s));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(s));
-  int st = QPSK_OK;
-  long long widest = 0;
-  for (int c = 0; c < e.channels; ++c) {
-    n_bytes[c] = np[(size_t)c];
-    if (np[(size_t)c] > cap) st = QPSK_ERR_CAPACITY;         // the frame stays in the ring: qpsk_demod_last_payload
-    else if (np[(size_t)c] > widest) widest = np[(size_t)c];
-  }
-  if (widest > 0) {
-    if (!payload_out) return QPSK_ERR_NULL;
-    QPSK_TRY(e.fetch_rows(payload_out, (size_t)cap, e.d_payload.p, (size_t)pcap, (size_t)widest, s));
-  }
+  // a frame longer than `cap` stays in the ring: qpsk_demod_last_payload
+  const int st = e.fetch_results(e.d_npayload.p, n_bytes, 8, payload_out, cap, e.d_payload.p, (size_t)pcap, s);
+  e.last_np.assign(n_bytes, n_bytes + e.channels);
   return st;
 }
 
@@ -1864,21 +1804,8 @@ int qpsk_demod_frame_bits(qpsk_demod* d, const uint8_t* bits, int64_t bits_strid
   const int64_t pcap = cap > 0 ? cap : 1;
   QPSK_TRY(e.d_payload.ensure((size_t)pcap * e.channels));
   QPSK_TRY(e.frame_dev(e.d_bits.p, ldb, e.d_nbits.p, start_marker, n_start, end_marker, n_end, e.d_payload.p, pcap, e.d_npayload.p, s));
-  std::vector<long long>& np = e.last_np;
-  np.assign((size_t)e.channels, 0);
-  QPSK_CUDA_TRY(cudaMemcpyAsync(np.data(), e.d_npayload.p, sizeof(long long) * e.channels, cudaMemcpyDeviceToHost, s));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(s));
-  int st = QPSK_OK;
-  long long widest = 0;
-  for (int c = 0; c < e.channels; ++c) {
-    n_bytes[c] = np[(size_t)c];
-    if (np[(size_t)c] > cap) st = QPSK_ERR_CAPACITY;
-    else if (np[(size_t)c] > widest) widest = np[(size_t)c];
-  }
-  if (widest > 0) {                                          // one 2-D copy as wide as the longest payload that fits
-    if (!payload_out) return QPSK_ERR_NULL;
-    QPSK_TRY(e.fetch_rows(payload_out, (size_t)cap, e.d_payload.p, (size_t)pcap, (size_t)widest, s));
-  }
+  const int st = e.fetch_results(e.d_npayload.p, n_bytes, 8, payload_out, cap, e.d_payload.p, (size_t)pcap, s);
+  e.last_np.assign(n_bytes, n_bytes + e.channels);
   return st;
 }
 
@@ -1891,28 +1818,14 @@ int qpsk_demod_constellation(qpsk_demod* d, const float* iq_in, int64_t n_floats
   if (n_floats == 0) return QPSK_OK;
   QPSK_TRY(ensure_device(d->eng.device));
   cudaStream_t s = e.stream;
-  const int64_t L = n_floats >> 1, ld = L + (L & 1);
-  QPSK_TRY(demod_stage_in(e, iq_in, L, s));
-  const long long lds = e.symbols_bound(L) > 0 ? e.symbols_bound(L) : 1;
+  const int64_t L = n_floats >> 1;
+  const long long lds = std::max(1LL, e.symbols_bound(L));
   QPSK_TRY(e.h_out.ensure((size_t)lds * e.channels));
-  DevBuf<int> dn;
-  QPSK_TRY(dn.alloc((size_t)e.channels));
-  QPSK_TRY(e.constellation_dev(e.h_in.p, L, ld, e.h_out.p, lds, dn.p, s));
-  std::vector<int> ns((size_t)e.channels);
-  QPSK_CUDA_TRY(cudaMemcpyAsync(ns.data(), dn.p, sizeof(int) * e.channels, cudaMemcpyDeviceToHost, s));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(s));
-  int st = QPSK_OK;
-  long long widest = 0;
-  for (int c = 0; c < e.channels; ++c) {
-    n_sym[c] = ns[(size_t)c];
-    if (2LL * ns[(size_t)c] > cap_floats) st = QPSK_ERR_CAPACITY;
-    else if (ns[(size_t)c] > widest) widest = ns[(size_t)c];
-  }
-  if (widest > 0) {
-    if (!sym_iq_out) return QPSK_ERR_NULL;
-    QPSK_TRY(e.fetch_rows(sym_iq_out, (size_t)cap_floats * 4, e.h_out.p, (size_t)lds * 8, (size_t)widest * 8, s));
-  }
-  return st;
+  QPSK_TRY(e.d_ncon.ensure((size_t)e.channels));
+  HostSrc hs;
+  hs.p = iq_in; hs.ld = L; hs.cs16 = false;
+  QPSK_TRY(e.constellation_dev(nullptr, L, 0, e.h_out.p, lds, e.d_ncon.p, s, &hs));
+  return e.fetch_results(e.d_ncon.p, n_sym, 64, sym_iq_out, cap_floats * 4, e.h_out.p, (size_t)lds * 8, s);
 }
 
 int qpsk_demod_device(const qpsk_demod* d, int* ordinal) {

@@ -121,3 +121,55 @@ def symsync_variants(names):
         if m:
             out.add(f"symsync_decode_kernel<{m.group(1)}, {m.group(2)}, {m.group(3)}>")
     return out
+
+
+# ---- call plan: time chunks and route of one DeModulate call ---------------------------------------------------------
+def pipeline_chunks(L, channels):
+    """DemodEngine::pipeline_chunks: time chunks of a fused call with the FLL on."""
+    n = 6 if channels <= 4096 else 4
+    if L < 2048:
+        n = 1
+    while n > 1 and L < n * 8 * K_SS_BLOCK:
+        n -= 1
+    return n
+
+
+def host_chunks(L, channels, cs16):
+    """DemodEngine::host_chunks: copy chunks of a fused call on host samples, >= 8 MiB each, at most 6."""
+    n = min(max(int(L * channels * (4.0 if cs16 else 8.0) / (8.0 * 1024 * 1024)), 1), 6)
+    while n > 1 and L < n * 8 * K_SS_BLOCK:
+        n -= 1
+    return n
+
+
+def chunks(L, channels, use_fll, host=False, cs16=False, fused=True):
+    """Time chunks one call runs in (DemodEngine::plan); an unfused call is always one."""
+    if not fused:
+        return 1
+    n = pipeline_chunks(L, channels) if use_fll else 1
+    return max(n, host_chunks(L, channels, cs16)) if host else n
+
+
+# rows of tests/test_gpu_demod_routes.py, span 10 and EXACT filter: one call of L samples each
+ROUTE_ROWS = {
+    "device_fll": dict(channels=256, fs=4000, rs=1000, L=4196, use_fll=True),
+    "device": dict(channels=256, fs=4000, rs=1000, L=4196),
+    "host_cf32": dict(channels=600, fs=4000, rs=1000, L=7200, host=True),
+    "host_cs16": dict(channels=600, fs=4000, rs=1000, L=7200, host=True, cs16=True),
+    "mf_separate": dict(channels=16, fs=4000, rs=1000, L=4196),
+    "eq": dict(channels=256, fs=4000, rs=1000, L=4196, eq=True),
+    "sps_1.05": dict(channels=256, fs=2100, rs=2000, L=4196),
+}
+ROUTES = ("pipeline_device", "pipeline_host", "single_mf_fused", "single_mf_separate", "unfused")
+
+
+def route(row):
+    """-> (route, chunks) of a ROUTE_ROWS row: the time-chunk pipeline from a device or a host source, a single launch of
+    the symbol-stage kernel with the matched filter inside or separate, or the unfused MM -> Costas -> decode chain."""
+    fused = not row.get("eq") and predict(row["channels"], row["fs"], row["rs"], 10) is not None
+    n = chunks(row["L"], row["channels"], row.get("use_fll", False), row.get("host", False), row.get("cs16", False), fused)
+    if not fused:
+        return "unfused", n
+    if n > 1:
+        return ("pipeline_host" if row.get("host") else "pipeline_device"), n
+    return ("single_mf_fused" if predict(row["channels"], row["fs"], row["rs"], 10)["mfw"] else "single_mf_separate"), n

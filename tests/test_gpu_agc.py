@@ -151,11 +151,17 @@ def _scene_batch(orc, C, n_total, seed=5):
     return rows, [pays[r % len(pays)] for r in range(C)]
 
 
-@pytest.mark.parametrize("use_fll", [False, True])
-def test_demod_stage_matches_oracle(gpu, orc, use_fll):
-    C, W = 256, 64
-    rows, pays = _scene_batch(orc, C, 4200)           # 4200 samples: with the FLL on, the time-chunk pipeline runs
-    cuts = [0, 30, 1500, 4200]                        # the first call is shorter than the AGC's discard
+# W = 4096 with the FLL: the first 4200-sample call runs the time-chunk pipeline and the AGC's discard takes its first five
+# chunks whole and part of the sixth
+@pytest.mark.parametrize("use_fll,W", [(False, 64), (True, 64), (True, 4096)], ids=["False", "True", "True-W4096"])
+def test_demod_stage_matches_oracle(gpu, orc, use_fll, W):
+    C = 256
+    if W == 64:
+        rows, pays = _scene_batch(orc, C, 4200)       # 4200 samples: with the FLL on, the time-chunk pipeline runs
+        cuts = [0, 30, 1500, 4200]                    # the first call is shorter than the AGC's discard
+    else:
+        rows, pays = _scene_batch(orc, C, 3 * 4200)
+        cuts = [0, 4200, 8400, 12600]
     dem = gpu.QPSKDeModulator(SCENE_FS, SCENE_RS, 0.35, 10, tsc=TSC, use_fll=use_fll, channels=C)
     dem.set_agc(W, 1.0, 65536.0)
     ref = AgcDemod(orc, SCENE_FS, SCENE_RS, 0.35, 10, channels=C, tsc=TSC, use_fll=use_fll)
@@ -163,11 +169,24 @@ def test_demod_stage_matches_oracle(gpu, orc, use_fll):
     for a, b in zip(cuts[:-1], cuts[1:]):
         part = np.ascontiguousarray(rows[:, a:b]).view(np.float32)
         assert dem.DeModulate(part) == ref.DeModulate(part), (a, b)
+    # host rows, cf32 and CS16, through the same calls: the payloads of the oracle on the values the device widens to
+    scale = float(np.float32(np.abs(rows.view(np.float32)).max() / 30000.0))
+    x16 = np.clip(np.round(rows.view(np.float32) / scale), -32768, 32767).astype(np.int16)
+    xf = (x16.astype(np.float32) * np.float32(scale)).astype(np.float32)
+    d32, d16 = (gpu.QPSKDeModulator(SCENE_FS, SCENE_RS, 0.35, 10, tsc=TSC, use_fll=use_fll, channels=C) for _ in range(2))
+    ref = AgcDemod(orc, SCENE_FS, SCENE_RS, 0.35, 10, channels=C, tsc=TSC, use_fll=use_fll)
+    for d in (d32, d16, ref):
+        d.set_agc(W, 1.0, 65536.0)
+    for a, b in zip(cuts[:-1], cuts[1:]):
+        want = ref.DeModulateBytes(np.ascontiguousarray(xf[:, 2 * a: 2 * b]), b"START", b"END")
+        assert d32.DeModulateBytes(np.ascontiguousarray(xf[:, 2 * a: 2 * b]), b"START", b"END") == want, (a, b)
+        assert d16.DeModulateBytesCs16(np.ascontiguousarray(x16[:, 2 * a: 2 * b]), scale, b"START", b"END") == want, (a, b)
     # the frames decode at every level
-    dem2 = gpu.QPSKDeModulator(SCENE_FS, SCENE_RS, 0.35, 10, tsc=TSC, use_fll=use_fll, channels=C)
-    dem2.set_agc(W, 1.0, 65536.0)
-    got = dem2.DeModulateBytes(np.ascontiguousarray(rows).view(np.float32), b"START", b"END")
-    assert got == pays
+    if W == 64:
+        dem2 = gpu.QPSKDeModulator(SCENE_FS, SCENE_RS, 0.35, 10, tsc=TSC, use_fll=use_fll, channels=C)
+        dem2.set_agc(W, 1.0, 65536.0)
+        got = dem2.DeModulateBytes(np.ascontiguousarray(rows).view(np.float32), b"START", b"END")
+        assert got == pays
 
 
 # The profiler runs in a child process: once a torch.profiler session has been opened in the pytest process, the profiled

@@ -90,43 +90,64 @@ def test_frame_grown_over_many_small_calls_is_not_lost(gpu, orc):
 
 def test_refused_device_call_leaves_the_stream_untouched(gpu, orc):
     """ADVICE r1: capacity / alignment errors of the *_dev entry points are reported before any stage consumes samples:
-    after a refused call the same samples still demodulate to the oracle's bits."""
+    after a refused call the same samples still demodulate to the oracle's bits.  With an opt-in stage on (AGC W = 64,
+    fractionally spaced or symbol-spaced equalizer) they demodulate to the bits of a twin handle that saw no refused call."""
     import torch
     fs, rs = 4000, 1000
     x, _ = _burst(orc, n_payload=200, tsc=None)
     kw = dict(RrcAlpha=0.35, rrcSpan=10, SymbolSyncBandwith=0.002)
-    want = orc.QPSKDeModulator(fs, rs, **kw).DeModulate(x)
-    for use_fll in (False, True):
-        if use_fll:
-            want = orc.QPSKDeModulator(fs, rs, use_fll=True, **kw).DeModulate(x)
-        gd = gpu.QPSKDeModulator(fs, rs, use_fll=use_fll, **kw)
-        gd.set_fir_mode(gpu.FIR_EXACT)
-        dx = torch.from_numpy(x).cuda()
-        cap = gd.bits_bound(x.size)
-        bits = torch.zeros(cap + 2, dtype=torch.uint8, device="cuda")
-        nb = torch.zeros(1, dtype=torch.int64, device="cuda")
-        with pytest.raises(gpu.QpskCudaError):                  # too small: QPSK_ERR_CAPACITY
-            gd.demod_bits_dev(dx.data_ptr(), x.size, x.size, bits.data_ptr(), 8, nb.data_ptr())
-        with pytest.raises(gpu.ArgumentException):              # odd output address (uchar2 stores): QPSK_ERR_ARG
-            gd.demod_bits_dev(dx.data_ptr(), x.size, x.size, bits.data_ptr() + 1, cap, nb.data_ptr())
-        gd.demod_bits_dev(dx.data_ptr(), x.size, x.size, bits.data_ptr(), cap, nb.data_ptr())
-        torch.cuda.synchronize()
-        got = "".join("1" if b else "0" for b in bits[: int(nb.item())].cpu().numpy())
-        assert got == want and len(want) > 100
-    # deModulateConstellation: short output refused before the matched filter / MM advance
-    gd = gpu.QPSKDeModulator(fs, rs, **kw)
-    gd.set_fir_mode(gpu.FIR_EXACT)
     L = gpu._native.lib()
     dx = torch.from_numpy(x).cuda()
-    sym = torch.zeros(x.size, dtype=torch.float32, device="cuda")
-    ns = torch.zeros(1, dtype=torch.int32, device="cuda")
-    assert L.qpsk_demod_constellation_dev(gd._h, dx.data_ptr(), x.size, x.size, sym.data_ptr(), 8, ns.data_ptr(), None) == gpu._native.ERR_CAPACITY
-    assert L.qpsk_demod_constellation_dev(gd._h, dx.data_ptr(), x.size, x.size, sym.data_ptr(), x.size, ns.data_ptr(), None) == 0
-    torch.cuda.synchronize()
+
+    def handle(use_fll, stage):
+        gd = gpu.QPSKDeModulator(fs, rs, use_fll=use_fll, **kw)
+        gd.set_fir_mode(gpu.FIR_EXACT)
+        if stage == "agc":
+            gd.set_agc(64)
+        elif stage == "fse":
+            gd.set_fractional_equalizer(11, 0.01)
+        elif stage == "eq":
+            gd.set_equalizer(11, 0.01)
+        return gd
+
+    def bits(gd, refuse):
+        cap = gd.bits_bound(x.size)
+        out = torch.zeros(cap + 2, dtype=torch.uint8, device="cuda")
+        nb = torch.zeros(1, dtype=torch.int64, device="cuda")
+        if refuse:
+            with pytest.raises(gpu.QpskCudaError):              # too small: QPSK_ERR_CAPACITY
+                gd.demod_bits_dev(dx.data_ptr(), x.size, x.size, out.data_ptr(), 8, nb.data_ptr())
+            with pytest.raises(gpu.ArgumentException):          # odd output address (uchar2 stores): QPSK_ERR_ARG
+                gd.demod_bits_dev(dx.data_ptr(), x.size, x.size, out.data_ptr() + 1, cap, nb.data_ptr())
+        gd.demod_bits_dev(dx.data_ptr(), x.size, x.size, out.data_ptr(), cap, nb.data_ptr())
+        torch.cuda.synchronize()
+        return "".join("1" if b else "0" for b in out[: int(nb.item())].cpu().numpy())
+
+    def constellation(gd, refuse):
+        # short output refused before the matched filter / MM advance
+        sym = torch.zeros(x.size, dtype=torch.float32, device="cuda")
+        ns = torch.zeros(1, dtype=torch.int32, device="cuda")
+        if refuse:
+            assert L.qpsk_demod_constellation_dev(gd._h, dx.data_ptr(), x.size, x.size, sym.data_ptr(), 8, ns.data_ptr(),
+                                                  None) == gpu._native.ERR_CAPACITY
+        assert L.qpsk_demod_constellation_dev(gd._h, dx.data_ptr(), x.size, x.size, sym.data_ptr(), x.size, ns.data_ptr(),
+                                              None) == 0
+        torch.cuda.synchronize()
+        return sym[: 2 * int(ns.item())].cpu().numpy()
+
+    for use_fll in (False, True):
+        want = orc.QPSKDeModulator(fs, rs, use_fll=use_fll, **kw).DeModulate(x)
+        assert bits(handle(use_fll, None), True) == want and len(want) > 100
+        for stage in ("agc", "fse", "eq"):
+            got = bits(handle(use_fll, stage), True)
+            assert got == bits(handle(use_fll, stage), False) and len(got) > 100, (use_fll, stage)
     wc = orc.QPSKDeModulator(fs, rs, **kw).deModulateConstellation(x)
-    n = int(ns.item())
-    assert 2 * n == wc.size
-    assert np.allclose(sym[: 2 * n].cpu().numpy(), wc, rtol=0, atol=1e-5 * np.abs(wc).max())
+    got = constellation(handle(False, None), True)
+    assert got.size == wc.size
+    assert np.allclose(got, wc, rtol=0, atol=1e-5 * np.abs(wc).max())
+    for stage in ("agc", "fse", "eq"):
+        got = constellation(handle(False, stage), True)
+        assert got.size > 100 and np.array_equal(got.view(np.uint32), constellation(handle(False, stage), False).view(np.uint32)), stage
 
 
 def test_handles_keep_the_device_they_were_created_on(gpu, orc):

@@ -52,6 +52,25 @@ def test_host_batch_demod_pipeline_matches_device_path_and_oracle(gpu, orc, use_
         for rep in range(2):
             w = od.DeModulateBytes(host[c], b"S", b"E")
         assert got[c] == w, c
+    # bits and packed bits from the same host rows, through the same copy chunks, against the device-resident path
+    gb, gp, gdb = (gpu.QPSKDeModulator(FS, RS, ALPHA, 10, **kw) for _ in range(3))
+    cap = gdb.bits_bound(ff)
+    d_bits = torch.zeros((C, cap), dtype=torch.uint8, device="cuda")
+    d_nb = torch.zeros(C, dtype=torch.int64, device="cuda")
+    for rep in range(2):
+        bits, packed = gb.DeModulate(host), gp.DeModulatePacked(host)
+        gdb.demod_bits_dev(rx.data_ptr(), ff, ff, d_bits.data_ptr(), cap, d_nb.data_ptr())
+        torch.cuda.synchronize()
+        db, dn = d_bits.cpu().numpy(), d_nb.cpu().numpy()
+        for c in range(C):
+            row = db[c, : dn[c]]
+            assert bits[c] == (row + ord("0")).tobytes().decode("ascii"), (rep, c)
+            assert packed[c] == (np.packbits(row).tobytes(), int(dn[c])), (rep, c)
+    for c in (0, 299, C - 1):
+        od = orc.QPSKDeModulator(FS, RS, ALPHA, 10, tsc=TSC, use_fll=use_fll)
+        for rep in range(2):
+            w = od.DeModulate(host[c])
+        assert bits[c] == w and len(w) > 1000, c
 
 
 def test_cs16_ingest_equals_cf32_of_the_same_values(gpu, orc):

@@ -77,3 +77,20 @@ def test_geometry_table_reaches_every_variant_the_dispatch_can_produce():
             assert why is not None, ("neither reached nor explained", (diff, mfw, dense, taps, ring))
     # DIFF x {MFW 0, 2, 2-DENSE, 4} x {NB 1, 2, 3, constant bank short, long} x {ring 96, 128}: 19 variants per DIFF
     assert len(reachable) == 2 * 19, len(reachable)
+
+
+def test_chunk_spot_values():
+    assert sd.chunks(2047, 256, True) == 1 and sd.chunks(2048, 256, True) == 6        # the pipeline starts at 2048 samples
+    assert sd.chunks(4196, 4096, True) == 6 and sd.chunks(4196, 4097, True) == 4
+    assert sd.chunks(4196, 256, False) == 1                                           # device source, no FLL: one launch
+    assert sd.chunks(4196, 1024, False, host=True) == 4 and sd.chunks(4196, 1024, False, host=True, cs16=True) == 2
+    assert sd.chunks(4196, 16384, False, host=True) == 6                              # at most six copy chunks
+    assert sd.chunks(300, 16384, False, host=True) == 1                               # chunks of >= 256 samples
+    assert sd.chunks(4196, 2048, True, host=True, fused=False) == 1                   # unfused calls: one chunk
+
+
+def test_route_rows_reach_every_route():
+    got = {name: sd.route(row) for name, row in sd.ROUTE_ROWS.items()}
+    assert {r for r, _ in got.values()} == set(sd.ROUTES), got
+    assert {n for _, n in got.values()} >= {1, 2, 4, 6}, got
+    assert all(n == 1 for r, n in got.values() if not r.startswith("pipeline")), got
