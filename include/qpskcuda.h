@@ -388,6 +388,73 @@ QPSK_API int qpsk_resamp_process(qpsk_resamp* p, const float* iq_in, int64_t n_f
 QPSK_API int qpsk_resamp_process_dev(qpsk_resamp* p, const float* d_in, int64_t n_floats, int64_t in_stride_floats,
                                      float* d_out, int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
 
+/* ---- convolutional code: K = 7, rate 1/2, encoder and soft-decision Viterbi decoder ---------------------------------- */
+/* Not in the reference; forward error correction for the coded receive path
+ *   qpsk_demod_constellation_dev -> qpsk_viterbi_decode_dev -> qpsk_demod_frame_bits_dev.
+ * The code (fixed): register s, the current input bit at bit 6 and the oldest at bit 0; each input bit emits the pair
+ * (c0, c1) = (parity(s & 0171), parity(s & 0133)) (octal), c0 first.  An impulse encodes to 11 10 11 11 00 01 11.  One
+ * pair is one QPSK symbol: c0 is the dibit's first bit (the I bit without differential encoding, the first bit of
+ * DibitToDelta with it), so one trellis step is one symbol.  Bits are bytes 0/1 ([channels][stride]), the format of
+ * qpsk_unpack_bits_dev and qpsk_ber_count_dev.  1..16384 channels (else QPSK_ERR_UNSUPPORTED).
+ * Encoder: the six-bit register of each channel persists across calls (zero at creation and reset), so any chunking of a
+ * stream gives the same bits.  A nonzero input byte is a 1. */
+typedef struct qpsk_conv qpsk_conv;
+QPSK_API int qpsk_conv_create(int channels, qpsk_conv** out);
+QPSK_API int qpsk_conv_destroy(qpsk_conv* p);
+QPSK_API int qpsk_conv_reset(qpsk_conv* p);
+/* host: bits [channels][n_bits] -> out [channels][2*n_bits] */
+QPSK_API int qpsk_conv_encode(qpsk_conv* p, const uint8_t* bits, int64_t n_bits, uint8_t* out);
+/* device: d_bits [channels][bits_stride] (bits_stride >= n_bits, else QPSK_ERR_ARG) -> d_out [channels][out_stride]
+ * (out_stride < 2*n_bits: QPSK_ERR_CAPACITY, nothing consumed); enqueued on `stream` (NULL = the handle's own) */
+QPSK_API int qpsk_conv_encode_dev(qpsk_conv* p, const uint8_t* d_bits, int64_t n_bits, int64_t bits_stride, uint8_t* d_out,
+                                  int64_t out_stride, void* stream);
+/* Decoder, per channel; every rule below is exact, and the GPU is bit-identical to tests/fec_oracle.py.
+ * 1. Soft values, int8, positive = bit 1: q(v) = clamp(rint_half_even(v), -127, 127) (NaN -> 0); every product and sum
+ *    is a separately rounded fp32 operation (no FMA contraction).
+ *      coherent:      s0 = q(scale*I), s1 = q(scale*Q)
+ *      differential:  z = y_k conj(y_{k-1}), re = yr*pr + yi*pi, im = yi*pr - yr*pi;
+ *                     s0 = q(-(scale*(re+im))), s1 = q(scale*(im-re))   (soft form of 00->+1, 01->+j, 11->-1, 10->-j)
+ *    y_{k-1} is carried across calls; the first symbol a handle sees after create, reset or flush yields no step (the
+ *    reference receiver drops its first symbol too).
+ * 2. Add-compare-select over the 64 states S (the last six inputs, the newest at bit 5): branch metric
+ *    sum_i (c_i ? -s_i : s_i), smaller is better; predecessors of a state in increasing state order, a tie keeps the lower;
+ *    every metric starts at 0 (unknown start state); integer metrics, renormalised by subtracting the minimum every 32 steps.
+ * 3. Decisions, B = 32, D = 64: once absolute step (k+1)*B + D - 1 of a channel has been processed, the bits of steps
+ *    [k*B, (k+1)*B) are read off the survivor path of the best state at that step (minimum metric, lowest state on ties).
+ *    A flush reads every step not yet emitted off the best state at the last step, then resets the handle.
+ * Default scales for symbols at unit amplitude (Costas output; the opt-in AGC stage delivers that level), from an oracle
+ * BER sweep (DESIGN.md §3 K13).  In differential mode z scales with the square of the amplitude. */
+#define QPSK_VITERBI_SCALE_COHERENT 32.0f
+#define QPSK_VITERBI_SCALE_DIFFERENTIAL 24.0f
+typedef struct qpsk_viterbi qpsk_viterbi;
+/* differential: 0 / 1; scale finite and > 0 (else QPSK_ERR_RANGE) */
+QPSK_API int qpsk_viterbi_create(int channels, int differential, float scale, qpsk_viterbi** out);
+QPSK_API int qpsk_viterbi_destroy(qpsk_viterbi* p);
+/* back to the state at creation.  Waits for the handle's own stream only. */
+QPSK_API int qpsk_viterbi_reset(qpsk_viterbi* p);
+/* the most bits one decode or flush call over at most max_sym symbols per channel can emit: max_sym + 96 rounded down
+ * to even (whole blocks of 32, plus the up to 95 steps a flush adds) */
+QPSK_API int qpsk_viterbi_bits_bound(const qpsk_viterbi* p, int64_t max_sym, int64_t* cap);
+/* Device: d_sym [channels][sym_stride_floats] cf32 and int d_n_sym[channels] (what qpsk_demod_constellation_dev writes;
+ * ragged, 0 allowed; a count past sym_stride_floats/2 is read as sym_stride_floats/2) -> decided bits d_bits
+ * [channels][bits_cap] and int64 d_n_bits[channels], the layout qpsk_ber_count_dev and qpsk_demod_frame_bits_dev read.
+ * Pointers 8-byte aligned and strides even (else QPSK_ERR_ARG); bits_cap < qpsk_viterbi_bits_bound(sym_stride_floats/2):
+ * QPSK_ERR_CAPACITY before any state advances.  Enqueued on `stream` (NULL = the handle's own); state lives on the device,
+ * so calls on one handle must run in issue order.  Bytes of a row past d_n_bits[c] are not written. */
+QPSK_API int qpsk_viterbi_decode_dev(qpsk_viterbi* p, const float* d_sym, int64_t sym_stride_floats, const int* d_n_sym,
+                                     uint8_t* d_bits, int64_t bits_cap, int64_t* d_n_bits, void* stream);
+/* decode the call's symbols, emit every step not yet emitted, reset the handle */
+QPSK_API int qpsk_viterbi_flush_dev(qpsk_viterbi* p, const float* d_sym, int64_t sym_stride_floats, const int* d_n_sym,
+                                    uint8_t* d_bits, int64_t bits_cap, int64_t* d_n_bits, void* stream);
+/* Host forms (as qpsk_demod_constellation): sym [channels][sym_stride_floats], int64 n_sym[channels] (each in
+ * 0..sym_stride_floats/2, else QPSK_ERR_RANGE) -> bits [channels][bits_cap], n_bits[channels]; bits_cap below
+ * qpsk_viterbi_bits_bound(max n_sym): QPSK_ERR_CAPACITY with that bound in every n_bits[c] and nothing consumed.
+ * Bytes of a row past n_bits[c], up to the longest row of the call, are overwritten. */
+QPSK_API int qpsk_viterbi_decode(qpsk_viterbi* p, const float* sym, int64_t sym_stride_floats, const int64_t* n_sym,
+                                 uint8_t* bits, int64_t bits_cap, int64_t* n_bits);
+QPSK_API int qpsk_viterbi_flush(qpsk_viterbi* p, const float* sym, int64_t sym_stride_floats, const int64_t* n_sym,
+                                uint8_t* bits, int64_t bits_cap, int64_t* n_bits);
+
 /* ---- a6  QPSKModulator  (MS/QPSKModulator.cs:18-168) ---------------------------------------- */
 /* tsc_bits: '0'/'1' string or NULL (null/whitespace = no TSC, :27) */
 QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha, int rrc_span,
@@ -519,6 +586,13 @@ QPSK_API int qpsk_demod_bytes_dev(qpsk_demod* d, const float* d_in, int64_t n_fl
 /* deModulateConstellation, batch/device: d_sym [channels][sym_stride_floats], d_n_sym[channels] */
 QPSK_API int qpsk_demod_constellation_dev(qpsk_demod* d, const float* d_in, int64_t n_floats, int64_t in_stride_floats,
                                           float* d_sym, int64_t sym_stride_floats, int* d_n_sym, void* stream);
+/* qpsk_demod_frame_bits on DEVICE bits: d_bits [channels][bits_stride], one byte 0/1 per bit, int64 d_n_bits[channels]
+ * (each in 0..bits_stride: device memory, not checked) -> d_payload [channels][payload_cap], d_n_bytes[channels] as
+ * qpsk_demod_bytes_dev.  Shares the framer state with the other framer calls.  With qpsk_viterbi_decode_dev it keeps the
+ * coded receive path on the device.  Enqueued on `stream` (NULL = the handle's own), no synchronisation. */
+QPSK_API int qpsk_demod_frame_bits_dev(qpsk_demod* d, const uint8_t* d_bits, int64_t bits_stride, const int64_t* d_n_bits,
+                                       const uint8_t* start_marker, int64_t n_start, const uint8_t* end_marker, int64_t n_end,
+                                       uint8_t* d_payload, int64_t payload_cap, int64_t* d_n_bytes, void* stream);
 /* per-channel loop state after the last call */
 QPSK_API int qpsk_demod_loop_state(qpsk_demod* d, double* costas_theta, double* costas_freq, double* mm_mu,
                                    double* mm_integral, float* fll_phase, float* fll_freq);

@@ -84,6 +84,19 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_resamp_reset(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_resamp_process(IntPtr h, float* iqIn, long nFloats, float* iqOut, long outStrideFloats, out long nOutFloats);
     [DllImport(Lib)] internal static extern int qpsk_resamp_process_dev(IntPtr h, float* dIn, long nFloats, long inStrideFloats, float* dOut, long outStrideFloats, out long nOutFloats, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_conv_create(int channels, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_conv_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_conv_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_conv_encode(IntPtr h, byte* bits, long nBits, byte* output);
+    [DllImport(Lib)] internal static extern int qpsk_conv_encode_dev(IntPtr h, byte* dBits, long nBits, long bitsStride, byte* dOut, long outStride, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_create(int channels, int differential, float scale, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_bits_bound(IntPtr h, long maxSym, out long cap);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_decode_dev(IntPtr h, float* dSym, long symStrideFloats, int* dNSym, byte* dBits, long bitsCap, long* dNBits, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_flush_dev(IntPtr h, float* dSym, long symStrideFloats, int* dNSym, byte* dBits, long bitsCap, long* dNBits, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_decode(IntPtr h, float* sym, long symStrideFloats, long* nSym, byte* bits, long bitsCap, long* nBits);
+    [DllImport(Lib)] internal static extern int qpsk_viterbi_flush(IntPtr h, float* sym, long symStrideFloats, long* nSym, byte* bits, long bitsCap, long* nBits);
     // a6  QPSKModulator                             (MS/QPSKModulator.cs:18,54,104)
     [DllImport(Lib, CharSet = CharSet.Ansi)]
     internal static extern int qpsk_mod_create(int fs, int rs, double alpha, int span, int diff, string? tsc, out IntPtr h);

@@ -483,6 +483,90 @@ namespace QPSK.Models
         }
         public void Dispose() => _o.Dispose();
     }
+
+    // Rate-1/2 K = 7 convolutional encoder (generators 171, 133 octal; not in the reference, definition in qpskcuda.h):
+    // Channels streams of bits as 0/1 bytes, each input bit -> the pair (c0, c1), one QPSK symbol.  The register persists
+    // across calls: any chunking gives the same bits.
+    public sealed unsafe class ConvEncoder : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Channels;
+        public ConvEncoder(int channels = 1)
+        {
+            if (channels < 1 || channels > 16384) throw new ArgumentOutOfRangeException(nameof(channels), "From 1 to 16384 channels.");
+            IntPtr h;
+            QpskCuda.Check(QpskCuda.qpsk_conv_create(channels, out h), nameof(channels));
+            _o = new QpskHandle(h, QpskCuda.qpsk_conv_destroy);
+            Channels = channels;
+        }
+        // bits: [Channels][nBits] 0/1 bytes, nBits = bits.Length / Channels; coded: [Channels][2 * nBits]
+        public void Encode(ReadOnlySpan<byte> bits, Span<byte> coded)
+        {
+            if (bits.Length % Channels != 0) throw new ArgumentException("Input must be Channels rows of equal length.", nameof(bits));
+            if (coded.Length < 2 * bits.Length) throw new ArgumentException("Output must hold two bits per input bit.", nameof(coded));
+            fixed (byte* i = bits) fixed (byte* o = coded)
+                QpskCuda.Check(QpskCuda.qpsk_conv_encode(_h, i, bits.Length / Channels, o), nameof(bits));
+            GC.KeepAlive(this);
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_conv_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
+
+    // Batched soft-decision Viterbi decoder of ConvEncoder's code (not in the reference; exact rules in qpskcuda.h): Costas
+    // output symbols in (deModulateConstellation), decided bits as 0/1 bytes out, one trellis step per symbol.  Bits come out
+    // in blocks of 32, 64 steps behind the newest symbol; Flush emits the rest and resets the decoder.
+    public sealed unsafe class ViterbiDecoder : IDisposable
+    {
+        public const float ScaleCoherent = 32.0f;       // QPSK_VITERBI_SCALE_COHERENT
+        public const float ScaleDifferential = 24.0f;   // QPSK_VITERBI_SCALE_DIFFERENTIAL
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Channels;
+        public ViterbiDecoder(int channels = 1, bool differential = true, float scale = 0.0f)
+        {
+            if (channels < 1 || channels > 16384) throw new ArgumentOutOfRangeException(nameof(channels), "From 1 to 16384 channels.");
+            if (scale == 0.0f) scale = differential ? ScaleDifferential : ScaleCoherent;
+            if (!(scale > 0.0f) || !float.IsFinite(scale)) throw new ArgumentOutOfRangeException(nameof(scale), "scale must be finite and > 0.");
+            IntPtr h;
+            QpskCuda.Check(QpskCuda.qpsk_viterbi_create(channels, differential ? 1 : 0, scale, out h), nameof(scale));
+            _o = new QpskHandle(h, QpskCuda.qpsk_viterbi_destroy);
+            Channels = channels;
+        }
+        public long BitsBound(long maxSymbols)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_viterbi_bits_bound(_h, maxSymbols, out long cap), nameof(maxSymbols));
+            GC.KeepAlive(this);
+            return cap;
+        }
+        // symIQ: [Channels][symStrideFloats] interleaved IQ, nSym[c] symbols used per row; bits: [Channels][bitsCap] with
+        // bitsCap >= BitsBound(max nSym); nBits[c] receives the bits written per row.
+        public void Decode(ReadOnlySpan<float> symIQ, long symStrideFloats, ReadOnlySpan<long> nSym, Span<byte> bits, long bitsCap, Span<long> nBits)
+            => Run(false, symIQ, symStrideFloats, nSym, bits, bitsCap, nBits);
+        public void Flush(ReadOnlySpan<float> symIQ, long symStrideFloats, ReadOnlySpan<long> nSym, Span<byte> bits, long bitsCap, Span<long> nBits)
+            => Run(true, symIQ, symStrideFloats, nSym, bits, bitsCap, nBits);
+        void Run(bool flush, ReadOnlySpan<float> symIQ, long symStrideFloats, ReadOnlySpan<long> nSym, Span<byte> bits, long bitsCap, Span<long> nBits)
+        {
+            if (symStrideFloats < 0 || (symStrideFloats & 1) != 0 || symIQ.Length < Channels * symStrideFloats)
+                throw new ArgumentException("Symbols must be Channels rows of symStrideFloats (even) floats.", nameof(symIQ));
+            if (nSym.Length < Channels || nBits.Length < Channels) throw new ArgumentException("One count per channel.", nameof(nSym));
+            if (bitsCap < 0 || bits.Length < Channels * bitsCap) throw new ArgumentException("Output span is too small for Channels rows of bitsCap.", nameof(bits));
+            fixed (float* s = symIQ) fixed (long* ns = nSym) fixed (byte* b = bits) fixed (long* nb = nBits)
+                QpskCuda.Check(flush ? QpskCuda.qpsk_viterbi_flush(_h, s, symStrideFloats, ns, b, bitsCap, nb)
+                                     : QpskCuda.qpsk_viterbi_decode(_h, s, symStrideFloats, ns, b, bitsCap, nb), nameof(bits));
+            GC.KeepAlive(this);
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_viterbi_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
 }
 
 namespace QPSK

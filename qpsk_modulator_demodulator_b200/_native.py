@@ -141,6 +141,19 @@ def _signatures():
         "qpsk_resamp_reset": (i, [vp]),
         "qpsk_resamp_process": (i, [vp, vp, i64, vp, i64, i64p]),
         "qpsk_resamp_process_dev": (i, [vp, vp, i64, i64, vp, i64, i64p, vp]),
+        "qpsk_conv_create": (i, [i, vpp]),
+        "qpsk_conv_destroy": (i, [vp]),
+        "qpsk_conv_reset": (i, [vp]),
+        "qpsk_conv_encode": (i, [vp, vp, i64, vp]),
+        "qpsk_conv_encode_dev": (i, [vp, vp, i64, i64, vp, i64, vp]),
+        "qpsk_viterbi_create": (i, [i, i, f, vpp]),
+        "qpsk_viterbi_destroy": (i, [vp]),
+        "qpsk_viterbi_reset": (i, [vp]),
+        "qpsk_viterbi_bits_bound": (i, [vp, i64, i64p]),
+        "qpsk_viterbi_decode_dev": (i, [vp, vp, i64, vp, vp, i64, vp, vp]),
+        "qpsk_viterbi_flush_dev": (i, [vp, vp, i64, vp, vp, i64, vp, vp]),
+        "qpsk_viterbi_decode": (i, [vp, vp, i64, vp, vp, i64, vp]),
+        "qpsk_viterbi_flush": (i, [vp, vp, i64, vp, vp, i64, vp]),
         "qpsk_mod_create": (i, [i, i, d, i, i, cp, vpp]),
         "qpsk_mod_destroy": (i, [vp]),
         "qpsk_mod_taps": (i, [vp, f64p, i, i32p]),
@@ -169,6 +182,7 @@ def _signatures():
         "qpsk_demod_bits_bound": (i, [vp, i64, i64p]),
         "qpsk_demod_bytes_dev": (i, [vp, vp, i64, i64, vp, i64, vp, i64, vp, i64, vp, vp]),
         "qpsk_demod_constellation_dev": (i, [vp, vp, i64, i64, vp, i64, vp, vp]),
+        "qpsk_demod_frame_bits_dev": (i, [vp, vp, i64, vp, vp, i64, vp, i64, vp, i64, vp, vp]),
         "qpsk_demod_loop_state": (i, [vp, f64p, f64p, f64p, f64p, f32p, f32p]),
         "qpsk_demod_in_frame": (i, [vp, i32p]),
         "qpsk_demod_channels": (i, [vp, i32p]),

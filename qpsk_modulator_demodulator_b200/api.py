@@ -616,3 +616,95 @@ class Resampler(_Handle):
 
     def reset(self):
         check(lib().qpsk_resamp_reset(self._h))
+
+
+# ---- convolutional code and Viterbi decoder (not in the reference) --------------------------------
+VITERBI_SCALE_COHERENT = 32.0          # QPSK_VITERBI_SCALE_COHERENT: symbols at unit amplitude (DESIGN.md §3 K13)
+VITERBI_SCALE_DIFFERENTIAL = 24.0      # QPSK_VITERBI_SCALE_DIFFERENTIAL
+
+
+class ConvEncoder(_Handle):
+    """Rate-1/2 K = 7 convolutional encoder (generators 171, 133 octal; csrc/fec.cu, definition in include/qpskcuda.h),
+    `channels` streams of bits as 0/1 bytes.  Each input bit gives the pair (c0, c1), c0 first; one pair is one QPSK
+    symbol.  The register persists across calls: any chunking gives the same bits."""
+    _destroy = "qpsk_conv_destroy"
+
+    def __init__(self, channels: int = 1):
+        super().__init__()
+        self.channels = channels
+        check(lib().qpsk_conv_create(channels, C.byref(self._h)))
+
+    def encode(self, bits) -> np.ndarray:
+        """bits: uint8 0/1 [channels, n] (or [n] for one channel) -> uint8 [channels, 2n] (or [2n])."""
+        a = np.ascontiguousarray(bits, np.uint8)
+        rows = a.reshape(self.channels, -1)
+        out = np.zeros((self.channels, 2 * rows.shape[1]), np.uint8)
+        check(lib().qpsk_conv_encode(self._h, _ptr(rows), rows.shape[1], _ptr(out)))
+        return out[0] if (self.channels == 1 and a.ndim == 1) else out
+
+    def encode_dev(self, d_bits: int, n_bits: int, d_out: int, out_stride: int, bits_stride: int = 0, stream: int = 0):
+        """Device pointers: [channels][bits_stride] (0 = n_bits) -> d_out [channels][out_stride], 2 * n_bits per row."""
+        check(lib().qpsk_conv_encode_dev(self._h, d_bits, n_bits, bits_stride or n_bits, d_out, out_stride, stream))
+
+    def reset(self):
+        check(lib().qpsk_conv_reset(self._h))
+
+
+class ViterbiDecoder(_Handle):
+    """Batched soft-decision Viterbi decoder of ConvEncoder's code (csrc/fec.cu; exact rules in include/qpskcuda.h): the
+    Costas output of every channel (QPSKDeModulator.constellation_dev) in, decided bits as 0/1 bytes out, one trellis step
+    per symbol.  `differential` decodes the differential map without a phase reference; `scale` (None = the default of
+    the mode) maps unit-amplitude symbols to int8 soft values.  Bits come out in blocks of 32, 64 steps behind the newest
+    symbol; flush() emits the rest and resets the handle."""
+    _destroy = "qpsk_viterbi_destroy"
+
+    def __init__(self, channels: int = 1, differential: bool = True, scale: float = None):
+        super().__init__()
+        if scale is None:
+            scale = VITERBI_SCALE_DIFFERENTIAL if differential else VITERBI_SCALE_COHERENT
+        self.channels, self.differential, self.scale = channels, bool(differential), float(scale)
+        check(lib().qpsk_viterbi_create(channels, int(differential), scale, C.byref(self._h)))
+
+    def bits_bound(self, max_sym: int) -> int:
+        b = C.c_int64(0)
+        check(lib().qpsk_viterbi_bits_bound(self._h, max_sym, C.byref(b)))
+        return b.value
+
+    def _host(self, fn, sym, n_sym):
+        if sym is None:
+            sym = np.zeros((self.channels, 0), np.complex64)
+        a = np.asarray(sym)
+        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        rows = np.ascontiguousarray(a.reshape(self.channels, -1))
+        stride = rows.shape[1]
+        ns = (np.full(self.channels, stride // 2, np.int64) if n_sym is None
+              else np.ascontiguousarray(np.broadcast_to(np.asarray(n_sym, np.int64), (self.channels,))))
+        cap = self.bits_bound(int(ns.max()) if ns.size else 0)
+        out = np.zeros((self.channels, cap), np.uint8)
+        nb = np.zeros(self.channels, np.int64)
+        check(getattr(lib(), fn)(self._h, _ptr(rows), stride, _ptr(ns), _ptr(out), cap, _ptr(nb)))
+        outs = [out[c, : nb[c]].copy() for c in range(self.channels)]
+        return outs[0] if (self.channels == 1 and np.ndim(sym) == 1) else outs
+
+    def decode(self, sym, n_sym=None):
+        """sym: complex64 [channels, n] (or [n]; interleaved float32 IQ also taken), n_sym: symbols used per channel
+        (default all) -> per channel the uint8 0/1 bits this call completes (a list, or one array for a 1-D input)."""
+        return self._host("qpsk_viterbi_decode", sym, n_sym)
+
+    def flush(self, sym=None, n_sym=None):
+        """decode(), then every bit not yet emitted; the handle is reset afterwards."""
+        return self._host("qpsk_viterbi_flush", sym, n_sym)
+
+    def decode_dev(self, d_sym: int, sym_stride: int, d_n_sym: int, d_bits: int, bits_cap: int, d_n_bits: int,
+                   stream: int = 0):
+        """Device pointers: d_sym [channels][sym_stride] floats with int32 d_n_sym[channels] (what
+        QPSKDeModulator.constellation_dev writes) -> d_bits [channels][bits_cap] uint8, int64 d_n_bits[channels].
+        bits_cap >= bits_bound(sym_stride // 2)."""
+        check(lib().qpsk_viterbi_decode_dev(self._h, d_sym, sym_stride, d_n_sym, d_bits, bits_cap, d_n_bits, stream))
+
+    def flush_dev(self, d_sym: int, sym_stride: int, d_n_sym: int, d_bits: int, bits_cap: int, d_n_bits: int,
+                  stream: int = 0):
+        check(lib().qpsk_viterbi_flush_dev(self._h, d_sym, sym_stride, d_n_sym, d_bits, bits_cap, d_n_bits, stream))
+
+    def reset(self):
+        check(lib().qpsk_viterbi_reset(self._h))

@@ -1880,6 +1880,21 @@ int qpsk_demod_bytes_dev(qpsk_demod* d, const float* d_in, int64_t n_floats, int
                      d_payload, payload_cap, (long long*)d_n_bytes, s);
 }
 
+int qpsk_demod_frame_bits_dev(qpsk_demod* d, const uint8_t* d_bits, int64_t bits_stride, const int64_t* d_n_bits,
+                              const uint8_t* start_marker, int64_t n_start, const uint8_t* end_marker, int64_t n_end,
+                              uint8_t* d_payload, int64_t payload_cap, int64_t* d_n_bytes, void* stream) {
+  if (!d) return QPSK_ERR_NULL;
+  if (n_start == 0 || n_end == 0) return QPSK_ERR_ARG;       // :174-175
+  if (!d_bits || !d_n_bits || !d_payload || !d_n_bytes) return QPSK_ERR_NULL;
+  if (bits_stride < 0) return QPSK_ERR_RANGE;
+  if (payload_cap <= 0) return QPSK_ERR_RANGE;
+  QPSK_TRY(ensure_device(d->eng.device));
+  DemodEngine& e = d->eng;
+  cudaStream_t s = stream ? (cudaStream_t)stream : e.stream;
+  return e.frame_dev(d_bits, bits_stride, (const long long*)d_n_bits, start_marker, n_start, end_marker, n_end, d_payload,
+                     payload_cap, (long long*)d_n_bytes, s);
+}
+
 int qpsk_demod_constellation_dev(qpsk_demod* d, const float* d_in, int64_t n_floats, int64_t in_stride_floats, float* d_sym,
                                  int64_t sym_stride_floats, int* d_n_sym, void* stream) {
   QPSK_TRY(demod_check_in(d, d_in, n_floats));

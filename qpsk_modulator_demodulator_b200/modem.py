@@ -12,7 +12,7 @@ import numpy as np
 
 from . import _native as N
 from ._native import ArgumentNullException, ChanParams, check, lib
-from .api import _Handle, _bytes_arr, _f32, _ptr
+from .api import ConvEncoder, _Handle, _bytes_arr, _f32, _ptr
 
 
 # ---- a6 ---------------------------------------------------------------------------------------
@@ -327,6 +327,22 @@ class QPSKDeModulator(_Handle):
         check(lib().qpsk_demod_bytes_dev(self._h, d_in, n_floats, in_stride or n_floats, _ptr(s), s.size, _ptr(e), e.size,
                                          d_payload, payload_cap, d_n_bytes, stream))
 
+    def constellation_dev(self, d_in: int, n_floats: int, in_stride: int, d_sym: int, sym_stride: int, d_n_sym: int,
+                          stream: int = 0):
+        """deModulateConstellation on device rows: d_in [channels][in_stride] floats (0 = n_floats) -> the Costas output
+        d_sym [channels][sym_stride] floats (sym_stride >= bits_bound(n_floats)) and int32 d_n_sym[channels] symbols, the
+        soft input of api.ViterbiDecoder.decode_dev."""
+        check(lib().qpsk_demod_constellation_dev(self._h, d_in, n_floats, in_stride or n_floats, d_sym, sym_stride, d_n_sym,
+                                                 stream))
+
+    def frame_bits_dev(self, d_bits: int, bits_stride: int, d_n_bits: int, startMarker: bytes, endMarker: bytes,
+                       d_payload: int, payload_cap: int, d_n_bytes: int, stream: int = 0):
+        """FrameBits on device bits: d_bits [channels][bits_stride] 0/1 bytes with int64 d_n_bits[channels] (e.g.
+        api.ViterbiDecoder.decode_dev's output) -> payloads as demod_bytes_dev writes them.  Shares the framer state."""
+        s, e = _bytes_arr(startMarker), _bytes_arr(endMarker)
+        check(lib().qpsk_demod_frame_bits_dev(self._h, d_bits, bits_stride, d_n_bits, _ptr(s), s.size, _ptr(e), e.size,
+                                              d_payload, payload_cap, d_n_bytes, stream))
+
     def loop_state(self):
         Cn = self.channels
         ct, cf, mu, mi = (np.empty(Cn, np.float64) for _ in range(4))
@@ -341,6 +357,24 @@ class QPSKDeModulator(_Handle):
         f = np.zeros(self.channels, np.int32)
         check(lib().qpsk_demod_in_frame(self._h, f.ctypes.data_as(N.i32p)))
         return bool(f[0]) if self.channels == 1 else f.astype(bool)
+
+
+CODED_LEAD_BITS = 32     # zero bits ahead of START: they absorb the decoder's acquisition after the uncoded TSC
+CODED_TAIL_BITS = 6      # zero bits after END: they drive the encoder back to state 0
+
+
+def coded_frame_bits(payload: bytes, startMarker: bytes, endMarker: bytes) -> str:
+    """The '0'/'1' string of one coded frame for QPSKModulator.Modulate, which sends it behind its TSC: 32 zero bits,
+    START, payload, END and 6 zero tail bits, encoded by a freshly reset api.ConvEncoder.  At one symbol rate the coded
+    frame takes twice the symbols of the uncoded one."""
+    raw = np.frombuffer(bytes(startMarker) + bytes(payload) + bytes(endMarker), np.uint8)
+    bits = np.concatenate([np.zeros(CODED_LEAD_BITS, np.uint8), np.unpackbits(raw), np.zeros(CODED_TAIL_BITS, np.uint8)])
+    enc = ConvEncoder(1)
+    try:
+        coded = enc.encode(bits)
+    finally:
+        enc.close()
+    return (coded + ord("0")).tobytes().decode("ascii")
 
 
 # ---- synthetic channel / BER (SURVEY 8f-1, K6, K7) ----------------------------------------------
