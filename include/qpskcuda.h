@@ -455,6 +455,49 @@ QPSK_API int qpsk_viterbi_decode(qpsk_viterbi* p, const float* sym, int64_t sym_
 QPSK_API int qpsk_viterbi_flush(qpsk_viterbi* p, const float* sym, int64_t sym_stride_floats, const int64_t* n_sym,
                                 uint8_t* bits, int64_t bits_cap, int64_t* n_bits);
 
+/* ---- Reed-Solomon outer code over bytes, with byte interleaving -------------------------------------------------------- */
+/* Not in the reference; the outer code around the convolutional code (the concatenated scheme): it corrects the short
+ * byte bursts the Viterbi decoder leaves.  Receive path, all on the device:
+ *   qpsk_demod_constellation_dev -> qpsk_viterbi_flush_dev -> qpsk_demod_frame_bits_dev -> qpsk_rs_decode_dev.
+ * The code (fixed at creation; the GPU is bit-identical to tests/rs_oracle.py):
+ *   field GF(2^8), primitive polynomial x^8 + x^4 + x^3 + x^2 + 1 (0x11d), alpha = 0x02;
+ *   generator g(x) = prod_{j=0}^{nroots-1} (x - alpha^j); nroots even, 2..32, t = nroots/2 symbol errors;
+ *   k >= 1 message bytes, n = k + nroots <= 255 (n < 255: a shortened code);
+ *   codeword bytes c_0..c_{n-1}, c_0 sent first and the coefficient of x^{n-1}; the message is c_0..c_{k-1} and the parity
+ *   c_k..c_{n-1} holds m(x) x^nroots mod g(x) (systematic).
+ * Block: depth I (1..8) codewords interleaved byte by byte into I*n bytes; block byte p is byte p / I of codeword p % I.
+ * So codeword i carries message bytes i, i+I, i+2I, ..., and the first I*k bytes of a block are its message in order.
+ * Decoding rule: a received codeword within Hamming distance t of a codeword of the shortened code becomes that codeword
+ * and its status is the distance (0..t); otherwise its status is -1 and its message bytes come out as received.  A
+ * correction that would fall in the shortened-away positions is a failure.  The kernels implement the rule exactly with
+ * Berlekamp-Massey, Chien search and Forney, accepting a result only when the LFSR length L <= t, deg Lambda = L, Lambda
+ * has exactly L distinct roots among the n valid positions, and every Forney magnitude is nonzero (miscorrections of a
+ * word more than t from the codeword sent are therefore the same on any implementation of the rule).
+ * Statuses are int32, one per codeword, in block order b*I + i.  nroots outside 2..32 or odd, depth outside 1..8:
+ * QPSK_ERR_UNSUPPORTED; k < 1 or n > 255: QPSK_ERR_RANGE.
+ * The handle holds constants only (generator and tables); calls keep no state, so unlike the other handles its calls may
+ * run on any stream, in any order, from any thread. */
+typedef struct qpsk_rs qpsk_rs;
+QPSK_API int qpsk_rs_create(int nroots, int k, int depth, qpsk_rs** out);
+QPSK_API int qpsk_rs_destroy(qpsk_rs* p);
+/* host: msg [n_blocks*I*k] -> code [n_blocks*I*n]; decode: code [n_blocks*I*n] -> msg [n_blocks*I*k], status [n_blocks*I] */
+QPSK_API int qpsk_rs_encode(qpsk_rs* p, const uint8_t* msg, int64_t n_blocks, uint8_t* code);
+QPSK_API int qpsk_rs_decode(qpsk_rs* p, const uint8_t* code, int64_t n_blocks, uint8_t* msg, int* status);
+/* device: n_blocks blocks in every row, d_msg [rows][msg_stride] (msg_stride < n_blocks*I*k: QPSK_ERR_ARG) -> d_code
+ * [rows][code_stride] (code_stride < n_blocks*I*n: QPSK_ERR_CAPACITY).  Enqueued on `stream` (NULL = the handle's own). */
+QPSK_API int qpsk_rs_encode_dev(qpsk_rs* p, const uint8_t* d_msg, int64_t msg_stride, int rows, int64_t n_blocks,
+                                uint8_t* d_code, int64_t code_stride, void* stream);
+/* device, the rows qpsk_demod_frame_bits_dev / qpsk_demod_bytes_dev write: d_code [rows][code_stride] bytes and int64
+ * d_n_bytes[rows], ragged (a count past code_stride is read as code_stride, the framer's "truncated"; a negative one as 0).
+ * Each row decodes count / (I*n) whole blocks and ignores a remainder -> d_msg [rows][msg_stride], int64 d_n_msg[rows] =
+ * blocks*I*k, int32 d_status [rows][status_stride].  msg_stride < (code_stride / (I*n))*I*k or status_stride <
+ * (code_stride / (I*n))*I: QPSK_ERR_CAPACITY before anything is enqueued.  d_n_bytes and d_n_msg 8-byte aligned, d_status
+ * 4-byte aligned (else QPSK_ERR_ARG).  Bytes and statuses of a row past what its count gives are not written.  Enqueued
+ * on `stream` (NULL = the handle's own). */
+QPSK_API int qpsk_rs_decode_dev(qpsk_rs* p, const uint8_t* d_code, int64_t code_stride, const int64_t* d_n_bytes, int rows,
+                                uint8_t* d_msg, int64_t msg_stride, int64_t* d_n_msg, int* d_status, int64_t status_stride,
+                                void* stream);
+
 /* ---- a6  QPSKModulator  (MS/QPSKModulator.cs:18-168) ---------------------------------------- */
 /* tsc_bits: '0'/'1' string or NULL (null/whitespace = no TSC, :27) */
 QPSK_API int qpsk_mod_create(int sample_rate, int symbol_rate, double rrc_alpha, int rrc_span,

@@ -97,6 +97,12 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_viterbi_flush_dev(IntPtr h, float* dSym, long symStrideFloats, int* dNSym, byte* dBits, long bitsCap, long* dNBits, IntPtr stream);
     [DllImport(Lib)] internal static extern int qpsk_viterbi_decode(IntPtr h, float* sym, long symStrideFloats, long* nSym, byte* bits, long bitsCap, long* nBits);
     [DllImport(Lib)] internal static extern int qpsk_viterbi_flush(IntPtr h, float* sym, long symStrideFloats, long* nSym, byte* bits, long bitsCap, long* nBits);
+    [DllImport(Lib)] internal static extern int qpsk_rs_create(int nroots, int k, int depth, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_rs_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_rs_encode(IntPtr h, byte* msg, long nBlocks, byte* code);
+    [DllImport(Lib)] internal static extern int qpsk_rs_decode(IntPtr h, byte* code, long nBlocks, byte* msg, int* status);
+    [DllImport(Lib)] internal static extern int qpsk_rs_encode_dev(IntPtr h, byte* dMsg, long msgStride, int rows, long nBlocks, byte* dCode, long codeStride, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_rs_decode_dev(IntPtr h, byte* dCode, long codeStride, long* dNBytes, int rows, byte* dMsg, long msgStride, long* dNMsg, int* dStatus, long statusStride, IntPtr stream);
     // a6  QPSKModulator                             (MS/QPSKModulator.cs:18,54,104)
     [DllImport(Lib, CharSet = CharSet.Ansi)]
     internal static extern int qpsk_mod_create(int fs, int rs, double alpha, int span, int diff, string? tsc, out IntPtr h);

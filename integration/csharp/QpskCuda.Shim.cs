@@ -567,6 +567,54 @@ namespace QPSK.Models
         }
         public void Dispose() => _o.Dispose();
     }
+
+    // Reed-Solomon outer code over GF(2^8) with depth-interleaved blocks (not in the reference; exact definition and
+    // decoding rule in qpskcuda.h): Nroots parity bytes per K message bytes, N = K + Nroots <= 255, T = Nroots / 2 byte
+    // errors corrected per codeword, Depth codewords interleaved byte by byte per block of BlockBytes.  Stateless: calls
+    // may run on any stream in any order.
+    public sealed unsafe class ReedSolomon : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Nroots, K, Depth;
+        public int N => K + Nroots;
+        public int T => Nroots / 2;
+        public int BlockBytes => Depth * N;
+        public ReedSolomon(int nroots = 32, int k = 223, int depth = 1)
+        {
+            if (nroots < 2 || nroots > 32 || (nroots & 1) != 0) throw new ArgumentOutOfRangeException(nameof(nroots), "nroots must be even, from 2 to 32.");
+            if (k < 1 || k + nroots > 255) throw new ArgumentOutOfRangeException(nameof(k), "k must be >= 1 with k + nroots <= 255.");
+            if (depth < 1 || depth > 8) throw new ArgumentOutOfRangeException(nameof(depth), "From 1 to 8 codewords per block.");
+            IntPtr h;
+            QpskCuda.Check(QpskCuda.qpsk_rs_create(nroots, k, depth, out h), nameof(nroots));
+            _o = new QpskHandle(h, QpskCuda.qpsk_rs_destroy);
+            Nroots = nroots; K = k; Depth = depth;
+        }
+        // message: whole blocks of Depth * K bytes -> code: Depth * N bytes per block
+        public byte[] Encode(ReadOnlySpan<byte> message)
+        {
+            if (message.Length % (Depth * K) != 0) throw new ArgumentException("Message must be whole blocks of Depth * K bytes.", nameof(message));
+            long nBlocks = message.Length / (Depth * K);
+            var code = new byte[nBlocks * BlockBytes];
+            fixed (byte* m = message) fixed (byte* c = code)
+                QpskCuda.Check(QpskCuda.qpsk_rs_encode(_h, m, nBlocks, c), nameof(message));
+            GC.KeepAlive(this);
+            return code;
+        }
+        // code: whole blocks (a remainder is ignored) -> message bytes; status: one per codeword in block order, the bytes
+        // corrected or -1 where the codeword passed through uncorrected
+        public byte[] Decode(ReadOnlySpan<byte> code, out int[] status)
+        {
+            long nBlocks = code.Length / BlockBytes;
+            var message = new byte[nBlocks * Depth * K];
+            status = new int[nBlocks * Depth];
+            fixed (byte* c = code) fixed (byte* m = message) fixed (int* s = status)
+                QpskCuda.Check(QpskCuda.qpsk_rs_decode(_h, c, nBlocks, m, s), nameof(code));
+            GC.KeepAlive(this);
+            return message;
+        }
+        public void Dispose() => _o.Dispose();
+    }
 }
 
 namespace QPSK

@@ -154,6 +154,12 @@ def _signatures():
         "qpsk_viterbi_flush_dev": (i, [vp, vp, i64, vp, vp, i64, vp, vp]),
         "qpsk_viterbi_decode": (i, [vp, vp, i64, vp, vp, i64, vp]),
         "qpsk_viterbi_flush": (i, [vp, vp, i64, vp, vp, i64, vp]),
+        "qpsk_rs_create": (i, [i, i, i, vpp]),
+        "qpsk_rs_destroy": (i, [vp]),
+        "qpsk_rs_encode": (i, [vp, vp, i64, vp]),
+        "qpsk_rs_decode": (i, [vp, vp, i64, vp, vp]),
+        "qpsk_rs_encode_dev": (i, [vp, vp, i64, i, i64, vp, i64, vp]),
+        "qpsk_rs_decode_dev": (i, [vp, vp, i64, vp, i, vp, i64, vp, vp, i64, vp]),
         "qpsk_mod_create": (i, [i, i, d, i, i, cp, vpp]),
         "qpsk_mod_destroy": (i, [vp]),
         "qpsk_mod_taps": (i, [vp, f64p, i, i32p]),

@@ -708,3 +708,66 @@ class ViterbiDecoder(_Handle):
 
     def reset(self):
         check(lib().qpsk_viterbi_reset(self._h))
+
+
+# ---- Reed-Solomon outer code (not in the reference) ------------------------------------------------
+class ReedSolomon(_Handle):
+    """Reed-Solomon code over GF(2^8) with depth-I byte interleaving (csrc/rs.cu; exact definition and decoding rule in
+    include/qpskcuda.h): `nroots` parity bytes (t = nroots / 2 correctable byte errors) per `k` message bytes, n = k +
+    nroots <= 255, `depth` codewords interleaved byte by byte per block.  The outer code around ConvEncoder /
+    ViterbiDecoder: transmit coded_frame_bits(rs.encode(payload), START, END); receive constellation_dev ->
+    ViterbiDecoder.flush_dev -> frame_bits_dev -> decode_dev.  The handle holds constants only: calls may run on any
+    stream in any order."""
+    _destroy = "qpsk_rs_destroy"
+
+    def __init__(self, nroots: int = 32, k: int = 223, depth: int = 1):
+        super().__init__()
+        self.nroots, self.k, self.depth = nroots, k, depth
+        check(lib().qpsk_rs_create(nroots, k, depth, C.byref(self._h)))
+
+    @property
+    def n(self) -> int:
+        return self.k + self.nroots
+
+    @property
+    def t(self) -> int:
+        return self.nroots // 2
+
+    @property
+    def block_bytes(self) -> int:
+        """code bytes per block, depth * n (depth * k of them the message)"""
+        return self.depth * self.n
+
+    def encode(self, msg) -> bytes:
+        """whole blocks of message bytes (a multiple of depth * k) -> their code bytes"""
+        a = _bytes_arr(msg)
+        mb = self.depth * self.k
+        if a.size % mb:
+            raise ArgumentException(f"message length {a.size} is not a multiple of depth * k = {mb}")
+        out = np.zeros(a.size // mb * self.block_bytes, np.uint8)
+        check(lib().qpsk_rs_encode(self._h, _ptr(a), a.size // mb, _ptr(out)))
+        return out.tobytes()
+
+    def decode(self, code):
+        """code bytes (whole blocks; a remainder is ignored) -> (message bytes, int32 status per codeword in block order:
+        the number of bytes corrected, or -1 where the codeword was not within t and passes through as received)"""
+        a = _bytes_arr(code)
+        nb = a.size // self.block_bytes
+        out = np.zeros(nb * self.depth * self.k, np.uint8)
+        st = np.zeros(nb * self.depth, np.int32)
+        check(lib().qpsk_rs_decode(self._h, _ptr(a), nb, _ptr(out), _ptr(st)))
+        return out.tobytes(), st
+
+    def encode_dev(self, d_msg: int, msg_stride: int, rows: int, n_blocks: int, d_code: int, code_stride: int,
+                   stream: int = 0):
+        """Device pointers: n_blocks blocks in every row, d_msg [rows][msg_stride] -> d_code [rows][code_stride]."""
+        check(lib().qpsk_rs_encode_dev(self._h, d_msg, msg_stride, rows, n_blocks, d_code, code_stride, stream))
+
+    def decode_dev(self, d_code: int, code_stride: int, d_n_bytes: int, rows: int, d_msg: int, msg_stride: int,
+                   d_n_msg: int, d_status: int, status_stride: int, stream: int = 0):
+        """Device pointers, the payload rows QPSKDeModulator.frame_bits_dev / demod_bytes_dev write: d_code
+        [rows][code_stride] with int64 d_n_bytes[rows] -> d_msg [rows][msg_stride], int64 d_n_msg[rows], int32 d_status
+        [rows][status_stride]; every row decodes its whole blocks.  msg_stride >= (code_stride // block_bytes) * depth * k,
+        status_stride >= (code_stride // block_bytes) * depth."""
+        check(lib().qpsk_rs_decode_dev(self._h, d_code, code_stride, d_n_bytes, rows, d_msg, msg_stride, d_n_msg, d_status,
+                                       status_stride, stream))
