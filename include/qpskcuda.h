@@ -455,6 +455,75 @@ QPSK_API int qpsk_viterbi_decode(qpsk_viterbi* p, const float* sym, int64_t sym_
 QPSK_API int qpsk_viterbi_flush(qpsk_viterbi* p, const float* sym, int64_t sym_stride_floats, const int64_t* n_sym,
                                 uint8_t* bits, int64_t bits_cap, int64_t* n_bits);
 
+/* ---- soft-decision frame synchronizer for coded frames ---------------------------------------------------------------- */
+/* Not in the reference; it finds coded frames by correlating their known encoded start against the Costas output, so a
+ * frame is found when bits of START are wrong, END is not needed, and in coherent mode the Costas lock phase is resolved.
+ * Receive path, all on the device (slots = qpsk_fsync_slots_bound(max symbols per call)):
+ *   qpsk_demod_constellation_dev -> qpsk_fsync_process_dev -> qpsk_viterbi_flush_dev (a decoder of channels*slots rows,
+ *   over the frame rows and d_frame_n_sym) -> qpsk_pack_bits_dev (d_bits + QPSK_CODED_LEAD_BITS + 8*n_start, max_bits =
+ *   8*payload_bytes) -> qpsk_rs_decode_dev (d_n_bytes from the synchronizer).
+ * Frame format (what modem.coded_frame_bits sends): QPSK_CODED_LEAD_BITS zero bits, START (n_start bytes), payload_bytes
+ * bytes, n_end bytes, QPSK_CODED_TAIL_BITS zero bits, MSB first, encoded from state 0 by the K = 7 code above.  One input
+ * bit is one symbol, so a frame is F = 32 + 8*(n_start + payload_bytes + n_end) + 6 symbols, and its first P = 32 +
+ * 8*n_start symbols are known: the pattern c_0..c_{2P-1}, the code bits of the 32 zeros and START from state 0.
+ * Every rule below is exact, and the GPU is bit-identical to tests/fsync_oracle.py.
+ * 1. Soft values s0(k), s1(k) of symbol k: rule 1 of the decoder above (same q, forms and scale; differential: symbol k
+ *    against symbol k-1).  Positions are absolute symbol indices since create or reset.
+ * 2. Correlation at position p, rotation r (the soft values of y*j^-r: r=1 (s1, -s0), r=2 (-s0, -s1), r=3 (-s1, s0)):
+ *      M_r(p) = sum_{i<P} (c_{2i} ? 1 : -1) s0_r(p+i) + (c_{2i+1} ? 1 : -1) s1_r(p+i);
+ *    coherent: M(p) = max over r = 0..3 (the lowest r on ties); differential: r = 0 only (it is rotation-invariant).
+ *    E(p) = sum_{i<P} |s0(p+i)| + |s1(p+i)|.  Integer arithmetic throughout.
+ * 3. Detection: the search starts at p = delta (delta = 1 differential, 0 coherent).  Position p is decided once symbols
+ *    up to p + 2P - 2 have arrived.  The crossing p0 is the first searched p with E(p) > 0 and 256*M(p) >= rho*E(p); the
+ *    frame is at p* = argmax M over [p0, p0 + P) (the lowest p on ties), with rotation r* and metric M(p*), energy
+ *    E(p*).  Its window is symbols [p* - delta, p* + F), derotated by j^-r* (an exact swap / negation of I and Q); the
+ *    search resumes at p* + F.  A frame goes out in the call after which symbol p* + F - 1 and symbol p0 + 2P - 2 have
+ *    both arrived.  qpsk_viterbi_flush_dev on a window (in the handle's mode) emits exactly F bits, and bit i is frame bit i.
+ * 4. State per channel (a raw-symbol history of 2P + 1 symbols, the search position, a partial frame of up to F + 1
+ *    symbols) lives on the device: any chunking of a stream gives the same frames.
+ * rho: 1..256, 0 = QPSK_FSYNC_RHO_DEFAULT (DESIGN.md §3 K15); scale finite and > 0 (the Viterbi defaults fit); n_start
+ * 1..24, payload_bytes 1..65536, n_end 0..32; outside: QPSK_ERR_RANGE.  1..16384 channels (else QPSK_ERR_UNSUPPORTED). */
+#define QPSK_CODED_LEAD_BITS 32
+#define QPSK_CODED_TAIL_BITS 6
+#define QPSK_FSYNC_RHO_DEFAULT 144
+typedef struct qpsk_fsync qpsk_fsync;
+/* one per slot; position -1 and the rest 0 (channel set) in an empty slot */
+typedef struct qpsk_fsync_frame {
+  int64_t position; /* p* */
+  int32_t metric;   /* M(p*) */
+  int32_t energy;   /* E(p*) */
+  int32_t rotation; /* r*: the window was multiplied by j^-r* */
+  int32_t channel;
+} qpsk_fsync_frame;
+QPSK_API int qpsk_fsync_create(int channels, int differential, float scale, const uint8_t* start_marker, int n_start,
+                               int payload_bytes, int n_end, int rho, qpsk_fsync** out);
+QPSK_API int qpsk_fsync_destroy(qpsk_fsync* p);
+/* back to the state at creation.  Waits for the handle's own stream only. */
+QPSK_API int qpsk_fsync_reset(qpsk_fsync* p);
+/* P, F, the window length F + delta, and the rho in use */
+QPSK_API int qpsk_fsync_shape(const qpsk_fsync* p, int* pattern_syms, int* frame_syms, int* window_syms, int* rho);
+/* the most frames one call over at most max_sym symbols per channel completes: ceil(max_sym / F) (frames do not overlap) */
+QPSK_API int qpsk_fsync_slots_bound(const qpsk_fsync* p, int64_t max_sym, int64_t* slots);
+/* Device: d_sym [channels][sym_stride_floats] cf32 and int d_n_sym[channels] (what qpsk_demod_constellation_dev writes;
+ * ragged, 0 allowed; a count past sym_stride_floats/2 is read as sym_stride_floats/2, a negative one as 0) -> per slot
+ * c*slots + j, the j-th frame channel c completed in this call: the window in d_frames [channels*slots]
+ * [frame_stride_floats] cf32, int d_frame_n_sym (F + delta; 0 for an empty slot; the d_n_sym of qpsk_viterbi_flush_dev),
+ * int64 d_n_bytes (payload_bytes; 0 for an empty slot; the count of qpsk_rs_decode_dev) and d_info.  Pointers 8-byte
+ * aligned and strides even (else QPSK_ERR_ARG); slots < qpsk_fsync_slots_bound(sym_stride_floats/2) or
+ * frame_stride_floats < 2*(F + delta): QPSK_ERR_CAPACITY before anything is enqueued.  Enqueued on `stream` (NULL = the
+ * handle's own); the state advances at enqueue, so calls on one handle must run in issue order.  Frame rows of empty
+ * slots, and floats of a row past its window, are not written. */
+QPSK_API int qpsk_fsync_process_dev(qpsk_fsync* p, const float* d_sym, int64_t sym_stride_floats, const int* d_n_sym,
+                                    int slots, float* d_frames, int64_t frame_stride_floats, int* d_frame_n_sym,
+                                    int64_t* d_n_bytes, qpsk_fsync_frame* d_info, void* stream);
+/* Host form (as qpsk_viterbi_decode): sym [channels][sym_stride_floats], int64 n_sym[channels] (each in
+ * 0..sym_stride_floats/2, else QPSK_ERR_RANGE) -> frames [channels*slots][frame_stride_floats], frame_n_sym, n_bytes and
+ * info [channels*slots]; slots below qpsk_fsync_slots_bound(max n_sym) or a short frame stride: QPSK_ERR_CAPACITY with
+ * that bound in *need_slots and nothing consumed. */
+QPSK_API int qpsk_fsync_process(qpsk_fsync* p, const float* sym, int64_t sym_stride_floats, const int64_t* n_sym, int slots,
+                                float* frames, int64_t frame_stride_floats, int* frame_n_sym, int64_t* n_bytes,
+                                qpsk_fsync_frame* info, int64_t* need_slots);
+
 /* ---- Reed-Solomon outer code over bytes, with byte interleaving -------------------------------------------------------- */
 /* Not in the reference; the outer code around the convolutional code (the concatenated scheme): it corrects the short
  * byte bursts the Viterbi decoder leaves.  Receive path, all on the device:

@@ -97,6 +97,13 @@ internal static unsafe partial class QpskCuda
     [DllImport(Lib)] internal static extern int qpsk_viterbi_flush_dev(IntPtr h, float* dSym, long symStrideFloats, int* dNSym, byte* dBits, long bitsCap, long* dNBits, IntPtr stream);
     [DllImport(Lib)] internal static extern int qpsk_viterbi_decode(IntPtr h, float* sym, long symStrideFloats, long* nSym, byte* bits, long bitsCap, long* nBits);
     [DllImport(Lib)] internal static extern int qpsk_viterbi_flush(IntPtr h, float* sym, long symStrideFloats, long* nSym, byte* bits, long bitsCap, long* nBits);
+    [DllImport(Lib)] internal static extern int qpsk_fsync_create(int channels, int differential, float scale, byte* startMarker, int nStart, int payloadBytes, int nEnd, int rho, out IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_fsync_destroy(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_fsync_reset(IntPtr h);
+    [DllImport(Lib)] internal static extern int qpsk_fsync_shape(IntPtr h, out int patternSyms, out int frameSyms, out int windowSyms, out int rho);
+    [DllImport(Lib)] internal static extern int qpsk_fsync_slots_bound(IntPtr h, long maxSym, out long slots);
+    [DllImport(Lib)] internal static extern int qpsk_fsync_process_dev(IntPtr h, float* dSym, long symStrideFloats, int* dNSym, int slots, float* dFrames, long frameStrideFloats, int* dFrameNSym, long* dNBytes, IntPtr dInfo, IntPtr stream);
+    [DllImport(Lib)] internal static extern int qpsk_fsync_process(IntPtr h, float* sym, long symStrideFloats, long* nSym, int slots, float* frames, long frameStrideFloats, int* frameNSym, long* nBytes, IntPtr info, out long needSlots);
     [DllImport(Lib)] internal static extern int qpsk_rs_create(int nroots, int k, int depth, out IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_rs_destroy(IntPtr h);
     [DllImport(Lib)] internal static extern int qpsk_rs_encode(IntPtr h, byte* msg, long nBlocks, byte* code);

@@ -568,6 +568,67 @@ namespace QPSK.Models
         public void Dispose() => _o.Dispose();
     }
 
+    // One frame found by FrameSync (qpsk_fsync_frame): the window was multiplied by j^-Rotation.
+    [StructLayout(LayoutKind.Sequential)]
+    public struct SyncedFrame
+    {
+        public long Position;   // p*, the absolute symbol index of the frame's first coded symbol
+        public int Metric, Energy, Rotation, Channel;
+    }
+
+    // Soft-decision frame synchronizer for coded frames (not in the reference; exact rules in qpskcuda.h): correlates the
+    // encoded start of a frame (32 zero bits and START) against the Costas output and cuts one window of WindowSymbols per
+    // frame, derotated by the lock phase it found in coherent mode.  Windows go to a ViterbiDecoder of Channels * slots
+    // rows (Flush), the payload starts at PayloadBitOffset of its bits, and ReedSolomon decodes it.
+    public sealed unsafe class FrameSync : IDisposable
+    {
+        readonly QpskHandle _o;
+        IntPtr _h => _o.Ptr;
+        public readonly int Channels, PatternSymbols, FrameSymbols, WindowSymbols, Rho;
+        public int PayloadBitOffset => PatternSymbols;
+        public FrameSync(int channels, bool differential, ReadOnlySpan<byte> startMarker, int payloadBytes, int nEnd, float scale = 0.0f, int rho = 0)
+        {
+            if (channels < 1 || channels > 16384) throw new ArgumentOutOfRangeException(nameof(channels), "From 1 to 16384 channels.");
+            if (startMarker.Length < 1 || startMarker.Length > 24) throw new ArgumentOutOfRangeException(nameof(startMarker), "START must be 1 to 24 bytes.");
+            if (scale == 0.0f) scale = differential ? ViterbiDecoder.ScaleDifferential : ViterbiDecoder.ScaleCoherent;
+            IntPtr h;
+            fixed (byte* s = startMarker)
+                QpskCuda.Check(QpskCuda.qpsk_fsync_create(channels, differential ? 1 : 0, scale, s, startMarker.Length, payloadBytes, nEnd, rho, out h), nameof(payloadBytes));
+            _o = new QpskHandle(h, QpskCuda.qpsk_fsync_destroy);
+            Channels = channels;
+            QpskCuda.Check(QpskCuda.qpsk_fsync_shape(h, out PatternSymbols, out FrameSymbols, out WindowSymbols, out Rho));
+        }
+        public long SlotsBound(long maxSymbols)
+        {
+            QpskCuda.Check(QpskCuda.qpsk_fsync_slots_bound(_h, maxSymbols, out long slots), nameof(maxSymbols));
+            GC.KeepAlive(this);
+            return slots;
+        }
+        // symIQ: [Channels][symStrideFloats] interleaved IQ, nSym[c] symbols per row; slot c * slots + j receives the j-th
+        // frame channel c completes: frames [Channels * slots][frameStrideFloats], frameNSym / nBytes / info per slot (0 and
+        // Position -1 in an empty slot).  slots >= SlotsBound(max nSym), frameStrideFloats >= 2 * WindowSymbols.
+        public void Process(ReadOnlySpan<float> symIQ, long symStrideFloats, ReadOnlySpan<long> nSym, int slots, Span<float> frames,
+                            long frameStrideFloats, Span<int> frameNSym, Span<long> nBytes, Span<SyncedFrame> info)
+        {
+            if (symStrideFloats < 0 || (symStrideFloats & 1) != 0 || symIQ.Length < Channels * symStrideFloats)
+                throw new ArgumentException("Symbols must be Channels rows of symStrideFloats (even) floats.", nameof(symIQ));
+            if (nSym.Length < Channels) throw new ArgumentException("One count per channel.", nameof(nSym));
+            long n = (long)Channels * slots;
+            if (slots < 0 || frames.Length < n * frameStrideFloats || frameNSym.Length < n || nBytes.Length < n || info.Length < n)
+                throw new ArgumentException("Output spans are too small for Channels * slots slots.", nameof(frames));
+            fixed (float* s = symIQ) fixed (long* ns = nSym) fixed (float* f = frames) fixed (int* fn = frameNSym)
+            fixed (long* nb = nBytes) fixed (SyncedFrame* inf = info)
+                QpskCuda.Check(QpskCuda.qpsk_fsync_process(_h, s, symStrideFloats, ns, slots, f, frameStrideFloats, fn, nb, (IntPtr)inf, out long _), nameof(slots));
+            GC.KeepAlive(this);
+        }
+        public void Reset()
+        {
+            QpskCuda.Check(QpskCuda.qpsk_fsync_reset(_h));
+            GC.KeepAlive(this);
+        }
+        public void Dispose() => _o.Dispose();
+    }
+
     // Reed-Solomon outer code over GF(2^8) with depth-interleaved blocks (not in the reference; exact definition and
     // decoding rule in qpskcuda.h): Nroots parity bytes per K message bytes, N = K + Nroots <= 255, T = Nroots / 2 byte
     // errors corrected per codeword, Depth codewords interleaved byte by byte per block of BlockBytes.  Stateless: calls

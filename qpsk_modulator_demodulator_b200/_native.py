@@ -154,6 +154,13 @@ def _signatures():
         "qpsk_viterbi_flush_dev": (i, [vp, vp, i64, vp, vp, i64, vp, vp]),
         "qpsk_viterbi_decode": (i, [vp, vp, i64, vp, vp, i64, vp]),
         "qpsk_viterbi_flush": (i, [vp, vp, i64, vp, vp, i64, vp]),
+        "qpsk_fsync_create": (i, [i, i, f, vp, i, i, i, i, vpp]),
+        "qpsk_fsync_destroy": (i, [vp]),
+        "qpsk_fsync_reset": (i, [vp]),
+        "qpsk_fsync_shape": (i, [vp, i32p, i32p, i32p, i32p]),
+        "qpsk_fsync_slots_bound": (i, [vp, i64, i64p]),
+        "qpsk_fsync_process_dev": (i, [vp, vp, i64, vp, i, vp, i64, vp, vp, vp, vp]),
+        "qpsk_fsync_process": (i, [vp, vp, i64, vp, i, vp, i64, vp, vp, vp, i64p]),
         "qpsk_rs_create": (i, [i, i, i, vpp]),
         "qpsk_rs_destroy": (i, [vp]),
         "qpsk_rs_encode": (i, [vp, vp, i64, vp]),

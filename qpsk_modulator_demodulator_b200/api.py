@@ -771,3 +771,85 @@ class ReedSolomon(_Handle):
         status_stride >= (code_stride // block_bytes) * depth."""
         check(lib().qpsk_rs_decode_dev(self._h, d_code, code_stride, d_n_bytes, rows, d_msg, msg_stride, d_n_msg, d_status,
                                        status_stride, stream))
+
+
+# ---- soft-decision frame synchronizer for coded frames (not in the reference) ------------------------------------------
+FSYNC_RHO_DEFAULT = 144                # QPSK_FSYNC_RHO_DEFAULT (DESIGN.md §3 K15)
+FSYNC_INFO = np.dtype([("position", "<i8"), ("metric", "<i4"), ("energy", "<i4"), ("rotation", "<i4"),
+                       ("channel", "<i4")])                     # qpsk_fsync_frame
+
+
+class FrameSync(_Handle):
+    """Soft-decision frame synchronizer for the coded frames of modem.coded_frame_bits (csrc/fsync.cu; exact rules in
+    include/qpskcuda.h): it correlates the known encoded start (32 zero bits and `start_marker`, P symbols) against the
+    soft values of the Costas output, and cuts one window of F + delta symbols per frame (delta = 1 differential, 0
+    coherent), derotated by the Costas lock phase it found in coherent mode.  `payload_bytes` and `n_end` (the END
+    marker's length) fix F; `rho` (0 = the default) is the detection threshold in 1/256 of the energy.  Receive path:
+    constellation_dev -> process_dev -> ViterbiDecoder(channels * slots).flush_dev -> pack_bits from payload_bit_offset
+    -> ReedSolomon.decode_dev.  State is carried per channel: any chunking of a stream gives the same frames."""
+    _destroy = "qpsk_fsync_destroy"
+
+    def __init__(self, channels: int = 1, differential: bool = True, start_marker: bytes = b"START",
+                 payload_bytes: int = 64, n_end: int = 3, scale: float = None, rho: int = 0):
+        super().__init__()
+        if scale is None:
+            scale = VITERBI_SCALE_DIFFERENTIAL if differential else VITERBI_SCALE_COHERENT
+        s = _bytes_arr(start_marker)
+        self.channels, self.differential, self.scale = channels, bool(differential), float(scale)
+        self.start_marker, self.payload_bytes, self.n_end = bytes(start_marker), payload_bytes, n_end
+        check(lib().qpsk_fsync_create(channels, int(differential), scale, _ptr(s), s.size, payload_bytes, n_end, rho,
+                                      C.byref(self._h)))
+        v = [C.c_int(0) for _ in range(4)]
+        check(lib().qpsk_fsync_shape(self._h, *(C.byref(x) for x in v)))
+        self.pattern_syms, self.frame_syms, self.window_syms, self.rho = (x.value for x in v)
+
+    @property
+    def payload_bit_offset(self) -> int:
+        """where the payload starts in the F bits ViterbiDecoder.flush_dev emits for a window: past the 32 lead bits and
+        START, which are the P pattern symbols"""
+        return self.pattern_syms
+
+    def layout(self) -> dict:
+        """P (pattern symbols), F (frame symbols), the window length F + delta, the payload bit offset and rho"""
+        return dict(P=self.pattern_syms, F=self.frame_syms, window=self.window_syms,
+                    payload_bit_offset=self.payload_bit_offset, rho=self.rho)
+
+    def slots_bound(self, max_sym: int) -> int:
+        b = C.c_int64(0)
+        check(lib().qpsk_fsync_slots_bound(self._h, max_sym, C.byref(b)))
+        return b.value
+
+    def process(self, sym, n_sym=None):
+        """sym: complex64 [channels, n] (or [n]; interleaved float32 IQ also taken), n_sym: symbols used per channel
+        (default all) -> per channel the frames this call completes, a list of (window complex64 [F + delta], info
+        record of FSYNC_INFO); a list per channel, or one list for a 1-D input."""
+        a = np.asarray(sym)
+        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        rows = np.ascontiguousarray(a.reshape(self.channels, -1))
+        stride = rows.shape[1]
+        ns = (np.full(self.channels, stride // 2, np.int64) if n_sym is None
+              else np.ascontiguousarray(np.broadcast_to(np.asarray(n_sym, np.int64), (self.channels,))))
+        slots = self.slots_bound(int(ns.max()) if ns.size else 0)
+        S, L = self.channels * slots, self.window_syms
+        frames = np.zeros((max(S, 1), L), np.complex64)
+        fn = np.zeros(max(S, 1), np.int32)
+        nb = np.zeros(max(S, 1), np.int64)
+        info = np.zeros(max(S, 1), FSYNC_INFO)
+        need = C.c_int64(0)
+        check(lib().qpsk_fsync_process(self._h, _ptr(rows), stride, _ptr(ns), slots, _ptr(frames), 2 * L, _ptr(fn),
+                                       _ptr(nb), _ptr(info), C.byref(need)))
+        outs = [[(frames[c * slots + j].copy(), info[c * slots + j]) for j in range(slots) if fn[c * slots + j] > 0]
+                for c in range(self.channels)]
+        return outs[0] if (self.channels == 1 and np.ndim(sym) == 1) else outs
+
+    def process_dev(self, d_sym: int, sym_stride: int, d_n_sym: int, slots: int, d_frames: int, frame_stride: int,
+                    d_frame_n_sym: int, d_n_bytes: int, d_info: int, stream: int = 0):
+        """Device pointers: d_sym [channels][sym_stride] floats with int32 d_n_sym[channels] (what
+        QPSKDeModulator.constellation_dev writes) -> slot c * slots + j: the j-th frame of channel c in this call, in
+        d_frames [channels * slots][frame_stride] floats, int32 d_frame_n_sym, int64 d_n_bytes and d_info (FSYNC_INFO)
+        per slot.  slots >= slots_bound(sym_stride // 2), frame_stride >= 2 * window_syms."""
+        check(lib().qpsk_fsync_process_dev(self._h, d_sym, sym_stride, d_n_sym, slots, d_frames, frame_stride,
+                                           d_frame_n_sym, d_n_bytes, d_info, stream))
+
+    def reset(self):
+        check(lib().qpsk_fsync_reset(self._h))

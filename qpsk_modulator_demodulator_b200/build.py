@@ -15,7 +15,7 @@ LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(HERE, "build")
 LIB = os.path.join(LIBDIR, "libqpskcuda.so")
 
-SOURCES = ["core.cu", "fir.cu", "util.cu", "loops.cu", "eq.cu", "pfb.cu", "ddc.cu", "agc.cu", "resamp.cu", "fec.cu", "rs.cu", "fll_duo.cu", "fll_pair.cu", "modulator.cu", "demod.cu", "chain.cu", "stream.cu", "channel.cu", "comm.cu"]
+SOURCES = ["core.cu", "fir.cu", "util.cu", "loops.cu", "eq.cu", "pfb.cu", "ddc.cu", "agc.cu", "resamp.cu", "fec.cu", "rs.cu", "fsync.cu", "fll_duo.cu", "fll_pair.cu", "modulator.cu", "demod.cu", "chain.cu", "stream.cu", "channel.cu", "comm.cu"]
 
 # serial-loop kernels restate C# arithmetic in which RyuJIT never fuses a*b+c: no FMA contraction there
 PER_FILE_FLAGS = {"loops.cu": ["--fmad=false"], "eq.cu": ["--fmad=false"], "fll_duo.cu": ["--fmad=false"], "fll_pair.cu": ["--fmad=false"], "demod.cu": ["--fmad=false"], "chain.cu": ["--fmad=false"], "channel.cu": ["--fmad=false"]}

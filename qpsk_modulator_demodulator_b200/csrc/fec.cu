@@ -24,6 +24,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "soft.cuh"
 
 namespace qpsk {
 
@@ -57,9 +58,6 @@ struct VitArgs {
   float scale;
   int flush;
 };
-
-// q(v) = clamp(rint_half_even(v), -127, 127); NaN -> 0 (cvt.rni.s32.f32 saturates and maps NaN to 0)
-__device__ __forceinline__ int vit_q(float v) { return max(-127, min(127, __float2int_rn(v))); }
 
 __device__ __forceinline__ int vit_pack(int s0, int s1) { return (s0 & 0xffff) | (s1 << 16); }
 
@@ -146,7 +144,7 @@ __global__ void __launch_bounds__(32 * kVitWarps) viterbi_kernel(const VitArgs a
   }
   while (i < n) {
     const int chunk = min(n - i, kVitB - (int)(nstep & (kVitB - 1)));
-    int packed = 0;
+    int2 s;
     float2 y = make_float2(0.0f, 0.0f);
     if (lane < chunk) y = x[i + lane];
     if (DIFF) {
@@ -155,14 +153,13 @@ __global__ void __launch_bounds__(32 * kVitWarps) viterbi_kernel(const VitArgs a
         pr = prev.x;
         pi = prev.y;
       }
-      const float re = __fadd_rn(__fmul_rn(y.x, pr), __fmul_rn(y.y, pi));
-      const float im = __fsub_rn(__fmul_rn(y.y, pr), __fmul_rn(y.x, pi));
-      packed = vit_pack(vit_q(-__fmul_rn(a.scale, __fadd_rn(re, im))), vit_q(__fmul_rn(a.scale, __fsub_rn(im, re))));
+      s = soft_differential(y, make_float2(pr, pi), a.scale);
       prev.x = __shfl_sync(kFull, y.x, chunk - 1);
       prev.y = __shfl_sync(kFull, y.y, chunk - 1);
     } else {
-      packed = vit_pack(vit_q(__fmul_rn(a.scale, y.x)), vit_q(__fmul_rn(a.scale, y.y)));
+      s = soft_coherent(y, a.scale);
     }
+    const int packed = vit_pack(s.x, s.y);
     for (int t = 0; t < chunk; ++t) {
       const int w = __shfl_sync(kFull, packed, t);
       const int s0 = (int)(short)(w & 0xffff), s1 = w >> 16;
