@@ -144,6 +144,7 @@ QPSK_API int qpsk_fll_destroy(qpsk_fll* f);
 /* Process(ReadOnlySpan<float>, Span<float>) :64-87 */
 QPSK_API int qpsk_fll_process(qpsk_fll* f, const float* iq_in, float* iq_out, int64_t n_floats,
                               int64_t out_cap_floats);
+/* device memory (8-byte aligned, else QPSK_ERR_ARG), strides in floats */
 QPSK_API int qpsk_fll_process_dev(qpsk_fll* f, const float* d_in, float* d_out, int64_t n_floats,
                                   int64_t in_stride_floats, int64_t out_stride_floats, void* stream);
 /* public fields phase/freq :25-26, per channel */
@@ -158,6 +159,7 @@ QPSK_API int qpsk_mm_destroy(qpsk_mm* m);
  * batch handles: n_sym[channels], out is [channels][cap_floats]). */
 QPSK_API int qpsk_mm_process(qpsk_mm* m, const float* mf_iq_in, int64_t n_floats, float* sym_iq_out,
                              int64_t cap_floats, int* n_sym);
+/* device memory (8-byte aligned, else QPSK_ERR_ARG), strides in floats; d_n_sym[channels] symbols written */
 QPSK_API int qpsk_mm_process_dev(qpsk_mm* m, const float* d_in, int64_t n_floats, int64_t in_stride_floats,
                                  float* d_out, int64_t cap_floats, int64_t out_stride_floats,
                                  int* d_n_sym, void* stream);
@@ -174,7 +176,8 @@ QPSK_API int qpsk_costas_destroy(qpsk_costas* c);
 /* Process(ReadOnlySpan<float>, Span<float>) :98-114 */
 QPSK_API int qpsk_costas_process(qpsk_costas* c, const float* iq_in, float* iq_out, int64_t n_floats,
                                  int64_t out_cap_floats);
-/* batch/device: n_sym[channels] valid complex samples per channel (NULL = n_floats/2 for all) */
+/* batch/device (8-byte aligned, else QPSK_ERR_ARG): n_sym[channels] valid complex samples per channel (NULL = n_floats/2
+ * for all) */
 QPSK_API int qpsk_costas_process_dev(qpsk_costas* c, const float* d_in, float* d_out, int64_t n_floats,
                                      int64_t in_stride_floats, int64_t out_stride_floats,
                                      const int* d_n_sym, void* stream);
@@ -212,7 +215,8 @@ QPSK_API int qpsk_eq_destroy(qpsk_eq* eq);
 QPSK_API int qpsk_eq_reset(qpsk_eq* eq);                      /* taps to the centre spike, window and sample counter zeroed */
 /* host memory, iq_in / iq_out [channels][n_floats]; odd n_floats -> QPSK_ERR_ARG, out_cap_floats < n_floats -> QPSK_ERR_CAPACITY */
 QPSK_API int qpsk_eq_process(qpsk_eq* eq, const float* iq_in, float* iq_out, int64_t n_floats, int64_t out_cap_floats);
-/* device memory, strides in floats; d_n_sym[channels] valid complex symbols per channel (NULL = n_floats/2 for all) */
+/* device memory (8-byte aligned, else QPSK_ERR_ARG), strides in floats; d_n_sym[channels] valid complex symbols per
+ * channel (NULL = n_floats/2 for all) */
 QPSK_API int qpsk_eq_process_dev(qpsk_eq* eq, const float* d_in, float* d_out, int64_t n_floats, int64_t in_stride_floats,
                                  int64_t out_stride_floats, const int* d_n_sym, void* stream);
 /* taps [channels][2*n_taps] interleaved IQ; get: cap_floats < channels*2*n_taps -> QPSK_ERR_CAPACITY; set: n_floats must be
@@ -259,10 +263,10 @@ QPSK_API int qpsk_pfb_reset(qpsk_pfb* p);
  * QPSK_ERR_CAPACITY, nothing consumed.  Floats of a row past *n_out_floats are not written. */
 QPSK_API int qpsk_pfb_process(qpsk_pfb* p, const float* iq_in, int64_t n_floats, float* iq_out,
                               int64_t out_stride_floats, int64_t* n_out_floats);
-/* device memory (8-byte aligned), out_stride_floats even: the [channels][out_stride] rows qpsk_demod_bits_dev /
- * qpsk_demod_bytes_dev read with in_stride = out_stride; pass both calls the same stream (NULL means each handle's own
- * stream, and nothing then orders the demodulator's reads after these writes).  Enqueued on `stream`; the handle's state
- * advances at enqueue, so calls on one handle must run in issue order. */
+/* device memory (8-byte aligned, else QPSK_ERR_ARG), out_stride_floats even: the [channels][out_stride] rows
+ * qpsk_demod_bits_dev / qpsk_demod_bytes_dev read with in_stride = out_stride; pass both calls the same stream (NULL means
+ * each handle's own stream, and nothing then orders the demodulator's reads after these writes).  Enqueued on `stream`;
+ * the handle's state advances at enqueue, so calls on one handle must run in issue order. */
 QPSK_API int qpsk_pfb_process_dev(qpsk_pfb* p, const float* d_in, int64_t n_floats, float* d_out,
                                   int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
 
@@ -303,10 +307,10 @@ QPSK_API int qpsk_ddc_reset(qpsk_ddc* p);
  * QPSK_ERR_CAPACITY, nothing consumed.  Floats of a row past *n_out_floats are not written. */
 QPSK_API int qpsk_ddc_process(qpsk_ddc* p, const float* iq_in, int64_t n_floats, float* iq_out,
                               int64_t out_stride_floats, int64_t* n_out_floats);
-/* device memory (8-byte aligned), out_stride_floats even: the [channels][out_stride] rows qpsk_demod_bits_dev /
- * qpsk_demod_bytes_dev read with in_stride = out_stride; pass both calls the same stream (NULL means each handle's own
- * stream, and nothing then orders the demodulator's reads after these writes).  Enqueued on `stream`; the handle's state
- * advances at enqueue, so calls on one handle must run in issue order. */
+/* device memory (8-byte aligned, else QPSK_ERR_ARG), out_stride_floats even: the [channels][out_stride] rows
+ * qpsk_demod_bits_dev / qpsk_demod_bytes_dev read with in_stride = out_stride; pass both calls the same stream (NULL means
+ * each handle's own stream, and nothing then orders the demodulator's reads after these writes).  Enqueued on `stream`;
+ * the handle's state advances at enqueue, so calls on one handle must run in issue order. */
 QPSK_API int qpsk_ddc_process_dev(qpsk_ddc* p, const float* d_in, int64_t n_floats, float* d_out,
                                   int64_t out_stride_floats, int64_t* n_out_floats, void* stream);
 

@@ -31,6 +31,38 @@ def _bytes_arr(b) -> np.ndarray:
     return np.frombuffer(bytes(b), dtype=np.uint8).copy() if len(b) else np.zeros(0, np.uint8)
 
 
+def _iq(x) -> np.ndarray:
+    """complex64 samples or interleaved float32 IQ -> contiguous interleaved float32 IQ"""
+    a = np.asarray(x)
+    return np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+
+
+def _row_floats(a: np.ndarray) -> int:
+    """floats per channel of a [channels, n] batch, or of a 1-D array"""
+    return a.shape[-1] if a.ndim == 2 else a.size
+
+
+def _sym_counts(n_sym, channels: int, stride: int) -> np.ndarray:
+    """int64 symbols used per channel: all `stride` floats of each row, or `n_sym` broadcast to every channel"""
+    if n_sym is None:
+        return np.full(channels, stride // 2, np.int64)
+    return np.ascontiguousarray(np.broadcast_to(np.asarray(n_sym, np.int64), (channels,)))
+
+
+def _bank_process(fn, h, a: np.ndarray, n_floats: int, rows: int, out_stride: int) -> np.ndarray:
+    """The host call of the blocks whose output count depends on their state: without `out_stride` the call is asked for
+    the floats per output row first (its QPSK_ERR_CAPACITY answer) -> complex64 [rows, n_out]."""
+    n = C.c_int64(0)
+    if not out_stride:
+        st = fn(h, None, n_floats, None, -1, C.byref(n))
+        if st != N.ERR_CAPACITY:
+            check(st)
+        out_stride = n.value
+    y = np.zeros((rows, max(out_stride, 0)), np.float32)
+    check(fn(h, _ptr(a), n_floats, _ptr(y), out_stride, C.byref(n)))
+    return np.ascontiguousarray(y[:, : n.value]).view(np.complex64)
+
+
 # ---- library / device ---------------------------------------------------------------------
 def device_count() -> int:
     n = C.c_int(0)
@@ -180,11 +212,10 @@ class ComplexFIRFilter(_Handle):
     def Filter(self, iqIn, iqOut=None, out_len=None) -> np.ndarray:
         """Filter(ReadOnlySpan<float>, Span<float>) :80-91.  Batch handles: shape [channels, n_floats]."""
         x = _f32(iqIn)
-        n = x.shape[-1] if x.ndim == 2 else x.size
+        n = _row_floats(x)
         if iqOut is None:
             iqOut = np.empty(x.shape if out_len is None else out_len, np.float32)
-        cap = iqOut.shape[-1] if iqOut.ndim == 2 else iqOut.size
-        check(lib().qpsk_fir_filter(self._h, _ptr(x), _ptr(iqOut), n, cap))
+        check(lib().qpsk_fir_filter(self._h, _ptr(x), _ptr(iqOut), n, _row_floats(iqOut)))
         return iqOut
 
     def fftFilter(self, iqData) -> np.ndarray:
@@ -192,7 +223,7 @@ class ComplexFIRFilter(_Handle):
         if iqData is None:
             raise ArgumentNullException("iqData")
         x = _f32(iqData)
-        n = x.shape[-1] if x.ndim == 2 else x.size
+        n = _row_floats(x)
         y = np.empty(x.shape if n % 2 == 0 else 0, np.float32)
         check(lib().qpsk_fir_fft_filter(self._h, _ptr(x), _ptr(y), n))
         return y
@@ -201,7 +232,7 @@ class ComplexFIRFilter(_Handle):
         """Decimate-by-D matched filter (north_star (2)): Filter() kept at stream indices 0, D, 2D, ... across calls.
         Returns the kept samples (interleaved IQ; [channels, n] for batch handles)."""
         x = _f32(iqIn)
-        n = x.shape[-1] if x.ndim == 2 else x.size
+        n = _row_floats(x)
         cap = (2 * ((n // 2 + decim - 1) // max(decim, 1)) + 2) if out_cap_floats is None else out_cap_floats
         y = np.zeros((self.channels, max(cap, 0)), np.float32)
         no = C.c_int64(0)
@@ -260,10 +291,9 @@ class FLLBandEdgeFilter(_Handle):
         """Process(float[]) :90-96 -> the output array; with `outputIQ` given it is Process(ReadOnlySpan<float>,
         Span<float>) :64-87: writes into the caller's array and returns the number of COMPLEX samples processed (:71, :86)."""
         x = _f32(inputIQ)
-        n = x.shape[-1] if x.ndim == 2 else x.size
+        n = _row_floats(x)
         y = outputIQ if outputIQ is not None else np.empty(x.shape if out_len is None else out_len, np.float32)
-        cap = y.shape[-1] if y.ndim == 2 else y.size
-        check(lib().qpsk_fll_process(self._h, _ptr(x), _ptr(y), n, cap))
+        check(lib().qpsk_fll_process(self._h, _ptr(x), _ptr(y), n, _row_floats(y)))
         return (n >> 1) if outputIQ is not None else y
 
     def process_dev(self, d_in, d_out, n_floats, in_stride=0, out_stride=0, stream=0):
@@ -316,12 +346,11 @@ class MuellerMuller(_Handle):
         caller's array ([channels][cap] for batch handles) and returns outSymbols, the number of complex SYMBOLS written
         (:135; an int for one channel, an int array per channel for batch handles)."""
         x = _f32(incomingMfSamplesIQ)
-        n = x.shape[-1] if x.ndim == 2 else x.size
+        n = _row_floats(x)
         ns = np.zeros(self.channels, np.int32)
         if outputSymbolsIQ is not None:
             y = outputSymbolsIQ
-            cap = y.shape[-1] if y.ndim == 2 else y.size
-            check(lib().qpsk_mm_process(self._h, _ptr(x), n, _ptr(y), cap, ns.ctypes.data_as(N.i32p)))
+            check(lib().qpsk_mm_process(self._h, _ptr(x), n, _ptr(y), _row_floats(y), ns.ctypes.data_as(N.i32p)))
             return int(ns[0]) if self.channels == 1 else ns
         cap = n if cap_floats is None else cap_floats
         y = np.zeros((self.channels, max(cap, 0)), np.float32)
@@ -362,10 +391,9 @@ class CostasLoopQpsk(_Handle):
         """Process(float[]) :119-125 -> the output array; with `iqOut` given it is Process(ReadOnlySpan<float>, Span<float>)
         :98-114: writes into the caller's array and returns the number of COMPLEX samples processed (:105, :113)."""
         x = _f32(iqIn)
-        n = x.shape[-1] if x.ndim == 2 else x.size
+        n = _row_floats(x)
         y = iqOut if iqOut is not None else np.empty(x.shape if out_len is None else out_len, np.float32)
-        cap = y.shape[-1] if y.ndim == 2 else y.size
-        check(lib().qpsk_costas_process(self._h, _ptr(x), _ptr(y), n, cap))
+        check(lib().qpsk_costas_process(self._h, _ptr(x), _ptr(y), n, _row_floats(y)))
         return (n >> 1) if iqOut is not None else y
 
     @staticmethod
@@ -397,10 +425,9 @@ class CmaEqualizer(_Handle):
         """-> the equalized symbols (interleaved IQ; [channels, n_floats] for batch handles).  With `iqOut` given the
         outputs go there and the number of complex symbols processed is returned."""
         x = _f32(iqIn)
-        n = x.shape[-1] if x.ndim == 2 else x.size
+        n = _row_floats(x)
         y = iqOut if iqOut is not None else np.empty(x.shape, np.float32)
-        cap = y.shape[-1] if y.ndim == 2 else y.size
-        check(lib().qpsk_eq_process(self._h, _ptr(x), _ptr(y), n, cap))
+        check(lib().qpsk_eq_process(self._h, _ptr(x), _ptr(y), n, _row_floats(y)))
         return (n >> 1) if iqOut is not None else y
 
     def process_dev(self, d_in: int, d_out: int, n_floats: int, in_stride: int = 0, out_stride: int = 0, d_n_sym: int = 0,
@@ -440,8 +467,7 @@ class Agc(_Handle):
     def process(self, x) -> np.ndarray:
         """x: complex64 [channels, n] (or [n] for one channel; interleaved float32 IQ also taken) -> complex64 outputs of
         the same shape, one per input sample."""
-        a = np.asarray(x)
-        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        a = _iq(x)
         rows = a.reshape(self.channels, -1)
         y = np.empty(rows.shape, np.float32)
         check(lib().qpsk_agc_process(self._h, _ptr(rows), _ptr(y), rows.shape[1], rows.shape[1]))
@@ -498,17 +524,8 @@ class PfbChannelizer(_Handle):
     def process(self, x, out_stride: int = 0) -> np.ndarray:
         """x: complex64 samples (or interleaved float32 IQ) of the wideband stream -> complex64 [channels, n_out], the
         outputs this call completes.  `out_stride` (floats) sizes the output rows like the C call; 0 = just enough."""
-        a = np.asarray(x)
-        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
-        n = C.c_int64(0)
-        if not out_stride:
-            st = lib().qpsk_pfb_process(self._h, None, a.size, None, -1, C.byref(n))
-            if st != N.ERR_CAPACITY:
-                check(st)
-            out_stride = n.value
-        y = np.zeros((self.channels, max(out_stride, 0)), np.float32)
-        check(lib().qpsk_pfb_process(self._h, _ptr(a), a.size, _ptr(y), out_stride, C.byref(n)))
-        return np.ascontiguousarray(y[:, : n.value]).view(np.complex64)
+        a = _iq(x)
+        return _bank_process(lib().qpsk_pfb_process, self._h, a, a.size, self.channels, out_stride)
 
     def process_dev(self, d_in: int, n_floats: int, d_out: int, out_stride: int, stream: int = 0) -> int:
         """Device pointers: n_floats of the wideband stream -> d_out [channels][out_stride] floats.  Returns the floats
@@ -546,17 +563,8 @@ class DdcBank(_Handle):
     def process(self, x, out_stride: int = 0) -> np.ndarray:
         """x: complex64 samples (or interleaved float32 IQ) of the wideband stream -> complex64 [channels, n_out], the
         outputs this call completes.  `out_stride` (floats) sizes the output rows like the C call; 0 = just enough."""
-        a = np.asarray(x)
-        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
-        n = C.c_int64(0)
-        if not out_stride:
-            st = lib().qpsk_ddc_process(self._h, None, a.size, None, -1, C.byref(n))
-            if st != N.ERR_CAPACITY:
-                check(st)
-            out_stride = n.value
-        y = np.zeros((self.channels, max(out_stride, 0)), np.float32)
-        check(lib().qpsk_ddc_process(self._h, _ptr(a), a.size, _ptr(y), out_stride, C.byref(n)))
-        return np.ascontiguousarray(y[:, : n.value]).view(np.complex64)
+        a = _iq(x)
+        return _bank_process(lib().qpsk_ddc_process, self._h, a, a.size, self.channels, out_stride)
 
     def process_dev(self, d_in: int, n_floats: int, d_out: int, out_stride: int, stream: int = 0) -> int:
         """Device pointers: n_floats of the wideband stream -> d_out [channels][out_stride] floats.  Returns the floats
@@ -590,18 +598,9 @@ class Resampler(_Handle):
         """x: complex64 [channels, n] (or [n] for one channel; interleaved float32 IQ also taken) -> complex64
         [channels, n_out] (or [n_out]), the outputs this call completes.  `out_stride` (floats) sizes the output rows like
         the C call; 0 = just enough."""
-        a = np.asarray(x)
-        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
+        a = _iq(x)
         rows = a.reshape(self.channels, -1)
-        n = C.c_int64(0)
-        if not out_stride:
-            st = lib().qpsk_resamp_process(self._h, None, rows.shape[1], None, -1, C.byref(n))
-            if st != N.ERR_CAPACITY:
-                check(st)
-            out_stride = n.value
-        y = np.zeros((self.channels, max(out_stride, 0)), np.float32)
-        check(lib().qpsk_resamp_process(self._h, _ptr(rows), rows.shape[1], _ptr(y), out_stride, C.byref(n)))
-        out = np.ascontiguousarray(y[:, : n.value]).view(np.complex64)
+        out = _bank_process(lib().qpsk_resamp_process, self._h, rows, rows.shape[1], self.channels, out_stride)
         return out[0] if (self.channels == 1 and a.ndim == 1) else out
 
     def process_dev(self, d_in: int, n_floats: int, d_out: int, out_stride: int, in_stride: int = 0,
@@ -673,12 +672,9 @@ class ViterbiDecoder(_Handle):
     def _host(self, fn, sym, n_sym):
         if sym is None:
             sym = np.zeros((self.channels, 0), np.complex64)
-        a = np.asarray(sym)
-        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
-        rows = np.ascontiguousarray(a.reshape(self.channels, -1))
+        rows = np.ascontiguousarray(_iq(sym).reshape(self.channels, -1))
         stride = rows.shape[1]
-        ns = (np.full(self.channels, stride // 2, np.int64) if n_sym is None
-              else np.ascontiguousarray(np.broadcast_to(np.asarray(n_sym, np.int64), (self.channels,))))
+        ns = _sym_counts(n_sym, self.channels, stride)
         cap = self.bits_bound(int(ns.max()) if ns.size else 0)
         out = np.zeros((self.channels, cap), np.uint8)
         nb = np.zeros(self.channels, np.int64)
@@ -823,12 +819,9 @@ class FrameSync(_Handle):
         """sym: complex64 [channels, n] (or [n]; interleaved float32 IQ also taken), n_sym: symbols used per channel
         (default all) -> per channel the frames this call completes, a list of (window complex64 [F + delta], info
         record of FSYNC_INFO); a list per channel, or one list for a 1-D input."""
-        a = np.asarray(sym)
-        a = np.ascontiguousarray(a, np.complex64).view(np.float32) if np.iscomplexobj(a) else _f32(a)
-        rows = np.ascontiguousarray(a.reshape(self.channels, -1))
+        rows = np.ascontiguousarray(_iq(sym).reshape(self.channels, -1))
         stride = rows.shape[1]
-        ns = (np.full(self.channels, stride // 2, np.int64) if n_sym is None
-              else np.ascontiguousarray(np.broadcast_to(np.asarray(n_sym, np.int64), (self.channels,))))
+        ns = _sym_counts(n_sym, self.channels, stride)
         slots = self.slots_bound(int(ns.max()) if ns.size else 0)
         S, L = self.channels * slots, self.window_syms
         frames = np.zeros((max(S, 1), L), np.complex64)

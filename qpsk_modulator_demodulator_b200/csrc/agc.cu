@@ -184,18 +184,12 @@ int agc_check_params(int window, float ref, float max_gain) {
   return QPSK_OK;
 }
 
-AgcEngine::~AgcEngine() {
-  if (stream) cudaStreamDestroy(stream);
-}
-
 int AgcEngine::init(int window, float ref_in, float max_gain_in, int channels_in) {
   W = window;
   ref = ref_in;
   max_gain = max_gain_in;
   channels = channels_in;
-  QPSK_TRY(ensure_device());
-  device = current_device();
-  QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+  QPSK_TRY(open());
   for (auto& hb : d_hist) QPSK_TRY(hb.alloc((size_t)channels * (W - 1)));
   QPSK_TRY(d_gain.alloc((size_t)channels));
   QPSK_TRY(reset(stream));
@@ -274,37 +268,15 @@ struct qpsk_agc {
 extern "C" {
 
 int qpsk_agc_create_batch(int window, float ref, float max_gain, int channels, qpsk_agc** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (channels < 1) return QPSK_ERR_RANGE;
   QPSK_TRY(agc_check_params(window, ref, max_gain));
-  qpsk_agc* p = new (std::nothrow) qpsk_agc();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(window, ref, max_gain, channels);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, window, ref, max_gain, channels);
 }
 
-int qpsk_agc_destroy(qpsk_agc* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_agc_destroy(qpsk_agc* p) { return destroy_handle(p); }
 
-int qpsk_agc_reset(qpsk_agc* p) {
-  if (!p) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(p->eng.device));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  QPSK_TRY(p->eng.reset(p->eng.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  return QPSK_OK;
-}
+int qpsk_agc_reset(qpsk_agc* p) { return reset_handle(p); }
 
 int qpsk_agc_process(qpsk_agc* p, const float* iq_in, float* iq_out, int64_t n_floats, int64_t out_cap_floats) {
   if (!p) return QPSK_ERR_NULL;
@@ -314,16 +286,10 @@ int qpsk_agc_process(qpsk_agc* p, const float* iq_in, float* iq_out, int64_t n_f
   if (n_floats == 0) return QPSK_OK;
   if (!iq_in || !iq_out) return QPSK_ERR_NULL;
   AgcEngine& g = p->eng;
-  QPSK_TRY(ensure_device(g.device));
   const int64_t n = n_floats >> 1;
-  const size_t tot = (size_t)n * g.channels;
-  QPSK_TRY(p->d_in.ensure(tot));
-  QPSK_TRY(p->d_out.ensure(tot));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(p->d_in.p, iq_in, tot * 8, cudaMemcpyHostToDevice, g.stream));
-  QPSK_TRY(g.process_dev(p->d_in.p, n, n, p->d_out.p, n, g.stream));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(iq_out, p->d_out.p, tot * 8, cudaMemcpyDeviceToHost, g.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(g.stream));
-  return QPSK_OK;
+  const size_t row = (size_t)n * 8;
+  return host_call(p, iq_in, g.channels, row, iq_out, row, g.channels, row,
+                   [&](const float2* x, float2* y) { return g.process_dev(x, n, n, y, n, g.stream); });
 }
 
 int qpsk_agc_process_dev(qpsk_agc* p, const float* d_in, float* d_out, int64_t n_floats, int64_t in_stride_floats,
@@ -335,7 +301,7 @@ int qpsk_agc_process_dev(qpsk_agc* p, const float* d_in, float* d_out, int64_t n
   if (out_stride_floats < n_floats) return QPSK_ERR_CAPACITY;
   if (n_floats == 0) return QPSK_OK;
   if (!d_in || !d_out) return QPSK_ERR_NULL;
-  if ((reinterpret_cast<uintptr_t>(d_in) & 7) || (reinterpret_cast<uintptr_t>(d_out) & 7)) return QPSK_ERR_ARG;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(p->eng.device));
   return p->eng.process_dev((const float2*)d_in, n_floats >> 1, in_stride_floats >> 1, (float2*)d_out,
                             out_stride_floats >> 1, (cudaStream_t)stream);

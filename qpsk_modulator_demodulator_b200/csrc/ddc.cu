@@ -32,7 +32,7 @@
 #include <algorithm>
 #include <vector>
 
-#include "common.cuh"
+#include "handle.cuh"
 
 namespace qpsk {
 
@@ -153,18 +153,13 @@ static unsigned long long ddc_phase_word(double f) { return (unsigned long long)
 
 static bool ddc_freq_ok(double f) { return isfinite(f) && f >= -0.5 && f < 0.5; }
 
-struct DdcEngine {
-  int device = 0;
+struct DdcEngine : EngineBase {
   int K = 0, D = 0, N = 0, NP = 0, ldg = 0;
   unsigned long long count = 0;          // samples since creation or the last reset
   int cur = 0;                           // which history buffer is live
   DevBuf<float2> d_g;                    // [NP][ldg]
   DevBuf<unsigned long long> d_inc;      // [ldg]
   DevBuf<float2> d_hist[2];              // [N-1 + D-1]
-  cudaStream_t stream = nullptr;
-  ~DdcEngine() {
-    if (stream) cudaStreamDestroy(stream);
-  }
   long long pending() const { return (long long)(count % (unsigned long long)D); }
   long long hist_len() const { return (long long)N - 1 + pending(); }
   int reset(cudaStream_t s) {
@@ -179,9 +174,7 @@ struct DdcEngine {
     N = n_taps;
     NP = (N + kDdcRowAlign - 1) / kDdcRowAlign * kDdcRowAlign;
     ldg = (K + kDdcColAlign - 1) / kDdcColAlign * kDdcColAlign;
-    QPSK_TRY(ensure_device());
-    device = current_device();
-    QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    QPSK_TRY(open());
     std::vector<unsigned long long> inc((size_t)ldg, 0ULL);
     for (int k = 0; k < K; ++k) inc[k] = ddc_phase_word(freqs[k]);
     std::vector<float2> gt((size_t)NP * ldg, make_float2(0.0f, 0.0f));
@@ -257,8 +250,7 @@ struct qpsk_ddc {
 extern "C" {
 
 int qpsk_ddc_create(const float* taps, int n_taps, const double* freqs, int channels, int decim, qpsk_ddc** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (!taps || !freqs) return QPSK_ERR_NULL;
   if (n_taps <= 0) return QPSK_ERR_ARG;
   if (n_taps > kDdcMaxTaps || channels < 1 || channels > kDdcMaxChannels || decim < 1 || decim > kDdcMaxDecim)
@@ -267,33 +259,12 @@ int qpsk_ddc_create(const float* taps, int n_taps, const double* freqs, int chan
     if (!isfinite(taps[i])) return QPSK_ERR_RANGE;
   for (int k = 0; k < channels; ++k)
     if (!ddc_freq_ok(freqs[k])) return QPSK_ERR_RANGE;
-  qpsk_ddc* p = new (std::nothrow) qpsk_ddc();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(taps, n_taps, freqs, channels, decim);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, taps, n_taps, freqs, channels, decim);
 }
 
-int qpsk_ddc_destroy(qpsk_ddc* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_ddc_destroy(qpsk_ddc* p) { return destroy_handle(p); }
 
-int qpsk_ddc_reset(qpsk_ddc* p) {
-  if (!p) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(p->eng.device));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  QPSK_TRY(p->eng.reset(p->eng.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  return QPSK_OK;
-}
+int qpsk_ddc_reset(qpsk_ddc* p) { return reset_handle(p); }
 
 int qpsk_ddc_process(qpsk_ddc* p, const float* iq_in, int64_t n_floats, float* iq_out, int64_t out_stride_floats,
                      int64_t* n_out_floats) {
@@ -306,16 +277,8 @@ int qpsk_ddc_process(qpsk_ddc* p, const float* iq_in, int64_t n_floats, float* i
   if (out_stride_floats < 2 * n_out) return QPSK_ERR_CAPACITY;
   if (n == 0) return QPSK_OK;
   if (!iq_in || (n_out > 0 && !iq_out)) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(g.device));
-  QPSK_TRY(p->d_in.ensure((size_t)n));
-  QPSK_TRY(p->d_out.ensure((size_t)g.K * (size_t)n_out));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(p->d_in.p, iq_in, (size_t)n * 8, cudaMemcpyHostToDevice, g.stream));
-  QPSK_TRY(g.process_dev(p->d_in.p, n, p->d_out.p, n_out, g.stream));
-  if (n_out > 0)
-    QPSK_CUDA_TRY(cudaMemcpy2DAsync(iq_out, (size_t)out_stride_floats * 4, p->d_out.p, (size_t)n_out * 8, (size_t)n_out * 8,
-                                    (size_t)g.K, cudaMemcpyDeviceToHost, g.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(g.stream));
-  return QPSK_OK;
+  return host_call(p, iq_in, 1, (size_t)n * 8, iq_out, (size_t)out_stride_floats * 4, g.K, (size_t)n_out * 8,
+                   [&](const float2* x, float2* y) { return g.process_dev(x, n, y, n_out, g.stream); });
 }
 
 int qpsk_ddc_process_dev(qpsk_ddc* p, const float* d_in, int64_t n_floats, float* d_out, int64_t out_stride_floats,
@@ -329,6 +292,7 @@ int qpsk_ddc_process_dev(qpsk_ddc* p, const float* d_in, int64_t n_floats, float
   if (out_stride_floats < 2 * n_out) return QPSK_ERR_CAPACITY;
   if (n == 0) return QPSK_OK;
   if (!d_in || (n_out > 0 && !d_out)) return QPSK_ERR_NULL;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(g.device));
   return g.process_dev((const float2*)d_in, n, (float2*)d_out, out_stride_floats >> 1, (cudaStream_t)stream);
 }

@@ -163,21 +163,15 @@ __global__ void __launch_bounds__(kEqThreads, S == 1 ? 0 : 8)
   }
 }
 
-EqEngine::~EqEngine() {
-  if (stream) cudaStreamDestroy(stream);
-}
-
 int EqEngine::init(int n_taps, float mu, float modulus, int sps, int channels_in) {
   QPSK_TRY(eq_check_params(n_taps, mu, modulus, sps));
   if (channels_in <= 0) return QPSK_ERR_RANGE;
-  QPSK_TRY(ensure_device());
-  device = current_device();
+  QPSK_TRY(open());
   channels = channels_in;
   P.n_taps = n_taps;
   P.mu = mu;
   P.modulus = modulus;
   P.sps = sps;
-  QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
   QPSK_TRY(d_taps.alloc((size_t)channels * n_taps));
   QPSK_TRY(d_win.alloc((size_t)channels * n_taps));
   QPSK_TRY(d_drop.alloc((size_t)channels));
@@ -245,15 +239,9 @@ struct qpsk_eq {
 extern "C" {
 
 int qpsk_eq_create_fractional(int n_taps, float mu, float modulus, int sps, int channels, qpsk_eq** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   QPSK_TRY(eq_check_params(n_taps, mu, modulus, sps));
-  qpsk_eq* e = new (std::nothrow) qpsk_eq();
-  if (!e) return QPSK_ERR_NOMEM;
-  int st = e->eng.init(n_taps, mu, modulus, sps, channels);
-  if (st != QPSK_OK) { delete e; return st; }
-  *out = e;
-  return QPSK_OK;
+  return create_handle(out, n_taps, mu, modulus, sps, channels);
 }
 int qpsk_eq_create_batch(int n_taps, float mu, float modulus, int channels, qpsk_eq** out) {
   return qpsk_eq_create_fractional(n_taps, mu, modulus, 1, channels, out);
@@ -261,20 +249,8 @@ int qpsk_eq_create_batch(int n_taps, float mu, float modulus, int channels, qpsk
 int qpsk_eq_create(int n_taps, float mu, float modulus, qpsk_eq** out) {
   return qpsk_eq_create_batch(n_taps, mu, modulus, 1, out);
 }
-int qpsk_eq_destroy(qpsk_eq* e) {
-  if (e) {
-    if (e->eng.stream) cudaStreamSynchronize(e->eng.stream);
-    delete e;
-  }
-  return QPSK_OK;
-}
-int qpsk_eq_reset(qpsk_eq* e) {
-  if (!e) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(e->eng.device));
-  QPSK_TRY(e->eng.reset(e->eng.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(e->eng.stream));
-  return QPSK_OK;
-}
+int qpsk_eq_destroy(qpsk_eq* e) { return destroy_handle(e); }
+int qpsk_eq_reset(qpsk_eq* e) { return reset_handle(e); }
 int qpsk_eq_process(qpsk_eq* e, const float* in, float* out, int64_t n_floats, int64_t out_cap_floats) {
   if (!e) return QPSK_ERR_NULL;
   if (n_floats < 0) return QPSK_ERR_RANGE;
@@ -282,23 +258,19 @@ int qpsk_eq_process(qpsk_eq* e, const float* in, float* out, int64_t n_floats, i
   if (out_cap_floats < n_floats) return QPSK_ERR_CAPACITY;
   if (n_floats == 0) return QPSK_OK;
   if (!in || !out) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(e->eng.device));
   EqEngine& g = e->eng;
   const int64_t L = n_floats >> 1;
-  const size_t tot = (size_t)L * g.channels;
-  QPSK_TRY(e->d_in.ensure(tot));
-  QPSK_TRY(e->d_out.ensure(tot));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(e->d_in.p, in, tot * 8, cudaMemcpyHostToDevice, g.stream));
-  QPSK_TRY(g.process_dev(e->d_in.p, e->d_out.p, L, L, L, nullptr, nullptr, false, g.stream));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(out, e->d_out.p, tot * 8, cudaMemcpyDeviceToHost, g.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(g.stream));
-  return QPSK_OK;
+  const size_t row = (size_t)L * 8;
+  return host_call(e, in, g.channels, row, out, row, g.channels, row, [&](const float2* x, float2* y) {
+    return g.process_dev(x, y, L, L, L, nullptr, nullptr, false, g.stream);
+  });
 }
 int qpsk_eq_process_dev(qpsk_eq* e, const float* d_in, float* d_out, int64_t n_floats, int64_t is, int64_t os, const int* d_n_sym,
                         void* stream) {
   if (!e) return QPSK_ERR_NULL;
   if (n_floats < 0) return QPSK_ERR_RANGE;
   if ((n_floats & 1) || (is & 1) || (os & 1)) return QPSK_ERR_ARG;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(e->eng.device));
   return e->eng.process_dev((const float2*)d_in, (float2*)d_out, n_floats >> 1, is >> 1, os >> 1, d_n_sym, nullptr, false,
                             (cudaStream_t)stream);

@@ -3,7 +3,7 @@
 // two CPU restatements in tests/cma_oracle.py (CmaScalar, CmaBatch) agree with it bit for bit; with an update stride,
 // FseScalar and FseBatch in tests/fse_oracle.py.
 #pragma once
-#include "common.cuh"
+#include "handle.cuh"
 
 namespace qpsk {
 
@@ -19,16 +19,13 @@ struct EqParams {
 // the status a parameter set gets: QPSK_ERR_RANGE for mu / modulus, QPSK_ERR_UNSUPPORTED for the tap count or stride
 int eq_check_params(int n_taps, float mu, float modulus, int sps);
 
-struct EqEngine {
+struct EqEngine : EngineBase {
   int channels = 1;
-  int device = 0;
   EqParams P{};
   DevBuf<float2> d_taps;     // [C][N]
   DevBuf<float2> d_win;      // [C][N]: d_win[c][k] = x_{n-k} after the last symbol n (k = N-1 is never read)
   DevBuf<int> d_drop;        // [C] outputs still to discard (process_dev with drop = true)
   DevBuf<int> d_phase;       // [C] stream sample counter mod sps (allocated for sps > 1 only)
-  cudaStream_t stream = nullptr;
-  ~EqEngine();
   int init(int n_taps, float mu, float modulus, int sps, int channels_in);
   // taps to the centre spike w[(N-1)/2] = 1, window zeroed, drop counter (N-1)/2, sample counter 0
   int reset(cudaStream_t s);

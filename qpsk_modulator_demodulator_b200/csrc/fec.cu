@@ -23,7 +23,7 @@
 
 #include <algorithm>
 
-#include "common.cuh"
+#include "handle.cuh"
 #include "soft.cuh"
 
 namespace qpsk {
@@ -232,20 +232,15 @@ __global__ void conv_encode_kernel(const uint8_t* __restrict__ in, long long n, 
   reg[c] = S;
 }
 
-struct ConvEngine {
-  int device = 0, C = 0;
+struct ConvEngine : EngineBase {
+  int C = 0;
   DevBuf<int> d_reg;
-  cudaStream_t stream = nullptr;
-  ~ConvEngine() {
-    if (stream) cudaStreamDestroy(stream);
-  }
+  int reset(cudaStream_t s) { return d_reg.zero(s); }
   int init(int channels) {
     C = channels;
-    QPSK_TRY(ensure_device());
-    device = current_device();
-    QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    QPSK_TRY(open());
     QPSK_TRY(d_reg.alloc((size_t)C));
-    QPSK_TRY(d_reg.zero(stream));
+    QPSK_TRY(reset(stream));
     QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
     return QPSK_OK;
   }
@@ -258,17 +253,13 @@ struct ConvEngine {
   }
 };
 
-struct VitEngine {
-  int device = 0, C = 0;
+struct VitEngine : EngineBase {
+  int C = 0;
   bool diff = false;
   float scale = 1.0f;
   DevBuf<int> d_metric;
   DevBuf<uint2> d_ring;
   DevBuf<VitState> d_st;
-  cudaStream_t stream = nullptr;
-  ~VitEngine() {
-    if (stream) cudaStreamDestroy(stream);
-  }
   int reset(cudaStream_t s) {
     QPSK_TRY(d_metric.zero(s));
     QPSK_TRY(d_ring.zero(s));
@@ -279,9 +270,7 @@ struct VitEngine {
     C = channels;
     diff = differential != 0;
     scale = sc;
-    QPSK_TRY(ensure_device());
-    device = current_device();
-    QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    QPSK_TRY(open());
     QPSK_TRY(d_metric.alloc((size_t)C * kVitStates));
     QPSK_TRY(d_ring.alloc((size_t)C * kVitRing));
     QPSK_TRY(d_st.alloc((size_t)C));
@@ -340,41 +329,17 @@ struct qpsk_viterbi {
   DevBuf<long long> d_nbits;
 };
 
-static bool misaligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7) != 0; }
-
 extern "C" {
 
 int qpsk_conv_create(int channels, qpsk_conv** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (channels < 1 || channels > kFecMaxChannels) return QPSK_ERR_UNSUPPORTED;
-  qpsk_conv* p = new (std::nothrow) qpsk_conv();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(channels);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, channels);
 }
 
-int qpsk_conv_destroy(qpsk_conv* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_conv_destroy(qpsk_conv* p) { return destroy_handle(p); }
 
-int qpsk_conv_reset(qpsk_conv* p) {
-  if (!p) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(p->eng.device));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  QPSK_TRY(p->eng.d_reg.zero(p->eng.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  return QPSK_OK;
-}
+int qpsk_conv_reset(qpsk_conv* p) { return reset_handle(p); }
 
 int qpsk_conv_encode(qpsk_conv* p, const uint8_t* bits, int64_t n_bits, uint8_t* out) {
   if (!p) return QPSK_ERR_NULL;
@@ -382,15 +347,9 @@ int qpsk_conv_encode(qpsk_conv* p, const uint8_t* bits, int64_t n_bits, uint8_t*
   if (n_bits == 0) return QPSK_OK;
   if (!bits || !out) return QPSK_ERR_NULL;
   ConvEngine& g = p->eng;
-  QPSK_TRY(ensure_device(g.device));
-  const size_t C = (size_t)g.C, n = (size_t)n_bits;
-  QPSK_TRY(p->d_in.ensure(C * n));
-  QPSK_TRY(p->d_out.ensure(2 * C * n));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(p->d_in.p, bits, C * n, cudaMemcpyHostToDevice, g.stream));
-  QPSK_TRY(g.encode_dev(p->d_in.p, n_bits, n_bits, p->d_out.p, 2 * n_bits, g.stream));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(out, p->d_out.p, 2 * C * n, cudaMemcpyDeviceToHost, g.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(g.stream));
-  return QPSK_OK;
+  const size_t n = (size_t)n_bits;
+  return host_call(p, bits, g.C, n, out, 2 * n, g.C, 2 * n,
+                   [&](const uint8_t* x, uint8_t* y) { return g.encode_dev(x, n_bits, n_bits, y, 2 * n_bits, g.stream); });
 }
 
 int qpsk_conv_encode_dev(qpsk_conv* p, const uint8_t* d_bits, int64_t n_bits, int64_t bits_stride, uint8_t* d_out,
@@ -406,37 +365,15 @@ int qpsk_conv_encode_dev(qpsk_conv* p, const uint8_t* d_bits, int64_t n_bits, in
 }
 
 int qpsk_viterbi_create(int channels, int differential, float scale, qpsk_viterbi** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (channels < 1 || channels > kFecMaxChannels) return QPSK_ERR_UNSUPPORTED;
   if (!(scale > 0.0f) || !isfinite(scale)) return QPSK_ERR_RANGE;
-  qpsk_viterbi* p = new (std::nothrow) qpsk_viterbi();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(channels, differential, scale);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, channels, differential, scale);
 }
 
-int qpsk_viterbi_destroy(qpsk_viterbi* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_viterbi_destroy(qpsk_viterbi* p) { return destroy_handle(p); }
 
-int qpsk_viterbi_reset(qpsk_viterbi* p) {
-  if (!p) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(p->eng.device));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  QPSK_TRY(p->eng.reset(p->eng.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  return QPSK_OK;
-}
+int qpsk_viterbi_reset(qpsk_viterbi* p) { return reset_handle(p); }
 
 int qpsk_viterbi_bits_bound(const qpsk_viterbi* p, int64_t max_sym, int64_t* cap) {
   if (!p || !cap) return QPSK_ERR_NULL;
@@ -451,7 +388,7 @@ static int viterbi_dev(qpsk_viterbi* p, const float* d_sym, int64_t sym_stride_f
   if (!d_sym || !d_n_sym || !d_bits || !d_n_bits) return QPSK_ERR_NULL;
   if (sym_stride_floats < 0 || bits_cap < 0) return QPSK_ERR_RANGE;
   if ((sym_stride_floats & 1) || (bits_cap & 1)) return QPSK_ERR_ARG;
-  if (misaligned8(d_sym) || misaligned8(d_n_sym) || misaligned8(d_bits) || misaligned8(d_n_bits)) return QPSK_ERR_ARG;
+  if (misaligned(d_sym) || misaligned(d_n_sym) || misaligned(d_bits) || misaligned(d_n_bits)) return QPSK_ERR_ARG;
   if (sym_stride_floats / 2 > INT_MAX) return QPSK_ERR_UNSUPPORTED;
   if (bits_cap < vit_bits_bound(sym_stride_floats / 2)) return QPSK_ERR_CAPACITY;
   QPSK_TRY(ensure_device(p->eng.device));
@@ -476,12 +413,8 @@ static int viterbi_host(qpsk_viterbi* p, const float* sym, int64_t sym_stride_fl
   if (sym_stride_floats & 1) return QPSK_ERR_ARG;
   VitEngine& g = p->eng;
   const size_t C = (size_t)g.C;
-  int64_t max_sym = 0;
-  for (size_t c = 0; c < C; ++c) {
-    if (n_sym[c] < 0 || n_sym[c] > sym_stride_floats / 2) return QPSK_ERR_RANGE;
-    max_sym = std::max(max_sym, n_sym[c]);
-  }
-  if (max_sym > INT_MAX) return QPSK_ERR_UNSUPPORTED;
+  int64_t max_sym;
+  QPSK_TRY(host_sym_counts(n_sym, C, sym_stride_floats, &max_sym));
   if (bits_cap < vit_bits_bound(max_sym)) {
     for (size_t c = 0; c < C; ++c) n_bits[c] = vit_bits_bound(max_sym);
     return QPSK_ERR_CAPACITY;
@@ -491,16 +424,9 @@ static int viterbi_host(qpsk_viterbi* p, const float* sym, int64_t sym_stride_fl
   QPSK_TRY(ensure_device(g.device));
   cudaStream_t s = g.stream;
   const long long lds = std::max<long long>(max_sym, 1), ldb = vit_bits_bound(max_sym);
-  QPSK_TRY(p->d_sym.ensure(C * (size_t)lds));
-  QPSK_TRY(p->d_nsym.ensure(C));
   QPSK_TRY(p->d_bits.ensure(C * (size_t)ldb));
   QPSK_TRY(p->d_nbits.ensure(C));
-  std::vector<int> ns(C);
-  for (size_t c = 0; c < C; ++c) ns[c] = (int)n_sym[c];
-  if (max_sym > 0)
-    QPSK_CUDA_TRY(cudaMemcpy2DAsync(p->d_sym.p, (size_t)lds * 8, sym, (size_t)sym_stride_floats * 4, (size_t)max_sym * 8, C,
-                                    cudaMemcpyHostToDevice, s));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(p->d_nsym.p, ns.data(), C * sizeof(int), cudaMemcpyHostToDevice, s));
+  QPSK_TRY(upload_syms(p->d_sym, p->d_nsym, sym, sym_stride_floats, n_sym, C, max_sym, s));
   QPSK_TRY(g.run(p->d_sym.p, lds, p->d_nsym.p, p->d_bits.p, ldb, p->d_nbits.p, flush, s));
   QPSK_CUDA_TRY(cudaMemcpyAsync(n_bits, p->d_nbits.p, C * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
   QPSK_CUDA_TRY(cudaStreamSynchronize(s));

@@ -17,7 +17,7 @@
 
 #include <algorithm>
 
-#include "common.cuh"
+#include "handle.cuh"
 #include "soft.cuh"
 
 namespace qpsk {
@@ -264,17 +264,13 @@ __global__ void __launch_bounds__(32 * kFsWarps) fsync_kernel(const FsArgs a) {
   }
 }
 
-struct FsEngine {
-  int device = 0, C = 0, P = 0, F = 0, H = 0, payload = 0, rho = 0;
+struct FsEngine : EngineBase {
+  int C = 0, P = 0, F = 0, H = 0, payload = 0, rho = 0;
   bool diff = false;
   float scale = 1.0f;
   DevBuf<int2> d_pattern;
   DevBuf<FsState> d_st;
   DevBuf<float2> d_hist, d_fbuf;
-  cudaStream_t stream = nullptr;
-  ~FsEngine() {
-    if (stream) cudaStreamDestroy(stream);
-  }
   int delta() const { return diff ? 1 : 0; }
   int reset(cudaStream_t s) {
     std::vector<FsState> st((size_t)C);
@@ -326,9 +322,7 @@ struct FsEngine {
         const unsigned wy = byte(-A[1]) | byte(A[0]) << 8 | byte(-B[1]) << 16 | byte(B[0]) << 24;
         pat[sh * kFsPatWords + i] = make_int2((int)wx, (int)wy);
       }
-    QPSK_TRY(ensure_device());
-    device = current_device();
-    QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    QPSK_TRY(open());
     QPSK_TRY(d_pattern.alloc(pat.size()));
     QPSK_TRY(d_st.alloc((size_t)C));
     QPSK_TRY(d_hist.alloc((size_t)C * 2 * H));
@@ -387,45 +381,23 @@ struct qpsk_fsync {
   DevBuf<qpsk_fsync_frame> d_info;
 };
 
-static bool fs_misaligned8(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 7) != 0; }
-
 extern "C" {
 
 int qpsk_fsync_create(int channels, int differential, float scale, const uint8_t* start_marker, int n_start,
                       int payload_bytes, int n_end, int rho, qpsk_fsync** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (!start_marker) return QPSK_ERR_NULL;
   if (channels < 1 || channels > kFsMaxChannels) return QPSK_ERR_UNSUPPORTED;
   if (!(scale > 0.0f) || !isfinite(scale)) return QPSK_ERR_RANGE;
   if (n_start < 1 || n_start > kFsMaxStart || payload_bytes < 1 || payload_bytes > kFsMaxPayload || n_end < 0 ||
       n_end > kFsMaxEnd || rho < 0 || rho > 256)
     return QPSK_ERR_RANGE;
-  qpsk_fsync* p = new (std::nothrow) qpsk_fsync();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(channels, differential, scale, start_marker, n_start, payload_bytes, n_end, rho);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, channels, differential, scale, start_marker, n_start, payload_bytes, n_end, rho);
 }
 
-int qpsk_fsync_destroy(qpsk_fsync* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_fsync_destroy(qpsk_fsync* p) { return destroy_handle(p); }
 
-int qpsk_fsync_reset(qpsk_fsync* p) {
-  if (!p) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(p->eng.device));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  return p->eng.reset(p->eng.stream);
-}
+int qpsk_fsync_reset(qpsk_fsync* p) { return reset_handle(p); }
 
 int qpsk_fsync_shape(const qpsk_fsync* p, int* pattern_syms, int* frame_syms, int* window_syms, int* rho) {
   if (!p || !pattern_syms || !frame_syms || !window_syms || !rho) return QPSK_ERR_NULL;
@@ -450,8 +422,8 @@ int qpsk_fsync_process_dev(qpsk_fsync* p, const float* d_sym, int64_t sym_stride
   if (!d_sym || !d_n_sym || !d_frames || !d_frame_n_sym || !d_n_bytes || !d_info) return QPSK_ERR_NULL;
   if (sym_stride_floats < 0 || frame_stride_floats < 0 || slots < 0) return QPSK_ERR_RANGE;
   if ((sym_stride_floats & 1) || (frame_stride_floats & 1)) return QPSK_ERR_ARG;
-  if (fs_misaligned8(d_sym) || fs_misaligned8(d_n_sym) || fs_misaligned8(d_frames) || fs_misaligned8(d_frame_n_sym) ||
-      fs_misaligned8(d_n_bytes) || fs_misaligned8(d_info))
+  if (misaligned(d_sym) || misaligned(d_n_sym) || misaligned(d_frames) || misaligned(d_frame_n_sym) ||
+      misaligned(d_n_bytes) || misaligned(d_info))
     return QPSK_ERR_ARG;
   if (sym_stride_floats / 2 > INT_MAX) return QPSK_ERR_UNSUPPORTED;
   const FsEngine& g = p->eng;
@@ -470,12 +442,8 @@ int qpsk_fsync_process(qpsk_fsync* p, const float* sym, int64_t sym_stride_float
   if ((sym_stride_floats & 1) || (frame_stride_floats & 1)) return QPSK_ERR_ARG;
   FsEngine& g = p->eng;
   const size_t C = (size_t)g.C;
-  int64_t max_sym = 0;
-  for (size_t c = 0; c < C; ++c) {
-    if (n_sym[c] < 0 || n_sym[c] > sym_stride_floats / 2) return QPSK_ERR_RANGE;
-    max_sym = std::max(max_sym, n_sym[c]);
-  }
-  if (max_sym > INT_MAX) return QPSK_ERR_UNSUPPORTED;
+  int64_t max_sym;
+  QPSK_TRY(host_sym_counts(n_sym, C, sym_stride_floats, &max_sym));
   *need_slots = g.slots_bound(max_sym);
   const long long L = g.F + g.delta();
   if (slots < *need_slots || frame_stride_floats < 2 * L) return QPSK_ERR_CAPACITY;
@@ -485,18 +453,11 @@ int qpsk_fsync_process(qpsk_fsync* p, const float* sym, int64_t sym_stride_float
   QPSK_TRY(ensure_device(g.device));
   cudaStream_t s = g.stream;
   const long long lds = std::max<long long>(max_sym, 1);
-  QPSK_TRY(p->d_sym.ensure(C * (size_t)lds));
-  QPSK_TRY(p->d_nsym.ensure(C));
   QPSK_TRY(p->d_frames.ensure(std::max<size_t>(S, 1) * (size_t)L));
   QPSK_TRY(p->d_fn.ensure(std::max<size_t>(S, 1)));
   QPSK_TRY(p->d_nb.ensure(std::max<size_t>(S, 1)));
   QPSK_TRY(p->d_info.ensure(std::max<size_t>(S, 1)));
-  std::vector<int> ns(C);
-  for (size_t c = 0; c < C; ++c) ns[c] = (int)n_sym[c];
-  if (max_sym > 0)
-    QPSK_CUDA_TRY(cudaMemcpy2DAsync(p->d_sym.p, (size_t)lds * 8, sym, (size_t)sym_stride_floats * 4, (size_t)max_sym * 8, C,
-                                    cudaMemcpyHostToDevice, s));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(p->d_nsym.p, ns.data(), C * sizeof(int), cudaMemcpyHostToDevice, s));
+  QPSK_TRY(upload_syms(p->d_sym, p->d_nsym, sym, sym_stride_floats, n_sym, C, max_sym, s));
   QPSK_TRY(g.run(p->d_sym.p, lds, p->d_nsym.p, slots, p->d_frames.p, L, p->d_fn.p, p->d_nb.p, p->d_info.p, s));
   if (S > 0) {
     QPSK_CUDA_TRY(cudaMemcpyAsync(frame_n_sym, p->d_fn.p, S * sizeof(int), cudaMemcpyDeviceToHost, s));

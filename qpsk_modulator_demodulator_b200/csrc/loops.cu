@@ -133,10 +133,6 @@ __global__ void __launch_bounds__(kFllCtaThreads)
   }
 }
 
-FllEngine::~FllEngine() {
-  if (stream) cudaStreamDestroy(stream);
-}
-
 int FllEngine::init(float sps, float rolloff, int size, float bw, int channels_in) {
   if (!(sps > 0.0f)) return QPSK_ERR_RANGE;                  // Band-Edge Filter.cs:42
   if (rolloff < 0 || rolloff > 1.0f) return QPSK_ERR_RANGE;  // :43
@@ -144,8 +140,7 @@ int FllEngine::init(float sps, float rolloff, int size, float bw, int channels_i
   if (!(bw > 0.0f)) return QPSK_ERR_RANGE;                   // :45
   if (channels_in <= 0) return QPSK_ERR_RANGE;
   if (fll_group_smem(size) > kFllGroupMaxSmem) return QPSK_ERR_UNSUPPORTED;   // the ring lives in shared memory: N <= 1430
-  QPSK_TRY(ensure_device());
-  device = current_device();
+  QPSK_TRY(open());
   channels = channels_in;
   n_taps = size;
   P.alpha = 0.0f;                        // :55
@@ -159,7 +154,6 @@ int FllEngine::init(float sps, float rolloff, int size, float bw, int channels_i
     rev[(size_t)i] = lower[2 * (size_t)(size - 1 - i)];
     rev[(size_t)size + i] = lower[2 * (size_t)(size - 1 - i) + 1];
   }
-  QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
   QPSK_TRY(d_taps.alloc(rev.size()));
   QPSK_TRY(d_ring.alloc((size_t)size * channels));
   QPSK_TRY(d_head.alloc((size_t)channels));
@@ -254,17 +248,11 @@ __global__ void mm_init_kernel(MmState* st, int C) {
   st[c] = S;
 }
 
-MmEngine::~MmEngine() {
-  if (stream) cudaStreamDestroy(stream);
-}
-
 int MmEngine::init(double sps, double kp, double ki, int channels_in) {
   if (channels_in <= 0) return QPSK_ERR_RANGE;
-  QPSK_TRY(ensure_device());
-  device = current_device();
+  QPSK_TRY(open());
   channels = channels_in;
   P.sps = sps; P.kp = kp; P.ki = ki;
-  QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
   QPSK_TRY(d_state.alloc((size_t)channels));
   mm_init_kernel<<<(channels + 127) / 128, 128, 0, stream>>>(d_state.p, channels);
   QPSK_LAUNCH_CHECK();
@@ -340,17 +328,11 @@ __global__ void __launch_bounds__(kLoopThreads)
   st_g[c] = S;
 }
 
-CostasEngine::~CostasEngine() {
-  if (stream) cudaStreamDestroy(stream);
-}
-
 int CostasEngine::init(double fs, double bw, double damping, int channels_in) {
   if (channels_in <= 0) return QPSK_ERR_RANGE;
-  QPSK_TRY(ensure_device());
-  device = current_device();
+  QPSK_TRY(open());
   channels = channels_in;
   costas_gains(fs, bw, damping, &P.alpha, &P.beta);
-  QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
   QPSK_TRY(d_state.alloc((size_t)channels));
   QPSK_TRY(d_state.zero(stream));   // theta = freq = 0 (:46-47)
   QPSK_CUDA_TRY(cudaStreamSynchronize(stream));
@@ -393,25 +375,13 @@ extern "C" {
 
 // ---- FLL ----
 int qpsk_fll_create_batch(float sps, float rolloff, int filter_size, float bandwidth, int channels, qpsk_fll** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
-  qpsk_fll* f = new (std::nothrow) qpsk_fll();
-  if (!f) return QPSK_ERR_NOMEM;
-  int st = f->eng.init(sps, rolloff, filter_size, bandwidth, channels);
-  if (st != QPSK_OK) { delete f; return st; }
-  *out = f;
-  return QPSK_OK;
+  QPSK_TRY(clear_out(out));
+  return create_handle(out, sps, rolloff, filter_size, bandwidth, channels);
 }
 int qpsk_fll_create(float sps, float rolloff, int filter_size, float bandwidth, qpsk_fll** out) {
   return qpsk_fll_create_batch(sps, rolloff, filter_size, bandwidth, 1, out);
 }
-int qpsk_fll_destroy(qpsk_fll* f) {
-  if (f) {
-    if (f->eng.stream) cudaStreamSynchronize(f->eng.stream);
-    delete f;
-  }
-  return QPSK_OK;
-}
+int qpsk_fll_destroy(qpsk_fll* f) { return destroy_handle(f); }
 int qpsk_fll_process(qpsk_fll* f, const float* in, float* out, int64_t n_floats, int64_t out_cap_floats) {
   if (!f) return QPSK_ERR_NULL;
   if (n_floats < 0) return QPSK_ERR_RANGE;
@@ -419,22 +389,17 @@ int qpsk_fll_process(qpsk_fll* f, const float* in, float* out, int64_t n_floats,
   if (out_cap_floats < n_floats) return QPSK_ERR_ARG;    // :68-69
   if (n_floats == 0) return QPSK_OK;
   if (!in || !out) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(f->eng.device));
   FllEngine& e = f->eng;
   const int64_t L = n_floats >> 1;
-  const size_t tot = (size_t)L * e.channels;
-  QPSK_TRY(f->d_in.ensure(tot));
-  QPSK_TRY(f->d_out.ensure(tot));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(f->d_in.p, in, tot * 8, cudaMemcpyHostToDevice, e.stream));
-  QPSK_TRY(e.process_dev(f->d_in.p, f->d_out.p, L, L, L, e.stream));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(out, f->d_out.p, tot * 8, cudaMemcpyDeviceToHost, e.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(e.stream));
-  return QPSK_OK;
+  const size_t row = (size_t)L * 8;
+  return host_call(f, in, e.channels, row, out, row, e.channels, row,
+                   [&](const float2* x, float2* y) { return e.process_dev(x, y, L, L, L, e.stream); });
 }
 int qpsk_fll_process_dev(qpsk_fll* f, const float* d_in, float* d_out, int64_t n_floats, int64_t is, int64_t os, void* stream) {
   if (!f) return QPSK_ERR_NULL;
   if (n_floats < 0) return QPSK_ERR_RANGE;
   if ((n_floats & 1) || (is & 1) || (os & 1)) return QPSK_ERR_ARG;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(f->eng.device));
   return f->eng.process_dev((const float2*)d_in, (float2*)d_out, n_floats >> 1, is >> 1, os >> 1, (cudaStream_t)stream);
 }
@@ -467,23 +432,11 @@ int qpsk_fll_set_state(qpsk_fll* f, const float* phase, const float* freq) {
 
 // ---- Mueller-Muller ----
 int qpsk_mm_create_batch(double sps, double kp, double ki, int channels, qpsk_mm** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
-  qpsk_mm* m = new (std::nothrow) qpsk_mm();
-  if (!m) return QPSK_ERR_NOMEM;
-  int st = m->eng.init(sps, kp, ki, channels);
-  if (st != QPSK_OK) { delete m; return st; }
-  *out = m;
-  return QPSK_OK;
+  QPSK_TRY(clear_out(out));
+  return create_handle(out, sps, kp, ki, channels);
 }
 int qpsk_mm_create(double sps, double kp, double ki, qpsk_mm** out) { return qpsk_mm_create_batch(sps, kp, ki, 1, out); }
-int qpsk_mm_destroy(qpsk_mm* m) {
-  if (m) {
-    if (m->eng.stream) cudaStreamSynchronize(m->eng.stream);
-    delete m;
-  }
-  return QPSK_OK;
-}
+int qpsk_mm_destroy(qpsk_mm* m) { return destroy_handle(m); }
 int qpsk_mm_process(qpsk_mm* m, const float* in, int64_t n_floats, float* out, int64_t cap_floats, int* n_sym) {
   if (!m || !n_sym) return QPSK_ERR_NULL;
   if (n_floats < 0 || cap_floats < 0) return QPSK_ERR_RANGE;
@@ -494,10 +447,9 @@ int qpsk_mm_process(qpsk_mm* m, const float* in, int64_t n_floats, float* out, i
   MmEngine& e = m->eng;
   const int64_t L = n_floats >> 1;
   const int64_t cap_sym = cap_floats >> 1;
-  QPSK_TRY(m->d_in.ensure((size_t)(L > 0 ? L : 1) * e.channels));
   QPSK_TRY(m->d_out.ensure((size_t)(cap_sym > 0 ? cap_sym : 1) * e.channels));
   QPSK_TRY(m->d_n.ensure((size_t)e.channels));
-  if (L > 0) QPSK_CUDA_TRY(cudaMemcpyAsync(m->d_in.p, in, (size_t)L * e.channels * 8, cudaMemcpyHostToDevice, e.stream));
+  QPSK_TRY(stage_in(m->d_in, in, (size_t)L * 8, (size_t)L * 8, e.channels, e.stream));
   QPSK_TRY(e.process_dev(m->d_in.p, L, L, m->d_out.p, cap_floats, cap_sym > 0 ? cap_sym : 1, m->d_n.p, e.stream));
   QPSK_CUDA_TRY(cudaMemcpyAsync(n_sym, m->d_n.p, sizeof(int) * e.channels, cudaMemcpyDeviceToHost, e.stream));
   QPSK_CUDA_TRY(cudaStreamSynchronize(e.stream));
@@ -516,6 +468,7 @@ int qpsk_mm_process_dev(qpsk_mm* m, const float* d_in, int64_t n_floats, int64_t
   if (!m) return QPSK_ERR_NULL;
   if (n_floats < 0 || cap_floats < 0) return QPSK_ERR_RANGE;
   if ((n_floats & 1) || (is & 1) || (os & 1)) return QPSK_ERR_ARG;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(m->eng.device));
   return m->eng.process_dev((const float2*)d_in, n_floats >> 1, is >> 1, (float2*)d_out, cap_floats, os >> 1, d_n_sym,
                             (cudaStream_t)stream);
@@ -538,25 +491,13 @@ int qpsk_mm_get_state(qpsk_mm* m, int* base_index, double* mu, double* integral,
 
 // ---- Costas ----
 int qpsk_costas_create_batch(double fs, double bw, double damping, int channels, qpsk_costas** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
-  qpsk_costas* c = new (std::nothrow) qpsk_costas();
-  if (!c) return QPSK_ERR_NOMEM;
-  int st = c->eng.init(fs, bw, damping, channels);
-  if (st != QPSK_OK) { delete c; return st; }
-  *out = c;
-  return QPSK_OK;
+  QPSK_TRY(clear_out(out));
+  return create_handle(out, fs, bw, damping, channels);
 }
 int qpsk_costas_create(double fs, double bw, double damping, qpsk_costas** out) {
   return qpsk_costas_create_batch(fs, bw, damping, 1, out);
 }
-int qpsk_costas_destroy(qpsk_costas* c) {
-  if (c) {
-    if (c->eng.stream) cudaStreamSynchronize(c->eng.stream);
-    delete c;
-  }
-  return QPSK_OK;
-}
+int qpsk_costas_destroy(qpsk_costas* c) { return destroy_handle(c); }
 int qpsk_costas_process(qpsk_costas* c, const float* in, float* out, int64_t n_floats, int64_t out_cap_floats) {
   if (!c) return QPSK_ERR_NULL;
   if (n_floats < 0) return QPSK_ERR_RANGE;
@@ -564,23 +505,18 @@ int qpsk_costas_process(qpsk_costas* c, const float* in, float* out, int64_t n_f
   if (out_cap_floats < n_floats) return QPSK_ERR_ARG;    // :102-103
   if (n_floats == 0) return QPSK_OK;
   if (!in || !out) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(c->eng.device));
   CostasEngine& e = c->eng;
   const int64_t L = n_floats >> 1;
-  const size_t tot = (size_t)L * e.channels;
-  QPSK_TRY(c->d_in.ensure(tot));
-  QPSK_TRY(c->d_out.ensure(tot));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(c->d_in.p, in, tot * 8, cudaMemcpyHostToDevice, e.stream));
-  QPSK_TRY(e.process_dev(c->d_in.p, c->d_out.p, L, L, L, nullptr, e.stream));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(out, c->d_out.p, tot * 8, cudaMemcpyDeviceToHost, e.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(e.stream));
-  return QPSK_OK;
+  const size_t row = (size_t)L * 8;
+  return host_call(c, in, e.channels, row, out, row, e.channels, row,
+                   [&](const float2* x, float2* y) { return e.process_dev(x, y, L, L, L, nullptr, e.stream); });
 }
 int qpsk_costas_process_dev(qpsk_costas* c, const float* d_in, float* d_out, int64_t n_floats, int64_t is, int64_t os,
                             const int* d_n_sym, void* stream) {
   if (!c) return QPSK_ERR_NULL;
   if (n_floats < 0) return QPSK_ERR_RANGE;
   if ((n_floats & 1) || (is & 1) || (os & 1)) return QPSK_ERR_ARG;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(c->eng.device));
   return c->eng.process_dev((const float2*)d_in, (float2*)d_out, n_floats >> 1, is >> 1, os >> 1, d_n_sym, (cudaStream_t)stream);
 }

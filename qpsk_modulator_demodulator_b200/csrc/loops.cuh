@@ -6,7 +6,7 @@
 //   MmState/mm_*           MuellerMuller.Process       MS/Models/MuellerMuller.cs:52-136,160-198
 //   CostasState/costas_step CostasLoopQpsk.Process     MS/Models/CostasLoopQpsk.cs:63-92
 #pragma once
-#include "common.cuh"
+#include "handle.cuh"
 #include "design.h"
 
 namespace qpsk {
@@ -238,9 +238,8 @@ __device__ __forceinline__ void costas_step(const CostasParams& P, const SinCosK
 // ---------------------------------------------------------------------------------------------
 // engines (host side)
 // ---------------------------------------------------------------------------------------------
-struct FllEngine {
+struct FllEngine : EngineBase {
   int channels = 1, n_taps = 0;
-  int device = 0;
   FllParams P{};
   std::vector<float> lower, upper;
   DevBuf<float> d_taps;      // [2][N] reversed lower taps, planar
@@ -249,8 +248,6 @@ struct FllEngine {
   DevBuf<float2> d_pf;       // [C] (phase, freq)
   bool state_wild = false;   // a caller-set (phase, freq) outside the fast kernel's range is pending
   bool state_far = false;    // a caller-set |phase| >= 32 is pending (the pair kernel's short-range sin/cos)
-  cudaStream_t stream = nullptr;
-  ~FllEngine();
   int init(float sps, float rolloff, int size, float bw, int channels_in);
   int process_dev(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t ldy, cudaStream_t s);
 };
@@ -265,30 +262,24 @@ bool fll_pair_supported(int n_taps);
 int fll_pair_launch(const FllParams& P, const std::vector<float>& lower, float2* ring, int* head, float2* pf, int C,
                     const float2* x, float2* y, long long L, long long ldx, long long ldy, cudaStream_t s);
 
-struct MmEngine {
+struct MmEngine : EngineBase {
   int channels = 1;
-  int device = 0;
   MmParams P{};
   DevBuf<MmState> d_state;
   DevBuf<float2> d_queue[2];  // [C][qcap], ping-pong
   int qcur = 0;
   int64_t qcap = 0;
   int64_t q_bound = 0;        // host-side upper bound of queued samples
-  cudaStream_t stream = nullptr;
-  ~MmEngine();
   int init(double sps, double kp, double ki, int channels_in);
   int ensure_queue(int64_t need, cudaStream_t s);
   int process_dev(const float2* x, int64_t L, int64_t ldx, float2* y, int64_t cap_sym, int64_t ldy, int* d_nsym,
                   cudaStream_t s);
 };
 
-struct CostasEngine {
+struct CostasEngine : EngineBase {
   int channels = 1;
-  int device = 0;
   CostasParams P{};
   DevBuf<CostasState> d_state;
-  cudaStream_t stream = nullptr;
-  ~CostasEngine();
   int init(double fs, double bw, double damping, int channels_in);
   int process_dev(const float2* x, float2* y, int64_t L, int64_t ldx, int64_t ldy, const int* d_nsym, cudaStream_t s);
 };

@@ -25,7 +25,7 @@
 #include <algorithm>
 #include <vector>
 
-#include "common.cuh"
+#include "handle.cuh"
 
 namespace qpsk {
 
@@ -173,18 +173,13 @@ static int pfb_run_blocks(int M) { return M <= kPfbThreads ? 32 : 65536 / (M * 8
 
 static bool pfb_pow2_channels(int M) { return M >= 2 && M <= kPfbMaxChannels && (M & (M - 1)) == 0; }
 
-struct PfbEngine {
-  int device = 0;
+struct PfbEngine : EngineBase {
   int M = 0, log2m = 0, P = 0;
   long long pending = 0;                 // samples of the open block
   int cur = 0;                           // which history buffer is live
   DevBuf<float> d_taps;                  // [P][M], zero-padded
   DevBuf<float2> d_tw;                   // [M/2] e^{+j 2 pi t / M}
   DevBuf<float2> d_hist[2];              // [(P-1)M + M - 1]
-  cudaStream_t stream = nullptr;
-  ~PfbEngine() {
-    if (stream) cudaStreamDestroy(stream);
-  }
   long long hist_len() const { return (long long)(P - 1) * M + pending; }
   int reset(cudaStream_t s) {
     pending = 0;
@@ -196,9 +191,7 @@ struct PfbEngine {
     M = channels;
     P = (n_taps + M - 1) / M;
     while ((1 << log2m) < M) ++log2m;
-    QPSK_TRY(ensure_device());
-    device = current_device();
-    QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    QPSK_TRY(open());
     std::vector<float> hp((size_t)P * M, 0.0f);
     for (int i = 0; i < n_taps; ++i) hp[i] = taps[i];
     std::vector<float2> tw((size_t)M / 2);
@@ -307,41 +300,19 @@ int qpsk_pfb_taps(int channels, int taps_per_branch, double cutoff, double atten
 }
 
 int qpsk_pfb_create(const float* taps, int n_taps, int channels, qpsk_pfb** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (!taps) return QPSK_ERR_NULL;
   if (n_taps <= 0) return QPSK_ERR_ARG;
   for (int i = 0; i < n_taps; ++i)
     if (!isfinite(taps[i])) return QPSK_ERR_RANGE;
   if (!pfb_pow2_channels(channels)) return QPSK_ERR_UNSUPPORTED;
   if ((n_taps + channels - 1) / channels > kPfbMaxTapsPerBranch) return QPSK_ERR_UNSUPPORTED;
-  qpsk_pfb* p = new (std::nothrow) qpsk_pfb();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(taps, n_taps, channels);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, taps, n_taps, channels);
 }
 
-int qpsk_pfb_destroy(qpsk_pfb* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_pfb_destroy(qpsk_pfb* p) { return destroy_handle(p); }
 
-int qpsk_pfb_reset(qpsk_pfb* p) {
-  if (!p) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(p->eng.device));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  QPSK_TRY(p->eng.reset(p->eng.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  return QPSK_OK;
-}
+int qpsk_pfb_reset(qpsk_pfb* p) { return reset_handle(p); }
 
 int qpsk_pfb_process(qpsk_pfb* p, const float* iq_in, int64_t n_floats, float* iq_out, int64_t out_stride_floats,
                      int64_t* n_out_floats) {
@@ -354,16 +325,8 @@ int qpsk_pfb_process(qpsk_pfb* p, const float* iq_in, int64_t n_floats, float* i
   if (out_stride_floats < 2 * n_out) return QPSK_ERR_CAPACITY;
   if (n == 0) return QPSK_OK;
   if (!iq_in || (n_out > 0 && !iq_out)) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(g.device));
-  QPSK_TRY(p->d_in.ensure((size_t)n));
-  QPSK_TRY(p->d_out.ensure((size_t)g.M * (size_t)n_out));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(p->d_in.p, iq_in, (size_t)n * 8, cudaMemcpyHostToDevice, g.stream));
-  QPSK_TRY(g.process_dev(p->d_in.p, n, p->d_out.p, n_out, g.stream));
-  if (n_out > 0)
-    QPSK_CUDA_TRY(cudaMemcpy2DAsync(iq_out, (size_t)out_stride_floats * 4, p->d_out.p, (size_t)n_out * 8, (size_t)n_out * 8,
-                                    (size_t)g.M, cudaMemcpyDeviceToHost, g.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(g.stream));
-  return QPSK_OK;
+  return host_call(p, iq_in, 1, (size_t)n * 8, iq_out, (size_t)out_stride_floats * 4, g.M, (size_t)n_out * 8,
+                   [&](const float2* x, float2* y) { return g.process_dev(x, n, y, n_out, g.stream); });
 }
 
 int qpsk_pfb_process_dev(qpsk_pfb* p, const float* d_in, int64_t n_floats, float* d_out, int64_t out_stride_floats,
@@ -377,6 +340,7 @@ int qpsk_pfb_process_dev(qpsk_pfb* p, const float* d_in, int64_t n_floats, float
   if (out_stride_floats < 2 * n_out) return QPSK_ERR_CAPACITY;
   if (n == 0) return QPSK_OK;
   if (!d_in || (n_out > 0 && !d_out)) return QPSK_ERR_NULL;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(g.device));
   return g.process_dev((const float2*)d_in, n, (float2*)d_out, out_stride_floats >> 1, (cudaStream_t)stream);
 }

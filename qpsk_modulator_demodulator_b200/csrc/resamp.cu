@@ -31,7 +31,7 @@
 #include <algorithm>
 #include <vector>
 
-#include "common.cuh"
+#include "handle.cuh"
 
 namespace qpsk {
 
@@ -183,17 +183,12 @@ static unsigned long long resamp_count(unsigned long long n, int L, int M) {
   return (n / (unsigned long long)M) * (unsigned long long)L + (r == 0 ? 0ULL : (r * (unsigned long long)L - 1) / (unsigned long long)M + 1);
 }
 
-struct ResampEngine {
-  int device = 0;
+struct ResampEngine : EngineBase {
   int C = 0, L = 0, M = 0, N = 0, P = 0;
   unsigned long long n_in = 0, n_outc = 0;   // inputs consumed and outputs produced since creation or the last reset
   int cur = 0;                               // which history buffer is live
   DevBuf<float> d_hT;                        // [L][P]
   DevBuf<float2> d_hist[2];                  // [C][P-1]
-  cudaStream_t stream = nullptr;
-  ~ResampEngine() {
-    if (stream) cudaStreamDestroy(stream);
-  }
   int reset(cudaStream_t s) {
     n_in = n_outc = 0;
     cur = 0;
@@ -206,9 +201,7 @@ struct ResampEngine {
     M = decim;
     N = n_taps;
     P = (N + L - 1) / L;
-    QPSK_TRY(ensure_device());
-    device = current_device();
-    QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    QPSK_TRY(open());
     std::vector<float> hT((size_t)L * P, 0.0f);
     for (int i = 0; i < N; ++i) hT[(size_t)(i % L) * P + i / L] = taps[i];
     QPSK_TRY(d_hT.alloc(hT.size()));
@@ -291,8 +284,7 @@ struct qpsk_resamp {
 extern "C" {
 
 int qpsk_resamp_create(const float* taps, int n_taps, int interp, int decim, int channels, qpsk_resamp** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (!taps) return QPSK_ERR_NULL;
   if (n_taps <= 0) return QPSK_ERR_ARG;
   if (n_taps > kResampMaxTaps || interp < 1 || interp > kResampMaxFactor || decim < 1 || decim > kResampMaxFactor ||
@@ -300,33 +292,12 @@ int qpsk_resamp_create(const float* taps, int n_taps, int interp, int decim, int
     return QPSK_ERR_UNSUPPORTED;
   for (int i = 0; i < n_taps; ++i)
     if (!isfinite(taps[i])) return QPSK_ERR_RANGE;
-  qpsk_resamp* p = new (std::nothrow) qpsk_resamp();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(taps, n_taps, interp, decim, channels);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, taps, n_taps, interp, decim, channels);
 }
 
-int qpsk_resamp_destroy(qpsk_resamp* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_resamp_destroy(qpsk_resamp* p) { return destroy_handle(p); }
 
-int qpsk_resamp_reset(qpsk_resamp* p) {
-  if (!p) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(p->eng.device));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  QPSK_TRY(p->eng.reset(p->eng.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(p->eng.stream));
-  return QPSK_OK;
-}
+int qpsk_resamp_reset(qpsk_resamp* p) { return reset_handle(p); }
 
 int qpsk_resamp_process(qpsk_resamp* p, const float* iq_in, int64_t n_floats, float* iq_out, int64_t out_stride_floats,
                         int64_t* n_out_floats) {
@@ -339,16 +310,8 @@ int qpsk_resamp_process(qpsk_resamp* p, const float* iq_in, int64_t n_floats, fl
   if (out_stride_floats < 2 * n_out) return QPSK_ERR_CAPACITY;
   if (n == 0) return QPSK_OK;
   if (!iq_in || (n_out > 0 && !iq_out)) return QPSK_ERR_NULL;
-  QPSK_TRY(ensure_device(g.device));
-  QPSK_TRY(p->d_in.ensure((size_t)g.C * (size_t)n));
-  QPSK_TRY(p->d_out.ensure((size_t)g.C * (size_t)n_out));
-  QPSK_CUDA_TRY(cudaMemcpyAsync(p->d_in.p, iq_in, (size_t)g.C * (size_t)n * 8, cudaMemcpyHostToDevice, g.stream));
-  QPSK_TRY(g.process_dev(p->d_in.p, n, n, p->d_out.p, n_out, g.stream));
-  if (n_out > 0)
-    QPSK_CUDA_TRY(cudaMemcpy2DAsync(iq_out, (size_t)out_stride_floats * 4, p->d_out.p, (size_t)n_out * 8, (size_t)n_out * 8,
-                                    (size_t)g.C, cudaMemcpyDeviceToHost, g.stream));
-  QPSK_CUDA_TRY(cudaStreamSynchronize(g.stream));
-  return QPSK_OK;
+  return host_call(p, iq_in, g.C, (size_t)n * 8, iq_out, (size_t)out_stride_floats * 4, g.C, (size_t)n_out * 8,
+                   [&](const float2* x, float2* y) { return g.process_dev(x, n, n, y, n_out, g.stream); });
 }
 
 int qpsk_resamp_process_dev(qpsk_resamp* p, const float* d_in, int64_t n_floats, int64_t in_stride_floats, float* d_out,
@@ -363,7 +326,7 @@ int qpsk_resamp_process_dev(qpsk_resamp* p, const float* d_in, int64_t n_floats,
   if (out_stride_floats < 2 * n_out) return QPSK_ERR_CAPACITY;
   if (n == 0) return QPSK_OK;
   if (!d_in || (n_out > 0 && !d_out)) return QPSK_ERR_NULL;
-  if ((reinterpret_cast<uintptr_t>(d_in) & 7) || (reinterpret_cast<uintptr_t>(d_out) & 7)) return QPSK_ERR_ARG;
+  if (misaligned(d_in) || misaligned(d_out)) return QPSK_ERR_ARG;
   if (n_out > 0) {                                              // the rows read and the rows written must not overlap
     const uintptr_t i0 = reinterpret_cast<uintptr_t>(d_in), o0 = reinterpret_cast<uintptr_t>(d_out);
     const uintptr_t i1 = i0 + (uintptr_t)(((int64_t)(g.C - 1) * in_stride_floats + n_floats) * 4);

@@ -17,7 +17,7 @@
 
 #include <algorithm>
 
-#include "common.cuh"
+#include "handle.cuh"
 
 namespace qpsk {
 
@@ -263,21 +263,15 @@ static void rs_build_tables(int nroots, RsTables* T) {
     }
 }
 
-struct RsEngine {
-  int device = 0, nroots = 0, k = 0, n = 0, depth = 0, grid_cap = 1;
+struct RsEngine : EngineBase {
+  int nroots = 0, k = 0, n = 0, depth = 0, grid_cap = 1;
   DevBuf<RsTables> d_tab;
-  cudaStream_t stream = nullptr;           // host forms and NULL-stream calls
-  ~RsEngine() {
-    if (stream) cudaStreamDestroy(stream);
-  }
   int init(int nr, int kk, int I) {
     nroots = nr;
     k = kk;
     n = kk + nr;
     depth = I;
-    QPSK_TRY(ensure_device());
-    device = current_device();
-    QPSK_CUDA_TRY(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
+    QPSK_TRY(open());
     RsTables* h = new (std::nothrow) RsTables();
     if (!h) return QPSK_ERR_NOMEM;
     rs_build_tables(nroots, h);
@@ -346,33 +340,16 @@ struct qpsk_rs {
   RsEngine eng;
 };
 
-static bool rs_misaligned(const void* p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
-
 extern "C" {
 
 int qpsk_rs_create(int nroots, int k, int depth, qpsk_rs** out) {
-  if (!out) return QPSK_ERR_NULL;
-  *out = nullptr;
+  QPSK_TRY(clear_out(out));
   if (nroots < 2 || nroots > 32 || (nroots & 1) || depth < 1 || depth > 8) return QPSK_ERR_UNSUPPORTED;
   if (k < 1 || k > kRsMaxN - nroots) return QPSK_ERR_RANGE;
-  qpsk_rs* p = new (std::nothrow) qpsk_rs();
-  if (!p) return QPSK_ERR_NOMEM;
-  const int st = p->eng.init(nroots, k, depth);
-  if (st != QPSK_OK) {
-    delete p;
-    return st;
-  }
-  *out = p;
-  return QPSK_OK;
+  return create_handle(out, nroots, k, depth);
 }
 
-int qpsk_rs_destroy(qpsk_rs* p) {
-  if (p) {
-    if (p->eng.stream) cudaStreamSynchronize(p->eng.stream);
-    delete p;
-  }
-  return QPSK_OK;
-}
+int qpsk_rs_destroy(qpsk_rs* p) { return destroy_handle(p); }
 
 int qpsk_rs_encode_dev(qpsk_rs* p, const uint8_t* d_msg, int64_t msg_stride, int rows, int64_t n_blocks, uint8_t* d_code,
                        int64_t code_stride, void* stream) {
@@ -398,7 +375,7 @@ int qpsk_rs_decode_dev(qpsk_rs* p, const uint8_t* d_code, int64_t code_stride, c
   if (msg_stride < blocks * g.depth * g.k || status_stride < blocks * g.depth) return QPSK_ERR_CAPACITY;
   if (rows == 0) return QPSK_OK;
   if (!d_code || !d_n_bytes || !d_msg || !d_n_msg || !d_status) return QPSK_ERR_NULL;
-  if (rs_misaligned(d_n_bytes, 8) || rs_misaligned(d_n_msg, 8) || rs_misaligned(d_status, 4)) return QPSK_ERR_ARG;
+  if (misaligned(d_n_bytes) || misaligned(d_n_msg) || misaligned(d_status, 4)) return QPSK_ERR_ARG;
   QPSK_TRY(ensure_device(g.device));
   return p->eng.decode(d_code, code_stride, (const long long*)d_n_bytes, rows, d_msg, msg_stride, (long long*)d_n_msg,
                        d_status, status_stride, stream ? (cudaStream_t)stream : g.stream);
